@@ -4,6 +4,12 @@ bench.py -- headline benchmark of the hot path (BASELINE.json: "BN254 MSM points
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K ...  # the CPU restatement of the reference's path (oracle)
+    python bench.py ... --dump-outputs DIR                   # also write the outputs of the last timed steps to DIR/*.npy
+
+With the same arguments the inputs are the same from run to run (seeded generators on the device), so the files of
+--dump-outputs from two builds can be compared array for array: msm, msm_witness, msm_e2e, msm_registered_pinned (the affine
+result point of each MSM leg, x and y in 32-bit limbs; the identity is all zero) and ntt, ntt_e2e (the rows ntt_rows of the
+device-resident and of the host-array NTT output, Montgomery form in 32-bit limbs).
 
 A *step* is one pass of the hot path over one batch of synthetic input: one BN254 G1 MSM over
 2^k points per GPU (k = 24 by default: BASELINE.json configs[3], the synthetic sweep; the other
@@ -52,7 +58,14 @@ def parse_args():
     ap.add_argument("--plain", action="store_true", help="do not use the precomputed window tables of the registered SRS")
     ap.add_argument("--no-inprocess", action="store_true", help="N > 1: skip the in-process h2b_init(N) parity + strong-scaling leg (tools/multi_gpu_inprocess.py)")
     ap.add_argument("--strong-k", type=int, nargs="*", default=[24, 26], help="total sizes 2^k of the strong-scaling leg at N > 1")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last timed step of each leg returned "
+                    "as DIR/<name>.npy (float64 32-bit limbs; the NTT outputs as a fixed, seeded sample of rows), rank 0 only")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
 
 
 def config_for(args, n_gpus):
@@ -109,6 +122,24 @@ class ClockSampler:
                     reasons.add(name)
         return {"sm_mhz": statistics.median(sm), "sm_max_mhz": float(rows[0][2]), "power_w_max": max(float(r[3]) for r in rows),
                 "samples": len(rows), "reasons": sorted(reasons)}
+
+
+DUMP_NTT_ROWS = 1 << 16        # --dump-outputs: rows of each 2^k NTT output written (4 MiB per array)
+DUMP_SEED = 0xB2D0
+
+
+def words_to_limbs(words):
+    """(m, 4) u64 field elements -> (m, 8) float64 of their 32-bit halves, least significant first (exact)"""
+    import numpy as np
+    return np.ascontiguousarray(words, dtype=np.uint64).view(np.uint32).reshape(-1, 8).astype(np.float64)
+
+
+def point_to_limbs(p):
+    """affine (x, y) as canonical ints, None for the identity -> (2, 8) float64 of 32-bit limbs, least significant first.
+    The identity is written as (0, 0), which is not on the curve."""
+    import numpy as np
+    x, y = p if p is not None else (0, 0)
+    return np.array([[(c >> (32 * i)) & 0xFFFFFFFF for i in range(8)] for c in (x, y)], dtype=np.float64)
 
 
 def omega_words(k):
@@ -298,7 +329,9 @@ def run_ours(args):
     msm_value = world * n * K / (msm_ms / 1e3)
     result_host = d_out.cpu().numpy().view(np.uint64)
     expect = expected_point(d_scal)
-    checks = {"device_resident_equals_checksum": V.jacobian_words_to_affine(result_host) == expect}
+    result_affine = V.jacobian_words_to_affine(result_host)
+    checks = {"device_resident_equals_checksum": result_affine == expect}
+    outputs = {"msm": point_to_limbs(result_affine)}          # what the last timed step of each leg returned (--dump-outputs)
 
     # ---- the same MSM over a witness-like column (SURVEY.md 8d: 50 % zero, 20 % one, 20 % < 2^19, 10 % r - small) ---------
     witness = None
@@ -325,8 +358,10 @@ def run_ours(args):
             L.msm_fold_partials_dev(0, d_blocks.data_ptr(), world, d_out.data_ptr(), st)
         else:
             L.msm_fold_partials_dev(0, d_block.data_ptr(), 1, d_out.data_ptr(), st)
-        wit_ok = V.jacobian_words_to_affine(d_out.cpu().numpy().view(np.uint64)) == expected_point(d_wit)
+        wit_affine = V.jacobian_words_to_affine(d_out.cpu().numpy().view(np.uint64))
+        wit_ok = wit_affine == expected_point(d_wit)
         checks["witness_like_equals_checksum"] = wit_ok
+        outputs["msm_witness"] = point_to_limbs(wit_affine)
         witness = {"value": world * n * K / (wit_ms / 1e3), "unit": "points/s", "ms_per_step": wit_ms / K,
                    "scalars": "50% zero, 20% one, 20% uniform < 2^19, 10% r - small", "verified": bool(wit_ok)}
         del d_wit
@@ -357,7 +392,9 @@ def run_ours(args):
     barrier()
     e2e_s = max_over_ranks(time.perf_counter() - t0)
     e2e_value = world * n * K / e2e_s
-    checks["e2e_equals_checksum"] = (V.jacobian_words_to_affine(r) if world == 1 else r) == expect
+    e2e_affine = V.jacobian_words_to_affine(r) if world == 1 else r
+    checks["e2e_equals_checksum"] = e2e_affine == expect
+    outputs["msm_e2e"] = point_to_limbs(e2e_affine)
     cache_stats = L.implicit_cache_stats()
     del base_np
     # (b) the friendlier variant of round 1: pinned scalars, explicitly registered SRS (what a patched ParamsKZG::commit does)
@@ -377,8 +414,10 @@ def run_ours(args):
         r = L.msm_registered(pin_np, handle)
     barrier()
     e2e_pinned_value = world * n * K / max_over_ranks(time.perf_counter() - t0)
+    pinned_affine = V.jacobian_words_to_affine(r)            # at N > 1: this rank's share of the points
     if world == 1:
-        checks["e2e_registered_pinned_equals_checksum"] = V.jacobian_words_to_affine(r) == expect
+        checks["e2e_registered_pinned_equals_checksum"] = pinned_affine == expect
+    outputs["msm_registered_pinned"] = point_to_limbs(pinned_affine)
     L.unregister_bases(handle)
     del scal_np
 
@@ -413,6 +452,9 @@ def run_ours(args):
         torch.cuda.synchronize()
         ntt_ok = ntt_ok and bool((d_ev.cpu() == d_ntt[4 * idx: 4 * idx + 4].cpu()).all())
     checks["ntt_spot_values"] = ntt_ok
+    ntt_rows = np.sort(np.random.default_rng(DUMP_SEED).choice(n, size=min(n, DUMP_NTT_ROWS), replace=False))
+    outputs["ntt_rows"] = ntt_rows.astype(np.float64)
+    outputs["ntt"] = words_to_limbs(d_in.view(n, 4)[torch.from_numpy(ntt_rows).to(dev)].cpu().numpy().view(np.uint64))
     del d_in
     a_np = np.empty((n, 4), dtype=np.uint64)                     # pageable, like the Vec<Fr> best_fft receives
     a_np[:] = h_scal.numpy().view(np.uint64).reshape(n, 4)
@@ -423,6 +465,7 @@ def run_ours(args):
         L.ntt(a_np, w_words, k)
     barrier()
     ntt_e2e_s = max_over_ranks(time.perf_counter() - t0)
+    outputs["ntt_e2e"] = words_to_limbs(a_np[ntt_rows])
     sampler.stop()
     clocks = sampler.summary(t_wall0, t_wall1)
 
@@ -621,6 +664,10 @@ def run_ours(args):
             line["witness_like"] = witness
         if cpu_baseline:
             line["cpu_baseline"] = cpu_baseline
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in outputs.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -527,3 +527,23 @@ def test_msm_pair_pre_reduction_forced(gpu, oc):
     for levels in ("1", "3"):
         out = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, H2B_MSM_PAIR_LEVELS=levels), capture_output=True, text=True, timeout=900)
         assert out.returncode == 0 and "ok" in out.stdout, (levels, out.stderr[-3000:])
+
+
+def test_bench_dump_outputs(tmp_path):
+    # bench.py --dump-outputs: the outputs of the last timed step of every leg; with one warm-up step both NTT legs have applied
+    # the same number of transforms to the same column, and every MSM leg sums the same points
+    import json, subprocess, sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--k", "12", "--steps", "2", "--warmup", "1", "--no-cpu-baseline",
+                          "--no-widened", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900)
+    assert out.returncode == 0, out.stderr[-3000:]
+    line = json.loads(out.stdout.strip().splitlines()[-1])
+    assert line["verified"] and line["steps"] == 2, line["checks"]
+    d = {f[:-4]: np.load(str(tmp_path / f)) for f in os.listdir(str(tmp_path))}
+    assert sorted(d) == ["msm", "msm_e2e", "msm_registered_pinned", "msm_witness", "ntt", "ntt_e2e", "ntt_rows"]
+    assert all(a.dtype == np.float64 for a in d.values()) and sum(a.nbytes for a in d.values()) <= 64 << 20
+    assert (d["ntt_rows"] == np.arange(1 << 12)).all() and d["ntt"].shape == (1 << 12, 8)
+    assert (d["ntt"] == d["ntt_e2e"]).all()
+    assert d["msm"].shape == (2, 8) and d["msm"].any()
+    assert (d["msm"] == d["msm_e2e"]).all() and (d["msm"] == d["msm_registered_pinned"]).all()
+    assert (d["msm_witness"] != d["msm"]).any()
