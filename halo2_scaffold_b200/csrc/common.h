@@ -63,7 +63,7 @@ struct DevBuf {
 
 // Optional per-kernel timing with CUDA events on the launching stream (bench.py's roofline numbers).
 enum ProfTag { PROF_BEGIN = 0, PROF_MSM_DECOMPOSE = 1, PROF_MSM_SCAN = 2, PROF_MSM_SCATTER = 3, PROF_MSM_PLAN = 4, PROF_MSM_ACCUMULATE = 5,
-               PROF_MSM_COMBINE = 6, PROF_MSM_REDUCE = 7, PROF_MSM_FINAL = 8, PROF_MSM_PRECOMPUTE = 9, PROF_MSM_PAIR = 10, PROF_NTT_TWIDDLE = 15, PROF_NTT_PASS0 = 16 };
+               PROF_MSM_COMBINE = 6, PROF_MSM_REDUCE = 7, PROF_MSM_FINAL = 8, PROF_MSM_PRECOMPUTE = 9, PROF_NTT_TWIDDLE = 15, PROF_NTT_PASS0 = 16 };
 struct Profiler {
     bool enabled = false;
     std::vector<cudaEvent_t> ev;

@@ -30,7 +30,6 @@
 namespace h2b {
 
 static const uint32_t SIGN_BIT = 0x80000000u;
-static const uint32_t PAIR_BIT = 0x40000000u;      // the entry names a pair sum (row of the pair buffer) instead of a table row
 
 // scattered 4-byte stores of the counting sort: evict-first, so that they do not push the bucket cursors out of L2
 #if defined(H2B_EMU) || defined(H2B_NO_STREAMING_STORES)
@@ -631,103 +630,11 @@ __global__ void __launch_bounds__(256) msm_scatter_kernel(MsmCols cols, MsmPlan 
     }
 }
 
-// ---- 2b. pair pre-reduction: batched affine additions ------------------------------------------------------
-// The mixed addition into an XYZZ accumulator costs 8M + 2S.  Two AFFINE points add in 2M + 1S plus one field inversion,
-// and Montgomery's trick shares one inversion among K independent additions (3M each): 5.9 multiplications + 341 / K
-// instead of 9.8.  Independent additions are there for the taking: inside a bucket of the sorted list, entries
-// (0,1), (2,3), ... can be summed pairwise, which halves the list; the sums are affine again, so the step repeats.
-// One thread owns K consecutive OUTPUT positions (balanced for any distribution, like the slices of the accumulation),
-// walks the buckets they fall into, multiplies the denominators up (x2 - x1; 2 y for P + P; 1 for the cases that need no
-// division: a lone last entry, an identity operand, P + (-P)), inverts once, and walks back writing the pair sums into
-// the pair buffer and entries that name them (PAIR_BIT) into the next list.  Lone entries and identity cases are passed
-// through by entry, so they cost no point write.  The accumulation then runs over a list 2^levels shorter.
-__device__ __forceinline__ Affine msm_entry_point(const uint4* __restrict__ tables, const uint4* __restrict__ pair_pts, uint32_t e) {
-    return (e & PAIR_BIT) ? affine_load(pair_pts + 4 * (size_t)(e & ~(SIGN_BIT | PAIR_BIT))) : affine_load(tables + 4 * (size_t)(e & ~SIGN_BIT));
-}
-__device__ __forceinline__ Affine msm_entry_point_signed(const uint4* __restrict__ tables, const uint4* __restrict__ pair_pts, uint32_t e) {
-    Affine p = msm_entry_point(tables, pair_pts, e);
-    if ((e & SIGN_BIT) && !affine_is_identity(p)) p.y = fp_neg(p.y);
-    return p;
-}
-
-__global__ void __launch_bounds__(256) msm_pair_counts_kernel(const uint32_t* __restrict__ offsets, uint32_t B, uint32_t* __restrict__ counts2) {
-    const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
-    if (b < B) counts2[b] = (offsets[b + 1] - offsets[b] + 1) >> 1;
-}
-
-// what the addition of the pair (p0, p1) needs: 0 = a division by d, 1 = a doubling (d = 2 y), 2 = p0 is the identity (result p1),
-// 3 = p1 is the identity (result p0), 4 = p1 = -p0 (result: identity)
-__device__ __forceinline__ int msm_pair_mode(const Affine& p0, const Affine& p1, Fq& d) {
-    if (affine_is_identity(p0)) return 2;
-    if (affine_is_identity(p1)) return 3;
-    d = fp_sub(p1.x, p0.x);
-    if (!fp_is_zero(d)) return 0;
-    if (!fp_eq(p0.y, p1.y)) return 4;
-    d = fp_dbl(p0.y);
-    return 1;
-}
-
-template <int K, int MINB>
-__global__ void __launch_bounds__(128, MINB) msm_pair_reduce_kernel(uint32_t B, const uint32_t* __restrict__ offsets, const uint32_t* __restrict__ sorted,
-                                                            const uint32_t* __restrict__ new_offsets, uint32_t* __restrict__ new_sorted,
-                                                            const uint4* __restrict__ tables, uint4* __restrict__ pair_pts, uint32_t out_base) {
-    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
-    const uint32_t total2 = new_offsets[B];
-    if ((uint64_t)t * K >= total2) return;
-    const uint32_t q0 = t * K, q1 = (total2 - q0 > (uint32_t)K) ? q0 + K : total2;
-    uint32_t lo = 0, hi = B;                       // the bucket that holds output position q0
-    while (hi - lo > 1) {
-        const uint32_t mid = (lo + hi) >> 1;
-        if (new_offsets[mid] <= q0) lo = mid; else hi = mid;
-    }
-    Fq prefix[K];
-    Fq run = fp_one<FQ>();
-    uint32_t b = lo, base2 = new_offsets[b], next2 = new_offsets[b + 1], src0 = offsets[b], src_end = offsets[b + 1];
-    for (uint32_t q = q0; q < q1; ++q) {
-        while (q >= next2) { ++b; base2 = next2; next2 = new_offsets[b + 1]; src0 = offsets[b]; src_end = offsets[b + 1]; }
-        const uint32_t src = src0 + 2 * (q - base2);
-        prefix[q - q0] = run;
-        if (src + 1 < src_end) {
-            const Affine p0 = msm_entry_point_signed(tables, pair_pts, sorted[src]), p1 = msm_entry_point_signed(tables, pair_pts, sorted[src + 1]);
-            Fq d;
-            if (msm_pair_mode(p0, p1, d) <= 1) run = fp_mul(run, d);
-        }
-    }
-    Fq inv = fp_inv(run);
-    for (uint32_t q = q1; q-- > q0;) {
-        while (q < base2) { --b; base2 = new_offsets[b]; next2 = new_offsets[b + 1]; src0 = offsets[b]; src_end = offsets[b + 1]; }
-        const uint32_t src = src0 + 2 * (q - base2);
-        const uint32_t e0 = sorted[src];
-        if (src + 1 >= src_end) { new_sorted[q] = e0; continue; }      // a lone last entry of its bucket
-        const uint32_t e1 = sorted[src + 1];
-        const Affine p0 = msm_entry_point_signed(tables, pair_pts, e0), p1 = msm_entry_point_signed(tables, pair_pts, e1);
-        Fq d;
-        const int mode = msm_pair_mode(p0, p1, d);
-        if (mode == 2) { new_sorted[q] = e1; continue; }
-        if (mode == 3) { new_sorted[q] = e0; continue; }
-        Affine r;
-        if (mode == 4) {
-            r.x = fp_zero<FQ>(); r.y = fp_zero<FQ>();
-        } else {
-            const Fq inv_d = fp_mul(inv, prefix[q - q0]);
-            inv = fp_mul(inv, d);
-            Fq lambda;
-            if (mode == 0) lambda = fp_mul(fp_sub(p1.y, p0.y), inv_d);
-            else { const Fq xx = fp_sqr(p0.x); lambda = fp_mul(fp_add(fp_dbl(xx), xx), inv_d); }
-            r.x = fp_sub(fp_sub(fp_sqr(lambda), p0.x), p1.x);
-            r.y = fp_sub(fp_mul(lambda, fp_sub(p0.x, r.x)), p0.y);
-        }
-        affine_store(pair_pts + 4 * (size_t)(out_base + q), r);
-        new_sorted[q] = PAIR_BIT | (out_base + q);
-    }
-}
-
 // ---- 3. accumulate: equal slices of the sorted list ----------------------------------------------------
 // slice length for `total` sorted entries cut into at most G slices.  The host sizes G for the worst case (every
 // digit non-zero); skewed columns sort far fewer entries, so slices never get shorter than SLICE_MIN and the
 // surplus threads simply exit.
 static const uint32_t SLICE_MIN = 16;
-static const int PAIR_K = 256;               // pair additions that share one inversion (one thread)
 __device__ __forceinline__ uint32_t slice_len(uint32_t total, uint32_t G) {
     uint32_t S = (total + G - 1) / G;
     return S < SLICE_MIN ? SLICE_MIN : S;
@@ -737,7 +644,7 @@ __device__ __forceinline__ uint32_t slice_len(uint32_t total, uint32_t G) {
 __global__ void __launch_bounds__(256) msm_accumulate_kernel(MsmPlan pl, const uint4* __restrict__ tables, const uint32_t* __restrict__ offsets,
                                                            const uint32_t* __restrict__ sorted, uint32_t* __restrict__ ctrl,
                                                            uint32_t* __restrict__ split_list, uint4* __restrict__ bucket_acc,
-                                                           uint4* __restrict__ head_partial, const uint4* __restrict__ pair_pts) {
+                                                           uint4* __restrict__ head_partial) {
     const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= pl.G) return;
     const uint32_t total = offsets[pl.B];
@@ -757,13 +664,13 @@ __global__ void __launch_bounds__(256) msm_accumulate_kernel(MsmPlan pl, const u
 
     XYZZ acc = xyzz_identity();
     uint32_t e = sorted[start];
-    Affine p = msm_entry_point(tables, pair_pts, e);
+    Affine p = affine_load(tables + 4 * (size_t)(e & ~SIGN_BIT));
     for (uint32_t j = start; j < end; ++j) {
         uint32_t e_next = 0;
         Affine p_next = p;
         if (j + 1 < end) {      // prefetch the next point while this one is added
             e_next = sorted[j + 1];
-            p_next = msm_entry_point(tables, pair_pts, e_next);
+            p_next = affine_load(tables + 4 * (size_t)(e_next & ~SIGN_BIT));
         }
         if (j == next) {        // bucket b is complete: flush, move to the next non-empty bucket
             if (head) xyzz_store(head_partial + 8 * (size_t)t, acc);
@@ -1066,13 +973,8 @@ int msm_precompute_run(DeviceCtx& ctx, const void* d_src, void* d_dst, size_t n,
 }
 
 // ---- host orchestration ----------------------------------------------------------------------------------
-// The sort of chunk j + 1 (L2-atomic bound) runs on its own high-priority stream while chunk j is accumulated
-// (integer-pipe bound): the two stages keep their outputs (offsets, sorted list) in alternating buffers.
 struct MsmScratch {
-    cudaStream_t sort_stream = nullptr;
-    cudaEvent_t ev_start = nullptr, ev_sorted[2] = {nullptr, nullptr}, ev_accumulated[2] = {nullptr, nullptr};
-    DevBuf digits, counts, offsets, offsets2, cursor, block_sums, sorted, sorted2, ctrl, split_list, heavy, chunk_desc, chunk_out, bucket_acc, bucket_tmp, head_partial, redA, redB, redC, redD, result;
-    DevBuf pair_pts, pair_counts, pair_offsets[3], pair_sorted[3];      // pair pre-reduction (batched affine additions)
+    DevBuf digits, counts, offsets, cursor, block_sums, sorted, ctrl, split_list, heavy, chunk_desc, chunk_out, bucket_acc, bucket_tmp, head_partial, redA, redB, redC, redD, result;
     DevBuf batch_out;                                                   // result blocks of a batched host-pointer call
     DevBuf part_counts, part_off, part_cursor, chunk0, chunk_hist, inter; // partitioned sort (section 2c)
     bool part_attr_set = false;
@@ -1215,7 +1117,7 @@ static void chunk_points(const MsmBases& bases, size_t done, const void** tables
 }
 
 // slices and scratch of one chunk
-static int msm_size_chunk(DeviceCtx& ctx, MsmScratch& s, MsmPlan& pl, size_t row0, uint32_t n, int b) {
+static int msm_size_chunk(DeviceCtx& ctx, MsmScratch& s, MsmPlan& pl, size_t row0, uint32_t n) {
     pl.n = n;
     pl.row0 = (uint32_t)row0;
     const uint64_t upper = (uint64_t)n * pl.W * pl.ncols;          // sorted entries, at most
@@ -1256,8 +1158,8 @@ static int msm_size_chunk(DeviceCtx& ctx, MsmScratch& s, MsmPlan& pl, size_t row
         }
     }
     H2B_TRY(s.digits.reserve((size_t)upper * 4));
-    H2B_TRY((b ? s.sorted2 : s.sorted).reserve((size_t)upper * 4 + 4));
-    H2B_TRY((b ? s.offsets2 : s.offsets).reserve(((size_t)pl.B + 1) * 4));
+    H2B_TRY(s.sorted.reserve((size_t)upper * 4 + 4));
+    H2B_TRY(s.offsets.reserve(((size_t)pl.B + 1) * 4));
     H2B_TRY(s.split_list.reserve((size_t)pl.G * 4));
     const size_t max_heavy = pl.G / COMBINE_HEAVY + 1, max_chunks = pl.G / COMBINE_CHUNK + max_heavy + 1;
     H2B_TRY(s.heavy.reserve(max_heavy * sizeof(HeavyDesc)));
@@ -1267,12 +1169,12 @@ static int msm_size_chunk(DeviceCtx& ctx, MsmScratch& s, MsmPlan& pl, size_t row
     return H2B_OK;
 }
 
-// stage 1 of a chunk: digits, histogram, scan, counting-sort scatter -> offsets[b], sorted[b]
-static int msm_sort_chunk(DeviceCtx& ctx, MsmScratch& s, const MsmPlan& pl, const MsmCols& cols, int b, cudaStream_t stream) {
+// stage 1 of a chunk: digits, histogram, scan, counting-sort scatter -> offsets, sorted
+static int msm_sort_chunk(DeviceCtx& ctx, MsmScratch& s, const MsmPlan& pl, const MsmCols& cols, cudaStream_t stream) {
     uint32_t* counts = (uint32_t*)s.counts.p;
-    uint32_t* offsets = (uint32_t*)(b ? s.offsets2 : s.offsets).p;
+    uint32_t* offsets = (uint32_t*)s.offsets.p;
     uint32_t* cursor = (uint32_t*)s.cursor.p;
-    uint32_t* sorted = (uint32_t*)(b ? s.sorted2 : s.sorted).p;
+    uint32_t* sorted = (uint32_t*)s.sorted.p;
     const uint32_t nblk = (pl.n + 255) / 256;
     if (pl.pb) {
         // partitioned sort (section 2c)
@@ -1330,62 +1232,15 @@ static int msm_sort_chunk(DeviceCtx& ctx, MsmScratch& s, const MsmPlan& pl, cons
 }
 
 // stage 2 of a chunk: accumulate the sorted list into the buckets, combine cut buckets, merge (chunked MSMs)
-static int msm_accumulate_chunk(DeviceCtx& ctx, MsmScratch& s, const MsmPlan& pl, const void* tables, int b, cudaStream_t stream) {
-    const uint32_t* offsets = (const uint32_t*)(b ? s.offsets2 : s.offsets).p;
-    const uint32_t* sorted = (const uint32_t*)(b ? s.sorted2 : s.sorted).p;
+static int msm_accumulate_chunk(DeviceCtx& ctx, MsmScratch& s, const MsmPlan& pl, const void* tables, cudaStream_t stream) {
+    const uint32_t* offsets = (const uint32_t*)s.offsets.p;
+    const uint32_t* sorted = (const uint32_t*)s.sorted.p;
     uint32_t* ctrl = (uint32_t*)s.ctrl.p;
     uint4* target = (uint4*)(pl.add_into ? s.bucket_tmp.p : s.bucket_acc.p);
     H2B_CUDA(cudaMemsetAsync(ctrl, 0, 16, stream));
     ctx.prof.mark(PROF_BEGIN, stream);
-    // pair pre-reduction (batched affine additions, section 2b): OFF by default.  Measured at 2^24 points (profiles/r01_msm_pair_stage.jsonl):
-    // every level halves the accumulation exactly as modelled (34.8 -> 17.5 -> 8.8 -> 4.4 ms), but one level costs 23.8 ms instead of the
-    // 10.3 ms its multiplications need -- its two passes gather every point twice, and the kernel runs at the random 64-byte access rate
-    // of HBM (~18 G gathers/s; more resident warps, software prefetch and 64-byte fetch hints change nothing), where the XYZZ
-    // accumulation hides ONE gather behind ten multiplications.  41.5 ms without, 48.0 / 48.8 / 50.1 ms with 1 / 2 / 3 levels.
-    // H2B_MSM_PAIR_LEVELS=1..3 turns it on (tests run it on the emulator).  Entries must leave bit 30 free for PAIR_BIT.
-    const uint64_t upper = (uint64_t)pl.n * pl.W * pl.ncols;
-    uint32_t levels = 0;
-    {
-        static int env_levels = -2;
-        if (env_levels == -2) env_levels = env_int("H2B_MSM_PAIR_LEVELS", 0);
-        if (env_levels > 0) levels = env_levels > 3 ? 3u : (uint32_t)env_levels;
-        const uint64_t table_rows = pl.stride ? (uint64_t)pl.stride * ((pl.W + pl.m - 1) / pl.m) : pl.n;
-        if (table_rows >= PAIR_BIT || upper + 3 * (uint64_t)pl.B >= PAIR_BIT) levels = 0;
-    }
-    const uint4* pair_pts = nullptr;
-    if (levels) {
-        // level l holds at most upper / 2^(l+1) + B entries; all levels share one pair buffer
-        uint64_t cap[3], base[3], total_cap = 0;
-        for (uint32_t l = 0; l < levels; ++l) { cap[l] = (upper >> (l + 1)) + pl.B + 1; base[l] = total_cap; total_cap += cap[l]; }
-        H2B_TRY(s.pair_pts.reserve(total_cap * 64 + 64));
-        H2B_TRY(s.pair_counts.reserve((size_t)pl.B * 4));
-        pair_pts = (const uint4*)s.pair_pts.p;
-        for (uint32_t l = 0; l < levels; ++l) {
-            H2B_TRY(s.pair_offsets[l].reserve(((size_t)pl.B + 1) * 4));
-            H2B_TRY(s.pair_sorted[l].reserve(cap[l] * 4 + 4));
-            uint32_t* offsets_l = (uint32_t*)s.pair_offsets[l].p;
-            uint32_t* sorted_l = (uint32_t*)s.pair_sorted[l].p;
-            H2B_LAUNCH(msm_pair_counts_kernel, (pl.B + 255) / 256, 256, 0, stream, offsets, pl.B, (uint32_t*)s.pair_counts.p);
-            H2B_TRY(exclusive_scan(s, (const uint32_t*)s.pair_counts.p, pl.B, offsets_l, sorted_l /* cursor copy: unused, overwritten below */, stream));
-            const uint64_t threads = (cap[l] + PAIR_K - 1) / PAIR_K;
-            static int env_occ = -1;
-            if (env_occ < 0) env_occ = env_int("H2B_MSM_PAIR_OCC", 5);
-            if (env_occ >= 8)
-                H2B_LAUNCH((msm_pair_reduce_kernel<PAIR_K, 8>), (unsigned)((threads + 127) / 128), 128, 0, stream, pl.B, offsets, sorted, (const uint32_t*)offsets_l,
-                           sorted_l, (const uint4*)tables, (uint4*)s.pair_pts.p, (uint32_t)base[l]);
-            else if (env_occ >= 6)
-                H2B_LAUNCH((msm_pair_reduce_kernel<PAIR_K, 6>), (unsigned)((threads + 127) / 128), 128, 0, stream, pl.B, offsets, sorted, (const uint32_t*)offsets_l,
-                           sorted_l, (const uint4*)tables, (uint4*)s.pair_pts.p, (uint32_t)base[l]);
-            else
-                H2B_LAUNCH((msm_pair_reduce_kernel<PAIR_K, 4>), (unsigned)((threads + 127) / 128), 128, 0, stream, pl.B, offsets, sorted, (const uint32_t*)offsets_l,
-                           sorted_l, (const uint4*)tables, (uint4*)s.pair_pts.p, (uint32_t)base[l]);
-            offsets = offsets_l;
-            sorted = sorted_l;
-        }
-        ctx.prof.mark(PROF_MSM_PAIR, stream);
-    }
     H2B_LAUNCH(msm_accumulate_kernel, (pl.G + 255) / 256, 256, 0, stream, pl, (const uint4*)tables, offsets, sorted, ctrl, (uint32_t*)s.split_list.p, target,
-               (uint4*)s.head_partial.p, pair_pts);
+               (uint4*)s.head_partial.p);
     ctx.prof.mark(PROF_MSM_ACCUMULATE, stream);
     H2B_LAUNCH(msm_combine_light_kernel, (pl.G + 127) / 128, 128, 0, stream, pl, offsets, ctrl, (const uint32_t*)s.split_list.p,
                (HeavyDesc*)s.heavy.p, (uint2*)s.chunk_desc.p, (const uint4*)s.head_partial.p, target);
@@ -1400,60 +1255,26 @@ static int msm_accumulate_chunk(DeviceCtx& ctx, MsmScratch& s, const MsmPlan& pl
     return H2B_OK;
 }
 
-static int msm_pipeline_init(MsmScratch& s) {
-    if (s.sort_stream) return H2B_OK;
-    int lo = 0, hi = 0;
-    H2B_CUDA(cudaDeviceGetStreamPriorityRange(&lo, &hi));
-    H2B_CUDA(cudaStreamCreateWithPriority(&s.sort_stream, cudaStreamNonBlocking, hi));     // numerically lowest = highest priority
-    H2B_CUDA(cudaEventCreateWithFlags(&s.ev_start, cudaEventDisableTiming));
-    for (int b = 0; b < 2; ++b) {
-        H2B_CUDA(cudaEventCreateWithFlags(&s.ev_sorted[b], cudaEventDisableTiming));
-        H2B_CUDA(cudaEventCreateWithFlags(&s.ev_accumulated[b], cudaEventDisableTiming));
-    }
-    return H2B_OK;
-}
-
-// All chunks of one MSM.  `stream` carries the accumulate stage (and is the stream the caller synchronises with);
-// with more than one chunk the sort stage of the next chunk overlaps it on s.sort_stream.  uploaded[j], when given, is
-// the event after which chunk j's scalars are in device memory.
+// All chunks of one MSM, each sorted and then accumulated on `stream`.  uploaded[j], when given, is the event after which
+// chunk j's scalars are in device memory.
 // bounds: nchunks + 1 ascending scalar indices, bounds[0] = 0, bounds[nchunks] = n
 static int msm_run_chunks(DeviceCtx& ctx, MsmScratch& s, MsmPlan pl, const void* d_scalars, const MsmBases& bases, const std::vector<size_t>& bounds,
                           const cudaEvent_t* uploaded, cudaStream_t stream, const std::function<int(size_t)>* before_chunk = nullptr) {
     const size_t nchunks = bounds.size() - 1;
-    // Measured at 2^24 (profiles/r01_msm_spacing.jsonl): overlapping the two stages gains nothing -- both want every SM,
-    // the sort slows down 2x and the accumulation 15 % while they share the GPU (41.4 ms unsplit, 43.3 ms as 4
-    // overlapped chunks).  Off by default; H2B_MSM_OVERLAP_SORT=1 turns it on.
-    static int env_overlap = -1;
-    if (env_overlap < 0) env_overlap = env_int("H2B_MSM_OVERLAP_SORT", 0);
-    const bool overlap = nchunks > 1 && env_overlap > 0;
-    if (overlap) {
-        H2B_TRY(msm_pipeline_init(s));
-        // the sort stage starts after everything already queued on the caller's stream (inputs, the previous MSM)
-        H2B_CUDA(cudaEventRecord(s.ev_start, stream));
-        H2B_CUDA(cudaStreamWaitEvent(s.sort_stream, s.ev_start, 0));
-    }
     for (size_t j = 0; j < nchunks; ++j) {
         const size_t done = bounds[j], m = bounds[j + 1] - bounds[j];
-        const int b = overlap ? (int)(j & 1) : 0;
         const void* tables;
         size_t row0;
         chunk_points(bases, done, &tables, &row0);
-        H2B_TRY(msm_size_chunk(ctx, s, pl, row0, (uint32_t)m, b));
-        cudaStream_t ss = overlap ? s.sort_stream : stream;
+        H2B_TRY(msm_size_chunk(ctx, s, pl, row0, (uint32_t)m));
         if (before_chunk) H2B_TRY((*before_chunk)(j));          // e.g. the staged upload of this chunk's scalars onto `stream`
-        if (uploaded) H2B_CUDA(cudaStreamWaitEvent(ss, uploaded[j], 0));
-        if (overlap && j >= 2) H2B_CUDA(cudaStreamWaitEvent(ss, s.ev_accumulated[b], 0));      // buffers b are free again
+        if (uploaded) H2B_CUDA(cudaStreamWaitEvent(stream, uploaded[j], 0));
         MsmCols cols;
         memset(&cols, 0, sizeof(cols));
         cols.scalars[0] = (const uint4*)((const char*)d_scalars + done * 32);
         cols.len[0] = (uint32_t)m;
-        H2B_TRY(msm_sort_chunk(ctx, s, pl, cols, b, ss));
-        if (overlap) {
-            H2B_CUDA(cudaEventRecord(s.ev_sorted[b], ss));
-            H2B_CUDA(cudaStreamWaitEvent(stream, s.ev_sorted[b], 0));
-        }
-        H2B_TRY(msm_accumulate_chunk(ctx, s, pl, tables, b, stream));
-        if (overlap) H2B_CUDA(cudaEventRecord(s.ev_accumulated[b], stream));
+        H2B_TRY(msm_sort_chunk(ctx, s, pl, cols, stream));
+        H2B_TRY(msm_accumulate_chunk(ctx, s, pl, tables, stream));
     }
     return H2B_OK;
 }
@@ -1700,9 +1521,9 @@ int msm_run_batch(DeviceCtx& ctx, const void* const* d_cols, const size_t* lens,
     const void* tables;
     size_t row0;
     chunk_points(bases, 0, &tables, &row0);
-    H2B_TRY(msm_size_chunk(ctx, s, pl, row0, (uint32_t)n_max, 0));
-    H2B_TRY(msm_sort_chunk(ctx, s, pl, cols, 0, stream));
-    H2B_TRY(msm_accumulate_chunk(ctx, s, pl, tables, 0, stream));
+    H2B_TRY(msm_size_chunk(ctx, s, pl, row0, (uint32_t)n_max));
+    H2B_TRY(msm_sort_chunk(ctx, s, pl, cols, stream));
+    H2B_TRY(msm_accumulate_chunk(ctx, s, pl, tables, stream));
     H2B_TRY(msm_finish(ctx, s, pl, s.result.p, false, stream));
     H2B_CUDA(cudaMemcpyAsync(d_out_blocks, s.result.p, 224 * (size_t)count, cudaMemcpyDeviceToDevice, stream));
     return H2B_OK;
@@ -1758,14 +1579,9 @@ int msm_sum_partials_run(DeviceCtx& ctx, const void* d_blocks, uint32_t count, v
 void msm_release(DeviceCtx& ctx) {
     if (!ctx.msm) return;
     MsmScratch& s = *ctx.msm;
-    if (s.sort_stream) {
-        cudaStreamDestroy(s.sort_stream);
-        cudaEventDestroy(s.ev_start);
-        for (int b = 0; b < 2; ++b) { cudaEventDestroy(s.ev_sorted[b]); cudaEventDestroy(s.ev_accumulated[b]); }
-    }
-    DevBuf* all[] = {&s.digits, &s.counts, &s.offsets, &s.offsets2, &s.sorted2, &s.cursor, &s.block_sums, &s.sorted, &s.ctrl, &s.split_list, &s.heavy, &s.chunk_desc, &s.chunk_out,
-                     &s.bucket_acc, &s.bucket_tmp, &s.head_partial, &s.redA, &s.redB, &s.redC, &s.redD, &s.result, &s.pair_pts, &s.pair_counts,
-                     &s.pair_offsets[0], &s.pair_offsets[1], &s.pair_offsets[2], &s.pair_sorted[0], &s.pair_sorted[1], &s.pair_sorted[2], &s.batch_out, &s.part_counts, &s.part_off, &s.part_cursor, &s.chunk0, &s.chunk_hist, &s.inter};
+    DevBuf* all[] = {&s.digits, &s.counts, &s.offsets, &s.cursor, &s.block_sums, &s.sorted, &s.ctrl, &s.split_list, &s.heavy, &s.chunk_desc, &s.chunk_out,
+                     &s.bucket_acc, &s.bucket_tmp, &s.head_partial, &s.redA, &s.redB, &s.redC, &s.redD, &s.result, &s.batch_out,
+                     &s.part_counts, &s.part_off, &s.part_cursor, &s.chunk0, &s.chunk_hist, &s.inter};
     for (DevBuf* b : all) b->release();
     delete ctx.msm;
     ctx.msm = nullptr;

@@ -129,7 +129,6 @@ __global__ void __launch_bounds__(512, 1) ntt_pass_kernel(NttPassParams p) {
     uint4* thi = tlo + tw_slots;
     const uint32_t tid = threadIdx.x, nthr = blockDim.x;
     const bool last = p.last != 0;
-    const uint32_t ntiles = 1u << (p.log_n - b - logT);
     // non-last pass: tile (q, t), q < N, t < T  <->  global base + q*M + t ; shared e = q*T + t
     // last pass: T segments that differ in the TOP logT bits of the position;
     //            element (q, t) <-> global ((t*nseg + tile) << b) + q ; shared e = t*N + q
@@ -143,54 +142,50 @@ __global__ void __launch_bounds__(512, 1) ntt_pass_kernel(NttPassParams p) {
         uint32_t half = idx & 1, j = idx >> 1;
         copy16_async((half ? thi : tlo) + sm_slot(j), p.tw_small + 2 * j + half);
     }
-    // first tile of this CTA (persistent: tiles blockIdx.x, blockIdx.x + gridDim.x, ...)
-    {
-        const uint32_t tile = blockIdx.x;
-        if (!last) {
-            const uint32_t seg = tile >> log_tiles_per_seg, tau = tile & ((1u << log_tiles_per_seg) - 1);
-            const uint32_t base = (seg << p.logL) + (tau << logT);
-            for (uint32_t idx = tid; idx < 2 * E; idx += nthr) {
-                uint32_t half = idx & 1, t = (idx >> 1) & (T - 1), q = idx >> (1 + logT);
-                copy16_async((half ? hi : lo) + sm_slot((q << logT) + t), p_in + 2 * (size_t)(base + q * M + t) + half);
-            }
-        } else {
-            for (uint32_t idx = tid; idx < 2 * E; idx += nthr) {
-                uint32_t half = idx & 1, q = (idx >> 1) & (N - 1), t = idx >> (1 + b);
-                copy16_async((half ? hi : lo) + sm_slot((t << b) + q), p_in + 2 * (size_t)(((t * nseg + tile) << b) + q) + half);
-            }
+    // this CTA's tile
+    const uint32_t tile = blockIdx.x;
+    if (!last) {
+        const uint32_t seg = tile >> log_tiles_per_seg, tau = tile & ((1u << log_tiles_per_seg) - 1);
+        const uint32_t base = (seg << p.logL) + (tau << logT);
+        for (uint32_t idx = tid; idx < 2 * E; idx += nthr) {
+            uint32_t half = idx & 1, t = (idx >> 1) & (T - 1), q = idx >> (1 + logT);
+            copy16_async((half ? hi : lo) + sm_slot((q << logT) + t), p_in + 2 * (size_t)(base + q * M + t) + half);
+        }
+    } else {
+        for (uint32_t idx = tid; idx < 2 * E; idx += nthr) {
+            uint32_t half = idx & 1, q = (idx >> 1) & (N - 1), t = idx >> (1 + b);
+            copy16_async((half ? hi : lo) + sm_slot((t << b) + q), p_in + 2 * (size_t)(((t * nseg + tile) << b) + q) + half);
         }
     }
+    copy_async_wait_all();
+    __syncthreads();
 
-    for (uint32_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-        copy_async_wait_all();
+    // b DIF stages: one partial round (b mod 3 stages) followed by radix-8 rounds, all out of registers
+    uint32_t s = 0;
+    if (b % 3 == 1) {
+        for (uint32_t item = tid; item < (E >> 1); item += nthr) ntt_round<1>(lo, hi, tlo, thi, item, b, 0, logT, last);
+        s = 1;
         __syncthreads();
+    } else if (b % 3 == 2) {
+        for (uint32_t item = tid; item < (E >> 2); item += nthr) ntt_round<2>(lo, hi, tlo, thi, item, b, 0, logT, last);
+        s = 2;
+        __syncthreads();
+    }
+    for (; s < b; s += 3) {
+        for (uint32_t item = tid; item < (E >> 3); item += nthr) ntt_round<3>(lo, hi, tlo, thi, item, b, s, logT, last);
+        __syncthreads();
+    }
 
-        // b DIF stages: one partial round (b mod 3 stages) followed by radix-8 rounds, all out of registers
-        uint32_t s = 0;
-        if (b % 3 == 1) {
-            for (uint32_t item = tid; item < (E >> 1); item += nthr) ntt_round<1>(lo, hi, tlo, thi, item, b, 0, logT, last);
-            s = 1;
-            __syncthreads();
-        } else if (b % 3 == 2) {
-            for (uint32_t item = tid; item < (E >> 2); item += nthr) ntt_round<2>(lo, hi, tlo, thi, item, b, 0, logT, last);
-            s = 2;
-            __syncthreads();
-        }
-        for (; s < b; s += 3) {
-            for (uint32_t item = tid; item < (E >> 3); item += nthr) ntt_round<3>(lo, hi, tlo, thi, item, b, s, logT, last);
-            __syncthreads();
-        }
-
-        // Write-out.  Every shared slot is read by exactly one thread, which right afterwards refills it with the
-        // matching element of this CTA's NEXT tile: the next tile's load overlaps the twiddle multiplications and
-        // stores of this one without a second buffer.
-        const uint32_t next = tile + gridDim.x;
-        const bool has_next = next < ntiles;
+    // Write-out: non-last passes multiply by the inter-pass twiddles, the last pass scatters to bit-reversed positions.
+    // The tile geometry is recomputed here: kept live across the radix-8 rounds, it spills at the 128-register cap.
+    {
+        const uint32_t logM = last ? 0u : p.logL - b;
+        const uint32_t M = 1u << logM;
+        const uint32_t log_tiles_per_seg = logM - (last ? 0u : logT);
+        const uint32_t nseg = (1u << (p.log_n - b)) >> logT;
         if (!last) {
             const uint32_t seg = tile >> log_tiles_per_seg, tau = tile & ((1u << log_tiles_per_seg) - 1);
             const uint32_t base = (seg << p.logL) + (tau << logT);
-            const uint32_t nseg2 = next >> log_tiles_per_seg, ntau = next & ((1u << log_tiles_per_seg) - 1);
-            const uint32_t nbase = (nseg2 << p.logL) + (ntau << logT);
             const uint32_t logS = p.log_n - p.logL;          // S_p = n / L_p
             const uint32_t hmask = (1u << p.h) - 1;
 #pragma unroll 2
@@ -212,11 +207,6 @@ __global__ void __launch_bounds__(512, 1) ntt_pass_kernel(NttPassParams p) {
                     v = fp_mul(v, w);
                 }
                 fp_store<FR>(p_out + 2 * (size_t)(base + q * M + t), v);
-                if (has_next) {
-                    const uint4* src = p_in + 2 * (size_t)(nbase + q * M + t);
-                    copy16_async(lo + sm_slot(i), src);
-                    copy16_async(hi + sm_slot(i), src + 1);
-                }
             }
         } else {
             for (uint32_t i = tid; i < E; i += nthr) {
@@ -227,15 +217,9 @@ __global__ void __launch_bounds__(512, 1) ntt_pass_kernel(NttPassParams p) {
                 uint32_t pos = ((t * nseg + tile) << b) + q;
                 uint32_t oidx = __brev(pos) >> (32 - p.log_n);
                 fp_store<FR>(p_out + 2 * (size_t)oidx, v);
-                if (has_next) {
-                    const uint4* src = p_in + 2 * (size_t)(((t * nseg + next) << b) + q);
-                    copy16_async(lo + sm_slot(e), src);
-                    copy16_async(hi + sm_slot(e), src + 1);
-                }
             }
         }
     }
-    copy_async_wait_all();
 }
 
 // ---- twiddle tables ---------------------------------------------------------------------------
@@ -500,22 +484,8 @@ static int ntt_run_group(DeviceCtx& ctx, void* const* d_polys, uint32_t count, c
         if (threads > 512) threads = 512;
         if (threads < 32) threads = 32;
         const size_t smem = 32 * ((size_t)sm_slot((1u << logE) - 1) + 1 + sm_slot(a.b > 1 ? (1u << (a.b - 1)) - 1 : 0) + 1);
-        // One tile per CTA by default: CTAs of different ages overlap their load, butterfly and store phases on an SM.
-        // H2B_NTT_PERSIST=1 instead keeps as many CTAs as fit on the GPU and lets each loop over tiles with the
-        // next tile prefetched into the slots the write-out frees (measured 7 % slower at 2^24: lock-step phases).
-        static int persist = -1;
-        if (persist < 0) { const char* e = getenv("H2B_NTT_PERSIST"); persist = e ? atoi(e) : 0; }
-        uint32_t per_sm = (uint32_t)(232448 / (smem + 1024));
-        const uint32_t by_regs = 65536 / (threads * 128);
-        if (per_sm > by_regs) per_sm = by_regs;
-        if (per_sm > 16) per_sm = 16;
-        if (per_sm < 1) per_sm = 1;
-        uint32_t grid = persist ? (uint32_t)ctx.sm_count * per_sm : ntiles;
-        static int grid_cap = -1;      // tests: force several tiles per CTA at small sizes
-        if (grid_cap < 0) { const char* e = getenv("H2B_NTT_GRID"); grid_cap = e ? atoi(e) : 0; }
-        if (grid_cap > 0 && grid > (uint32_t)grid_cap) grid = (uint32_t)grid_cap;
-        if (grid > ntiles) grid = ntiles;
-        H2B_LAUNCH(kfn, dim3(grid, count), threads, smem, stream, a);
+        // one CTA per tile: CTAs of different ages overlap their load, butterfly and store phases on an SM
+        H2B_LAUNCH(kfn, dim3(ntiles, count), threads, smem, stream, a);
         H2B_CUDA(cudaGetLastError());
         ctx.prof.mark(PROF_NTT_PASS0 + (int)p, stream);
     }

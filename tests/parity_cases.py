@@ -230,6 +230,24 @@ def check_golden_ntt(L, g):
             assert (got == g["k%d_%s" % (k, tag)]).all(), (k, tag)
 
 
+def check_msm_opposite_points(L, oc, n, kind):
+    """A duplicate point, an identity base, and P and -P with equal scalars (one bucket, the pair cancels), through a registered
+    base set and the plain call."""
+    s, P = L.gen_scalars(n, n, kind), oc.gen_points(n + 1, n)
+    P[5] = P[4]
+    P[7] = 0
+    P[9, :4] = P[8, :4]
+    P[9, 4:] = oc.field_op("fq", "sub", np.zeros((1, 4), dtype=np.uint64), P[8:9, 4:])[0]
+    s[9] = s[8]
+    want = affine_of(oc, oc.best_multiexp(s, P))
+    h = L.register_bases(P)
+    try:
+        assert (affine_of(oc, L.msm_registered(s, h, 0)) == want).all(), (n, kind)
+    finally:
+        L.unregister_bases(h)
+    assert (affine_of(oc, L.msm(s, P)) == want).all(), (n, kind, "plain")
+
+
 def check_golden_msm(L, oc, g):
     for tag in ("n1", "n2", "n8", "n64", "n200", "cancel", "anchor"):
         got = affine_of(oc, L.msm(g[tag + "_scalars"], g[tag + "_bases"]))

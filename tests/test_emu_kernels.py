@@ -47,8 +47,8 @@ def test_ntt_three_and_four_pass_plans(emu, oc, monkeypatch):
     env = dict(os.environ, H2B_NTT_BMAX="4")
     out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=600)
     assert out.returncode == 0 and "ok" in out.stdout, out.stderr[-2000:]
-    # persistent CTAs looping over several tiles (the next tile is prefetched into the slots the write-out frees)
-    env = dict(os.environ, H2B_NTT_BMAX="5", H2B_NTT_GRID="3")
+    # B_MAX = 5: passes of 3 to 5 stages
+    env = dict(os.environ, H2B_NTT_BMAX="5")
     out = subprocess.run([sys.executable, "-c", code.replace("(12, 13, 14, 16)", "(11, 13, 15, 16)")], env=env, capture_output=True, text=True, timeout=600)
     assert out.returncode == 0 and "ok" in out.stdout, out.stderr[-2000:]
     # one CTA holding a full 2^11 / 2^12 tile (the tile size of the two-pass plan at 2^22..2^24)
@@ -161,7 +161,7 @@ def test_msm_chunked_upload_pipeline(emu):
     env = dict(os.environ, H2B_MSM_UPLOAD_MIN_LOG="10")
     out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=900)
     assert out.returncode == 0 and "ok" in out.stdout, out.stderr[-2000:]
-    # device-resident scalars: 4 (or 3) chunks whose sort overlaps the previous chunk's accumulation
+    # device-resident scalars: 4 (or 3) chunks accumulated into the same buckets
     code2 = (
         "import sys; sys.path[:0]=[%r,%r,%r]\n"
         "import numpy as np, oracle_c as oc, parity_cases as pc\n"
@@ -179,7 +179,7 @@ def test_msm_chunked_upload_pipeline(emu):
         "    L.msm_dev_partial(0, d_s, d_p, n, d_o); L.dev_sync(0); L.d2h(0, out, d_o)\n"
         "    assert (pc.affine_of(oc, out[:12]) == want).all()\n"
         "print('ok')\n") % (root, root + '/oracle', root + '/tests', emu.path)
-    env = dict(os.environ, H2B_MSM_DEVICE_CHUNK_MIN_LOG="10", H2B_MSM_DEVICE_CHUNKS="4", H2B_MSM_OVERLAP_SORT="1")
+    env = dict(os.environ, H2B_MSM_DEVICE_CHUNK_MIN_LOG="10", H2B_MSM_DEVICE_CHUNKS="4")
     out = subprocess.run([sys.executable, "-c", code2], env=env, capture_output=True, text=True, timeout=900)
     assert out.returncode == 0 and "ok" in out.stdout, out.stderr[-2000:]
 
@@ -444,31 +444,13 @@ def test_evaluate_graph_property(emu, oc):
     pc.check_evaluate_graph_property(emu, oc, examples=80, max_rows=70, max_calcs=160)
 
 
-def test_msm_pair_pre_reduction(emu, oc):
-    # the batched-affine pair stage only switches on for long lists; H2B_MSM_PAIR_LEVELS forces it at CPU-friendly sizes
-    # (fresh library instance per setting: the knob is read once per process).  Golden vectors (identity bases, duplicate points,
-    # P and -P in one bucket), random shapes with forced windows and table spacings, and witness-like columns.
-    import os, subprocess, sys
-    root = pc.__file__.rsplit('/tests/', 1)[0]
-    code = (
-        "import sys; sys.path[:0]=[%r,%r,%r]\n"
-        "import numpy as np, oracle_c as oc, parity_cases as pc\n"
-        "from halo2_scaffold_b200._lib import Lib\n"
-        "L=Lib(%r, allow_emulator=True); L.init(1)\n"
-        "g=np.load(%r)\n"
-        "pc.check_golden_msm(L, oc, g)\n"
-        "pc.check_msm_random(L, oc, examples=8, max_n=600, spacings=(-1, 4, 6, 8), windows=(0, 2, 3, 4, 6))\n"
-        "for n, kind in ((3000, 1), (2500, 0)):\n"
-        "    s, P = L.gen_scalars(n, n, kind), oc.gen_points(n + 1, n)\n"
-        "    P[5] = P[4]; P[7] = 0; P[9, :4] = P[8, :4]; P[9, 4:] = oc.field_op('fq', 'sub', np.zeros((1, 4), dtype=np.uint64), P[8:9, 4:])[0]; s[9] = s[8]\n"
-        "    h = L.register_bases(P)\n"
-        "    assert (pc.affine_of(oc, L.msm_registered(s, h, 0)) == pc.affine_of(oc, oc.best_multiexp(s, P))).all(), (n, kind)\n"
-        "    assert (pc.affine_of(oc, L.msm(s, P)) == pc.affine_of(oc, oc.best_multiexp(s, P))).all(), (n, kind, 'plain')\n"
-        "print('ok')\n") % (root, root + '/oracle', root + '/tests', emu.path, root + '/tests/golden/msm_golden.npz')
-    for levels in ("1", "3"):      # (an off-by-default stage: one level and the multi-level bookkeeping)
-        env = dict(os.environ, H2B_MSM_PAIR_LEVELS=levels)
-        out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=900)
-        assert out.returncode == 0 and "ok" in out.stdout, (levels, out.stderr[-3000:])
+def test_msm_duplicate_identity_and_opposite_points(emu, oc, golden):
+    # golden vectors (identity bases, duplicate points, P and -P in one bucket), random shapes with forced windows and table
+    # spacings, and witness-like columns
+    pc.check_golden_msm(emu, oc, golden["msm"])
+    pc.check_msm_random(emu, oc, examples=8, max_n=600, spacings=(-1, 4, 6, 8), windows=(0, 2, 3, 4, 6))
+    for n, kind in ((3000, 1), (2500, 0)):
+        pc.check_msm_opposite_points(emu, oc, n, kind)
 
 
 def test_quotient_of_a_satisfied_circuit_is_a_polynomial(emu, oc):
@@ -586,10 +568,10 @@ def test_one_ntt_across_emulated_devices(emu, devices):
                          "for k in (4, 5, 8, 11, 12, 13):\n"
                          "    pc.check_ntt(L, oc, k)\n" % devices,
                     dict(H2B_EMU_DEVICES=devices, H2B_NTT_MULTI_MIN_LOG="4", H2B_STAGE_PIECE_LOG="10", H2B_STAGE_THREADS="3"))
-    # the strided-batch mode of the multi-pass plans (2, 3 and 4 passes per row / column transform; several tiles per CTA)
+    # the strided-batch mode of the multi-pass plans (2, 3 and 4 passes per row / column transform)
     _emu_subprocess(emu, "for k in (12, 14, 15):\n"
                          "    pc.check_ntt(L, oc, k)\n",
-                    dict(H2B_EMU_DEVICES=devices, H2B_NTT_MULTI_MIN_LOG="4", H2B_NTT_BMAX="2", H2B_NTT_GRID="3"))
+                    dict(H2B_EMU_DEVICES=devices, H2B_NTT_MULTI_MIN_LOG="4", H2B_NTT_BMAX="2"))
 
 
 @pytest.mark.parametrize("n,ncols,spacing,window", [(600, 6, 8, 0), (600, 5, 8, 4), (257, 9, 0, 0), (1200, 4, 12, 6), (40, 33, 6, 0), (300, 4, -1, 0)])

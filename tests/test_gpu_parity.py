@@ -506,27 +506,10 @@ def test_async_upload_overlaps_and_delivers(gpu, oc):
         gpu.dev_free(0, d_b)
 
 
-def test_msm_pair_pre_reduction_forced(gpu, oc):
-    # the batched-affine pair stage is off by default (measured slower, DESIGN.md 5.1); its CUDA build is still checked against the
-    # oracle with forced levels, in fresh processes (the knob is read once per process)
-    import subprocess, sys
-    root = pc.__file__.rsplit('/tests/', 1)[0]
-    code = (
-        "import sys; sys.path[:0]=[%r,%r,%r]\n"
-        "import numpy as np, oracle_c as oc, parity_cases as pc\n"
-        "import halo2_scaffold_b200 as h2\n"
-        "L=h2.load(); L.init_device(0)\n"
-        "pc.check_golden_msm(L, oc, np.load(%r))\n"
-        "for n, kind in ((1 << 17, 0), (200001, 1)):\n"
-        "    s, P = L.gen_scalars(n, n, kind), oc.gen_points(n + 1, n)\n"
-        "    P[5] = P[4]; P[7] = 0; P[9, :4] = P[8, :4]; P[9, 4:] = oc.field_op('fq', 'sub', np.zeros((1, 4), dtype=np.uint64), P[8:9, 4:])[0]; s[9] = s[8]\n"
-        "    h = L.register_bases(P)\n"
-        "    assert (pc.affine_of(oc, L.msm_registered(s, h, 0)) == pc.affine_of(oc, oc.best_multiexp(s, P))).all(), (n, kind)\n"
-        "    assert (pc.affine_of(oc, L.msm(s, P)) == pc.affine_of(oc, oc.best_multiexp(s, P))).all(), (n, kind, 'plain')\n"
-        "print('ok')\n") % (root, root + '/oracle', root + '/tests', root + '/tests/golden/msm_golden.npz')
-    for levels in ("1", "3"):
-        out = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, H2B_MSM_PAIR_LEVELS=levels), capture_output=True, text=True, timeout=900)
-        assert out.returncode == 0 and "ok" in out.stdout, (levels, out.stderr[-3000:])
+def test_msm_duplicate_identity_and_opposite_points(gpu, oc, golden):
+    pc.check_golden_msm(gpu, oc, golden["msm"])
+    for n, kind in ((1 << 17, 0), (200001, 1)):
+        pc.check_msm_opposite_points(gpu, oc, n, kind)
 
 
 def test_bench_dump_outputs(tmp_path):

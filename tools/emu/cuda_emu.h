@@ -190,8 +190,6 @@ static inline cudaError_t cudaMemsetAsync(void* d, int v, size_t n, cudaStream_t
 static inline cudaError_t cudaStreamCreateWithFlags(cudaStream_t* s, unsigned) { *s = nullptr; return cudaSuccess; }
 static inline cudaError_t cudaStreamCreate(cudaStream_t* s) { *s = nullptr; return cudaSuccess; }
 static inline cudaError_t cudaStreamDestroy(cudaStream_t) { return cudaSuccess; }
-static inline cudaError_t cudaStreamCreateWithPriority(cudaStream_t* s, unsigned, int) { *s = (cudaStream_t)1; return cudaSuccess; }
-static inline cudaError_t cudaDeviceGetStreamPriorityRange(int* lo, int* hi) { *lo = 0; *hi = -1; return cudaSuccess; }
 static inline cudaError_t cudaStreamSynchronize(cudaStream_t) { return cudaSuccess; }
 static inline cudaError_t cudaDeviceSynchronize() { return cudaSuccess; }
 static inline cudaError_t cudaGetLastError() { return cudaSuccess; }
