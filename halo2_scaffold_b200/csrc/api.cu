@@ -1663,11 +1663,11 @@ static int elementwise_host(int which, int field, int op, const uint64_t* a, con
     return rc;
 }
 int h2b_field_op(int field, int op, const uint64_t* a, const uint64_t* b, size_t n, uint64_t* out) {
-    if (field < 0 || field > 1 || op < 0 || op > 6) { set_error("h2b_field_op: bad field/op"); return H2B_ERR_BAD_ARGUMENT; }
+    if (field < 0 || field > 1 || op < 0 || op > 12) { set_error("h2b_field_op: bad field/op"); return H2B_ERR_BAD_ARGUMENT; }
     return elementwise_host(0, field, op, a, b, n, out, 32);
 }
 int h2b_ec_op(int op, const uint64_t* p, const uint64_t* q, size_t n, uint64_t* out) {
-    if (op < 0 || op > 3) { set_error("h2b_ec_op: bad op"); return H2B_ERR_BAD_ARGUMENT; }
+    if (op < 0 || op > 4) { set_error("h2b_ec_op: bad op"); return H2B_ERR_BAD_ARGUMENT; }
     return elementwise_host(1, 0, op, p, q, n, out, 64);
 }
 

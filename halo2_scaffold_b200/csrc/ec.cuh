@@ -140,6 +140,44 @@ __device__ __forceinline__ void xyzz_add_affine(XYZZ& acc, const Affine& q_in, b
     acc.zzz = fp_mul(acc.zzz, ppp);
 }
 
+// The same mixed addition on a lazily reduced accumulator (every coordinate in [0, 2p), see field.cuh); q is canonical.
+// It drops the final conditional subtraction of all ten products (17 ALU instructions each).  The
+// exceptional cases are tested modulo p: P == 0 or P == p.  ZZ of a non-identity accumulator is never 0 mod p, so the
+// identity test on ZZ == 0 stays exact.  Pass the result through xyzz_canon before it is stored.
+__device__ __forceinline__ void xyzz_add_affine_lazy(XYZZ& acc, const Affine& q_in, bool neg) {
+    if (affine_is_identity(q_in)) return;
+    Affine q = q_in;
+    if (neg) q.y = fp_neg(q.y);
+    if (xyzz_is_identity(acc)) {
+        acc.x = q.x; acc.y = q.y; acc.zz = fp_one<FQ>(); acc.zzz = fp_one<FQ>();
+        return;
+    }
+    Fq u2 = fp_mul_lazy(q.x, acc.zz);
+    Fq s2 = fp_mul_lazy(q.y, acc.zzz);
+    Fq p = fp_sub_lazy(u2, acc.x);
+    Fq r = fp_sub_lazy(s2, acc.y);
+    if (fp_is_zero_lazy(p)) {
+        if (fp_is_zero_lazy(r)) acc = xyzz_double_affine(q);
+        else acc = xyzz_identity();
+        return;
+    }
+    Fq pp = fp_sqr_lazy(p);
+    Fq ppp = fp_mul_lazy(p, pp);
+    Fq qq = fp_mul_lazy(acc.x, pp);
+    Fq yppp = fp_mul_lazy(acc.y, ppp);      // before X3: in the order of xyzz_add_affine this kernel spills at 128 registers
+    Fq x3 = fp_sub_lazy(fp_sub_lazy(fp_sqr_lazy(r), ppp), fp_add_lazy(qq, qq));
+    Fq y3 = fp_sub_lazy(fp_mul_lazy(r, fp_sub_lazy(qq, x3)), yppp);
+    acc.x = x3;
+    acc.y = y3;
+    acc.zz = fp_mul_lazy(acc.zz, pp);
+    acc.zzz = fp_mul_lazy(acc.zzz, ppp);
+}
+__device__ __forceinline__ XYZZ xyzz_canon(const XYZZ& a) {
+    XYZZ r;
+    r.x = fp_canon(a.x); r.y = fp_canon(a.y); r.zz = fp_canon(a.zz); r.zzz = fp_canon(a.zzz);
+    return r;
+}
+
 // acc += b, both XYZZ  (EFD add-2008-s: 12M + 2S)
 template <bool SHARED> __device__ __forceinline__ void xyzz_add_body(XYZZ& acc, const XYZZ& b);
 // ONE copy of the general addition for the latency-bound kernels: with the addition inlined at every call site the loop of

@@ -5,6 +5,11 @@
 //
 // The multiply/add/sub bodies are the generated IMAD.WIDE carry chains in field_asm.inc
 // (tools/gen_field_ptx.py, which also proves them against big-int arithmetic).
+//
+// The *_lazy operations keep values in [0, 2p) instead: BN254's p and r are below 2^256 / 5.29, so a Montgomery
+// product of two values < 2p is (ab + Mp) / 2^256 < 1.76p and needs no final conditional subtraction, and sums and
+// differences are corrected by 2p.  Loops that chain many products (the MSM bucket accumulation, the NTT butterflies)
+// run on them and call fp_canon before a value leaves the loop; everything stored in memory stays canonical.
 #pragma once
 #include <cstdint>
 
@@ -138,6 +143,37 @@ template <int F> __device__ __forceinline__ Fp<F> fp_sub(const Fp<F>& a, const F
     if (F == FR) fr_sub_asm(r.l, a.l, b.l); else fq_sub_asm(r.l, a.l, b.l);
     return r;
 }
+// lazily reduced: a, b < 2p -> result < 2p; products are the Montgomery value before the final subtraction
+template <int F> __device__ __forceinline__ Fp<F> fp_mul_lazy(const Fp<F>& a, const Fp<F>& b) {
+    Fp<F> r;
+    if (F == FR) fr_mul_lazy_asm(r.l, a.l, b.l); else fq_mul_lazy_asm(r.l, a.l, b.l);
+    return r;
+}
+template <int F> __device__ __forceinline__ Fp<F> fp_sqr_lazy(const Fp<F>& a) {
+#ifdef H2B_SQR_AS_MUL
+    return fp_mul_lazy(a, a);
+#else
+    Fp<F> r;
+    if (F == FR) fr_sqr_lazy_asm(r.l, a.l); else fq_sqr_lazy_asm(r.l, a.l);
+    return r;
+#endif
+}
+template <int F> __device__ __forceinline__ Fp<F> fp_add_lazy(const Fp<F>& a, const Fp<F>& b) {
+    Fp<F> r;
+    if (F == FR) fr_add_lazy_asm(r.l, a.l, b.l); else fq_add_lazy_asm(r.l, a.l, b.l);
+    return r;
+}
+template <int F> __device__ __forceinline__ Fp<F> fp_sub_lazy(const Fp<F>& a, const Fp<F>& b) {
+    Fp<F> r;
+    if (F == FR) fr_sub_lazy_asm(r.l, a.l, b.l); else fq_sub_lazy_asm(r.l, a.l, b.l);
+    return r;
+}
+// [0, 2p) -> [0, p)
+template <int F> __device__ __forceinline__ Fp<F> fp_canon(const Fp<F>& a) {
+    Fp<F> r;
+    if (F == FR) fr_canon_asm(r.l, a.l); else fq_canon_asm(r.l, a.l);
+    return r;
+}
 #else
 // portable bodies for the kernel-logic emulator (tools/emu); same contract, canonical in/out
 template <int F> inline bool fp_geq_p(const uint32_t* t) {
@@ -155,8 +191,8 @@ template <int F> inline void fp_sub_p(uint32_t* t) {
         bw = d >> 32;
     }
 }
-template <int F> inline Fp<F> fp_mul(const Fp<F>& a, const Fp<F>& b) {
-    uint32_t t[10] = {0};
+// Montgomery product without the final subtraction: t[0..8] = (ab + Mp) / 2^256
+template <int F> inline void fp_mont_emu(const Fp<F>& a, const Fp<F>& b, uint32_t (&t)[10]) {
     for (int i = 0; i < 8; ++i) {
         uint64_t c = 0;
         for (int j = 0; j < 8; ++j) { c += (uint64_t)a.l[j] * b.l[i] + t[j]; t[j] = (uint32_t)c; c >>= 32; }
@@ -166,6 +202,10 @@ template <int F> inline Fp<F> fp_mul(const Fp<F>& a, const Fp<F>& b) {
         for (int j = 1; j < 8; ++j) { c += (uint64_t)m * FpParams<F>::P(j) + t[j]; t[j - 1] = (uint32_t)c; c >>= 32; }
         c += t[8]; t[7] = (uint32_t)c; t[8] = t[9] + (uint32_t)(c >> 32);
     }
+}
+template <int F> inline Fp<F> fp_mul(const Fp<F>& a, const Fp<F>& b) {
+    uint32_t t[10] = {0};
+    fp_mont_emu(a, b, t);
     Fp<F> r;
     if (t[8] || fp_geq_p<F>(t)) fp_sub_p<F>(t);
     for (int i = 0; i < 8; ++i) r.l[i] = t[i];
@@ -188,7 +228,49 @@ template <int F> inline Fp<F> fp_sub(const Fp<F>& a, const Fp<F>& b) {
     Fp<F> r; for (int i = 0; i < 8; ++i) r.l[i] = t[i];
     return r;
 }
+// lazily reduced bodies: the same bits as the generated chains ((ab + Mp) / 2^256 is unique; sums and differences
+// are corrected by 2p exactly when the chains correct them)
+template <int F> inline void fp_2p(uint32_t (&q)[8]) {
+    uint64_t c = 0;
+    for (int i = 0; i < 8; ++i) { c += 2 * (uint64_t)FpParams<F>::P(i); q[i] = (uint32_t)c; c >>= 32; }
+}
+template <int F> inline Fp<F> fp_mul_lazy(const Fp<F>& a, const Fp<F>& b) {
+    uint32_t t[10] = {0};
+    fp_mont_emu(a, b, t);
+    Fp<F> r; for (int i = 0; i < 8; ++i) r.l[i] = t[i];
+    return r;
+}
+template <int F> inline Fp<F> fp_sqr_lazy(const Fp<F>& a) { return fp_mul_lazy(a, a); }
+template <int F> inline Fp<F> fp_add_lazy(const Fp<F>& a, const Fp<F>& b) {
+    uint32_t q[8], t[8], s[8]; fp_2p<F>(q);
+    uint64_t c = 0; int64_t bw = 0;
+    for (int i = 0; i < 8; ++i) { c += (uint64_t)a.l[i] + b.l[i]; t[i] = (uint32_t)c; c >>= 32; }
+    for (int i = 0; i < 8; ++i) { int64_t d = (int64_t)t[i] - q[i] + bw; s[i] = (uint32_t)d; bw = d >> 32; }
+    Fp<F> r; for (int i = 0; i < 8; ++i) r.l[i] = bw ? t[i] : s[i];
+    return r;
+}
+template <int F> inline Fp<F> fp_sub_lazy(const Fp<F>& a, const Fp<F>& b) {
+    uint32_t q[8], t[8]; fp_2p<F>(q);
+    int64_t bw = 0;
+    for (int i = 0; i < 8; ++i) { int64_t d = (int64_t)a.l[i] - b.l[i] + bw; t[i] = (uint32_t)d; bw = d >> 32; }
+    if (bw) { uint64_t c = 0; for (int i = 0; i < 8; ++i) { c += (uint64_t)t[i] + q[i]; t[i] = (uint32_t)c; c >>= 32; } }
+    Fp<F> r; for (int i = 0; i < 8; ++i) r.l[i] = t[i];
+    return r;
+}
+template <int F> inline Fp<F> fp_canon(const Fp<F>& a) {
+    Fp<F> r = a;
+    if (fp_geq_p<F>(r.l)) fp_sub_p<F>(r.l);
+    return r;
+}
 #endif
+
+// x == 0 (mod p) for x in [0, 2p): x == 0 or x == p
+template <int F> __device__ __forceinline__ bool fp_is_zero_lazy(const Fp<F>& a) {
+    uint32_t o = 0, d = 0;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) { o |= a.l[i]; d |= a.l[i] ^ FpParams<F>::P(i); }
+    return o == 0 || d == 0;
+}
 
 template <int F> __device__ __forceinline__ Fp<F> fp_neg(const Fp<F>& a) { return fp_sub(fp_zero<F>(), a); }
 template <int F> __device__ __forceinline__ Fp<F> fp_dbl(const Fp<F>& a) { return fp_add(a, a); }

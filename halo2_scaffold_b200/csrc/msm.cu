@@ -673,20 +673,20 @@ __global__ void __launch_bounds__(256) msm_accumulate_kernel(MsmPlan pl, const u
             p_next = affine_load(tables + 4 * (size_t)(e_next & ~SIGN_BIT));
         }
         if (j == next) {        // bucket b is complete: flush, move to the next non-empty bucket
-            if (head) xyzz_store(head_partial + 8 * (size_t)t, acc);
-            else xyzz_store(bucket_acc + 8 * (size_t)b, acc);
+            if (head) xyzz_store(head_partial + 8 * (size_t)t, xyzz_canon(acc));
+            else xyzz_store(bucket_acc + 8 * (size_t)b, xyzz_canon(acc));
             head = false;
             acc = xyzz_identity();
             do { ++b; next = offsets[b + 1]; } while (next <= j);
         }
-        xyzz_add_affine(acc, p, (e & SIGN_BIT) != 0);
+        xyzz_add_affine_lazy(acc, p, (e & SIGN_BIT) != 0);      // acc lazily reduced, canonical when stored
         e = e_next;
         p = p_next;
     }
     if (head) {
-        xyzz_store(head_partial + 8 * (size_t)t, acc);
+        xyzz_store(head_partial + 8 * (size_t)t, xyzz_canon(acc));
     } else {
-        xyzz_store(bucket_acc + 8 * (size_t)b, acc);
+        xyzz_store(bucket_acc + 8 * (size_t)b, xyzz_canon(acc));
         if (next > end) split_list[atomicAdd(&ctrl[0], 1u)] = b;      // continues in later slices
     }
 }

@@ -103,8 +103,10 @@ __device__ __forceinline__ void ntt_round(uint4* lo, uint4* hi, const uint4* tlo
             if (j & dj) continue;
             const uint32_t r = ((uint32_t)(j & (dj - 1)) << loghmin) + lo_part;
             const uint32_t twi = r << (s + st);
-            Fr sum = fp_add(x[j], x[j + dj]), dif = fp_sub(x[j], x[j + dj]);
-            if (twi != 0) dif = fp_mul(dif, sm_get(tlo, thi, twi));
+            // lazily reduced (field.cuh): x stays in [0, 2p) through all rounds, in shared memory too.  (Leaving the
+            // twiddled difference uncorrected, a - b + 2p < 4p, also keeps the product < 2p but spills at 128 registers.)
+            Fr sum = fp_add_lazy(x[j], x[j + dj]), dif = fp_sub_lazy(x[j], x[j + dj]);
+            if (twi != 0) dif = fp_mul_lazy(dif, sm_get(tlo, thi, twi));
             x[j] = sum;
             x[j + dj] = dif;
         }
@@ -191,7 +193,7 @@ __global__ void __launch_bounds__(512, 1) ntt_pass_kernel(NttPassParams p) {
 #pragma unroll 2
             for (uint32_t i = tid; i < E; i += nthr) {
                 uint32_t t = i & (T - 1), q = i >> logT;
-                Fr v = sm_get(lo, hi, i);
+                Fr v = sm_get(lo, hi, i);      // in [0, 2p): the canonical inter-pass product, or fp_canon, reduces it
                 uint32_t ip = __brev(q) >> (32 - b);
                 uint32_t jr = (tau << logT) + t;
                 uint32_t ex = (jr * ip) << logS;
@@ -205,6 +207,8 @@ __global__ void __launch_bounds__(512, 1) ntt_pass_kernel(NttPassParams p) {
                         if (eh != 0) w = fp_mul(w, fp_load<FR>(p.tw_hi + 2 * (size_t)eh));
                     }
                     v = fp_mul(v, w);
+                } else {
+                    v = fp_canon(v);
                 }
                 fp_store<FR>(p_out + 2 * (size_t)(base + q * M + t), v);
             }
@@ -213,7 +217,7 @@ __global__ void __launch_bounds__(512, 1) ntt_pass_kernel(NttPassParams p) {
                 uint32_t tr = i & (T - 1), q = i >> logT;
                 uint32_t t = logT ? (__brev(tr) >> (32 - logT)) : 0u;
                 const uint32_t e = (t << b) + q;
-                Fr v = sm_get(lo, hi, e);
+                Fr v = fp_canon(sm_get(lo, hi, e));
                 uint32_t pos = ((t * nseg + tile) << b) + q;
                 uint32_t oidx = __brev(pos) >> (32 - p.log_n);
                 fp_store<FR>(p_out + 2 * (size_t)oidx, v);

@@ -163,7 +163,8 @@ int msm_checksum_run(DeviceCtx& ctx, const void* d_scalars, uint64_t seed, uint6
 }
 
 // ---- arithmetic self-tests -------------------------------------------------------------------------------
-// op: 0 add, 1 sub, 2 mul, 3 sqr(a), 4 inv(a), 5 from_mont(a), 6 to_mont(a)
+// op: 0 add, 1 sub, 2 mul, 3 sqr(a), 4 inv(a), 5 from_mont(a), 6 to_mont(a); lazily reduced (operands < 2p):
+// 7 mul_lazy, 8 sqr_lazy(a), 9 add_lazy, 10 sub_lazy, 11 canon(a), 12 is_zero_lazy(a) (1 or 0 in the low limb)
 template <int F>
 __global__ void __launch_bounds__(128) field_selftest_kernel(int op, const uint4* __restrict__ a, const uint4* __restrict__ b, uint32_t n, uint4* __restrict__ out) {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -176,7 +177,13 @@ __global__ void __launch_bounds__(128) field_selftest_kernel(int op, const uint4
         case 3: r = fp_sqr(x); break;
         case 4: r = fp_inv(x); break;
         case 5: r = fp_from_mont(x); break;
-        default: r = fp_to_mont(x); break;
+        case 6: r = fp_to_mont(x); break;
+        case 7: r = fp_mul_lazy(x, y); break;
+        case 8: r = fp_sqr_lazy(x); break;
+        case 9: r = fp_add_lazy(x, y); break;
+        case 10: r = fp_sub_lazy(x, y); break;
+        case 11: r = fp_canon(x); break;
+        default: r = fp_zero<F>(); r.l[0] = fp_is_zero_lazy(x) ? 1u : 0u; break;
     }
     fp_store<F>(out + 2 * (size_t)i, r);
 }
@@ -191,7 +198,17 @@ int field_selftest_run(DeviceCtx& ctx, int field, int op, const void* d_a, const
 }
 
 // op 0: affine p + affine q (mixed-add path, through XYZZ);  op 1: p - q;  op 2: general XYZZ add of 2p+q and q
-// (exercises xyzz_add / xyzz_double);  op 3: Jacobian conversion round trip of p+q.  Output affine (64 B).
+// (exercises xyzz_add / xyzz_double);  op 3: Jacobian conversion round trip of p+q;  op 4: p + q by the lazily reduced
+// mixed addition of the MSM accumulation, on an accumulator that holds p with every coordinate offset by the modulus
+// (non-canonical, as a lazily reduced accumulator may be).  Output affine (64 B).
+__device__ __forceinline__ Fq fq_plus_modulus(const Fq& a) {
+    Fq r;
+    uint64_t c = 0;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) { c += (uint64_t)a.l[i] + FpParams<FQ>::P(i); r.l[i] = (uint32_t)c; c >>= 32; }
+    return r;
+}
+
 __global__ void __launch_bounds__(128) ec_selftest_kernel(int op, const uint4* __restrict__ P, const uint4* __restrict__ Q, uint32_t n, uint4* __restrict__ out) {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
@@ -210,6 +227,13 @@ __global__ void __launch_bounds__(128) ec_selftest_kernel(int op, const uint4* _
         xyzz_add(acc, o);                      // 2p + 2q
         xyzz_add(acc, acc);                    // 4p + 4q (doubling branch of the general add)
         res = xyzz_to_affine(acc);
+    } else if (op == 4) {
+        if (!affine_is_identity(p)) {
+            acc.x = fq_plus_modulus(p.x); acc.y = fq_plus_modulus(p.y);
+            acc.zz = fq_plus_modulus(fp_one<FQ>()); acc.zzz = fq_plus_modulus(fp_one<FQ>());
+        }
+        xyzz_add_affine_lazy(acc, q, false);
+        res = xyzz_to_affine(xyzz_canon(acc));
     } else {
         xyzz_add_affine(acc, p, false);
         xyzz_add_affine(acc, q, false);
@@ -293,7 +317,7 @@ __global__ void __launch_bounds__(256) imad_bench_kernel(int iters, uint32_t* si
         g.y = fp_dbl(fp_one<FQ>());
         XYZZ acc = xyzz_double_affine(g);
         acc.x.l[0] ^= 0;   // keep the point valid: 2G, then repeatedly add G
-        for (int i = 0; i < iters; ++i) xyzz_add_affine(acc, g, (i & 7) == 7 && t == 0xffffffffu);
+        for (int i = 0; i < iters; ++i) xyzz_add_affine_lazy(acc, g, (i & 7) == 7 && t == 0xffffffffu);     // the MSM accumulation's addition
         sink[t] = acc.x.l[0] ^ acc.zzz.l[3];
     }
 }

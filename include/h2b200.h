@@ -359,13 +359,15 @@ int h2b_gen_scalars_dev(int device, uint64_t seed, size_t n, int kind, void* d_o
  * field arithmetic only, so it shares no code with the MSM it checks (bench.py `verified`). */
 int h2b_msm_checksum_dev(int device, const void* d_scalars /* n x 32 B Montgomery */, uint64_t seed, uint64_t first, size_t n, void* d_out, void* stream);
 /* element-wise field op on host arrays.  field: 0 Fr, 1 Fq.  op: 0 add, 1 sub, 2 mul, 3 sqr(a), 4 inv(a),
- * 5 from_mont(a), 6 to_mont(a) */
+ * 5 from_mont(a), 6 to_mont(a); the lazily reduced operations of the MSM and NTT loops (operands in [0, 2p)):
+ * 7 mul, 8 sqr(a), 9 add, 10 sub (results in [0, 2p)), 11 canonical form of a, 12 a == 0 mod p (1 or 0 in limb 0) */
 int h2b_field_op(int field, int op, const uint64_t* a, const uint64_t* b, size_t n, uint64_t* out);
 /* element-wise group op on host arrays of affine points; op: 0 p+q, 1 p-q, 2 4(p+q) via the general
- * XYZZ adder and doubling, 3 p+q through the Jacobian conversion.  out: affine. */
+ * XYZZ adder and doubling, 3 p+q through the Jacobian conversion, 4 p+q by the lazily reduced mixed addition
+ * on a non-canonical accumulator.  out: affine. */
 int h2b_ec_op(int op, const uint64_t* p, const uint64_t* q, size_t n, uint64_t* out);
 /* integer-pipe micro-benchmark; kind 0 IMAD, 1 IMAD.WIDE, 2 dependent Fq multiplications, 3 dependent
- * XYZZ mixed additions, 4 dependent Fq squarings, 5 dependent a*b + c*d with one reduction.  Returns elapsed milliseconds and the number of operations executed. */
+ * XYZZ mixed additions (the lazily reduced one of the MSM accumulation), 4 dependent Fq squarings, 5 dependent a*b + c*d with one reduction.  Returns elapsed milliseconds and the number of operations executed. */
 int h2b_imad_bench(int device, int kind, int iters, float* ms_out, double* ops_out);
 /* number of CUDA kernels this library has launched since it was loaded */
 unsigned long long h2b_launch_count(void);

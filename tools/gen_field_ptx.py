@@ -148,7 +148,7 @@ class Prog:
 #   After each row the low limb of E is zero, T is divided by 2^32 by *renaming*:
 #   new E = old O (+ old e1 at limb 0), new O = old E >> 64.
 # =====================================================================================
-def gen_mont_mul(name, mod, square=False):
+def gen_mont_mul(name, mod, square=False, lazy=False):
     p = limbs(mod)
     inv = (-pow(mod, -1, 1 << 32)) & M32
     A = ["a%d" % i for i in range(NL)]
@@ -197,11 +197,13 @@ def gen_mont_mul(name, mod, square=False):
         chain_mad(O, p_odd, m)
         chain_mad(E, p_even, m)
         P.emit("addc", O[NL - 1], O[NL - 1], 0)
-    # T = (E >> 32) + O   (E[0] == 0)
-    t = [P.tmp("t%d" % i) for i in range(NL)]
+    # T = (E >> 32) + O   (E[0] == 0);  T < 2p whenever a*b < p * 2^256
+    t = R if lazy else [P.tmp("t%d" % i) for i in range(NL)]
     for i in range(NL):
         op = "add.cc" if i == 0 else ("addc.cc" if i < NL - 1 else "addc")
         P.emit(op, t[i], O[i], E[i + 1] if i + 1 < NL else 0)
+    if lazy:
+        return P
     # canonical: r = T - p if T >= p
     s = [P.tmp("s%d" % i) for i in range(NL)]
     bw = P.tmp("bw")
@@ -289,8 +291,8 @@ class WideAcc:
                 P.emit("shl1", regs[k], regs[k - 1] if (k > 0 and touched[k - 1]) else 0, regs[k])
 
 
-def redc_tail(P, acc, p, inv, R):
-    """Montgomery reduction of the value held in acc (< p * 2^256) into R (canonical)."""
+def redc_tail(P, acc, p, inv, R, lazy=False):
+    """Montgomery reduction of the value held in acc (< p * 2^256) into R (canonical; lazy: < 2p, no final subtraction)."""
     NLp = NL
     p_even = [p[0], p[2], p[4], p[6]]
     p_odd = [p[1], p[3], p[5], p[7]]
@@ -326,13 +328,15 @@ def redc_tail(P, acc, p, inv, R):
     P.emit("add", creg, csrc, cw8)
     # t = limbs 8..15 of AE + (AO << 32) + counters
     x = [P.tmp("q%d" % k) for k in range(NLp)]
-    t = [P.tmp("t%d" % k) for k in range(NLp)]
+    t = R if lazy else [P.tmp("t%d" % k) for k in range(NLp)]
     for k in range(NLp):
         op = "add.cc" if k == 0 else ("addc.cc" if k < NLp - 1 else "addc")
         P.emit(op, x[k], acc.limb_e(NLp + k), acc.limb_o(NLp + k))
     for k in range(NLp):
         op = "add.cc" if k == 0 else ("addc.cc" if k < NLp - 1 else "addc")
         P.emit(op, t[k], x[k], acc.c.get(NLp + k, 0))
+    if lazy:
+        return
     s = [P.tmp("s%d" % i) for i in range(NLp)]
     bw = P.tmp("bw")
     for i in range(NLp):
@@ -349,7 +353,7 @@ def product_rows(acc, X, Y):
         acc.chain(i + 1, [(X[j], Y[i]) for j in (1, 3, 5, 7)])
 
 
-def gen_mont_sqr_sep(name, mod):
+def gen_mont_sqr_sep(name, mod, lazy=False):
     p = limbs(mod)
     inv = (-pow(mod, -1, 1 << 32)) & M32
     A = ["a%d" % i for i in range(NL)]
@@ -365,7 +369,7 @@ def gen_mont_sqr_sep(name, mod):
     acc.double()
     # squares a_i^2 at limb 2i: one chain over the whole even accumulator
     acc.chain(0, [(A[i], A[i]) for i in range(NL)])
-    redc_tail(P, acc, p, inv, R)
+    redc_tail(P, acc, p, inv, R, lazy)
     return P
 
 
@@ -388,8 +392,8 @@ def gen_mont_mul2_sep(name, mod):
 
 
 
-def gen_add(name, mod):
-    p = limbs(mod)
+def gen_add(name, mod, lazy=False):
+    p = limbs(2 * mod if lazy else mod)      # lazy: inputs and output in [0, 2p), correction by 2p
     A = ["a%d" % i for i in range(NL)]
     B = ["b%d" % i for i in range(NL)]
     R = ["r%d" % i for i in range(NL)]
@@ -407,8 +411,8 @@ def gen_add(name, mod):
     return P
 
 
-def gen_sub(name, mod):
-    p = limbs(mod)
+def gen_sub(name, mod, lazy=False):
+    p = limbs(2 * mod if lazy else mod)
     A = ["a%d" % i for i in range(NL)]
     B = ["b%d" % i for i in range(NL)]
     R = ["r%d" % i for i in range(NL)]
@@ -423,6 +427,22 @@ def gen_sub(name, mod):
         P.emit("and", q[i], bw, p[i])
     for i in range(NL):
         P.emit("add.cc" if i == 0 else ("addc.cc" if i < NL - 1 else "addc"), R[i], t[i], q[i])
+    return P
+
+
+def gen_canon(name, mod):
+    """[0, 2p) -> [0, p): r = a - p if a >= p."""
+    p = limbs(mod)
+    A = ["a%d" % i for i in range(NL)]
+    R = ["r%d" % i for i in range(NL)]
+    P = Prog(name, A, R)
+    s = [P.tmp("s%d" % i) for i in range(NL)]
+    bw = P.tmp("bw")
+    for i in range(NL):
+        P.emit("sub.cc" if i == 0 else "subc.cc", s[i], A[i], p[i])
+    P.emit("subc", bw, 0, 0)
+    for i in range(NL):
+        P.emit("selnz", R[i], bw, A[i], s[i])
     return P
 
 
@@ -474,6 +494,43 @@ def check(prog, mod, kind, trials=3000):
     return len(cases)
 
 
+def check_lazy(prog, mod, kind, trials=3000):
+    """Lazily reduced operations: operands in [0, 2p).  Checks the
+    congruence, the output bound and, for products, the exact value: (a*b + M*p) / 2^256 with M = -a*b/p mod 2^256
+    is the unique Montgomery value before a final subtraction, so every other implementation must give these bits."""
+    rng = random.Random(0x1A2B + mod % 9973 + len(prog.ins))
+    R = 1 << 256
+    Rinv = pow(R, -1, mod)
+    pinv = pow(mod, -1, R)
+    two_p = 2 * mod
+    edge = [0, 1, 2, mod - 1, mod, mod + 1, two_p - 1, two_p - 2, R % mod, mod + R % mod, (mod - 1) // 2, (mod + 1) // 2,
+            0xFFFFFFFF, 0xFFFFFFFF00000000, (1 << 224) - 1, mod - 0xFFFFFFFF, mod + 0xFFFFFFFF, two_p - 0xFFFFFFFF]
+    for sh in range(0, 256, 16):                     # long runs of one-bits at every limb position
+        edge += [((1 << 256) - 1 - ((1 << sh) - 1)) % two_p, ((1 << sh) - 1) % two_p]
+    cases = [(x, y) for x in edge for y in edge]
+    cases += [(rng.randrange(two_p), rng.randrange(two_p)) for _ in range(trials)]
+    for x, y in cases:
+        if kind == "sqr":
+            y = x
+        env = {"z0": 0}
+        for i, l in enumerate(limbs(x)):
+            env["a%d" % i] = l
+        for i, l in enumerate(limbs(y)):
+            env["b%d" % i] = l
+        got = sum(v << (32 * i) for i, v in enumerate(prog.run(env)))
+        if kind in ("mul", "sqr"):
+            ok = got == (x * y + (-x * y * pinv % R) * mod) // R and got < two_p and got % mod == x * y * Rinv % mod
+        elif kind == "add":
+            ok = got < two_p and got % mod == (x + y) % mod
+        elif kind == "sub":
+            ok = got < two_p and got % mod == (x - y) % mod
+        elif kind == "canon":
+            ok = got == x % mod
+        if not ok:
+            raise SystemExit("FAIL %s: x=%x y=%x got=%x" % (prog.name, x, y, got))
+    return len(cases)
+
+
 def main():
     out_path = os.path.join(os.path.dirname(os.path.abspath(__file__)), "..", "halo2_scaffold_b200", "csrc", "field_asm.inc")
     chunks = [
@@ -494,6 +551,23 @@ def main():
                 sig = "__device__ __forceinline__ void %s_%s_asm(uint32_t (&r)[8], const uint32_t (&a)[8])" % (tag, kind)
             else:
                 sig = "__device__ __forceinline__ void %s_%s_asm(uint32_t (&r)[8], const uint32_t (&a)[8], const uint32_t (&b)[8])" % (tag, kind)
+            chunks.append("// %s: %d PTX instructions\n" % (prog.name, len(prog.ins)))
+            chunks.append(prog.to_cuda(sig))
+            chunks.append("\n")
+    chunks.append("// Lazily reduced operations: operands and results in [0, 2p) (canon: result in [0, p)).\n"
+                  "// BN254's p and r are below 2^256 / 5.29, so a Montgomery product of two values < 2p is already < 2p\n"
+                  "// without the final conditional subtraction.\n\n")
+    for tag, mod in (("fr", FR), ("fq", FQ)):
+        for kind, gen in (("mul", lambda n, m: gen_mont_mul(n, m, lazy=True)), ("sqr", lambda n, m: gen_mont_sqr_sep(n, m, lazy=True)),
+                          ("add", lambda n, m: gen_add(n, m, lazy=True)), ("sub", lambda n, m: gen_sub(n, m, lazy=True)),
+                          ("canon", gen_canon)):
+            name = "%s_%s" % (tag, kind) if kind == "canon" else "%s_%s_lazy" % (tag, kind)
+            prog = gen(name, mod)
+            total += check_lazy(prog, mod, kind)
+            if kind in ("sqr", "canon"):
+                sig = "__device__ __forceinline__ void %s_asm(uint32_t (&r)[8], const uint32_t (&a)[8])" % name
+            else:
+                sig = "__device__ __forceinline__ void %s_asm(uint32_t (&r)[8], const uint32_t (&a)[8], const uint32_t (&b)[8])" % name
             chunks.append("// %s: %d PTX instructions\n" % (prog.name, len(prog.ins)))
             chunks.append(prog.to_cuda(sig))
             chunks.append("\n")
