@@ -39,6 +39,7 @@ _EXPORTS = [
     "h2b_fr_lincomb_dev", "h2b_fr_transpose_dev", "h2b_permutation_product_dev", "h2b_lookup_product_dev", "h2b_lookup_permute_dev", "h2b_lookup_permute_async_dev", "h2b_g1_decode_dev", "h2b_g1_encode_dev", "h2b_srs_read", "h2b_srs_write", "h2b_srs_cache_clear",
     "h2b_evaluate_graph_dev", "h2b_evaluate_graph_shard_dev", "h2b_evaluate_h_permutation_shard_dev", "h2b_evaluate_h_lookup_shard_dev", "h2b_evaluate_h_permutation_dev", "h2b_evaluate_h_lookup_dev", "h2b_evaluate_graph_info",
     "h2b_register_bases_sharded", "h2b_msm_bn254_g1_dev_batch_registered", "h2b_implicit_cache_stats", "h2b_msm_checksum_dev", "h2b_ntt_bn254_fr_dev_batch", "h2b_lagrange_to_coeff_dev_batch", "h2b_coeff_to_extended_dev_batch", "h2b_memcpy_d2d_async", "h2b_memset_zero_async", "h2b_column_pipeline",
+    "h2b_srs_setup", "h2b_g1_generator_mul_dev",
 ]
 
 
@@ -172,6 +173,8 @@ class Lib:
         L.h2b_g1_encode_dev.argtypes = [i32, vp, sz, vp, vp]
         L.h2b_srs_read.argtypes = [ctypes.c_char_p, i32, ctypes.POINTER(u32), vp, vp, vp, sz, ctypes.POINTER(sz), ctypes.POINTER(u64), ctypes.POINTER(u64)]
         L.h2b_srs_write.argtypes = [ctypes.c_char_p, i32, u32, vp, vp, vp, sz]
+        L.h2b_srs_setup.argtypes = [u32, vp, vp, vp, ctypes.POINTER(u64), ctypes.POINTER(u64)]
+        L.h2b_g1_generator_mul_dev.argtypes = [i32, vp, sz, vp, vp]
         L.h2b_evaluate_graph_dev.argtypes = [i32, vp, vp, vp, u32, i32, vp]
         L.h2b_evaluate_h_permutation_dev.argtypes = [i32, vp, u32, i32, vp, u32, vp, vp, u32, u32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
         L.h2b_evaluate_h_lookup_dev.argtypes = [i32, vp, vp, vp, u32, i32, vp, vp, vp, vp, vp, vp, vp]
@@ -606,6 +609,37 @@ class Lib:
         assert g.shape[0] == 1 << k and g_lagrange.shape[0] == 1 << k
         buf = np.frombuffer(g2_bytes, dtype=np.uint8).copy()
         self.check(self.L.h2b_srs_write(path.encode(), fmt, k, g.ctypes.data, g_lagrange.ctypes.data, buf.ctypes.data if buf.size else None, buf.size))
+
+    def srs_setup(self, k: int, s, want_host: bool = True, register: bool = True):
+        """ParamsKZG::setup with toxic waste s (4 words, Montgomery) -> the dict of srs_read (g2_bytes empty: G2 is the caller's)"""
+        s = _u64(s).reshape(4)
+        n = 1 << k if 0 <= k <= 28 else 0
+        g = np.empty((n, 8), dtype=np.uint64) if want_host else None
+        gl = np.empty((n, 8), dtype=np.uint64) if want_host else None
+        hg, hl = ctypes.c_uint64(0), ctypes.c_uint64(0)
+        self.check(self.L.h2b_srs_setup(k, s.ctypes.data, g.ctypes.data if want_host else None, gl.ctypes.data if want_host else None,
+                                        ctypes.byref(hg) if register else None, ctypes.byref(hl) if register else None))
+        return dict(k=k, g=g, g_lagrange=gl, g2_bytes=b"", handle_g=hg.value, handle_g_lagrange=hl.value)
+
+    def g1_generator_mul_dev(self, device: int, d_scalars: int, n: int, d_out: int, stream: int = 0):
+        self.check(self.L.h2b_g1_generator_mul_dev(device, d_scalars, n, d_out, stream))
+
+    def g1_generator_mul(self, scalars: np.ndarray, device: int = 0) -> np.ndarray:
+        """(n, 4) Montgomery scalars -> (n, 8) affine [scalar] G, through device memory"""
+        scalars = _u64(scalars).reshape(-1, 4)
+        n = scalars.shape[0]
+        out = np.empty((n, 8), dtype=np.uint64)
+        d_s, d_o = self.dev_alloc(device, max(n, 1) * 32), self.dev_alloc(device, max(n, 1) * 64)
+        try:
+            if n:
+                self.h2d(device, d_s, scalars)
+                self.g1_generator_mul_dev(device, d_s, n, d_o)
+                self.dev_sync(device)
+                self.d2h(device, out, d_o)
+        finally:
+            self.dev_free(device, d_s)
+            self.dev_free(device, d_o)
+        return out
 
     # ---- quotient evaluation (evaluate_h) on device-resident extended-coset columns ------------------
     def evaluate_graph_dev(self, device: int, graph: GraphArrays, cols: EvalColumns, d_values: int, size: int, rot_scale: int, stream: int = 0,

@@ -616,6 +616,8 @@ void h2b_shutdown(void) {
         c->srs_status.release();
         c->lookup_scratch.release();
         c->srs_io.release();
+        c->gen_table.release();
+        c->gen_scratch.release();
         for (cudaEvent_t e : c->copy_events) cudaEventDestroy(e);
         c->copy_events.clear();
         if (c->copy_stream) { cudaStreamDestroy(c->copy_stream); c->copy_stream = nullptr; }
@@ -1290,6 +1292,31 @@ namespace {
 struct FileCloser { FILE* f; ~FileCloser() { if (f) fclose(f); } };
 }  // namespace
 
+// points on device 0 (d_pts, n x 64 B + 64, owned by the new set from here on) -> a registered, replicated base set: peer
+// copies to the other devices, window tables, a handle.  Caller holds G.mu.
+static int adopt_device0_points_locked(void* d_pts, size_t n, const char* caller, const char* what, uint64_t* handle) {
+    DeviceCtx& c = *G.devs[0];
+    SetRef bs(new BaseSet());
+    bs->last_use = ++G.use_counter;
+    bs->n = n;
+    layout_rows(n, false, bs->lo, bs->rows);
+    bs->dev.assign(G.devs.size(), nullptr);
+    for (size_t d = 0; d < G.devs.size(); ++d) bs->ordinal.push_back(G.devs[d]->device);
+    bs->dev[0] = d_pts;
+    for (size_t d = 1; d < G.devs.size(); ++d) {        // the other devices take a peer copy of the points
+        std::lock_guard<std::mutex> lk(G.devs[d]->mu);
+        cudaError_t e = cudaSetDevice(G.devs[d]->device);
+        if (e == cudaSuccess) e = cudaMalloc(&bs->dev[d], n * 64 + 64);
+        if (e == cudaSuccess) e = cudaMemcpyPeer(bs->dev[d], G.devs[d]->device, d_pts, c.device, n * 64);
+        if (e != cudaSuccess) { set_error("%s: copy of %s to device %zu: %s", caller, what, d, cudaGetErrorString(e)); return H2B_ERR_CUDA; }
+    }
+    bs = build_tables(bs);
+    bs->handle = G.next_handle++;
+    *handle = bs->handle;
+    G.sets.push_back(bs);
+    return H2B_OK;
+}
+
 // one vector of the file: bytes -> device 0 -> decoded points; optionally downloaded and / or registered on every device
 static int srs_read_vector(const unsigned char* raw, const char* what, size_t n, int format, uint64_t* host_out, uint64_t* handle) {
     const size_t ps = format == H2B_SERDE_PROCESSED ? 32 : 64;
@@ -1310,25 +1337,29 @@ static int srs_read_vector(const unsigned char* raw, const char* what, size_t n,
         if (!rc && cudaStreamSynchronize(c.stream) != cudaSuccess) { set_error("h2b_srs_read: %s", cudaGetErrorString(cudaGetLastError())); rc = H2B_ERR_CUDA; }
         if (rc || !handle) { cudaFree(d_pts); if (rc) set_error("%s: %s", what, std::string(get_error()).c_str()); return rc; }
     }
-    SetRef bs(new BaseSet());
-    bs->last_use = ++G.use_counter;
-    bs->n = n;
-    layout_rows(n, false, bs->lo, bs->rows);
-    bs->dev.assign(G.devs.size(), nullptr);
-    for (size_t d = 0; d < G.devs.size(); ++d) bs->ordinal.push_back(G.devs[d]->device);
-    bs->dev[0] = d_pts;
-    for (size_t d = 1; d < G.devs.size(); ++d) {        // the other devices take a peer copy of the decoded points
-        std::lock_guard<std::mutex> lk(G.devs[d]->mu);
-        cudaError_t e = cudaSetDevice(G.devs[d]->device);
-        if (e == cudaSuccess) e = cudaMalloc(&bs->dev[d], n * 64 + 64);
-        if (e == cudaSuccess) e = cudaMemcpyPeer(bs->dev[d], G.devs[d]->device, d_pts, c.device, n * 64);
-        if (e != cudaSuccess) { set_error("h2b_srs_read: copy of %s to device %zu: %s", what, d, cudaGetErrorString(e)); return H2B_ERR_CUDA; }
+    return adopt_device0_points_locked(d_pts, n, "h2b_srs_read", what, handle);
+}
+
+// one vector of ParamsKZG::setup (which 0: g, 1: g_lagrange) computed on device 0; optionally downloaded and / or registered
+static int srs_setup_vector(uint32_t k, const uint64_t s[4], int which, uint64_t* host_out, uint64_t* handle) {
+    const size_t n = (size_t)1 << k;
+    const char* what = which ? "g_lagrange" : "g";
+    std::lock_guard<std::mutex> glk(G.mu);
+    DeviceCtx& c = *G.devs[0];
+    void* d_pts = nullptr;
+    {
+        std::lock_guard<std::mutex> lk(c.mu);
+        H2B_CUDA(cudaSetDevice(c.device));
+        cudaError_t e = cudaMalloc(&d_pts, n * 64 + 64);
+        if (e != cudaSuccess) { set_error("cudaMalloc of %zu bytes for %s failed: %s", n * 64, what, cudaGetErrorString(e)); return H2B_ERR_OOM; }
+        const size_t scan_cap = c.scan_scratch.cap;
+        int rc = srs_setup_run(c, k, s, which, d_pts, c.stream);
+        if (!rc && host_out) rc = host_download(c, host_out, d_pts, n * 64, c.stream);
+        if (!rc && cudaStreamSynchronize(c.stream) != cudaSuccess) { set_error("h2b_srs_setup: %s", cudaGetErrorString(cudaGetLastError())); rc = H2B_ERR_CUDA; }
+        if (!rc) g1gen_release_scratch(c, scan_cap);
+        if (rc || !handle) { cudaFree(d_pts); if (rc) set_error("%s: %s", what, std::string(get_error()).c_str()); return rc; }
     }
-    bs = build_tables(bs);
-    bs->handle = G.next_handle++;
-    *handle = bs->handle;
-    G.sets.push_back(bs);
-    return H2B_OK;
+    return adopt_device0_points_locked(d_pts, n, "h2b_srs_setup", what, handle);
 }
 
 namespace {
@@ -1451,6 +1482,26 @@ int h2b_srs_read(const char* path, int format, uint32_t* k, uint64_t* out_g, uin
     if (handle_g) *handle_g = hg;
     if (handle_g_lagrange) *handle_g_lagrange = hl;
     return H2B_OK;
+}
+
+int h2b_srs_setup(uint32_t k, const uint64_t s[4], uint64_t* out_g, uint64_t* out_g_lagrange, uint64_t* handle_g, uint64_t* handle_g_lagrange) {
+    H2B_TRY(require_init());
+    if (!s) { set_error("h2b_srs_setup: null s"); return H2B_ERR_BAD_ARGUMENT; }
+    H2B_TRY(srs_setup_check(k, s));
+    uint64_t hg = 0, hl = 0;
+    H2B_TRY(srs_setup_vector(k, s, 0, out_g, handle_g ? &hg : nullptr));
+    int rc = srs_setup_vector(k, s, 1, out_g_lagrange, handle_g_lagrange ? &hl : nullptr);
+    if (rc != H2B_OK) { if (hg) h2b_unregister_bases(hg); return rc; }
+    if (handle_g) *handle_g = hg;
+    if (handle_g_lagrange) *handle_g_lagrange = hl;
+    return H2B_OK;
+}
+
+int h2b_g1_generator_mul_dev(int device, const void* d_scalars, size_t n, void* d_out_affine, void* stream) {
+    DeviceCtx* c = nullptr;
+    H2B_TRY(get_ctx(device, &c));
+    std::lock_guard<std::mutex> lk(c->mu);
+    return g1_generator_mul_run(*c, d_scalars, n, d_out_affine, (cudaStream_t)stream);
 }
 
 int h2b_srs_cache_clear(void) {
@@ -1623,6 +1674,7 @@ int h2b_dev_sync(int device) {
 int h2b_gen_points_dev(int device, uint64_t seed, size_t n, void* d_out_affine, void* stream) {
     DeviceCtx* c = nullptr;
     H2B_TRY(get_ctx(device, &c));
+    std::lock_guard<std::mutex> lk(c->mu);
     return gen_points_run(*c, seed, n, d_out_affine, (cudaStream_t)stream);
 }
 int h2b_gen_scalars_dev(int device, uint64_t seed, size_t n, int kind, void* d_out, void* stream) {

@@ -61,9 +61,18 @@ struct DevBuf {
     }
 };
 
+// value #index (0-based) of the SplitMix64 stream `seed`: the synthetic points and scalars (g1gen.cu, testgen.cu)
+__host__ __device__ __forceinline__ uint64_t splitmix64_at(uint64_t seed, uint64_t index) {
+    uint64_t z = seed + (index + 1) * 0x9E3779B97F4A7C15ULL;
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ULL;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBULL;
+    return z ^ (z >> 31);
+}
+
 // Optional per-kernel timing with CUDA events on the launching stream (bench.py's roofline numbers).
 enum ProfTag { PROF_BEGIN = 0, PROF_MSM_DECOMPOSE = 1, PROF_MSM_SCAN = 2, PROF_MSM_SCATTER = 3, PROF_MSM_PLAN = 4, PROF_MSM_ACCUMULATE = 5,
-               PROF_MSM_COMBINE = 6, PROF_MSM_REDUCE = 7, PROF_MSM_FINAL = 8, PROF_MSM_PRECOMPUTE = 9, PROF_NTT_TWIDDLE = 15, PROF_NTT_PASS0 = 16 };
+               PROF_MSM_COMBINE = 6, PROF_MSM_REDUCE = 7, PROF_MSM_FINAL = 8, PROF_MSM_PRECOMPUTE = 9, PROF_NTT_TWIDDLE = 15, PROF_NTT_PASS0 = 16,
+               PROF_SRS_SCALARS = 24, PROF_SRS_FIXED_BASE = 25, PROF_SRS_NORMALISE = 26, PROF_SRS_TABLE = 27 };
 struct Profiler {
     bool enabled = false;
     std::vector<cudaEvent_t> ev;
@@ -102,6 +111,8 @@ struct DeviceCtx {
     DevBuf scan_scratch;               // batch inversion / prefix product scratch (scan.cu)
     DevBuf srs_status, srs_io;         // first-invalid-point flag and encoded-bytes staging of the SRS reader (srs.cu)
     DevBuf lookup_scratch;             // sorted keys, flags and ranks of permute_expression_pair (lookup.cu)
+    DevBuf gen_table;                  // fixed-base table of the G1 generator, built on first use (g1gen.cu)
+    DevBuf gen_scratch;                // normalisation denominators and SRS scalars of one chunk (g1gen.cu)
     EvalScratch* eval = nullptr;       // compiled-program ring of the quotient evaluation (evaluate.cu)
     std::vector<NttTwiddles*> twiddles;  // small LRU cache keyed by (omega, log_n)
     MsmScratch* msm = nullptr;
@@ -121,6 +132,7 @@ void stager_release(DeviceCtx& ctx);
 bool host_is_pageable(const void* p);
 // ---- scan.cu ----
 int fr_batch_invert_run(DeviceCtx& ctx, void* d_a, size_t n, cudaStream_t stream);
+int fq_batch_invert_run(DeviceCtx& ctx, void* d_a, size_t n, cudaStream_t stream);
 int fr_prefix_product_run(DeviceCtx& ctx, const void* d_in, void* d_out, size_t n, cudaStream_t stream);
 int fr_eval_polynomial_run(DeviceCtx& ctx, const void* d_coeffs, size_t n, const uint64_t x[4], void* d_out, cudaStream_t stream);
 int fr_kate_division_run(DeviceCtx& ctx, const void* d_a, size_t n, const uint64_t b[4], void* d_q, cudaStream_t stream);
@@ -181,8 +193,14 @@ uint32_t msm_tables_for(uint32_t c0);
 int msm_sum_partials_run(DeviceCtx& ctx, const void* d_blocks, uint32_t count, void* d_out_jac, cudaStream_t stream);
 void msm_release(DeviceCtx& ctx);
 int msm_set_window(int c);   // 0 = automatic
-// ---- testgen.cu ----
+// ---- g1gen.cu ----
 int gen_points_run(DeviceCtx& ctx, uint64_t seed, size_t n, void* d_out_affine, cudaStream_t stream);
+int g1_generator_mul_run(DeviceCtx& ctx, const void* d_scalars, size_t n, void* d_out_affine, cudaStream_t stream);
+int srs_setup_check(uint32_t k, const uint64_t s[4]);
+int srs_setup_run(DeviceCtx& ctx, uint32_t k, const uint64_t s[4], int which, void* d_out_affine, cudaStream_t stream);
+// after a synchronous call: drop the chunk scratch, and scan_scratch if the call grew it (the generator table stays)
+void g1gen_release_scratch(DeviceCtx& ctx, size_t scan_cap_before);
+// ---- testgen.cu ----
 int msm_checksum_run(DeviceCtx& ctx, const void* d_scalars, uint64_t seed, uint64_t first, size_t n, void* d_out, cudaStream_t stream);
 int gen_scalars_run(DeviceCtx& ctx, uint64_t seed, size_t n, int kind, void* d_out, cudaStream_t stream);
 int field_selftest_run(DeviceCtx& ctx, int field, int op, const void* d_a, const void* d_b, size_t n, void* d_out, cudaStream_t stream);

@@ -10,31 +10,33 @@
 
 namespace h2b {
 
-// ---- batch inversion -----------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128) fr_batch_invert_kernel(uint4* __restrict__ a, uint4* __restrict__ pre, size_t n, uint32_t K, uint32_t G) {
+// ---- batch inversion (Fr; Fq for the point normalisation of g1gen.cu) ---------------------------------------------
+template <int F>
+__global__ void __launch_bounds__(128) fp_batch_invert_kernel(uint4* __restrict__ a, uint4* __restrict__ pre, size_t n, uint32_t K, uint32_t G) {
     const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= G) return;
-    Fr run = fp_one<FR>();
+    Fp<F> run = fp_one<F>();
     for (uint32_t j = 0; j < K; ++j) {
         const size_t idx = (size_t)j * G + t;
         if (idx >= n) break;
-        Fr x = fp_load<FR>(a + 2 * idx);
-        fp_store<FR>(pre + 2 * idx, run);
+        Fp<F> x = fp_load<F>(a + 2 * idx);
+        fp_store<F>(pre + 2 * idx, run);
         if (!fp_is_zero(x)) run = fp_mul(run, x);
     }
-    Fr inv = fp_inv(run);
+    Fp<F> inv = fp_inv(run);
     for (uint32_t j = K; j-- > 0;) {
         const size_t idx = (size_t)j * G + t;
         if (idx >= n) continue;
-        Fr x = fp_load<FR>(a + 2 * idx);
+        Fp<F> x = fp_load<F>(a + 2 * idx);
         if (fp_is_zero(x)) continue;
-        Fr p = fp_load<FR>(pre + 2 * idx);
-        fp_store<FR>(a + 2 * idx, fp_mul(inv, p));
+        Fp<F> p = fp_load<F>(pre + 2 * idx);
+        fp_store<F>(a + 2 * idx, fp_mul(inv, p));
         inv = fp_mul(inv, x);
     }
 }
 
-int fr_batch_invert_run(DeviceCtx& ctx, void* d_a, size_t n, cudaStream_t stream) {
+template <int F>
+static int batch_invert_run(DeviceCtx& ctx, void* d_a, size_t n, cudaStream_t stream) {
     if (n == 0) return H2B_OK;
     if (!d_a) { set_error("batch_invert: null pointer"); return H2B_ERR_BAD_ARGUMENT; }
     H2B_TRY(ctx.scan_scratch.reserve(n * 32));
@@ -45,10 +47,12 @@ int fr_batch_invert_run(DeviceCtx& ctx, void* d_a, size_t n, cudaStream_t stream
     if (K < 8) K = 8;
     if (K > 128) K = 128;
     const uint32_t G = (uint32_t)((n + K - 1) / K);
-    H2B_LAUNCH(fr_batch_invert_kernel, (G + 127) / 128, 128, 0, stream, (uint4*)d_a, (uint4*)ctx.scan_scratch.p, n, (uint32_t)K, G);
+    H2B_LAUNCH(fp_batch_invert_kernel<F>, (G + 127) / 128, 128, 0, stream, (uint4*)d_a, (uint4*)ctx.scan_scratch.p, n, (uint32_t)K, G);
     H2B_CUDA(cudaGetLastError());
     return H2B_OK;
 }
+int fr_batch_invert_run(DeviceCtx& ctx, void* d_a, size_t n, cudaStream_t stream) { return batch_invert_run<FR>(ctx, d_a, n, stream); }
+int fq_batch_invert_run(DeviceCtx& ctx, void* d_a, size_t n, cudaStream_t stream) { return batch_invert_run<FQ>(ctx, d_a, n, stream); }
 
 // ---- exclusive prefix product ----------------------------------------------------------------------------------------
 static const uint32_t SCAN_K = 16;          // consecutive elements per thread

@@ -1,6 +1,6 @@
 // Synthetic inputs, device self-tests and integer-pipe micro-benchmarks.
 //
-// * gen_points / gen_scalars build the benchmark workload of SURVEY.md section 8(d) on the device
+// * gen_scalars (and gen_points, g1gen.cu) build the benchmark workload of SURVEY.md section 8(d) on the device
 //   (valid distinct G1 points, uniform or witness-like Fr scalars) so that bench.py never needs the
 //   CPU oracle to produce inputs.  The definitions match oracle/h2_oracle.cpp (orc_gen_points,
 //   orc_random_fr) bit for bit, which the parity tests exploit.
@@ -12,42 +12,6 @@
 #include "ec.cuh"
 
 namespace h2b {
-
-__host__ __device__ __forceinline__ uint64_t splitmix64_at(uint64_t seed, uint64_t index) {
-    uint64_t z = seed + (index + 1) * 0x9E3779B97F4A7C15ULL;
-    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ULL;
-    z = (z ^ (z >> 27)) * 0x94D049BB133111EBULL;
-    return z ^ (z >> 31);
-}
-
-// table[j] = 2^j * G (affine), j < 64.  One thread; runs once per call.
-__global__ void gen_pow2_table_kernel(uint4* table) {
-    if (blockIdx.x != 0 || threadIdx.x != 0) return;
-    Affine g;
-    g.x = fp_one<FQ>();
-    g.y = fp_dbl(fp_one<FQ>());
-    XYZZ t = xyzz_from_affine(g);
-    for (int j = 0; j < 64; ++j) {
-        Affine a = xyzz_to_affine(t);
-        affine_store(table + 4 * j, a);
-        t = xyzz_double(t);
-    }
-}
-
-// P_i = [z_i] G, z_i = SplitMix64 value #(first + i) of stream `seed`
-__global__ void __launch_bounds__(128) gen_points_kernel(const uint4* __restrict__ table, uint64_t seed, uint64_t first, uint32_t n, uint4* __restrict__ out) {
-    uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    uint64_t z = splitmix64_at(seed, first + i);
-    XYZZ acc = xyzz_identity();
-    for (int j = 0; j < 64; ++j) {
-        if ((z >> j) & 1) {
-            Affine p = affine_load(table + 4 * j);
-            xyzz_add_affine(acc, p, false);
-        }
-    }
-    affine_store(out + 4 * (size_t)i, xyzz_to_affine(acc));
-}
 
 // kind 0: uniform in [0, r): 512-bit SplitMix64 draw (big-endian word order) reduced mod r.
 // kind 1: witness-like skew (SURVEY.md 8d): 50 % zero, 20 % one, 20 % uniform < 2^19, 10 % r - small.
@@ -79,24 +43,6 @@ __global__ void __launch_bounds__(256) gen_scalars_kernel(uint64_t seed, uint64_
         if (sel == 9) r = fp_neg(r);
     }
     fp_store<FR>(out + 2 * (size_t)i, r);
-}
-
-int gen_points_run(DeviceCtx& ctx, uint64_t seed, size_t n, void* d_out, cudaStream_t stream) {
-    (void)ctx;
-    if (n == 0) return H2B_OK;
-    DevBuf table;
-    H2B_TRY(table.reserve(64 * 64));
-    H2B_LAUNCH(gen_pow2_table_kernel, 1, 32, 0, stream, (uint4*)table.p);
-    for (size_t done = 0; done < n; done += (size_t)1 << 24) {
-        uint32_t m = (uint32_t)((n - done < ((size_t)1 << 24)) ? n - done : (size_t)1 << 24);
-        H2B_LAUNCH(gen_points_kernel, (m + 127) / 128, 128, 0, stream, (const uint4*)table.p, seed, (uint64_t)done, m, (uint4*)d_out + 4 * done);
-    }
-    cudaError_t e = cudaGetLastError();
-    cudaError_t e2 = cudaStreamSynchronize(stream);
-    table.release();
-    H2B_CUDA(e);
-    H2B_CUDA(e2);
-    return H2B_OK;
 }
 
 int gen_scalars_run(DeviceCtx& ctx, uint64_t seed, size_t n, int kind, void* d_out, cudaStream_t stream) {

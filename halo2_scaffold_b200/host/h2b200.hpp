@@ -309,6 +309,11 @@ class ParamsKZG {
                            g2_bytes_.data(), g2_bytes_.size(), &g2_len, &g_, &g_lagrange_), "ParamsKZG::read_custom");
         g2_bytes_.resize(g2_len);
     }
+    // pub fn setup<R: RngCore>(k: u32, rng: R) -> Self with the toxic waste s = Fr::random(rng) drawn by the caller: both vectors are
+    // computed on the device and stay resident there.  g2_bytes (g2 | s_g2 as write_custom stores them) are the caller's (G2 is host work).
+    static std::unique_ptr<ParamsKZG> setup(uint32_t k, const Fr& s, std::vector<uint8_t> g2_bytes = {}) {
+        return std::unique_ptr<ParamsKZG>(new ParamsKZG(k, s, std::move(g2_bytes)));
+    }
     // pub fn write_custom<W: io::Write>(&self, writer, format)
     void write_custom(const std::string& path, SerdeFormat format) const {
         check(h2b_srs_write(path.c_str(), (int)format, k_, reinterpret_cast<const uint64_t*>(host_g_.data()), reinterpret_cast<const uint64_t*>(host_g_lagrange_.data()),
@@ -352,6 +357,14 @@ class ParamsKZG {
     }
 
   private:
+    ParamsKZG(uint32_t k, const Fr& s, std::vector<uint8_t> g2_bytes) : k_(k), g2_bytes_(std::move(g2_bytes)) {
+        ensure_init();
+        if (k > 28) throw Panic("ParamsKZG::setup: k out of range");
+        n_ = (uint64_t)1 << k;
+        host_g_.resize(n_); host_g_lagrange_.resize(n_);
+        check(h2b_srs_setup(k, s.l, reinterpret_cast<uint64_t*>(host_g_.data()), reinterpret_cast<uint64_t*>(host_g_lagrange_.data()), &g_, &g_lagrange_),
+              "ParamsKZG::setup");
+    }
     std::vector<G1> msm_many(const std::vector<std::vector<Fr>>& polys, uint64_t handle) const {
         std::vector<const uint64_t*> ptrs;
         std::vector<size_t> lens;

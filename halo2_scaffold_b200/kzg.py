@@ -45,6 +45,17 @@ class ParamsKZG:
         return cls(r["k"], r["g"], r["g_lagrange"], lib, r["g2_bytes"], (r["handle_g"], r["handle_g_lagrange"]))
 
     @classmethod
+    def setup(cls, k: int, s, lib=None, g2_bytes: bytes = b"") -> "ParamsKZG":
+        """ParamsKZG::setup with the caller's toxic waste s (4 words, Montgomery): both vectors are computed on the device and
+        stay resident there as registered base sets.  g2_bytes (g2 | s_g2 as write_custom stores them) come from the caller:
+        G2 arithmetic is the host's business."""
+        lib = lib or _lib.load()
+        if lib.device_count() == 0:
+            lib.init(0)
+        r = lib.srs_setup(k, s)
+        return cls(k, r["g"], r["g_lagrange"], lib, g2_bytes, (r["handle_g"], r["handle_g_lagrange"]))
+
+    @classmethod
     def read(cls, path: str, lib=None) -> "ParamsKZG":
         """ParamsKZG::read = read_custom(reader, SerdeFormat::RawBytes)"""
         return cls.read_custom(path, SerdeFormat.RawBytes, lib)

@@ -335,6 +335,20 @@ int h2b_srs_cache_clear(void);
 /* ParamsKZG::write_custom for host arrays (Processed: compressed on the device) */
 int h2b_srs_write(const char* path, int format, uint32_t k, const uint64_t* g, const uint64_t* g_lagrange, const uint8_t* g2_bytes, size_t g2_len);
 
+/* ParamsKZG::setup ([UP] halo2_proofs/src/poly/kzg/commitment.rs) with the caller's toxic waste s (Montgomery, < r):
+ * g[i] = [s^i] G, g_lagrange[i] = [L_i(s)] G for i < 2^k, k <= 28, G = (1, 2), computed on device 0 by fixed-base
+ * multiplication (w = ROOT_OF_UNITY^(2^(28 - k)) is derived on the device).  Output convention of h2b_srs_read:
+ * out_g / out_g_lagrange (2^k x 8 words, may be NULL) receive the points; handle_g / handle_g_lagrange (may be NULL)
+ * receive registered, replicated base sets with window tables.  Synchronous.  k > 28, s >= r and s^(2^k) = 1 (s a power
+ * of w, s = 1 included: a denominator s - w^i vanishes) fail with H2B_ERR_BAD_ARGUMENT before anything is allocated;
+ * s = 0 is legal (g = [G, O, O, ...], g_lagrange[i] = [1/n] G). */
+int h2b_srs_setup(uint32_t k, const uint64_t s[4], uint64_t* out_g, uint64_t* out_g_lagrange, uint64_t* handle_g, uint64_t* handle_g_lagrange);
+/* out[i] = [scalars[i]] G (G = (1, 2)); scalars n x 4 words Montgomery (< r), out n x 8 words affine, identity (0, 0);
+ * asynchronous on `stream`.  The first call on a device builds its fixed-base table (32 MiB, kept until h2b_shutdown, as are
+ * h2b_srs_setup's and h2b_gen_points_dev's); being asynchronous, this call also keeps its scratch (64 B per point up to 2^24
+ * points, plus the batch-inversion scratch) reserved until h2b_shutdown, as the other device-pointer entry points do. */
+int h2b_g1_generator_mul_dev(int device, const void* d_scalars, size_t n, void* d_out_affine, void* stream);
+
 /* ---- raw device memory helpers (so that non-CUDA hosts -- ctypes, Rust -- can hold device buffers) --- */
 int h2b_dev_alloc(int device, size_t bytes, void** out);
 int h2b_dev_free(int device, void* p);
@@ -374,7 +388,9 @@ unsigned long long h2b_launch_count(void);
 /* per-kernel timing with CUDA events recorded on the launching stream. After h2b_profile_enable(device, 1) every
  * MSM / NTT call records one event per phase; h2b_profile_read synchronises the device and returns (tag, ms) pairs
  * in launch order.  MSM tags: 1 decompose, 2 scan, 3 scatter, 4 plan, 5 accumulate, 6 combine, 7 bucket reduction,
- * 8 final;  NTT tags: 15 twiddle tables, 16 + p = pass p. */
+ * 8 final;  NTT tags: 15 twiddle tables, 16 + p = pass p;  h2b_srs_setup tags (per vector and chunk of 2^24 points):
+ * 24 scalars (powers, inversion, scaling), 25 fixed-base multiplication, 26 normalisation, 27 generator table (first use
+ * on the device only); registering the results records 9 (window tables) as every registered base set does. */
 int h2b_profile_enable(int device, int on);
 int h2b_profile_read(int device, int* tags, float* ms, int cap, int* count);
 /* force the MSM window size (0 = automatic) -- tuning / tests only */

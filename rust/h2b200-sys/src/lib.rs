@@ -100,6 +100,9 @@ extern "C" {
                         g2_len: *mut usize, handle_g: *mut u64, handle_g_lagrange: *mut u64) -> c_int;
     pub fn h2b_srs_write(path: *const c_char, format: c_int, k: u32, g: *const u64, g_lagrange: *const u64, g2_bytes: *const u8, g2_len: usize) -> c_int;
     pub fn h2b_srs_cache_clear() -> c_int;
+    // ParamsKZG::setup on the device and the fixed-base multiples of the generator it is built on
+    pub fn h2b_srs_setup(k: u32, s: *const u64, out_g: *mut u64, out_g_lagrange: *mut u64, handle_g: *mut u64, handle_g_lagrange: *mut u64) -> c_int;
+    pub fn h2b_g1_generator_mul_dev(device: c_int, d_scalars: *const c_void, n: usize, d_out_affine: *mut c_void, stream: *mut c_void) -> c_int;
     pub fn h2b_dev_alloc(device: c_int, bytes: usize, out: *mut *mut c_void) -> c_int;
     pub fn h2b_dev_free(device: c_int, p: *mut c_void) -> c_int;
     pub fn h2b_memcpy_h2d(device: c_int, d_dst: *mut c_void, h_src: *const c_void, bytes: usize) -> c_int;
@@ -163,4 +166,21 @@ pub fn ntt_bn254_fr(a: &mut [[u64; 4]], omega: &[u64; 4], log_n: u32) {
     if rc != 0 {
         panic!("h2b_ntt_bn254_fr failed ({rc}): {}", last_error());
     }
+}
+
+/// The G1 half of `ParamsKZG::<Bn256>::setup(k, rng)` for the toxic waste `s` (Montgomery limbs, `Fr::random(rng)` drawn by
+/// the caller): `g[i] = [s^i] G`, `g_lagrange[i] = [L_i(s)] G` as `2^k x 8` u64 each, plus the handles of both vectors as
+/// registered base sets (window tables built on every device).  Panics like upstream's `invert().unwrap()` when `s` is a
+/// `2^k`-th root of unity, and on `k > 28`.
+pub fn srs_setup(k: u32, s: &[u64; 4]) -> (Vec<[u64; 8]>, Vec<[u64; 8]>, u64, u64) {
+    assert!(k <= 28);
+    ensure_init();
+    let n = 1usize << k;
+    let (mut g, mut g_lagrange) = (vec![[0u64; 8]; n], vec![[0u64; 8]; n]);
+    let (mut hg, mut hl) = (0u64, 0u64);
+    let rc = unsafe { h2b_srs_setup(k, s.as_ptr(), g.as_mut_ptr() as *mut u64, g_lagrange.as_mut_ptr() as *mut u64, &mut hg, &mut hl) };
+    if rc != 0 {
+        panic!("h2b_srs_setup failed ({rc}): {}", last_error());
+    }
+    (g, g_lagrange, hg, hl)
 }
