@@ -39,7 +39,7 @@ _EXPORTS = [
     "h2b_fr_lincomb_dev", "h2b_fr_transpose_dev", "h2b_permutation_product_dev", "h2b_lookup_product_dev", "h2b_lookup_permute_dev", "h2b_lookup_permute_async_dev", "h2b_g1_decode_dev", "h2b_g1_encode_dev", "h2b_srs_read", "h2b_srs_write", "h2b_srs_cache_clear",
     "h2b_evaluate_graph_dev", "h2b_evaluate_graph_shard_dev", "h2b_evaluate_h_permutation_shard_dev", "h2b_evaluate_h_lookup_shard_dev", "h2b_evaluate_h_permutation_dev", "h2b_evaluate_h_lookup_dev", "h2b_evaluate_graph_info",
     "h2b_register_bases_sharded", "h2b_msm_bn254_g1_dev_batch_registered", "h2b_implicit_cache_stats", "h2b_msm_checksum_dev", "h2b_ntt_bn254_fr_dev_batch", "h2b_lagrange_to_coeff_dev_batch", "h2b_coeff_to_extended_dev_batch", "h2b_memcpy_d2d_async", "h2b_memset_zero_async", "h2b_column_pipeline",
-    "h2b_srs_setup", "h2b_g1_generator_mul_dev",
+    "h2b_srs_setup", "h2b_g1_generator_mul_dev", "h2b_g1_to_lagrange_dev", "h2b_srs_downsize",
 ]
 
 
@@ -175,6 +175,8 @@ class Lib:
         L.h2b_srs_write.argtypes = [ctypes.c_char_p, i32, u32, vp, vp, vp, sz]
         L.h2b_srs_setup.argtypes = [u32, vp, vp, vp, ctypes.POINTER(u64), ctypes.POINTER(u64)]
         L.h2b_g1_generator_mul_dev.argtypes = [i32, vp, sz, vp, vp]
+        L.h2b_g1_to_lagrange_dev.argtypes = [i32, vp, u32, vp, vp]
+        L.h2b_srs_downsize.argtypes = [u64, u32, vp, ctypes.POINTER(u64), ctypes.POINTER(u64)]
         L.h2b_evaluate_graph_dev.argtypes = [i32, vp, vp, vp, u32, i32, vp]
         L.h2b_evaluate_h_permutation_dev.argtypes = [i32, vp, u32, i32, vp, u32, vp, vp, u32, u32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
         L.h2b_evaluate_h_lookup_dev.argtypes = [i32, vp, vp, vp, u32, i32, vp, vp, vp, vp, vp, vp, vp]
@@ -640,6 +642,34 @@ class Lib:
             self.dev_free(device, d_s)
             self.dev_free(device, d_o)
         return out
+
+    def g1_to_lagrange_dev(self, device: int, d_g: int, k: int, d_out: int, stream: int = 0):
+        self.check(self.L.h2b_g1_to_lagrange_dev(device, d_g, k, d_out, stream))
+
+    def g1_to_lagrange(self, points: np.ndarray, k: int, device: int = 0) -> np.ndarray:
+        """g_to_lagrange of the first 2^k of the (n, 8) affine points -> (2^k, 8) affine, through device memory"""
+        points = _u64(points).reshape(-1, 8)
+        n = 1 << k
+        assert points.shape[0] >= n
+        out = np.empty((n, 8), dtype=np.uint64)
+        d_p = self.dev_alloc(device, n * 64)
+        try:
+            self.h2d(device, d_p, points[:n])
+            self.g1_to_lagrange_dev(device, d_p, k, d_p)
+            self.dev_sync(device)
+            self.d2h(device, out, d_p)
+        finally:
+            self.dev_free(device, d_p)
+        return out
+
+    def srs_downsize(self, handle_g: int, k: int, want_host: bool = True, register: bool = True):
+        """ParamsKZG::downsize of the resident g of a replicated set -> dict(g_lagrange (host copy or None), handle_g,
+        handle_g_lagrange) with new sets for the 2^k-point prefix of g and its g_lagrange (0 when not registered)"""
+        gl = np.empty((1 << k, 8), dtype=np.uint64) if want_host and 0 <= k <= 28 else None
+        hg, hl = ctypes.c_uint64(0), ctypes.c_uint64(0)
+        self.check(self.L.h2b_srs_downsize(handle_g, k, gl.ctypes.data if gl is not None else None,
+                                           ctypes.byref(hg) if register else None, ctypes.byref(hl) if register else None))
+        return dict(g_lagrange=gl, handle_g=hg.value, handle_g_lagrange=hl.value)
 
     # ---- quotient evaluation (evaluate_h) on device-resident extended-coset columns ------------------
     def evaluate_graph_dev(self, device: int, graph: GraphArrays, cols: EvalColumns, d_values: int, size: int, rot_scale: int, stream: int = 0,

@@ -1504,6 +1504,66 @@ int h2b_g1_generator_mul_dev(int device, const void* d_scalars, size_t n, void* 
     return g1_generator_mul_run(*c, d_scalars, n, d_out_affine, (cudaStream_t)stream);
 }
 
+int h2b_g1_to_lagrange_dev(int device, const void* d_g_affine, uint32_t k, void* d_out_affine, void* stream) {
+    DeviceCtx* c = nullptr;
+    H2B_TRY(get_ctx(device, &c));
+    std::lock_guard<std::mutex> lk(c->mu);
+    return g1_to_lagrange_run(*c, d_g_affine, k, d_out_affine, (cudaStream_t)stream);
+}
+
+int h2b_srs_downsize(uint64_t handle_g, uint32_t k, uint64_t* out_g_lagrange, uint64_t* handle_g_out, uint64_t* handle_g_lagrange_out) {
+    H2B_TRY(require_init());
+    if (k > 28) { set_error("h2b_srs_downsize: k = %u (at most 28)", k); return H2B_ERR_BAD_ARGUMENT; }
+    const size_t n = (size_t)1 << k;
+    std::lock_guard<std::mutex> glk(G.mu);
+    SetRef src = find_set_locked(handle_g);
+    if (!src || src->implicit) { set_error("h2b_srs_downsize: unknown base-set handle %llu", (unsigned long long)handle_g); return H2B_ERR_BAD_ARGUMENT; }
+    if (src->sharded) { set_error("h2b_srs_downsize: handle %llu is a sharded set (g must be whole on device 0)", (unsigned long long)handle_g); return H2B_ERR_BAD_ARGUMENT; }
+    if (n > src->n) { set_error("h2b_srs_downsize: 2^%u points requested from a set of %zu", k, src->n); return H2B_ERR_BAD_ARGUMENT; }
+    const bool want_gl = out_g_lagrange || handle_g_lagrange_out;
+    DeviceCtx& c = *G.devs[0];
+    void* d_g = nullptr;
+    void* d_gl = nullptr;
+    {
+        std::lock_guard<std::mutex> lk(c.mu);
+        H2B_CUDA(cudaSetDevice(c.device));
+        int rc = H2B_OK;
+        if (handle_g_out && cudaMalloc(&d_g, n * 64 + 64) != cudaSuccess) rc = H2B_ERR_OOM;
+        if (!rc && want_gl && cudaMalloc(&d_gl, n * 64 + 64) != cudaSuccess) rc = H2B_ERR_OOM;
+        if (rc) set_error("h2b_srs_downsize: cudaMalloc of %zu bytes failed", n * 64);
+        if (!rc && d_g && cudaMemcpyAsync(d_g, src->dev[0], n * 64, cudaMemcpyDeviceToDevice, c.stream) != cudaSuccess) {
+            set_error("h2b_srs_downsize: copy of g: %s", cudaGetErrorString(cudaGetLastError()));
+            rc = H2B_ERR_CUDA;
+        }
+        const size_t scan_cap = c.scan_scratch.cap;
+        if (!rc && d_gl) rc = g1_to_lagrange_run(c, src->dev[0], k, d_gl, c.stream);
+        if (!rc && out_g_lagrange) rc = host_download(c, out_g_lagrange, d_gl, n * 64, c.stream);
+        if (!rc && cudaStreamSynchronize(c.stream) != cudaSuccess) { set_error("h2b_srs_downsize: %s", cudaGetErrorString(cudaGetLastError())); rc = H2B_ERR_CUDA; }
+        g1gen_release_scratch(c, scan_cap);
+        if (rc) {
+            if (d_g) cudaFree(d_g);
+            if (d_gl) cudaFree(d_gl);
+            return rc;
+        }
+        if (d_gl && !handle_g_lagrange_out) { cudaFree(d_gl); d_gl = nullptr; }
+    }
+    uint64_t hg = 0, hl = 0;
+    if (d_g) {
+        int rc = adopt_device0_points_locked(d_g, n, "h2b_srs_downsize", "g", &hg);
+        if (rc) { if (d_gl) cudaFree(d_gl); return rc; }
+    }
+    if (d_gl) {
+        int rc = adopt_device0_points_locked(d_gl, n, "h2b_srs_downsize", "g_lagrange", &hl);
+        if (rc) {
+            if (hg) drop_locked(hg);
+            return rc;
+        }
+    }
+    if (handle_g_out) *handle_g_out = hg;
+    if (handle_g_lagrange_out) *handle_g_lagrange_out = hl;
+    return H2B_OK;
+}
+
 int h2b_srs_cache_clear(void) {
     H2B_TRY(require_init());
     std::vector<uint64_t> drop;
@@ -1719,7 +1779,7 @@ int h2b_field_op(int field, int op, const uint64_t* a, const uint64_t* b, size_t
     return elementwise_host(0, field, op, a, b, n, out, 32);
 }
 int h2b_ec_op(int op, const uint64_t* p, const uint64_t* q, size_t n, uint64_t* out) {
-    if (op < 0 || op > 4) { set_error("h2b_ec_op: bad op"); return H2B_ERR_BAD_ARGUMENT; }
+    if (op < 0 || op > 5) { set_error("h2b_ec_op: bad op"); return H2B_ERR_BAD_ARGUMENT; }
     return elementwise_host(1, 0, op, p, q, n, out, 64);
 }
 

@@ -72,7 +72,8 @@ __host__ __device__ __forceinline__ uint64_t splitmix64_at(uint64_t seed, uint64
 // Optional per-kernel timing with CUDA events on the launching stream (bench.py's roofline numbers).
 enum ProfTag { PROF_BEGIN = 0, PROF_MSM_DECOMPOSE = 1, PROF_MSM_SCAN = 2, PROF_MSM_SCATTER = 3, PROF_MSM_PLAN = 4, PROF_MSM_ACCUMULATE = 5,
                PROF_MSM_COMBINE = 6, PROF_MSM_REDUCE = 7, PROF_MSM_FINAL = 8, PROF_MSM_PRECOMPUTE = 9, PROF_NTT_TWIDDLE = 15, PROF_NTT_PASS0 = 16,
-               PROF_SRS_SCALARS = 24, PROF_SRS_FIXED_BASE = 25, PROF_SRS_NORMALISE = 26, PROF_SRS_TABLE = 27 };
+               PROF_SRS_SCALARS = 24, PROF_SRS_FIXED_BASE = 25, PROF_SRS_NORMALISE = 26, PROF_SRS_TABLE = 27,
+               PROF_G1NTT_TWIDDLE = 28, PROF_G1NTT_STAGES = 29, PROF_G1NTT_NORMALISE = 30 };
 struct Profiler {
     bool enabled = false;
     std::vector<cudaEvent_t> ev;
@@ -112,7 +113,7 @@ struct DeviceCtx {
     DevBuf srs_status, srs_io;         // first-invalid-point flag and encoded-bytes staging of the SRS reader (srs.cu)
     DevBuf lookup_scratch;             // sorted keys, flags and ranks of permute_expression_pair (lookup.cu)
     DevBuf gen_table;                  // fixed-base table of the G1 generator, built on first use (g1gen.cu)
-    DevBuf gen_scratch;                // normalisation denominators and SRS scalars of one chunk (g1gen.cu)
+    DevBuf gen_scratch;                // normalisation denominators and SRS scalars of one chunk; the G1 NTT work buffer (g1gen.cu)
     EvalScratch* eval = nullptr;       // compiled-program ring of the quotient evaluation (evaluate.cu)
     std::vector<NttTwiddles*> twiddles;  // small LRU cache keyed by (omega, log_n)
     MsmScratch* msm = nullptr;
@@ -198,6 +199,8 @@ int gen_points_run(DeviceCtx& ctx, uint64_t seed, size_t n, void* d_out_affine, 
 int g1_generator_mul_run(DeviceCtx& ctx, const void* d_scalars, size_t n, void* d_out_affine, cudaStream_t stream);
 int srs_setup_check(uint32_t k, const uint64_t s[4]);
 int srs_setup_run(DeviceCtx& ctx, uint32_t k, const uint64_t s[4], int which, void* d_out_affine, cudaStream_t stream);
+// g_to_lagrange of the first 2^k affine points of d_g into d_out (may equal d_g); asynchronous, scratch in gen_scratch
+int g1_to_lagrange_run(DeviceCtx& ctx, const void* d_g, uint32_t k, void* d_out_affine, cudaStream_t stream);
 // after a synchronous call: drop the chunk scratch, and scan_scratch if the call grew it (the generator table stays)
 void g1gen_release_scratch(DeviceCtx& ctx, size_t scan_cap_before);
 // ---- testgen.cu ----

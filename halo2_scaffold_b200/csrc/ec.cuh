@@ -218,6 +218,53 @@ __device__ __forceinline__ void xyzz_add_body(XYZZ& acc, const XYZZ& b) {
     acc.zzz = fq_m<SHARED>(fq_m<SHARED>(acc.zzz, b.zzz), ppp);
 }
 
+// [e] P for a canonical (non-Montgomery) e < 2^254 and any P, the variable-base multiplication of the G1 NTT (g1gen.cu).
+// Left to right over Booth (signed radix-2^W) digits d_j = ((x + 1) >> 1) - 2^W (x >> W) in [-2^(W-1), 2^(W-1)], x the W + 1
+// bits [jW - 1, jW + W - 1] of e (bit -1 = 0): each digit is read straight off the scalar, with no carry from the digits
+// below, so the loop consumes them top down.  A per-thread table T[m - 1] = m P, m = 1 .. 2^(W-1); per window W doublings
+// and one complete general addition of +-T[|d| - 1].  W = H2B_G1_MUL_WINDOW is chosen by measurement (DESIGN.md 5.8).
+#ifndef H2B_G1_MUL_WINDOW
+#define H2B_G1_MUL_WINDOW 4
+#endif
+static const int G1_MUL_W = H2B_G1_MUL_WINDOW;
+static const int G1_MUL_WINDOWS = (255 + G1_MUL_W - 1) / G1_MUL_W;     // W * windows >= 255: the top digit is never negative
+static_assert(G1_MUL_W >= 1 && G1_MUL_W <= 6, "variable-base window out of range");
+
+__device__ __forceinline__ XYZZ xyzz_mul_scalar(const XYZZ& p, const Fp<FR>& e) {
+    const int TAB = 1 << (G1_MUL_W - 1);
+    XYZZ tab[TAB];
+    tab[0] = p;
+    if (TAB > 1) tab[1] = xyzz_double(p);
+#pragma unroll 1
+    for (int m = 2; m < TAB; ++m) { tab[m] = tab[m - 1]; xyzz_add(tab[m], p); }
+    // z = 2 e in 9 words; after t windows it is shifted left by t W, so the field of the current window is always at bit TOP
+    uint32_t z[9];
+    z[0] = e.l[0] << 1;
+#pragma unroll
+    for (int i = 1; i < 8; ++i) z[i] = __funnelshift_l(e.l[i - 1], e.l[i], 1);
+    z[8] = e.l[7] >> 31;
+    const int TOP = G1_MUL_W * (G1_MUL_WINDOWS - 1), TW = TOP / 32, TS = TOP % 32;
+    XYZZ acc = xyzz_identity();
+#pragma unroll 1
+    for (int t = 0; t < G1_MUL_WINDOWS; ++t) {
+        if (t) {
+#pragma unroll
+            for (int b = 0; b < G1_MUL_W; ++b) acc = xyzz_double(acc);
+        }
+        const uint32_t x = __funnelshift_r(z[TW], z[TW + 1], TS) & ((2u << G1_MUL_W) - 1);
+#pragma unroll
+        for (int i = 8; i > 0; --i) z[i] = __funnelshift_l(z[i - 1], z[i], G1_MUL_W);
+        z[0] <<= G1_MUL_W;
+        const int d = (int)((x + 1) >> 1) - (int)((x >> G1_MUL_W) << G1_MUL_W);
+        if (d != 0) {
+            XYZZ q = tab[(d < 0 ? -d : d) - 1];
+            if (d < 0) q.y = fp_neg(q.y);
+            xyzz_add(acc, q);
+        }
+    }
+    return acc;
+}
+
 // XYZZ -> a Jacobian representative (X', Y', Z') of the same point without an inversion:
 // Z' = ZZ*ZZZ, X' = X*ZZ*ZZZ^2, Y' = Y*ZZ^3*ZZZ^2  (then X'/Z'^2 = X/ZZ and Y'/Z'^3 = Y/ZZZ).
 // Identity -> (0, 1, 0), matching halo2curves' G1::identity().

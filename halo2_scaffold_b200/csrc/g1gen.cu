@@ -13,6 +13,8 @@
 //   g_lagrange[i] = [L_i(s)] G, L_i(s) = w^i (s^n - 1) / (n (s - w^i)), by one scalar multiplication per point on the CPU.
 //   Here L_i(s) = c / (s w^-i - 1) with c = (s^n - 1) / n: the denominators are one power table, one batch inversion and
 //   one scaling, and both vectors go through the fixed-base kernel.
+// * g1_to_lagrange (ParamsKZG::downsize): a radix-2 NTT over G1 points, see the section at the end; it shares the
+//   normalisation with the two above.
 #include "common.h"
 #include "ec.cuh"
 
@@ -302,6 +304,115 @@ int srs_setup_run(DeviceCtx& ctx, uint32_t k, const uint64_t s_words[4], int whi
         return H2B_OK;
     };
     return g1gen_run(ctx, n, (uint4*)d_out, stream, [&](size_t) { return ScalarArray{scal}; }, fill, true);
+}
+
+// ---- g_to_lagrange: a radix-2 NTT over G1 points -----------------------------------------------------------------------
+// [UP] halo2_proofs/src/arithmetic.rs g_to_lagrange: g_lagrange[i] = n^-1 sum_j w^(-ij) g[j] (best_fft over C::Curve with
+// omega_inv, *= n_inv, batch_normalize).  One butterfly is two general additions and one variable-base scalar multiplication
+// (xyzz_mul_scalar, ~3300 Fq multiplications) on 256 bytes of points, so the transform is arithmetic-bound by three orders of
+// magnitude: one launch per radix-2 stage, one thread per butterfly, in place on an n x 128 B XYZZ work buffer.
+// Decimation in frequency on the natural-order input: stage s pairs i and i + n / 2^(s+1) and gives (a + b, w^(-j 2^s) (a - b)).
+// Stage 0 reads the affine input and folds n^-1 in (n^-1 (a + b), (n^-1 w^-j) (a - b): n / 2 extra multiplications instead of
+// n); the last stage has only trivial twiddles and stores the projective half of the normalisation at the bit-reversed index.
+
+// consts[0] = w (from ntt_root_powers_run) -> consts[0] = w^-1, consts[1] = 1 / 2^k
+__global__ void g1ntt_constants_kernel(uint32_t k, uint4* consts) {
+    if (blockIdx.x != 0 || threadIdx.x != 0) return;
+    Fr n = fp_zero<FR>();
+    n.l[0] = 1u << k;
+    fp_store<FR>(consts, fp_inv(fp_load<FR>(consts)));
+    fp_store<FR>(consts + 2, fp_inv(fp_to_mont(n)));
+}
+
+// tw[i] = w^-i for i < m (Montgomery), SRS_RUN consecutive powers per thread as srs_powers_kernel does; the base is read
+// from the device, so the call stays asynchronous
+__global__ void __launch_bounds__(128) g1ntt_twiddle_kernel(const uint4* __restrict__ consts, uint32_t m, uint4* __restrict__ tw) {
+    const uint32_t i0 = (blockIdx.x * blockDim.x + threadIdx.x) * SRS_RUN;
+    if (i0 >= m) return;
+    const Fr base = fp_load<FR>(consts);
+    Fr cur = fp_pow_u32(base, i0);
+    for (uint32_t i = i0; i < i0 + SRS_RUN && i < m; ++i) {
+        fp_store<FR>(tw + 2 * (size_t)i, cur);
+        cur = fp_mul(cur, base);
+    }
+}
+
+// one DIF stage; MODE bit 0: the first stage (affine input, n^-1 folded in), bit 1: the last (projective normalisation half
+// stored at the bit-reversed index into out / den)
+template <int MODE>
+__global__ void __launch_bounds__(128) g1ntt_stage_kernel(const uint4* __restrict__ in, uint4* __restrict__ work, const uint4* __restrict__ tw,
+                                                           const uint4* __restrict__ consts, uint32_t log_n, uint32_t s, uint4* __restrict__ out,
+                                                           uint4* __restrict__ den) {
+    const bool FIRST = MODE & 1, LAST = MODE & 2;
+    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= (1u << (log_n - 1))) return;
+    const uint32_t lh = log_n - 1 - s, j = t & ((1u << lh) - 1);
+    const uint32_t i0 = ((t >> lh) << (lh + 1)) | j, i1 = i0 + (1u << lh);
+    XYZZ a, b;
+    if (FIRST) {
+        a = xyzz_from_affine(affine_load(in + 4 * (size_t)i0));
+        b = xyzz_from_affine(affine_load(in + 4 * (size_t)i1));
+    } else {
+        a = xyzz_load(work + 8 * (size_t)i0);
+        b = xyzz_load(work + 8 * (size_t)i1);
+    }
+    XYZZ sum = a;
+    xyzz_add(sum, b);
+    b.y = fp_neg(b.y);
+    xyzz_add(a, b);                                 // a - b
+    if (FIRST) {
+        const Fr ninv = fp_load<FR>(consts + 2);
+        sum = xyzz_mul_scalar(sum, fp_from_mont(ninv));
+        a = xyzz_mul_scalar(a, fp_from_mont(fp_mul(ninv, fp_load<FR>(tw + 2 * (size_t)j))));
+    } else if (j != 0) {
+        a = xyzz_mul_scalar(a, fp_from_mont(fp_load<FR>(tw + 2 * ((size_t)j << s))));
+    }
+    if (LAST) {
+        const uint32_t r0 = __brev(i0) >> (32 - log_n), r1 = __brev(i1) >> (32 - log_n);
+        gen_store_projective(sum, out + 4 * (size_t)r0, den + 2 * (size_t)r0);
+        gen_store_projective(a, out + 4 * (size_t)r1, den + 2 * (size_t)r1);
+    } else {
+        xyzz_store(work + 8 * (size_t)i0, sum);
+        xyzz_store(work + 8 * (size_t)i1, a);
+    }
+}
+
+// d_out[i] = g_to_lagrange(d_g)[i] for i < 2^k (d_out may be d_g); asynchronous, the scratch stays reserved in gen_scratch
+int g1_to_lagrange_run(DeviceCtx& ctx, const void* d_g, uint32_t k, void* d_out, cudaStream_t stream) {
+    if (k > 28) { set_error("g1_to_lagrange: k = %u (at most 28)", k); return H2B_ERR_BAD_ARGUMENT; }
+    if (!d_g || !d_out) { set_error("g1_to_lagrange: null pointer"); return H2B_ERR_BAD_ARGUMENT; }
+    if (k == 0) {                                   // n^-1 = 1, a transform of length one
+        if (d_out != d_g) H2B_CUDA(cudaMemcpyAsync(d_out, d_g, 64, cudaMemcpyDeviceToDevice, stream));
+        return H2B_OK;
+    }
+    const size_t n = (size_t)1 << k;
+    H2B_TRY(ctx.gen_scratch.reserve(n * 128 + n * 32 + (n / 2) * 32 + 64));      // work | den | twiddles | constants
+    H2B_TRY(ctx.scan_scratch.reserve(n * 32));
+    uint4* work = (uint4*)ctx.gen_scratch.p;
+    uint4* den = work + 8 * n;
+    uint4* tw = den + 2 * n;
+    uint4* consts = tw + n;
+    ctx.prof.mark(PROF_BEGIN, stream);
+    H2B_TRY(ntt_root_powers_run(ctx, FR_ROOT_OF_UNITY_MONT, 28 - k, 28 - k, consts, stream));
+    H2B_LAUNCH(g1ntt_constants_kernel, 1, 32, 0, stream, k, consts);
+    const uint32_t half = (uint32_t)(n / 2);
+    H2B_LAUNCH(g1ntt_twiddle_kernel, (half + 128 * SRS_RUN - 1) / (128 * SRS_RUN), 128, 0, stream, (const uint4*)consts, half, tw);
+    ctx.prof.mark(PROF_G1NTT_TWIDDLE, stream);
+    const unsigned grid = (half + 127) / 128;
+    const uint4* g = (const uint4*)d_g;
+    uint4* out = (uint4*)d_out;
+    if (k == 1) {
+        H2B_LAUNCH(g1ntt_stage_kernel<3>, grid, 128, 0, stream, g, work, (const uint4*)tw, (const uint4*)consts, k, 0u, out, den);
+    } else {
+        H2B_LAUNCH(g1ntt_stage_kernel<1>, grid, 128, 0, stream, g, work, (const uint4*)tw, (const uint4*)consts, k, 0u, out, den);
+        for (uint32_t s = 1; s + 1 < k; ++s)
+            H2B_LAUNCH(g1ntt_stage_kernel<0>, grid, 128, 0, stream, g, work, (const uint4*)tw, (const uint4*)consts, k, s, out, den);
+        H2B_LAUNCH(g1ntt_stage_kernel<2>, grid, 128, 0, stream, g, work, (const uint4*)tw, (const uint4*)consts, k, k - 1, out, den);
+    }
+    ctx.prof.mark(PROF_G1NTT_STAGES, stream);
+    H2B_TRY(g1gen_normalise(ctx, out, den, n, stream));
+    ctx.prof.mark(PROF_G1NTT_NORMALISE, stream);
+    return H2B_OK;
 }
 
 }  // namespace h2b

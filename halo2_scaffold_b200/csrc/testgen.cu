@@ -146,7 +146,8 @@ int field_selftest_run(DeviceCtx& ctx, int field, int op, const void* d_a, const
 // op 0: affine p + affine q (mixed-add path, through XYZZ);  op 1: p - q;  op 2: general XYZZ add of 2p+q and q
 // (exercises xyzz_add / xyzz_double);  op 3: Jacobian conversion round trip of p+q;  op 4: p + q by the lazily reduced
 // mixed addition of the MSM accumulation, on an accumulator that holds p with every coordinate offset by the modulus
-// (non-canonical, as a lazily reduced accumulator may be).  Output affine (64 B).
+// (non-canonical, as a lazily reduced accumulator may be);  op 5: [e] p by the variable-base multiplication of the G1 NTT,
+// e = the first 4 words of q (Fr, Montgomery).  Output affine (64 B).
 __device__ __forceinline__ Fq fq_plus_modulus(const Fq& a) {
     Fq r;
     uint64_t c = 0;
@@ -173,6 +174,11 @@ __global__ void __launch_bounds__(128) ec_selftest_kernel(int op, const uint4* _
         xyzz_add(acc, o);                      // 2p + 2q
         xyzz_add(acc, acc);                    // 4p + 4q (doubling branch of the general add)
         res = xyzz_to_affine(acc);
+    } else if (op == 5) {
+        Fr e;
+#pragma unroll
+        for (int l = 0; l < 8; ++l) e.l[l] = q.x.l[l];
+        res = xyzz_to_affine(xyzz_mul_scalar(xyzz_from_affine(p), fp_from_mont(e)));
     } else if (op == 4) {
         if (!affine_is_identity(p)) {
             acc.x = fq_plus_modulus(p.x); acc.y = fq_plus_modulus(p.y);

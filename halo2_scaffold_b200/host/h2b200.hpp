@@ -319,6 +319,20 @@ class ParamsKZG {
         check(h2b_srs_write(path.c_str(), (int)format, k_, reinterpret_cast<const uint64_t*>(host_g_.data()), reinterpret_cast<const uint64_t*>(host_g_lagrange_.data()),
                             g2_bytes_.data(), g2_bytes_.size()), "ParamsKZG::write_custom");
     }
+    // fn downsize(&mut self, k: u32): g keeps its first 2^k points, g_lagrange is recomputed from them on the device
+    // (g_to_lagrange); both become new resident sets and the old ones are given back.  g2_bytes are kept.
+    void downsize(uint32_t k) {
+        if (k > k_) throw Panic("ParamsKZG::downsize: k above the params' k");
+        uint64_t hg = 0, hl = 0;
+        std::vector<G1Affine> gl((size_t)1 << k);
+        check(h2b_srs_downsize(g_, k, reinterpret_cast<uint64_t*>(gl.data()), &hg, &hl), "ParamsKZG::downsize");
+        h2b_unregister_bases(g_);
+        h2b_unregister_bases(g_lagrange_);
+        g_ = hg; g_lagrange_ = hl;
+        k_ = k; n_ = (uint64_t)1 << k;
+        host_g_.resize(n_);
+        host_g_lagrange_ = std::move(gl);
+    }
     const std::vector<G1Affine>& get_g() const { return host_g_; }
     const std::vector<G1Affine>& get_g_lagrange() const { return host_g_lagrange_; }
     const std::vector<uint8_t>& g2_bytes() const { return g2_bytes_; }

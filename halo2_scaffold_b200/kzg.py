@@ -60,6 +60,20 @@ class ParamsKZG:
         """ParamsKZG::read = read_custom(reader, SerdeFormat::RawBytes)"""
         return cls.read_custom(path, SerdeFormat.RawBytes, lib)
 
+    def downsize(self, k: int):
+        """ParamsKZG::downsize: keep the first 2^k points of g and recompute g_lagrange from them on the device
+        (g_to_lagrange); both become new resident sets and the old ones are given back.  g2_bytes are kept."""
+        assert k <= self.k, "downsize: k = %d above the params' k = %d" % (k, self.k)
+        r = self.lib.srs_downsize(self._g, k)
+        old = (self._g, self._g_lagrange)
+        self.k, self.n = k, 1 << k
+        self.g = self.g[:self.n].copy()
+        self.g_lagrange = r["g_lagrange"]
+        self._g, self._g_lagrange = r["handle_g"], r["handle_g_lagrange"]
+        for h in old:
+            if h:
+                self.lib.unregister_bases(h)
+
     def write_custom(self, path: str, fmt: int):
         self.lib.srs_write(path, fmt, self.k, self.g, self.g_lagrange, self.g2_bytes)
 

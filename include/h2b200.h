@@ -348,6 +348,20 @@ int h2b_srs_setup(uint32_t k, const uint64_t s[4], uint64_t* out_g, uint64_t* ou
  * h2b_srs_setup's and h2b_gen_points_dev's); being asynchronous, this call also keeps its scratch (64 B per point up to 2^24
  * points, plus the batch-inversion scratch) reserved until h2b_shutdown, as the other device-pointer entry points do. */
 int h2b_g1_generator_mul_dev(int device, const void* d_scalars, size_t n, void* d_out_affine, void* stream);
+/* g_to_lagrange ([UP] halo2_proofs/src/arithmetic.rs) of the first 2^k affine points at d_g_affine (n x 8 words, identity
+ * (0, 0) allowed anywhere): d_out[i] = n^-1 sum_j w^(-ij) g[j], w = ROOT_OF_UNITY^(2^(28 - k)) the root of the Fr NTT of the
+ * same k, batch-normalised affine, bit-identical to upstream's.  d_out may equal d_g.  Asynchronous on `stream`; its
+ * scratch (about 200 B per point) stays reserved until h2b_shutdown, as h2b_g1_generator_mul_dev's does.  k > 28 and null
+ * pointers fail with H2B_ERR_BAD_ARGUMENT. */
+int h2b_g1_to_lagrange_dev(int device, const void* d_g_affine, uint32_t k, void* d_out_affine, void* stream);
+/* ParamsKZG::downsize(k) ([UP] halo2_proofs/src/poly/kzg/commitment.rs) of the resident g of a REPLICATED registered set
+ * (h2b_srs_read, h2b_srs_setup, h2b_register_bases): handle_g_out (may be NULL) receives a new registered set holding the
+ * 2^k-point prefix of g (a device-to-device copy, window tables sized for 2^k), handle_g_lagrange_out (may be NULL) a new
+ * registered set of g_to_lagrange of that prefix, and out_g_lagrange (2^k x 8 words, may be NULL) its host copy.  The caller
+ * truncates its own host g and drops the old handles when it wants to.  Synchronous; gives its scratch back before it returns.
+ * k > 28, 2^k above the set's n, an unknown handle and a sharded set fail with H2B_ERR_BAD_ARGUMENT before anything is
+ * allocated, and leave the output handles untouched. */
+int h2b_srs_downsize(uint64_t handle_g, uint32_t k, uint64_t* out_g_lagrange, uint64_t* handle_g_out, uint64_t* handle_g_lagrange_out);
 
 /* ---- raw device memory helpers (so that non-CUDA hosts -- ctypes, Rust -- can hold device buffers) --- */
 int h2b_dev_alloc(int device, size_t bytes, void** out);
@@ -378,7 +392,8 @@ int h2b_msm_checksum_dev(int device, const void* d_scalars /* n x 32 B Montgomer
 int h2b_field_op(int field, int op, const uint64_t* a, const uint64_t* b, size_t n, uint64_t* out);
 /* element-wise group op on host arrays of affine points; op: 0 p+q, 1 p-q, 2 4(p+q) via the general
  * XYZZ adder and doubling, 3 p+q through the Jacobian conversion, 4 p+q by the lazily reduced mixed addition
- * on a non-canonical accumulator.  out: affine. */
+ * on a non-canonical accumulator, 5 [e] p by the variable-base multiplication of h2b_g1_to_lagrange_dev with e the
+ * first 4 words of q (Fr, Montgomery).  out: affine. */
 int h2b_ec_op(int op, const uint64_t* p, const uint64_t* q, size_t n, uint64_t* out);
 /* integer-pipe micro-benchmark; kind 0 IMAD, 1 IMAD.WIDE, 2 dependent Fq multiplications, 3 dependent
  * XYZZ mixed additions (the lazily reduced one of the MSM accumulation), 4 dependent Fq squarings, 5 dependent a*b + c*d with one reduction.  Returns elapsed milliseconds and the number of operations executed. */
@@ -390,7 +405,9 @@ unsigned long long h2b_launch_count(void);
  * in launch order.  MSM tags: 1 decompose, 2 scan, 3 scatter, 4 plan, 5 accumulate, 6 combine, 7 bucket reduction,
  * 8 final;  NTT tags: 15 twiddle tables, 16 + p = pass p;  h2b_srs_setup tags (per vector and chunk of 2^24 points):
  * 24 scalars (powers, inversion, scaling), 25 fixed-base multiplication, 26 normalisation, 27 generator table (first use
- * on the device only); registering the results records 9 (window tables) as every registered base set does. */
+ * on the device only); registering the results records 9 (window tables) as every registered base set does;
+ * h2b_g1_to_lagrange_dev / h2b_srs_downsize tags: 28 twiddles (w^-1, n^-1 and the power table), 29 butterfly stages (all
+ * k of them), 30 normalisation (batch inversion and the affine finish). */
 int h2b_profile_enable(int device, int on);
 int h2b_profile_read(int device, int* tags, float* ms, int cap, int* count);
 /* force the MSM window size (0 = automatic) -- tuning / tests only */

@@ -103,6 +103,9 @@ extern "C" {
     // ParamsKZG::setup on the device and the fixed-base multiples of the generator it is built on
     pub fn h2b_srs_setup(k: u32, s: *const u64, out_g: *mut u64, out_g_lagrange: *mut u64, handle_g: *mut u64, handle_g_lagrange: *mut u64) -> c_int;
     pub fn h2b_g1_generator_mul_dev(device: c_int, d_scalars: *const c_void, n: usize, d_out_affine: *mut c_void, stream: *mut c_void) -> c_int;
+    // ParamsKZG::downsize on the device and the G1 NTT (g_to_lagrange) it is built on
+    pub fn h2b_g1_to_lagrange_dev(device: c_int, d_g_affine: *const c_void, k: u32, d_out_affine: *mut c_void, stream: *mut c_void) -> c_int;
+    pub fn h2b_srs_downsize(handle_g: u64, k: u32, out_g_lagrange: *mut u64, handle_g_out: *mut u64, handle_g_lagrange_out: *mut u64) -> c_int;
     pub fn h2b_dev_alloc(device: c_int, bytes: usize, out: *mut *mut c_void) -> c_int;
     pub fn h2b_dev_free(device: c_int, p: *mut c_void) -> c_int;
     pub fn h2b_memcpy_h2d(device: c_int, d_dst: *mut c_void, h_src: *const c_void, bytes: usize) -> c_int;
@@ -183,4 +186,20 @@ pub fn srs_setup(k: u32, s: &[u64; 4]) -> (Vec<[u64; 8]>, Vec<[u64; 8]>, u64, u6
         panic!("h2b_srs_setup failed ({rc}): {}", last_error());
     }
     (g, g_lagrange, hg, hl)
+}
+
+/// The G1 half of `ParamsKZG::<Bn256>::downsize(k)` on the resident g of the registered, replicated set `handle_g`:
+/// `g_lagrange` of the `2^k`-point prefix of g (`g_to_lagrange`, computed on the device) as `2^k x 8` u64, plus the handles of
+/// two new registered sets, the prefix of g and that g_lagrange.  The old handles stay valid; the caller gives them back.
+/// Panics like upstream's `assert!(k <= self.k)` when `2^k` exceeds the set.
+pub fn srs_downsize(handle_g: u64, k: u32) -> (Vec<[u64; 8]>, u64, u64) {
+    assert!(k <= 28);
+    ensure_init();
+    let mut g_lagrange = vec![[0u64; 8]; 1usize << k];
+    let (mut hg, mut hl) = (0u64, 0u64);
+    let rc = unsafe { h2b_srs_downsize(handle_g, k, g_lagrange.as_mut_ptr() as *mut u64, &mut hg, &mut hl) };
+    if rc != 0 {
+        panic!("h2b_srs_downsize failed ({rc}): {}", last_error());
+    }
+    (g_lagrange, hg, hl)
 }

@@ -151,6 +151,10 @@ static inline unsigned __funnelshift_r(unsigned lo, unsigned hi, unsigned s) {
     uint64_t v = ((uint64_t)hi << 32) | lo;
     return (unsigned)(v >> (s & 31));
 }
+static inline unsigned __funnelshift_l(unsigned lo, unsigned hi, unsigned s) {
+    uint64_t v = ((uint64_t)hi << 32) | lo;
+    return (unsigned)((v << (s & 31)) >> 32);
+}
 
 // atomics: blocks may run on different OS threads
 static inline unsigned atomicAdd(unsigned* p, unsigned v) { return __atomic_fetch_add(p, v, __ATOMIC_RELAXED); }
