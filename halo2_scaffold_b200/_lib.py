@@ -40,6 +40,7 @@ _EXPORTS = [
     "h2b_evaluate_graph_dev", "h2b_evaluate_graph_shard_dev", "h2b_evaluate_h_permutation_shard_dev", "h2b_evaluate_h_lookup_shard_dev", "h2b_evaluate_h_permutation_dev", "h2b_evaluate_h_lookup_dev", "h2b_evaluate_graph_info",
     "h2b_register_bases_sharded", "h2b_msm_bn254_g1_dev_batch_registered", "h2b_implicit_cache_stats", "h2b_msm_checksum_dev", "h2b_ntt_bn254_fr_dev_batch", "h2b_lagrange_to_coeff_dev_batch", "h2b_coeff_to_extended_dev_batch", "h2b_memcpy_d2d_async", "h2b_memset_zero_async", "h2b_column_pipeline",
     "h2b_srs_setup", "h2b_g1_generator_mul_dev", "h2b_g1_to_lagrange_dev", "h2b_srs_downsize",
+    "h2b_permutation_sigma_dev", "h2b_keygen_lagrange_indicators_dev", "h2b_permutation_build_vk", "h2b_permutation_build_pk",
 ]
 
 
@@ -118,6 +119,18 @@ def _u64(a: np.ndarray) -> np.ndarray:
     return a
 
 
+def _ptr_array(ptrs):
+    return (ctypes.c_void_p * len(ptrs))(*ptrs)
+
+
+def _mapping_columns(mapping, k: int):
+    """a permutation mapping -- (P, 2^k, 2) uint64 or a list of (2^k, 2) columns of (column, row) pairs -> contiguous columns"""
+    cols = [_u64(c).reshape(-1, 2) for c in mapping]
+    for c in cols:
+        assert c.shape[0] == 1 << k, "mapping column of %d rows, expected 2^%d" % (c.shape[0], k)
+    return cols
+
+
 class Lib:
     def __init__(self, path: str | None = None, allow_emulator: bool = False):
         path = path or os.environ.get("H2B200_LIB", DEFAULT_LIB)
@@ -177,6 +190,10 @@ class Lib:
         L.h2b_g1_generator_mul_dev.argtypes = [i32, vp, sz, vp, vp]
         L.h2b_g1_to_lagrange_dev.argtypes = [i32, vp, u32, vp, vp]
         L.h2b_srs_downsize.argtypes = [u64, u32, vp, ctypes.POINTER(u64), ctypes.POINTER(u64)]
+        L.h2b_permutation_sigma_dev.argtypes = [i32, vp, u32, u32, vp, vp, vp, vp, vp]
+        L.h2b_keygen_lagrange_indicators_dev.argtypes = [i32, u32, u32, u32, vp, vp, vp, vp, vp, vp, vp, vp]
+        L.h2b_permutation_build_vk.argtypes = [vp, u32, u32, vp, vp, u64, vp]
+        L.h2b_permutation_build_pk.argtypes = [vp, u32, u32, u32, vp, vp, vp, vp, vp, vp, vp, vp, vp]
         L.h2b_evaluate_graph_dev.argtypes = [i32, vp, vp, vp, u32, i32, vp]
         L.h2b_evaluate_h_permutation_dev.argtypes = [i32, vp, u32, i32, vp, u32, vp, vp, u32, u32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
         L.h2b_evaluate_h_lookup_dev.argtypes = [i32, vp, vp, vp, u32, i32, vp, vp, vp, vp, vp, vp, vp]
@@ -670,6 +687,61 @@ class Lib:
         self.check(self.L.h2b_srs_downsize(handle_g, k, gl.ctypes.data if gl is not None else None,
                                            ctypes.byref(hg) if register else None, ctypes.byref(hl) if register else None))
         return dict(g_lagrange=gl, handle_g=hg.value, handle_g_lagrange=hl.value)
+
+    # ---- key generation: permutation sigma columns and keygen_pk's indicator columns -------------------------------
+    def permutation_sigma_dev(self, device: int, d_mapping, k: int, delta, omega, d_sigma, d_status: int, stream: int = 0):
+        """sigma of len(d_mapping) mapping columns (device pointers, n x 16 B each) into d_sigma; the status word at d_status is
+        1 + the flat index of an out-of-range entry, 0 when all are valid (read it after synchronising `stream`)"""
+        m, s = _ptr_array(d_mapping), _ptr_array(d_sigma)
+        w = [_u64(x).reshape(4) for x in (delta, omega)]
+        self.check(self.L.h2b_permutation_sigma_dev(device, m, len(d_mapping), k, w[0].ctypes.data, w[1].ctypes.data, s, d_status, stream))
+
+    def keygen_lagrange_indicators_dev(self, device: int, k: int, extended_k: int, blinding_factors: int, omega_inv, ifft_divisor, extended_omega,
+                                       zeta_powers, d_l0: int, d_l_last: int, d_l_active_row: int, stream: int = 0):
+        w = [_u64(x).reshape(4) for x in (omega_inv, ifft_divisor, extended_omega)]
+        zp = _u64(zeta_powers).reshape(3, 4)
+        self.check(self.L.h2b_keygen_lagrange_indicators_dev(device, k, extended_k, blinding_factors, w[0].ctypes.data, w[1].ctypes.data, w[2].ctypes.data,
+                                                             zp.ctypes.data, d_l0, d_l_last, d_l_active_row, stream))
+
+    def keygen_lagrange_indicators(self, k: int, extended_k: int, blinding_factors: int, omega_inv, ifft_divisor, extended_omega, zeta_powers,
+                                   device: int = 0):
+        """(l0, l_last, l_active_row) of keygen_pk, each (2^extended_k, 4), computed on the device and downloaded"""
+        en = 1 << extended_k
+        outs = [np.empty((en, 4), dtype=np.uint64) for _ in range(3)]
+        d = [self.dev_alloc(device, en * 32) for _ in range(3)]
+        try:
+            self.keygen_lagrange_indicators_dev(device, k, extended_k, blinding_factors, omega_inv, ifft_divisor, extended_omega, zeta_powers, *d)
+            self.dev_sync(device)
+            for o, p in zip(outs, d):
+                self.d2h(device, o, p)
+        finally:
+            for p in d:
+                self.dev_free(device, p)
+        return tuple(outs)
+
+    def permutation_build_vk(self, mapping, k: int, delta, omega, handle_g_lagrange: int) -> np.ndarray:
+        """Assembly::build_vk: mapping (P, 2^k, 2) uint64 (or a list of (2^k, 2) columns) -> (P, 12) Jacobian commitments"""
+        cols = _mapping_columns(mapping, k)
+        w = [_u64(x).reshape(4) for x in (delta, omega)]
+        out = np.zeros((len(cols), 12), dtype=np.uint64)
+        self.check(self.L.h2b_permutation_build_vk(_ptr_array([c.ctypes.data for c in cols]), len(cols), k, w[0].ctypes.data, w[1].ctypes.data,
+                                                   handle_g_lagrange, out.ctypes.data))
+        return out
+
+    def permutation_build_pk(self, mapping, k: int, extended_k: int, delta, omega, omega_inv, ifft_divisor, extended_omega, zeta_powers,
+                             want_permutations: bool = True, want_polys: bool = True, want_cosets: bool = True):
+        """Assembly::build_pk -> dict(permutations, polys, cosets): lists of (2^k, 4), (2^k, 4) and (2^extended_k, 4) arrays (None when not wanted)"""
+        cols = _mapping_columns(mapping, k)
+        P, n = len(cols), 1 << k
+        w = [_u64(x).reshape(4) for x in (delta, omega, omega_inv, ifft_divisor, extended_omega)]
+        zp = _u64(zeta_powers).reshape(3, 4)
+        perms = [np.empty((n, 4), dtype=np.uint64) for _ in range(P)] if want_permutations else None
+        polys = [np.empty((n, 4), dtype=np.uint64) for _ in range(P)] if want_polys else None
+        cosets = [np.empty((1 << extended_k, 4), dtype=np.uint64) for _ in range(P)] if want_cosets else None
+        arr = lambda xs: _ptr_array([x.ctypes.data for x in xs]) if xs is not None else None
+        self.check(self.L.h2b_permutation_build_pk(_ptr_array([c.ctypes.data for c in cols]), P, k, extended_k, *[x.ctypes.data for x in w],
+                                                   zp.ctypes.data, arr(perms), arr(polys), arr(cosets)))
+        return dict(permutations=perms, polys=polys, cosets=cosets)
 
     # ---- quotient evaluation (evaluate_h) on device-resident extended-coset columns ------------------
     def evaluate_graph_dev(self, device: int, graph: GraphArrays, cols: EvalColumns, d_values: int, size: int, rot_scale: int, stream: int = 0,

@@ -1119,8 +1119,7 @@ int h2b_lagrange_to_coeff_dev_batch(int device, void* const* d_cols, size_t coun
     if (count == 0) return H2B_OK;
     if (!d_cols || !omega_inv || !ifft_divisor) { set_error("h2b_lagrange_to_coeff_dev_batch: null pointer"); return H2B_ERR_BAD_ARGUMENT; }
     std::lock_guard<std::mutex> lk(c->mu);
-    H2B_TRY(ntt_run_batch(*c, d_cols, count, omega_inv, k, (cudaStream_t)stream));
-    return ntt_scale_batch_run(*c, d_cols, count, (size_t)1 << k, ifft_divisor, 1, (cudaStream_t)stream);
+    return lagrange_to_coeff_batch_run(*c, d_cols, count, k, omega_inv, ifft_divisor, (cudaStream_t)stream);
 }
 
 int h2b_coeff_to_extended_dev_batch(int device, void* const* d_cols, size_t count, uint32_t k, uint32_t extended_k, const uint64_t extended_omega[4],
@@ -1131,11 +1130,7 @@ int h2b_coeff_to_extended_dev_batch(int device, void* const* d_cols, size_t coun
     if (!d_cols || !extended_omega || !zeta_powers) { set_error("h2b_coeff_to_extended_dev_batch: null pointer"); return H2B_ERR_BAD_ARGUMENT; }
     if (extended_k < k || extended_k > 28) { set_error("h2b_coeff_to_extended_dev_batch: need k <= extended_k <= 28"); return H2B_ERR_BAD_ARGUMENT; }
     std::lock_guard<std::mutex> lk(c->mu);
-    const size_t n = (size_t)1 << k, en = (size_t)1 << extended_k;
-    H2B_TRY(ntt_scale_batch_run(*c, d_cols, count, n, zeta_powers, 3, (cudaStream_t)stream));
-    if (en > n)
-        for (size_t j = 0; j < count; ++j) H2B_CUDA(cudaMemsetAsync((char*)d_cols[j] + n * 32, 0, (en - n) * 32, (cudaStream_t)stream));
-    return ntt_run_batch(*c, d_cols, count, extended_omega, extended_k, (cudaStream_t)stream);
+    return coeff_to_extended_batch_run(*c, d_cols, count, k, extended_k, extended_omega, zeta_powers, (cudaStream_t)stream);
 }
 
 // One witness / product column through the three steps such a column takes in create_proof ([UP] plonk/prover.rs: commit_lagrange,
@@ -1562,6 +1557,246 @@ int h2b_srs_downsize(uint64_t handle_g, uint32_t k, uint64_t* out_g_lagrange, ui
     if (handle_g_out) *handle_g_out = hg;
     if (handle_g_lagrange_out) *handle_g_lagrange_out = hl;
     return H2B_OK;
+}
+
+// ---- key generation: the permutation argument's sigma columns and keygen_pk's indicator columns ---------------------------------
+// ([UP] halo2_proofs/src/plonk/permutation/keygen.rs Assembly::{build_vk, build_pk}, plonk/keygen.rs keygen_pk)
+int h2b_permutation_sigma_dev(int device, const void* const* d_mapping, uint32_t n_columns, uint32_t k, const uint64_t delta[4], const uint64_t omega[4],
+                              void* const* d_sigma, void* d_status, void* stream) {
+    DeviceCtx* c = nullptr;
+    H2B_TRY(get_ctx(device, &c));
+    if (k > 28 || n_columns == 0) { set_error("h2b_permutation_sigma_dev: k = %u, %u columns (need k <= 28 and at least one column)", k, n_columns); return H2B_ERR_BAD_ARGUMENT; }
+    if (!d_mapping || !delta || !omega || !d_sigma || !d_status) { set_error("h2b_permutation_sigma_dev: null pointer"); return H2B_ERR_BAD_ARGUMENT; }
+    for (uint32_t i = 0; i < n_columns; ++i)
+        if (!d_mapping[i] || !d_sigma[i]) { set_error("h2b_permutation_sigma_dev: column %u: null pointer", i); return H2B_ERR_BAD_ARGUMENT; }
+    std::lock_guard<std::mutex> lk(c->mu);
+    const cudaStream_t st = (cudaStream_t)stream;
+    H2B_CUDA(cudaMemsetAsync(d_status, 0, 4, st));
+    H2B_TRY(permutation_sigma_tables_run(*c, n_columns, k, delta, omega, st));
+    return permutation_sigma_run(*c, d_mapping, n_columns, 0, n_columns, k, d_sigma, d_status, st);
+}
+
+int h2b_keygen_lagrange_indicators_dev(int device, uint32_t k, uint32_t extended_k, uint32_t blinding_factors, const uint64_t omega_inv[4],
+                                       const uint64_t ifft_divisor[4], const uint64_t extended_omega[4], const uint64_t zeta_powers[12], void* d_l0,
+                                       void* d_l_last, void* d_l_active_row, void* stream) {
+    DeviceCtx* c = nullptr;
+    H2B_TRY(get_ctx(device, &c));
+    if (extended_k > 28 || extended_k < k || (uint64_t)blinding_factors + 1 >= ((uint64_t)1 << k)) {
+        set_error("h2b_keygen_lagrange_indicators_dev: k = %u, extended_k = %u, %u blinding factors (need k <= extended_k <= 28 and bf + 1 < 2^k)", k,
+                  extended_k, blinding_factors);
+        return H2B_ERR_BAD_ARGUMENT;
+    }
+    if (!omega_inv || !ifft_divisor || !extended_omega || !zeta_powers || !d_l0 || !d_l_last || !d_l_active_row) {
+        set_error("h2b_keygen_lagrange_indicators_dev: null pointer");
+        return H2B_ERR_BAD_ARGUMENT;
+    }
+    std::lock_guard<std::mutex> lk(c->mu);
+    void* cols[3] = {d_l0, d_l_last, d_l_active_row};
+    return keygen_indicators_run(*c, k, extended_k, blinding_factors, omega_inv, ifft_divisor, extended_omega, zeta_powers, cols, (cudaStream_t)stream);
+}
+
+// One build_vk / build_pk pass over the mapping columns [col_begin, col_end); column i runs on device i mod D.
+struct KeygenJob {
+    const uint64_t* const* mapping = nullptr;
+    uint32_t n_columns = 0, k = 0, extended_k = 0, col_begin = 0, col_end = 0;
+    const uint64_t *delta = nullptr, *omega = nullptr, *omega_inv = nullptr, *ifft_divisor = nullptr, *extended_omega = nullptr, *zeta_powers = nullptr;
+    bool validate_only = false;                 // sigma and its status word only: nothing leaves the device
+    const BaseSet* commit_set = nullptr;        // a replicated set: commitments of sigma over its first n points
+    uint64_t* commitments = nullptr;            // n_columns x 12 words (Jacobian), indexed by column
+    uint64_t* const* sigma_out = nullptr;       // per column (indexed by column), or null
+    uint64_t* const* poly_out = nullptr;
+    uint64_t* const* coset_out = nullptr;
+};
+
+// scratch of one device's share, given back on every return path
+struct KeygenScratch {
+    std::vector<void*> bufs;
+    cudaEvent_t ev[2] = {nullptr, nullptr};
+    DeviceCtx* ctx = nullptr;
+    int alloc(size_t bytes, void** out) {
+        cudaError_t e = cudaMalloc(out, bytes);
+        if (e != cudaSuccess) { cudaGetLastError(); set_error("key generation: cudaMalloc(%zu): %s", bytes, cudaGetErrorString(e)); return H2B_ERR_OOM; }
+        bufs.push_back(*out);
+        return H2B_OK;
+    }
+    ~KeygenScratch() {
+        if (ctx) cudaStreamSynchronize(ctx->stream);
+        for (void* p : bufs) cudaFree(p);
+        for (cudaEvent_t e : ev) if (e) cudaEventDestroy(e);
+        if (ctx) ctx->keygen_tables.release();
+        cudaGetLastError();
+    }
+};
+
+static const size_t KEYGEN_GROUP_BYTES = (size_t)1 << 31;      // device memory of one group of columns (sigma / coefficients / cosets)
+
+// device d's columns of the job, in groups that share the batched MSM / NTT launches.  The mapping of column i + 1 is staged while the
+// sigma kernel of column i runs (two mapping buffers).  *bad receives the status word of the first group that holds an invalid entry; no
+// output of that group or a later one is written.
+static int keygen_device(size_t d, const KeygenJob& job, uint32_t* bad) {
+    const size_t nd = G.devs.size();
+    std::vector<uint32_t> mine;
+    for (uint32_t i = job.col_begin; i < job.col_end; ++i) if (i % nd == d) mine.push_back(i);
+    if (mine.empty()) return H2B_OK;
+    DeviceCtx& c = *G.devs[d];
+    std::lock_guard<std::mutex> lk(c.mu);
+    H2B_CUDA(cudaSetDevice(c.device));
+    const cudaStream_t st = c.stream;
+    const uint32_t k = job.k;
+    const size_t n = (size_t)1 << k;
+    const bool pk = job.poly_out || job.coset_out;
+    const size_t col_bytes = (job.coset_out && !job.validate_only ? (size_t)1 << job.extended_k : n) * 32;
+    size_t group = ntt_batch_max();
+    while (group > 1 && group * col_bytes > KEYGEN_GROUP_BYTES) group >>= 1;
+    if (job.commit_set && group > msm_batch_max()) group = msm_batch_max();
+    KeygenScratch s;
+    s.ctx = &c;
+    void *d_map[2], *d_cols, *d_status, *d_blocks;
+    H2B_TRY(s.alloc(n * 16, &d_map[0]));
+    H2B_TRY(s.alloc(n * 16, &d_map[1]));
+    H2B_TRY(s.alloc(group * col_bytes, &d_cols));
+    H2B_TRY(s.alloc(group * 224 + 32, &d_blocks));
+    d_status = (char*)d_blocks + group * 224;
+    for (cudaEvent_t& e : s.ev) H2B_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    c.prof.mark(PROF_BEGIN, st);
+    H2B_CUDA(cudaMemsetAsync(d_status, 0, 4, st));
+    H2B_TRY(permutation_sigma_tables_run(c, job.n_columns, k, job.delta, job.omega, st));
+    size_t seq = 0;
+    for (size_t g0 = 0; g0 < mine.size(); g0 += group) {
+        const size_t m = mine.size() - g0 < group ? mine.size() - g0 : group;
+        std::vector<void*> cols(m);
+        for (size_t t = 0; t < m; ++t) {
+            const uint32_t i = mine[g0 + t];
+            const int slot = (int)(seq++ & 1);
+            cols[t] = (char*)d_cols + t * col_bytes;
+            H2B_CUDA(cudaEventSynchronize(s.ev[slot]));          // the sigma kernel that last read this mapping buffer is done
+            H2B_TRY(host_upload(c, d_map[slot], job.mapping[i], n * 16, st, false));
+            c.prof.mark(PROF_KEYGEN_UPLOAD, st);
+            H2B_TRY(permutation_sigma_run(c, &d_map[slot], 1, i, job.n_columns, k, &cols[t], d_status, st));
+            H2B_CUDA(cudaEventRecord(s.ev[slot], st));
+            c.prof.mark(PROF_KEYGEN_SIGMA, st);
+        }
+        uint32_t status = 0;
+        H2B_CUDA(cudaMemcpyAsync(&status, d_status, 4, cudaMemcpyDeviceToHost, st));
+        H2B_CUDA(cudaStreamSynchronize(st));
+        if (status) { *bad = status; return H2B_OK; }
+        if (job.validate_only) continue;
+        if (job.commit_set) {
+            const MsmBases b = bases_of(*job.commit_set, d, 0);
+            if (n > BATCH_COLUMN_MAX) {
+                for (size_t t = 0; t < m; ++t) H2B_TRY(msm_run(c, cols[t], b, n, (char*)d_blocks + 224 * t, false, st));
+            } else {
+                std::vector<size_t> lens(m, n);
+                H2B_TRY(msm_run_batch(c, cols.data(), lens.data(), (uint32_t)m, b, d_blocks, st));
+            }
+            c.prof.mark(PROF_KEYGEN_COMMIT, st);
+            std::vector<uint64_t> blocks(28 * m);
+            H2B_CUDA(cudaMemcpyAsync(blocks.data(), d_blocks, 224 * m, cudaMemcpyDeviceToHost, st));
+            H2B_CUDA(cudaStreamSynchronize(st));
+            for (size_t t = 0; t < m; ++t) memcpy(job.commitments + 12 * (size_t)mine[g0 + t], &blocks[28 * t], 96);
+        }
+        if (job.sigma_out) {
+            for (size_t t = 0; t < m; ++t) H2B_TRY(host_download(c, job.sigma_out[mine[g0 + t]], cols[t], n * 32, st));
+            c.prof.mark(PROF_KEYGEN_DOWNLOAD, st);
+        }
+        if (!pk) continue;
+        H2B_TRY(lagrange_to_coeff_batch_run(c, cols.data(), m, k, job.omega_inv, job.ifft_divisor, st));
+        c.prof.mark(PROF_KEYGEN_INTT, st);
+        if (job.poly_out) {
+            for (size_t t = 0; t < m; ++t) H2B_TRY(host_download(c, job.poly_out[mine[g0 + t]], cols[t], n * 32, st));
+            c.prof.mark(PROF_KEYGEN_DOWNLOAD, st);
+        }
+        if (job.coset_out) {
+            H2B_TRY(coeff_to_extended_batch_run(c, cols.data(), m, k, job.extended_k, job.extended_omega, job.zeta_powers, st));
+            c.prof.mark(PROF_KEYGEN_COSET, st);
+            for (size_t t = 0; t < m; ++t) H2B_TRY(host_download(c, job.coset_out[mine[g0 + t]], cols[t], col_bytes, st));
+            c.prof.mark(PROF_KEYGEN_DOWNLOAD, st);
+        }
+    }
+    return H2B_OK;
+}
+
+// every device's share of the job; an invalid mapping entry fails with H2B_ERR_BAD_ARGUMENT
+static int keygen_run(const char* who, const KeygenJob& job) {
+    const size_t nd = G.devs.size();
+    std::vector<uint32_t> bad(nd, 0);
+    H2B_TRY(on_all_devices(nd, [&](size_t d) { return keygen_device(d, job, &bad[d]); }));
+    for (size_t d = 0; d < nd; ++d) {
+        if (!bad[d]) continue;
+        const uint64_t flat = bad[d] - 1, n = (uint64_t)1 << job.k;
+        if (bad[d] == 0xFFFFFFFFu) set_error("%s: the mapping holds an entry outside %u columns x 2^%u rows", who, job.n_columns, job.k);
+        else set_error("%s: mapping[%llu][%llu] is outside %u columns x 2^%u rows", who, (unsigned long long)(flat / n), (unsigned long long)(flat % n),
+                       job.n_columns, job.k);
+        return H2B_ERR_BAD_ARGUMENT;
+    }
+    return H2B_OK;
+}
+
+static int keygen_check(const char* who, const uint64_t* const* mapping, uint32_t n_columns, uint32_t k, const uint64_t* delta, const uint64_t* omega) {
+    H2B_TRY(require_init());
+    if (k > 28 || n_columns == 0) { set_error("%s: k = %u, %u columns (need k <= 28 and at least one column)", who, k, n_columns); return H2B_ERR_BAD_ARGUMENT; }
+    if (!mapping || !delta || !omega) { set_error("%s: null pointer", who); return H2B_ERR_BAD_ARGUMENT; }
+    for (uint32_t i = 0; i < n_columns; ++i) if (!mapping[i]) { set_error("%s: mapping column %u is null", who, i); return H2B_ERR_BAD_ARGUMENT; }
+    return H2B_OK;
+}
+
+int h2b_permutation_build_vk(const uint64_t* const* mapping, uint32_t n_columns, uint32_t k, const uint64_t delta[4], const uint64_t omega[4],
+                             uint64_t handle_g_lagrange, uint64_t* out_commitments) {
+    static const char* who = "h2b_permutation_build_vk";
+    H2B_TRY(keygen_check(who, mapping, n_columns, k, delta, omega));
+    if (!out_commitments) { set_error("%s: null output", who); return H2B_ERR_BAD_ARGUMENT; }
+    const size_t n = (size_t)1 << k;
+    SetRef bs = find_set(handle_g_lagrange);
+    if (!bs) { set_error("%s: unknown base-set handle %llu", who, (unsigned long long)handle_g_lagrange); return H2B_ERR_BAD_ARGUMENT; }
+    if (n > bs->n) { set_error("%s: 2^%u points requested from a set of %zu", who, k, bs->n); return H2B_ERR_BAD_ARGUMENT; }
+    std::vector<uint64_t> com((size_t)n_columns * 12);
+    KeygenJob job;
+    job.mapping = mapping; job.n_columns = n_columns; job.k = k; job.delta = delta; job.omega = omega;
+    if (!bs->sharded) {
+        job.commit_set = bs.get();
+        job.commitments = com.data();
+        job.col_begin = 0; job.col_end = n_columns;
+        H2B_TRY(keygen_run(who, job));
+    } else {
+        // a sharded set holds every point on one device only: sigma comes back to the host and each commitment is split by point
+        // range over the devices, as h2b_msm_bn254_g1_batch_registered does with such a set
+        const uint32_t chunk = (uint32_t)ntt_batch_max();
+        std::vector<std::vector<uint64_t>> sigma(chunk, std::vector<uint64_t>(4 * n));
+        std::vector<uint64_t*> ptrs(n_columns, nullptr);
+        job.sigma_out = ptrs.data();
+        for (uint32_t c0 = 0; c0 < n_columns; c0 += chunk) {
+            const uint32_t c1 = n_columns - c0 < chunk ? n_columns : c0 + chunk;
+            for (uint32_t i = c0; i < c1; ++i) ptrs[i] = sigma[i - c0].data();
+            job.col_begin = c0; job.col_end = c1;
+            H2B_TRY(keygen_run(who, job));
+            for (uint32_t i = c0; i < c1; ++i) H2B_TRY(msm_host(ptrs[i], *bs, 0, n, com.data() + 12 * (size_t)i));
+        }
+    }
+    memcpy(out_commitments, com.data(), com.size() * 8);
+    return H2B_OK;
+}
+
+int h2b_permutation_build_pk(const uint64_t* const* mapping, uint32_t n_columns, uint32_t k, uint32_t extended_k, const uint64_t delta[4],
+                             const uint64_t omega[4], const uint64_t omega_inv[4], const uint64_t ifft_divisor[4], const uint64_t extended_omega[4],
+                             const uint64_t zeta_powers[12], uint64_t* const* out_permutations, uint64_t* const* out_polys, uint64_t* const* out_cosets) {
+    static const char* who = "h2b_permutation_build_pk";
+    H2B_TRY(keygen_check(who, mapping, n_columns, k, delta, omega));
+    if (extended_k > 28 || extended_k < k) { set_error("%s: need k <= extended_k <= 28 (k = %u, extended_k = %u)", who, k, extended_k); return H2B_ERR_BAD_ARGUMENT; }
+    if (!omega_inv || !ifft_divisor || !extended_omega || !zeta_powers) { set_error("%s: null pointer", who); return H2B_ERR_BAD_ARGUMENT; }
+    for (uint64_t* const* outs : {out_permutations, out_polys, out_cosets})
+        if (outs)
+            for (uint32_t i = 0; i < n_columns; ++i) if (!outs[i]) { set_error("%s: output column %u is null", who, i); return H2B_ERR_BAD_ARGUMENT; }
+    KeygenJob job;
+    job.mapping = mapping; job.n_columns = n_columns; job.k = k; job.extended_k = extended_k; job.delta = delta; job.omega = omega;
+    job.omega_inv = omega_inv; job.ifft_divisor = ifft_divisor; job.extended_omega = extended_omega; job.zeta_powers = zeta_powers;
+    job.col_begin = 0; job.col_end = n_columns;
+    // every entry is checked before the first byte of caller memory is written: a pass that only builds sigma, then the real one
+    job.validate_only = true;
+    H2B_TRY(keygen_run(who, job));
+    if (!out_permutations && !out_polys && !out_cosets) return H2B_OK;
+    job.validate_only = false;
+    job.sigma_out = out_permutations; job.poly_out = out_polys; job.coset_out = out_cosets;
+    return keygen_run(who, job);
 }
 
 int h2b_srs_cache_clear(void) {

@@ -73,7 +73,9 @@ __host__ __device__ __forceinline__ uint64_t splitmix64_at(uint64_t seed, uint64
 enum ProfTag { PROF_BEGIN = 0, PROF_MSM_DECOMPOSE = 1, PROF_MSM_SCAN = 2, PROF_MSM_SCATTER = 3, PROF_MSM_PLAN = 4, PROF_MSM_ACCUMULATE = 5,
                PROF_MSM_COMBINE = 6, PROF_MSM_REDUCE = 7, PROF_MSM_FINAL = 8, PROF_MSM_PRECOMPUTE = 9, PROF_NTT_TWIDDLE = 15, PROF_NTT_PASS0 = 16,
                PROF_SRS_SCALARS = 24, PROF_SRS_FIXED_BASE = 25, PROF_SRS_NORMALISE = 26, PROF_SRS_TABLE = 27,
-               PROF_G1NTT_TWIDDLE = 28, PROF_G1NTT_STAGES = 29, PROF_G1NTT_NORMALISE = 30 };
+               PROF_G1NTT_TWIDDLE = 28, PROF_G1NTT_STAGES = 29, PROF_G1NTT_NORMALISE = 30,
+               PROF_KEYGEN_UPLOAD = 31, PROF_KEYGEN_SIGMA = 32, PROF_KEYGEN_COMMIT = 33, PROF_KEYGEN_INTT = 34, PROF_KEYGEN_COSET = 35,
+               PROF_KEYGEN_DOWNLOAD = 36 };
 struct Profiler {
     bool enabled = false;
     std::vector<cudaEvent_t> ev;
@@ -114,6 +116,7 @@ struct DeviceCtx {
     DevBuf lookup_scratch;             // sorted keys, flags and ranks of permute_expression_pair (lookup.cu)
     DevBuf gen_table;                  // fixed-base table of the G1 generator, built on first use (g1gen.cu)
     DevBuf gen_scratch;                // normalisation denominators and SRS scalars of one chunk; the G1 NTT work buffer (g1gen.cu)
+    DevBuf keygen_tables;              // the two-level delta^c omega^r tables of the sigma kernel (keygen.cu)
     EvalScratch* eval = nullptr;       // compiled-program ring of the quotient evaluation (evaluate.cu)
     std::vector<NttTwiddles*> twiddles;  // small LRU cache keyed by (omega, log_n)
     MsmScratch* msm = nullptr;
@@ -172,6 +175,10 @@ int ntt_fourstep_twiddle_run(DeviceCtx& ctx, void* d_y, uint32_t rows, uint32_t 
 int ntt_root_powers_run(DeviceCtx& ctx, const uint64_t omega[4], uint32_t e0, uint32_t e1, void* d_out, cudaStream_t stream);
 int ntt_scale_run(DeviceCtx& ctx, void* d_a, size_t n, const uint64_t* factors /*host, count x 4*/, int count, cudaStream_t stream);
 int ntt_scale_batch_run(DeviceCtx& ctx, void* const* d_cols, size_t ncols, size_t n, const uint64_t* factors, int count, cudaStream_t stream);
+int lagrange_to_coeff_batch_run(DeviceCtx& ctx, void* const* d_cols, size_t count, uint32_t k, const uint64_t omega_inv[4], const uint64_t ifft_divisor[4],
+                                cudaStream_t stream);
+int coeff_to_extended_batch_run(DeviceCtx& ctx, void* const* d_cols, size_t count, uint32_t k, uint32_t extended_k, const uint64_t extended_omega[4],
+                                const uint64_t zeta_powers[12], cudaStream_t stream);
 void ntt_release(DeviceCtx& ctx);
 // ---- msm.cu ----
 // The points of an MSM: table j (j < n_tables) holds 2^(c0*j) * P_i at rows [0, stride); the call uses rows
@@ -203,6 +210,16 @@ int srs_setup_run(DeviceCtx& ctx, uint32_t k, const uint64_t s[4], int which, vo
 int g1_to_lagrange_run(DeviceCtx& ctx, const void* d_g, uint32_t k, void* d_out_affine, cudaStream_t stream);
 // after a synchronous call: drop the chunk scratch, and scan_scratch if the call grew it (the generator table stays)
 void g1gen_release_scratch(DeviceCtx& ctx, size_t scan_cap_before);
+// ---- keygen.cu ----
+// the lo / hi tables of sigma for n_columns columns at k into ctx.keygen_tables (stream-ordered; must precede permutation_sigma_run)
+int permutation_sigma_tables_run(DeviceCtx& ctx, uint32_t n_columns, uint32_t k, const uint64_t delta[4], const uint64_t omega[4], cudaStream_t stream);
+// sigma of `count` mapping columns (flat column index col0 + y for the status word), with the tables of the last permutation_sigma_tables_run
+int permutation_sigma_run(DeviceCtx& ctx, const void* const* d_mapping, uint32_t count, uint32_t col0, uint32_t n_columns, uint32_t k,
+                          void* const* d_sigma, void* d_status, cudaStream_t stream);
+// l0, l_last, l_active_row (d_cols[0..3), 2^extended_k elements each) of keygen_pk
+int keygen_indicators_run(DeviceCtx& ctx, uint32_t k, uint32_t extended_k, uint32_t blinding_factors, const uint64_t omega_inv[4],
+                          const uint64_t ifft_divisor[4], const uint64_t extended_omega[4], const uint64_t zeta_powers[12], void* const* d_cols,
+                          cudaStream_t stream);
 // ---- testgen.cu ----
 int msm_checksum_run(DeviceCtx& ctx, const void* d_scalars, uint64_t seed, uint64_t first, size_t n, void* d_out, cudaStream_t stream);
 int gen_scalars_run(DeviceCtx& ctx, uint64_t seed, size_t n, int kind, void* d_out, cudaStream_t stream);

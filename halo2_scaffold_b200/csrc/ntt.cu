@@ -758,6 +758,23 @@ int ntt_scale_run(DeviceCtx& ctx, void* d_a, size_t n, const uint64_t* factors, 
     return H2B_OK;
 }
 
+// EvaluationDomain::lagrange_to_coeff / coeff_to_extended ([UP] halo2_proofs/src/poly/domain.rs) of `count` columns in place: the (i)NTT
+// passes and the scaling are launched once for the whole batch.  coeff_to_extended needs 2^extended_k elements per column.
+int lagrange_to_coeff_batch_run(DeviceCtx& ctx, void* const* d_cols, size_t count, uint32_t k, const uint64_t omega_inv[4], const uint64_t ifft_divisor[4],
+                                cudaStream_t stream) {
+    H2B_TRY(ntt_run_batch(ctx, d_cols, count, omega_inv, k, stream));
+    return ntt_scale_batch_run(ctx, d_cols, count, (size_t)1 << k, ifft_divisor, 1, stream);
+}
+
+int coeff_to_extended_batch_run(DeviceCtx& ctx, void* const* d_cols, size_t count, uint32_t k, uint32_t extended_k, const uint64_t extended_omega[4],
+                                const uint64_t zeta_powers[12], cudaStream_t stream) {
+    const size_t n = (size_t)1 << k, en = (size_t)1 << extended_k;
+    H2B_TRY(ntt_scale_batch_run(ctx, d_cols, count, n, zeta_powers, 3, stream));                     // a[i] *= zeta^(i mod 3)
+    if (en > n)
+        for (size_t j = 0; j < count; ++j) H2B_CUDA(cudaMemsetAsync((char*)d_cols[j] + n * 32, 0, (en - n) * 32, stream));   // zero-pad
+    return ntt_run_batch(ctx, d_cols, count, extended_omega, extended_k, stream);
+}
+
 void ntt_release(DeviceCtx& ctx) {
     for (NttTwiddles* t : ctx.twiddles) { t->buf.release(); t->direct.release(); delete t; }
     ctx.twiddles.clear();

@@ -336,6 +336,8 @@ class ParamsKZG {
     const std::vector<G1Affine>& get_g() const { return host_g_; }
     const std::vector<G1Affine>& get_g_lagrange() const { return host_g_lagrange_; }
     const std::vector<uint8_t>& g2_bytes() const { return g2_bytes_; }
+    // the registered g_lagrange set (what Assembly::build_vk commits sigma over)
+    uint64_t g_lagrange_handle() const { return g_lagrange_; }
     ~ParamsKZG() {
         if (g_) h2b_unregister_bases(g_);
         if (g_lagrange_) h2b_unregister_bases(g_lagrange_);
@@ -623,7 +625,76 @@ inline std::vector<Fr> commit_product(const std::vector<std::vector<Fr>>& values
           "permutation::commit");
     return dev.download(z, n);
 }
+
+// Assembly::build_vk / build_pk (plonk/permutation/keygen.rs) from the mapping that Assembly::copy built on the host:
+// mapping[i][j] = (column, row), sigma_i[j] = DELTA^column omega^row, all per-row work on the device.
+namespace keygen {
+typedef std::vector<std::vector<std::pair<uint64_t, uint64_t>>> Mapping;      // upstream's Vec<Vec<(usize, usize)>>
+static_assert(sizeof(std::pair<uint64_t, uint64_t>) == 16, "a mapping entry is two u64");
+
+inline Fr delta() {                      // Fr::DELTA = GENERATOR^(2^S)
+    const uint64_t e[4] = {(uint64_t)1 << fr::S, 0, 0, 0};
+    return fr::pow(fr::from_u64(7), e);
+}
+inline std::vector<const uint64_t*> columns_of(const Mapping& mapping, size_t n) {
+    std::vector<const uint64_t*> cols;
+    for (const auto& c : mapping) {
+        if (c.size() != n) throw Panic("permutation keygen: mapping column length != 2^k");
+        cols.push_back(reinterpret_cast<const uint64_t*>(c.data()));
+    }
+    return cols;
+}
+// VerifyingKey { commitments }: commit_lagrange(sigma_i) for every column
+inline std::vector<G1> build_vk(const poly::kzg::ParamsKZG& params, const poly::EvaluationDomain& domain, const Mapping& mapping) {
+    ensure_init();
+    const auto cols = columns_of(mapping, (size_t)1 << domain.k());
+    std::vector<G1> out(cols.size());
+    check(h2b_permutation_build_vk(cols.data(), (uint32_t)cols.size(), domain.k(), delta().l, domain.get_omega().l, params.g_lagrange_handle(),
+                                   reinterpret_cast<uint64_t*>(out.data())), "permutation::keygen::build_vk");
+    return out;
+}
+// ProvingKey { permutations, polys, cosets }
+struct ProvingKey { std::vector<std::vector<Fr>> permutations, polys, cosets; };
+inline ProvingKey build_pk(const poly::kzg::ParamsKZG&, const poly::EvaluationDomain& domain, const Mapping& mapping) {
+    ensure_init();
+    const size_t n = (size_t)1 << domain.k();
+    const auto cols = columns_of(mapping, n);
+    ProvingKey pk;
+    std::vector<uint64_t*> p, c, e;
+    for (size_t i = 0; i < cols.size(); ++i) {
+        pk.permutations.emplace_back(n); pk.polys.emplace_back(n); pk.cosets.emplace_back(domain.extended_len());
+        p.push_back(reinterpret_cast<uint64_t*>(pk.permutations.back().data()));
+        c.push_back(reinterpret_cast<uint64_t*>(pk.polys.back().data()));
+        e.push_back(reinterpret_cast<uint64_t*>(pk.cosets.back().data()));
+    }
+    const Fr z[3] = {fr::one(), domain.get_g_coset(), domain.get_g_coset_inv()};
+    check(h2b_permutation_build_pk(cols.data(), (uint32_t)cols.size(), domain.k(), domain.extended_k(), delta().l, domain.get_omega().l,
+                                   domain.get_omega_inv().l, domain.get_ifft_divisor().l, domain.get_extended_omega().l, z[0].l, p.data(), c.data(), e.data()),
+          "permutation::keygen::build_pk");
+    return pk;
+}
+}  // namespace keygen
 }  // namespace permutation
+
+// keygen_pk's l0, l_last and l_active_row on the extended coset (plonk/keygen.rs), computed on the device
+namespace keygen {
+struct LagrangeIndicators { std::vector<Fr> l0, l_last, l_active_row; };
+inline LagrangeIndicators lagrange_indicators(const poly::EvaluationDomain& domain, uint32_t blinding_factors) {
+    ensure_init();
+    const size_t en = domain.extended_len();
+    DeviceBuffer d0(domain.device(), en * sizeof(Fr)), d1(domain.device(), en * sizeof(Fr)), d2(domain.device(), en * sizeof(Fr));
+    const Fr z[3] = {fr::one(), domain.get_g_coset(), domain.get_g_coset_inv()};
+    check(h2b_keygen_lagrange_indicators_dev(domain.device(), domain.k(), domain.extended_k(), blinding_factors, domain.get_omega_inv().l,
+                                             domain.get_ifft_divisor().l, domain.get_extended_omega().l, z[0].l, d0.get(), d1.get(), d2.get(), nullptr),
+          "keygen_pk: lagrange indicators");
+    check(h2b_dev_sync(domain.device()), "sync");
+    LagrangeIndicators out{std::vector<Fr>(en), std::vector<Fr>(en), std::vector<Fr>(en)};
+    check(h2b_memcpy_d2h(domain.device(), out.l0.data(), d0.get(), en * sizeof(Fr)), "d2h");
+    check(h2b_memcpy_d2h(domain.device(), out.l_last.data(), d1.get(), en * sizeof(Fr)), "d2h");
+    check(h2b_memcpy_d2h(domain.device(), out.l_active_row.data(), d2.get(), en * sizeof(Fr)), "d2h");
+    return out;
+}
+}  // namespace keygen
 
 namespace lookup {
 // fn permute_expression_pair(..) -> Result<(Vec<F>, Vec<F>), Error>: the first usable_rows rows of (A', S')

@@ -363,6 +363,42 @@ int h2b_g1_to_lagrange_dev(int device, const void* d_g_affine, uint32_t k, void*
  * allocated, and leave the output handles untouched. */
 int h2b_srs_downsize(uint64_t handle_g, uint32_t k, uint64_t* out_g_lagrange, uint64_t* handle_g_out, uint64_t* handle_g_lagrange_out);
 
+/* ---- key generation: the permutation argument's sigma columns and keygen_pk's indicator columns -------------------------
+ * [UP] halo2_proofs/src/plonk/permutation/keygen.rs (Assembly::build_vk / build_pk) and plonk/keygen.rs (keygen_pk).  A mapping
+ * column is upstream's Vec<(usize, usize)> as it sits in memory: n = 2^k pairs of u64 (column, row).  sigma_i[j] = delta^c * omega^r
+ * for (c, r) = mapping[i][j], Montgomery form, canonical; delta is Fr::DELTA and omega the domain's root, both from the caller. */
+/* sigma of n_columns mapping columns (d_mapping[i]: n x 16 B on `device`) into d_sigma[i] (n x 32 B), for every column in one launch
+ * sequence.  An entry with c >= n_columns or r >= n is refused as upstream's out-of-range index panics: the 32-bit word at d_status
+ * receives 1 + the flat index i * n + j of the last such entry (saturated at 2^32 - 1), 0 when every entry is valid; sigma is
+ * unspecified when it is non-zero (the convention of h2b_lookup_permute_async_dev).  Asynchronous on `stream`; the twiddle tables
+ * (2^ceil(k/2) + n_columns * 2^floor(k/2) entries of 32 B) stay reserved until h2b_shutdown.  k > 28, n_columns = 0 and null pointers
+ * fail with H2B_ERR_BAD_ARGUMENT before anything is launched. */
+int h2b_permutation_sigma_dev(int device, const void* const* d_mapping, uint32_t n_columns, uint32_t k, const uint64_t delta[4], const uint64_t omega[4],
+                              void* const* d_sigma, void* d_status, void* stream);
+/* keygen_pk's l0 = ext(coeff(e_0)), l_last = ext(coeff(e_(n-bf-1))) and l_active_row = 1 - (l_last + l_blind) = ext(coeff(1 on rows
+ * 0 .. n-bf-2)), each 2^extended_k x 32 B on `device`, with ext / coeff the EvaluationDomain conversions of
+ * h2b_lagrange_to_coeff_dev_batch / h2b_coeff_to_extended_dev_batch (same constants).  Nothing is uploaded.  Asynchronous on `stream`.
+ * bf + 1 >= n, extended_k < k, extended_k > 28 and null pointers fail with H2B_ERR_BAD_ARGUMENT. */
+int h2b_keygen_lagrange_indicators_dev(int device, uint32_t k, uint32_t extended_k, uint32_t blinding_factors, const uint64_t omega_inv[4],
+                                       const uint64_t ifft_divisor[4], const uint64_t extended_omega[4], const uint64_t zeta_powers[12], void* d_l0,
+                                       void* d_l_last, void* d_l_active_row, void* stream);
+/* Assembly::build_vk: out_commitments[12 i ..] = commit_lagrange(sigma_i) (Jacobian) over the registered set handle_g_lagrange (the
+ * handles h2b_msm_bn254_g1_batch_registered accepts: replicated or sharded, at least n points).  mapping[i]: the caller's n x 2 u64
+ * column (pageable is fine); columns go round-robin over the devices, and each is staged through pinned buffers while the previous
+ * one's sigma kernel runs.  Synchronous; gives its scratch back before it returns.  k > 28, n_columns = 0, null pointers, an unknown
+ * handle, a set shorter than n and an invalid mapping entry fail with H2B_ERR_BAD_ARGUMENT and leave out_commitments untouched. */
+int h2b_permutation_build_vk(const uint64_t* const* mapping, uint32_t n_columns, uint32_t k, const uint64_t delta[4], const uint64_t omega[4],
+                             uint64_t handle_g_lagrange, uint64_t* out_commitments);
+/* Assembly::build_pk: per column i, out_permutations[i] = sigma_i (n x 32 B), out_polys[i] = lagrange_to_coeff(sigma_i) (n x 32 B) and
+ * out_cosets[i] = coeff_to_extended(out_polys[i]) (2^extended_k x 32 B); any of the three arrays may be NULL.  The domain constants
+ * are those of h2b_lagrange_to_coeff_dev_batch / h2b_coeff_to_extended_dev_batch.  Columns are dealt as in h2b_permutation_build_vk
+ * and processed a bounded number (at most 2 GiB of device memory per device) at a time.  Every entry is checked before any caller
+ * memory is written: bad arguments and invalid entries fail with H2B_ERR_BAD_ARGUMENT and leave every output untouched.  Synchronous;
+ * gives its scratch back before it returns. */
+int h2b_permutation_build_pk(const uint64_t* const* mapping, uint32_t n_columns, uint32_t k, uint32_t extended_k, const uint64_t delta[4],
+                             const uint64_t omega[4], const uint64_t omega_inv[4], const uint64_t ifft_divisor[4], const uint64_t extended_omega[4],
+                             const uint64_t zeta_powers[12], uint64_t* const* out_permutations, uint64_t* const* out_polys, uint64_t* const* out_cosets);
+
 /* ---- raw device memory helpers (so that non-CUDA hosts -- ctypes, Rust -- can hold device buffers) --- */
 int h2b_dev_alloc(int device, size_t bytes, void** out);
 int h2b_dev_free(int device, void* p);
@@ -407,7 +443,10 @@ unsigned long long h2b_launch_count(void);
  * 24 scalars (powers, inversion, scaling), 25 fixed-base multiplication, 26 normalisation, 27 generator table (first use
  * on the device only); registering the results records 9 (window tables) as every registered base set does;
  * h2b_g1_to_lagrange_dev / h2b_srs_downsize tags: 28 twiddles (w^-1, n^-1 and the power table), 29 butterfly stages (all
- * k of them), 30 normalisation (batch inversion and the affine finish). */
+ * k of them), 30 normalisation (batch inversion and the affine finish);  h2b_permutation_build_vk / h2b_permutation_build_pk tags
+ * (per column or group of columns): 31 mapping upload, 32 sigma kernel (the first also builds the twiddle tables), 33 commitments,
+ * 34 inverse NTTs (lagrange_to_coeff), 35 coset NTTs (coeff_to_extended), 36 downloads; the MSM / NTT tags recorded inside a phase
+ * belong to the keygen tag that follows them. */
 int h2b_profile_enable(int device, int on);
 int h2b_profile_read(int device, int* tags, float* ms, int cap, int* count);
 /* force the MSM window size (0 = automatic) -- tuning / tests only */

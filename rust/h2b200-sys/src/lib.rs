@@ -106,6 +106,17 @@ extern "C" {
     // ParamsKZG::downsize on the device and the G1 NTT (g_to_lagrange) it is built on
     pub fn h2b_g1_to_lagrange_dev(device: c_int, d_g_affine: *const c_void, k: u32, d_out_affine: *mut c_void, stream: *mut c_void) -> c_int;
     pub fn h2b_srs_downsize(handle_g: u64, k: u32, out_g_lagrange: *mut u64, handle_g_out: *mut u64, handle_g_lagrange_out: *mut u64) -> c_int;
+    // the permutation argument's sigma columns (Assembly::build_vk / build_pk) and keygen_pk's l0 / l_last / l_active_row
+    pub fn h2b_permutation_sigma_dev(device: c_int, d_mapping: *const *const c_void, n_columns: u32, k: u32, delta: *const u64, omega: *const u64,
+                                     d_sigma: *const *mut c_void, d_status: *mut c_void, stream: *mut c_void) -> c_int;
+    pub fn h2b_keygen_lagrange_indicators_dev(device: c_int, k: u32, extended_k: u32, blinding_factors: u32, omega_inv: *const u64, ifft_divisor: *const u64,
+                                              extended_omega: *const u64, zeta_powers: *const u64, d_l0: *mut c_void, d_l_last: *mut c_void,
+                                              d_l_active_row: *mut c_void, stream: *mut c_void) -> c_int;
+    pub fn h2b_permutation_build_vk(mapping: *const *const u64, n_columns: u32, k: u32, delta: *const u64, omega: *const u64, handle_g_lagrange: u64,
+                                    out_commitments: *mut u64) -> c_int;
+    pub fn h2b_permutation_build_pk(mapping: *const *const u64, n_columns: u32, k: u32, extended_k: u32, delta: *const u64, omega: *const u64,
+                                    omega_inv: *const u64, ifft_divisor: *const u64, extended_omega: *const u64, zeta_powers: *const u64,
+                                    out_permutations: *const *mut u64, out_polys: *const *mut u64, out_cosets: *const *mut u64) -> c_int;
     pub fn h2b_dev_alloc(device: c_int, bytes: usize, out: *mut *mut c_void) -> c_int;
     pub fn h2b_dev_free(device: c_int, p: *mut c_void) -> c_int;
     pub fn h2b_memcpy_h2d(device: c_int, d_dst: *mut c_void, h_src: *const c_void, bytes: usize) -> c_int;
@@ -202,4 +213,101 @@ pub fn srs_downsize(handle_g: u64, k: u32) -> (Vec<[u64; 8]>, u64, u64) {
         panic!("h2b_srs_downsize failed ({rc}): {}", last_error());
     }
     (g_lagrange, hg, hl)
+}
+
+/// The domain constants the keygen calls take, as Montgomery limbs (`EvaluationDomain`'s fields; `zeta_powers` = 1, g_coset,
+/// g_coset_inv).
+pub struct KeygenDomain {
+    pub k: u32,
+    pub extended_k: u32,
+    pub omega: [u64; 4],
+    pub omega_inv: [u64; 4],
+    pub ifft_divisor: [u64; 4],
+    pub extended_omega: [u64; 4],
+    pub zeta_powers: [[u64; 4]; 3],
+}
+
+/// A mapping column as the C ABI reads it: `2^k` pairs of u64 (column, row).  Upstream's `Vec<(usize, usize)>` is passed as is
+/// when `(usize, usize)` is laid out that way on this target (64-bit usize, field 0 first); otherwise it is converted once.
+fn mapping_columns(mapping: &[Vec<(usize, usize)>], n: usize) -> (Vec<Vec<[u64; 2]>>, Vec<*const u64>) {
+    let same_layout = std::mem::size_of::<(usize, usize)>() == 16
+        && std::mem::size_of::<usize>() == 8
+        && std::mem::offset_of!((usize, usize), 0) == 0
+        && std::mem::offset_of!((usize, usize), 1) == 8;
+    let mut owned = Vec::new();
+    let mut ptrs = Vec::with_capacity(mapping.len());
+    for col in mapping {
+        assert_eq!(col.len(), n, "mapping column length != 2^k");
+        if same_layout {
+            ptrs.push(col.as_ptr() as *const u64);
+        } else {
+            owned.push(col.iter().map(|&(c, r)| [c as u64, r as u64]).collect::<Vec<_>>());
+            ptrs.push(owned.last().unwrap().as_ptr() as *const u64);
+        }
+    }
+    (owned, ptrs)
+}
+
+/// `Assembly::build_vk`: `commit_lagrange(sigma_i)` (Jacobian, 12 u64) for every column of `mapping`, over the registered set
+/// `handle_g_lagrange`.  Panics like upstream's out-of-range index on an invalid mapping entry.
+pub fn permutation_build_vk(mapping: &[Vec<(usize, usize)>], delta: &[u64; 4], dom: &KeygenDomain, handle_g_lagrange: u64) -> Vec<[u64; 12]> {
+    ensure_init();
+    let (_owned, ptrs) = mapping_columns(mapping, 1usize << dom.k);
+    let mut out = vec![[0u64; 12]; mapping.len()];
+    let rc = unsafe {
+        h2b_permutation_build_vk(ptrs.as_ptr(), ptrs.len() as u32, dom.k, delta.as_ptr(), dom.omega.as_ptr(), handle_g_lagrange, out.as_mut_ptr() as *mut u64)
+    };
+    if rc != 0 {
+        panic!("h2b_permutation_build_vk failed ({rc}): {}", last_error());
+    }
+    out
+}
+
+/// `Assembly::build_pk`: per column sigma (Lagrange), its coefficients and its extended coset, as `2^k`, `2^k` and `2^extended_k`
+/// Montgomery scalars.  Panics like upstream's out-of-range index on an invalid mapping entry.
+#[allow(clippy::type_complexity)]
+pub fn permutation_build_pk(mapping: &[Vec<(usize, usize)>], delta: &[u64; 4], dom: &KeygenDomain) -> (Vec<Vec<[u64; 4]>>, Vec<Vec<[u64; 4]>>, Vec<Vec<[u64; 4]>>) {
+    ensure_init();
+    let n = 1usize << dom.k;
+    let (_owned, ptrs) = mapping_columns(mapping, n);
+    let mut perms = vec![vec![[0u64; 4]; n]; mapping.len()];
+    let mut polys = vec![vec![[0u64; 4]; n]; mapping.len()];
+    let mut cosets = vec![vec![[0u64; 4]; 1usize << dom.extended_k]; mapping.len()];
+    let outs = |v: &mut Vec<Vec<[u64; 4]>>| v.iter_mut().map(|c| c.as_mut_ptr() as *mut u64).collect::<Vec<_>>();
+    let (p, c, e) = (outs(&mut perms), outs(&mut polys), outs(&mut cosets));
+    let rc = unsafe {
+        h2b_permutation_build_pk(ptrs.as_ptr(), ptrs.len() as u32, dom.k, dom.extended_k, delta.as_ptr(), dom.omega.as_ptr(), dom.omega_inv.as_ptr(),
+                                 dom.ifft_divisor.as_ptr(), dom.extended_omega.as_ptr(), dom.zeta_powers.as_ptr() as *const u64, p.as_ptr(), c.as_ptr(),
+                                 e.as_ptr())
+    };
+    if rc != 0 {
+        panic!("h2b_permutation_build_pk failed ({rc}): {}", last_error());
+    }
+    (perms, polys, cosets)
+}
+
+/// keygen_pk's `(l0, l_last, l_active_row)` on the extended coset, each `2^extended_k` Montgomery scalars, computed on device 0.
+pub fn keygen_lagrange_indicators(dom: &KeygenDomain, blinding_factors: u32) -> [Vec<[u64; 4]>; 3] {
+    ensure_init();
+    let en = 1usize << dom.extended_k;
+    let mut d = [std::ptr::null_mut::<c_void>(); 3];
+    for p in d.iter_mut() {
+        assert_eq!(unsafe { h2b_dev_alloc(0, en * 32, p) }, 0, "h2b_dev_alloc: {}", last_error());
+    }
+    let mut out = [vec![[0u64; 4]; en], vec![[0u64; 4]; en], vec![[0u64; 4]; en]];
+    let rc = unsafe {
+        h2b_keygen_lagrange_indicators_dev(0, dom.k, dom.extended_k, blinding_factors, dom.omega_inv.as_ptr(), dom.ifft_divisor.as_ptr(),
+                                           dom.extended_omega.as_ptr(), dom.zeta_powers.as_ptr() as *const u64, d[0], d[1], d[2], std::ptr::null_mut())
+    };
+    let mut ok = rc == 0 && unsafe { h2b_dev_sync(0) } == 0;
+    for (o, p) in out.iter_mut().zip(d.iter()) {
+        ok = ok && unsafe { h2b_memcpy_d2h(0, o.as_mut_ptr() as *mut c_void, *p, en * 32) } == 0;
+    }
+    for p in d {
+        unsafe { h2b_dev_free(0, p) };
+    }
+    if !ok {
+        panic!("keygen_pk indicators failed: {}", last_error());
+    }
+    out
 }
