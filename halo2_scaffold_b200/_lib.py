@@ -41,6 +41,7 @@ _EXPORTS = [
     "h2b_register_bases_sharded", "h2b_msm_bn254_g1_dev_batch_registered", "h2b_implicit_cache_stats", "h2b_msm_checksum_dev", "h2b_ntt_bn254_fr_dev_batch", "h2b_lagrange_to_coeff_dev_batch", "h2b_coeff_to_extended_dev_batch", "h2b_memcpy_d2d_async", "h2b_memset_zero_async", "h2b_column_pipeline",
     "h2b_srs_setup", "h2b_g1_generator_mul_dev", "h2b_g1_to_lagrange_dev", "h2b_srs_downsize",
     "h2b_permutation_sigma_dev", "h2b_keygen_lagrange_indicators_dev", "h2b_permutation_build_vk", "h2b_permutation_build_pk",
+    "h2b_selector_exclusion", "h2b_keygen_fixed_build_vk", "h2b_keygen_fixed_build_pk",
 ]
 
 
@@ -131,6 +132,25 @@ def _mapping_columns(mapping, k: int):
     return cols
 
 
+def _activation_rows(activations, k: int):
+    """selector activations -- (S, 2^k) bool / uint8 or a list of such rows -> contiguous uint8 rows (Rust's Vec<bool> layout)"""
+    rows = [np.ascontiguousarray(np.asarray(a).reshape(-1), dtype=np.uint8) for a in activations]
+    for r in rows:
+        assert r.shape[0] == 1 << k, "activation row of %d entries, expected 2^%d" % (r.shape[0], k)
+    return rows
+
+
+def _fixed_args(fixed, activations, combination_of, root_of, k: int):
+    fx = [_u64(c).reshape(-1, 4) for c in fixed]
+    for c in fx:
+        assert c.shape[0] == 1 << k, "fixed column of %d rows, expected 2^%d" % (c.shape[0], k)
+    acts = _activation_rows(activations, k)
+    co = np.ascontiguousarray(np.asarray(combination_of, dtype=np.uint32).reshape(-1))
+    ro = np.ascontiguousarray(np.asarray(root_of, dtype=np.uint32).reshape(-1))
+    assert co.shape[0] == len(acts) and ro.shape[0] == len(acts), "one combination and one root per selector"
+    return fx, acts, co, ro
+
+
 class Lib:
     def __init__(self, path: str | None = None, allow_emulator: bool = False):
         path = path or os.environ.get("H2B200_LIB", DEFAULT_LIB)
@@ -194,6 +214,9 @@ class Lib:
         L.h2b_keygen_lagrange_indicators_dev.argtypes = [i32, u32, u32, u32, vp, vp, vp, vp, vp, vp, vp, vp]
         L.h2b_permutation_build_vk.argtypes = [vp, u32, u32, vp, vp, u64, vp]
         L.h2b_permutation_build_pk.argtypes = [vp, u32, u32, u32, vp, vp, vp, vp, vp, vp, vp, vp, vp]
+        L.h2b_selector_exclusion.argtypes = [vp, u32, u32, vp]
+        L.h2b_keygen_fixed_build_vk.argtypes = [vp, u32, vp, u32, vp, vp, u32, u32, u64, vp]
+        L.h2b_keygen_fixed_build_pk.argtypes = [vp, u32, vp, u32, vp, vp, u32, u32, u32, vp, vp, vp, vp, vp, vp, vp]
         L.h2b_evaluate_graph_dev.argtypes = [i32, vp, vp, vp, u32, i32, vp]
         L.h2b_evaluate_h_permutation_dev.argtypes = [i32, vp, u32, i32, vp, u32, vp, vp, u32, u32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
         L.h2b_evaluate_h_lookup_dev.argtypes = [i32, vp, vp, vp, u32, i32, vp, vp, vp, vp, vp, vp, vp]
@@ -742,6 +765,41 @@ class Lib:
         self.check(self.L.h2b_permutation_build_pk(_ptr_array([c.ctypes.data for c in cols]), P, k, extended_k, *[x.ctypes.data for x in w],
                                                    zp.ctypes.data, arr(perms), arr(polys), arr(cosets)))
         return dict(permutations=perms, polys=polys, cosets=cosets)
+
+    # ---- key generation: compress_selectors' exclusion matrix and the fixed columns of keygen_vk / keygen_pk ---------------------
+    def selector_exclusion(self, activations, k: int) -> np.ndarray:
+        """process's exclusion matrix: activations (S, 2^k) bool / uint8 (or a list of such rows) -> (S, S) bool, True where two
+        selectors are active on a common row (symmetric, False on the diagonal)"""
+        acts = _activation_rows(activations, k)
+        out = np.zeros((len(acts), len(acts)), dtype=np.uint8)
+        self.check(self.L.h2b_selector_exclusion(_ptr_array([a.ctypes.data for a in acts]) if acts else None, len(acts), k, out.ctypes.data))
+        return out.astype(bool)
+
+    def keygen_fixed_build_vk(self, fixed, activations, combination_of, root_of, n_combinations: int, k: int, handle_g_lagrange: int) -> np.ndarray:
+        """keygen_vk's fixed commitments: fixed (F, 2^k, 4) Montgomery words (or a list of (2^k, 4) columns), activations (S, 2^k) and
+        the assignment -> (F + n_combinations, 12) Jacobian commitments of the fixed columns, then the combination columns"""
+        fx, acts, co, ro = _fixed_args(fixed, activations, combination_of, root_of, k)
+        out = np.zeros((len(fx) + n_combinations, 12), dtype=np.uint64)
+        self.check(self.L.h2b_keygen_fixed_build_vk(_ptr_array([c.ctypes.data for c in fx]) if fx else None, len(fx),
+                                                    _ptr_array([a.ctypes.data for a in acts]) if acts else None, len(acts), co.ctypes.data,
+                                                    ro.ctypes.data, n_combinations, k, handle_g_lagrange, out.ctypes.data))
+        return out
+
+    def keygen_fixed_build_pk(self, fixed, activations, combination_of, root_of, n_combinations: int, k: int, extended_k: int, omega_inv, ifft_divisor,
+                              extended_omega, zeta_powers, want_values: bool = True, want_polys: bool = True, want_cosets: bool = True):
+        """keygen_pk's fixed columns -> dict(combination_values, polys, cosets): the n_combinations combination columns (2^k, 4), and
+        lagrange_to_coeff / coeff_to_extended of all F + n_combinations columns ((2^k, 4) and (2^extended_k, 4)); None when not wanted"""
+        fx, acts, co, ro = _fixed_args(fixed, activations, combination_of, root_of, k)
+        n, T = 1 << k, len(fx) + n_combinations
+        w = [_u64(x).reshape(4) for x in (omega_inv, ifft_divisor, extended_omega)]
+        zp = _u64(zeta_powers).reshape(3, 4)
+        vals = [np.empty((n, 4), dtype=np.uint64) for _ in range(n_combinations)] if want_values else None
+        polys = [np.empty((n, 4), dtype=np.uint64) for _ in range(T)] if want_polys else None
+        cosets = [np.empty((1 << extended_k, 4), dtype=np.uint64) for _ in range(T)] if want_cosets else None
+        arr = lambda xs: _ptr_array([x.ctypes.data for x in xs]) if xs else None
+        self.check(self.L.h2b_keygen_fixed_build_pk(arr(fx), len(fx), arr(acts), len(acts), co.ctypes.data, ro.ctypes.data, n_combinations, k, extended_k,
+                                                    *[x.ctypes.data for x in w], zp.ctypes.data, arr(vals), arr(polys), arr(cosets)))
+        return dict(combination_values=vals, polys=polys, cosets=cosets)
 
     # ---- quotient evaluation (evaluate_h) on device-resident extended-coset columns ------------------
     def evaluate_graph_dev(self, device: int, graph: GraphArrays, cols: EvalColumns, d_values: int, size: int, rot_scale: int, stream: int = 0,

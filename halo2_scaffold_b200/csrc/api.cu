@@ -1595,17 +1595,33 @@ int h2b_keygen_lagrange_indicators_dev(int device, uint32_t k, uint32_t extended
     return keygen_indicators_run(*c, k, extended_k, blinding_factors, omega_inv, ifft_divisor, extended_omega, zeta_powers, cols, (cudaStream_t)stream);
 }
 
-// One build_vk / build_pk pass over the mapping columns [col_begin, col_end); column i runs on device i mod D.
+// The combination columns of compress_selectors: combination c's members are the selectors s with combination_of[s] = c, and
+// member s writes root_of[s] on its active rows.  Built (and validated) on the host before any device work.
+struct SelectorCombinations {
+    const uint8_t* const* activations = nullptr;
+    uint32_t n_selectors = 0, n_combinations = 0;
+    std::vector<std::vector<uint32_t>> members;     // per combination: its selectors, in increasing order
+    const uint32_t* root_of = nullptr;
+};
+
+// One build_vk / build_pk pass over the columns [col_begin, col_end); column i runs on device i mod D.  Column i's Lagrange values
+// come from, in this order: sigma of mapping[i] for i < n_sigma, the caller's fixed[i - n_sigma] for the next n_fixed, and the
+// combination columns of `comb` after those.
 struct KeygenJob {
     const uint64_t* const* mapping = nullptr;
-    uint32_t n_columns = 0, k = 0, extended_k = 0, col_begin = 0, col_end = 0;
+    uint32_t n_sigma = 0;
+    const uint64_t* const* fixed = nullptr;
+    uint32_t n_fixed = 0;
+    const SelectorCombinations* comb = nullptr;
+    uint32_t k = 0, extended_k = 0, col_begin = 0, col_end = 0;
     const uint64_t *delta = nullptr, *omega = nullptr, *omega_inv = nullptr, *ifft_divisor = nullptr, *extended_omega = nullptr, *zeta_powers = nullptr;
-    bool validate_only = false;                 // sigma and its status word only: nothing leaves the device
-    const BaseSet* commit_set = nullptr;        // a replicated set: commitments of sigma over its first n points
-    uint64_t* commitments = nullptr;            // n_columns x 12 words (Jacobian), indexed by column
-    uint64_t* const* sigma_out = nullptr;       // per column (indexed by column), or null
+    bool validate_only = false;                 // the columns that can be invalid (sigma, combinations) and the status word only
+    const BaseSet* commit_set = nullptr;        // a replicated set: commitments of the columns over its first n points
+    uint64_t* commitments = nullptr;            // 12 words (Jacobian) per column, indexed by column
+    uint64_t* const* values_out = nullptr;      // per column (indexed by column; an entry may be null), or null
     uint64_t* const* poly_out = nullptr;
     uint64_t* const* coset_out = nullptr;
+    uint32_t n_columns() const { return n_sigma + n_fixed + (comb ? comb->n_combinations : 0); }
 };
 
 // scratch of one device's share, given back on every return path
@@ -1628,11 +1644,30 @@ struct KeygenScratch {
     }
 };
 
-static const size_t KEYGEN_GROUP_BYTES = (size_t)1 << 31;      // device memory of one group of columns (sigma / coefficients / cosets)
+static const size_t KEYGEN_GROUP_BYTES = (size_t)1 << 31;      // device memory of one group of columns (values / coefficients / cosets)
 
-// device d's columns of the job, in groups that share the batched MSM / NTT launches.  The mapping of column i + 1 is staged while the
-// sigma kernel of column i runs (two mapping buffers).  *bad receives the status word of the first group that holds an invalid entry; no
-// output of that group or a later one is written.
+// Uploads each selector of `sel` (n bytes, pageable) and packs it into d_bits + slot * selector_words(n); the upload of selector t + 1
+// goes through the other of the two staging buffers while the pack kernel of selector t runs.
+static int keygen_pack_selectors(DeviceCtx& c, KeygenScratch& s, const uint8_t* const* activations, const std::vector<uint32_t>& sel, size_t n,
+                                 void* d_bits, cudaStream_t st) {
+    if (sel.empty()) return H2B_OK;
+    void* d_act[2];
+    H2B_TRY(s.alloc(n, &d_act[0]));
+    H2B_TRY(s.alloc(n, &d_act[1]));
+    for (size_t t = 0; t < sel.size(); ++t) {
+        const int slot = (int)(t & 1);
+        H2B_CUDA(cudaEventSynchronize(s.ev[slot]));            // the pack kernel that last read this buffer is done
+        H2B_TRY(host_upload(c, d_act[slot], activations[sel[t]], n, st, false));
+        H2B_TRY(selector_pack_run(c, d_act[slot], n, (uint32_t*)d_bits + t * selector_words(n), st));
+        H2B_CUDA(cudaEventRecord(s.ev[slot], st));
+    }
+    return H2B_OK;
+}
+
+// device d's columns of the job, in groups that share the batched MSM / NTT launches.  The mapping of sigma column i + 1 is staged
+// while the sigma kernel of column i runs (two mapping buffers); the selectors of this device's combination columns are uploaded and
+// packed once, before the first group.  *bad receives the status word of the first group that holds an invalid entry; no output of
+// that group or a later one is written.
 static int keygen_device(size_t d, const KeygenJob& job, uint32_t* bad) {
     const size_t nd = G.devs.size();
     std::vector<uint32_t> mine;
@@ -1644,6 +1679,7 @@ static int keygen_device(size_t d, const KeygenJob& job, uint32_t* bad) {
     const cudaStream_t st = c.stream;
     const uint32_t k = job.k;
     const size_t n = (size_t)1 << k;
+    const uint32_t comb0 = job.n_sigma + job.n_fixed;
     const bool pk = job.poly_out || job.coset_out;
     const size_t col_bytes = (job.coset_out && !job.validate_only ? (size_t)1 << job.extended_k : n) * 32;
     size_t group = ntt_batch_max();
@@ -1651,30 +1687,68 @@ static int keygen_device(size_t d, const KeygenJob& job, uint32_t* bad) {
     if (job.commit_set && group > msm_batch_max()) group = msm_batch_max();
     KeygenScratch s;
     s.ctx = &c;
-    void *d_map[2], *d_cols, *d_status, *d_blocks;
-    H2B_TRY(s.alloc(n * 16, &d_map[0]));
-    H2B_TRY(s.alloc(n * 16, &d_map[1]));
+    for (cudaEvent_t& e : s.ev) H2B_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    void *d_map[2] = {nullptr, nullptr}, *d_cols, *d_status, *d_blocks, *d_bits = nullptr, *d_members = nullptr;
+    const bool any_sigma = mine.front() < job.n_sigma;
+    // this device's combinations: the selectors they use get consecutive bitset slots, members become (slot, root) pairs
+    std::vector<uint32_t> sel, member_pairs, member_off;
+    if (job.comb) {
+        std::vector<uint32_t> slot_of(job.comb->n_selectors, UINT32_MAX);
+        for (uint32_t i : mine) {
+            if (i < comb0) continue;
+            member_off.push_back((uint32_t)member_pairs.size() / 2);
+            for (uint32_t sidx : job.comb->members[i - comb0]) {
+                if (slot_of[sidx] == UINT32_MAX) { slot_of[sidx] = (uint32_t)sel.size(); sel.push_back(sidx); }
+                member_pairs.push_back(slot_of[sidx]);
+                member_pairs.push_back(job.comb->root_of[sidx]);
+            }
+        }
+        member_off.push_back((uint32_t)member_pairs.size() / 2);
+    }
+    if (any_sigma) {
+        H2B_TRY(s.alloc(n * 16, &d_map[0]));
+        H2B_TRY(s.alloc(n * 16, &d_map[1]));
+    }
+    if (!sel.empty()) {
+        H2B_TRY(s.alloc(sel.size() * selector_words(n) * 4, &d_bits));
+        H2B_TRY(s.alloc(member_pairs.size() * 4, &d_members));
+    }
     H2B_TRY(s.alloc(group * col_bytes, &d_cols));
     H2B_TRY(s.alloc(group * 224 + 32, &d_blocks));
     d_status = (char*)d_blocks + group * 224;
-    for (cudaEvent_t& e : s.ev) H2B_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     c.prof.mark(PROF_BEGIN, st);
     H2B_CUDA(cudaMemsetAsync(d_status, 0, 4, st));
-    H2B_TRY(permutation_sigma_tables_run(c, job.n_columns, k, job.delta, job.omega, st));
-    size_t seq = 0;
+    if (any_sigma) H2B_TRY(permutation_sigma_tables_run(c, job.n_sigma, k, job.delta, job.omega, st));
+    if (!sel.empty()) {
+        H2B_CUDA(cudaMemcpyAsync(d_members, member_pairs.data(), member_pairs.size() * 4, cudaMemcpyHostToDevice, st));
+        H2B_TRY(keygen_pack_selectors(c, s, job.comb->activations, sel, n, d_bits, st));
+        c.prof.mark(PROF_KEYGEN_PACK, st);
+    }
+    size_t seq = 0, comb_seq = 0;
     for (size_t g0 = 0; g0 < mine.size(); g0 += group) {
         const size_t m = mine.size() - g0 < group ? mine.size() - g0 : group;
         std::vector<void*> cols(m);
         for (size_t t = 0; t < m; ++t) {
             const uint32_t i = mine[g0 + t];
-            const int slot = (int)(seq++ & 1);
             cols[t] = (char*)d_cols + t * col_bytes;
-            H2B_CUDA(cudaEventSynchronize(s.ev[slot]));          // the sigma kernel that last read this mapping buffer is done
-            H2B_TRY(host_upload(c, d_map[slot], job.mapping[i], n * 16, st, false));
-            c.prof.mark(PROF_KEYGEN_UPLOAD, st);
-            H2B_TRY(permutation_sigma_run(c, &d_map[slot], 1, i, job.n_columns, k, &cols[t], d_status, st));
-            H2B_CUDA(cudaEventRecord(s.ev[slot], st));
-            c.prof.mark(PROF_KEYGEN_SIGMA, st);
+            if (i < job.n_sigma) {
+                const int slot = (int)(seq++ & 1);
+                H2B_CUDA(cudaEventSynchronize(s.ev[slot]));          // the sigma kernel that last read this mapping buffer is done
+                H2B_TRY(host_upload(c, d_map[slot], job.mapping[i], n * 16, st, false));
+                c.prof.mark(PROF_KEYGEN_UPLOAD, st);
+                H2B_TRY(permutation_sigma_run(c, &d_map[slot], 1, i, job.n_sigma, k, &cols[t], d_status, st));
+                H2B_CUDA(cudaEventRecord(s.ev[slot], st));
+                c.prof.mark(PROF_KEYGEN_SIGMA, st);
+            } else if (i < comb0) {
+                if (job.validate_only) continue;                     // the caller's values need no check
+                H2B_TRY(host_upload(c, cols[t], job.fixed[i - job.n_sigma], n * 32, st, t == 0));
+                c.prof.mark(PROF_KEYGEN_FIXED_UPLOAD, st);
+            } else {
+                const size_t q = comb_seq++;
+                H2B_TRY(combination_column_run(c, d_bits, (const uint32_t*)d_members + 2 * (size_t)member_off[q], member_off[q + 1] - member_off[q],
+                                               i - comb0, k, cols[t], d_status, st));
+                c.prof.mark(PROF_KEYGEN_COMBINATION, st);
+            }
         }
         uint32_t status = 0;
         H2B_CUDA(cudaMemcpyAsync(&status, d_status, 4, cudaMemcpyDeviceToHost, st));
@@ -1695,8 +1769,9 @@ static int keygen_device(size_t d, const KeygenJob& job, uint32_t* bad) {
             H2B_CUDA(cudaStreamSynchronize(st));
             for (size_t t = 0; t < m; ++t) memcpy(job.commitments + 12 * (size_t)mine[g0 + t], &blocks[28 * t], 96);
         }
-        if (job.sigma_out) {
-            for (size_t t = 0; t < m; ++t) H2B_TRY(host_download(c, job.sigma_out[mine[g0 + t]], cols[t], n * 32, st));
+        if (job.values_out) {
+            for (size_t t = 0; t < m; ++t)
+                if (job.values_out[mine[g0 + t]]) H2B_TRY(host_download(c, job.values_out[mine[g0 + t]], cols[t], n * 32, st));
             c.prof.mark(PROF_KEYGEN_DOWNLOAD, st);
         }
         if (!pk) continue;
@@ -1716,7 +1791,7 @@ static int keygen_device(size_t d, const KeygenJob& job, uint32_t* bad) {
     return H2B_OK;
 }
 
-// every device's share of the job; an invalid mapping entry fails with H2B_ERR_BAD_ARGUMENT
+// every device's share of the job; an invalid mapping entry or two members of a combination on one row fail with H2B_ERR_BAD_ARGUMENT
 static int keygen_run(const char* who, const KeygenJob& job) {
     const size_t nd = G.devs.size();
     std::vector<uint32_t> bad(nd, 0);
@@ -1724,11 +1799,57 @@ static int keygen_run(const char* who, const KeygenJob& job) {
     for (size_t d = 0; d < nd; ++d) {
         if (!bad[d]) continue;
         const uint64_t flat = bad[d] - 1, n = (uint64_t)1 << job.k;
-        if (bad[d] == 0xFFFFFFFFu) set_error("%s: the mapping holds an entry outside %u columns x 2^%u rows", who, job.n_columns, job.k);
-        else set_error("%s: mapping[%llu][%llu] is outside %u columns x 2^%u rows", who, (unsigned long long)(flat / n), (unsigned long long)(flat % n),
-                       job.n_columns, job.k);
+        if (job.comb) {
+            if (bad[d] == 0xFFFFFFFFu) set_error("%s: two selectors of one combination are active on the same row", who);
+            else set_error("%s: two selectors of combination %llu are active on row %llu", who, (unsigned long long)(flat / n), (unsigned long long)(flat % n));
+        } else if (bad[d] == 0xFFFFFFFFu) {
+            set_error("%s: the mapping holds an entry outside %u columns x 2^%u rows", who, job.n_sigma, job.k);
+        } else {
+            set_error("%s: mapping[%llu][%llu] is outside %u columns x 2^%u rows", who, (unsigned long long)(flat / n), (unsigned long long)(flat % n),
+                      job.n_sigma, job.k);
+        }
         return H2B_ERR_BAD_ARGUMENT;
     }
+    return H2B_OK;
+}
+
+// commitments of every column of `job` over a registered g_lagrange set (the caller has checked that it holds at least n points)
+static int keygen_commit(const char* who, KeygenJob& job, const BaseSet& bs, uint64_t* out_commitments) {
+    const size_t n = (size_t)1 << job.k;
+    const uint32_t total = job.n_columns();
+    std::vector<uint64_t> com((size_t)total * 12);
+    if (!bs.sharded) {
+        job.commit_set = &bs;
+        job.commitments = com.data();
+        job.col_begin = 0; job.col_end = total;
+        H2B_TRY(keygen_run(who, job));
+    } else {
+        // a sharded set holds every point on one device only: the columns come back to the host (the caller's fixed columns are
+        // there already) and each commitment is split by point range over the devices, as h2b_msm_bn254_g1_batch_registered does
+        for (uint32_t i = 0; i < job.n_fixed; ++i) H2B_TRY(msm_host(job.fixed[i], bs, 0, n, com.data() + 12 * (size_t)(job.n_sigma + i)));
+        const uint32_t chunk = (uint32_t)ntt_batch_max();
+        std::vector<std::vector<uint64_t>> values(chunk, std::vector<uint64_t>(4 * n));
+        std::vector<uint64_t*> ptrs(total, nullptr);
+        job.values_out = ptrs.data();
+        const uint32_t ranges[2][2] = {{0, job.n_sigma}, {job.n_sigma + job.n_fixed, total}};
+        for (const auto& r : ranges) {
+            for (uint32_t c0 = r[0]; c0 < r[1]; c0 += chunk) {
+                const uint32_t c1 = r[1] - c0 < chunk ? r[1] : c0 + chunk;
+                for (uint32_t i = c0; i < c1; ++i) ptrs[i] = values[i - c0].data();
+                job.col_begin = c0; job.col_end = c1;
+                H2B_TRY(keygen_run(who, job));
+                for (uint32_t i = c0; i < c1; ++i) H2B_TRY(msm_host(ptrs[i], bs, 0, n, com.data() + 12 * (size_t)i));
+            }
+        }
+    }
+    memcpy(out_commitments, com.data(), com.size() * 8);
+    return H2B_OK;
+}
+
+static int keygen_lookup_set(const char* who, uint64_t handle_g_lagrange, uint32_t k, SetRef* out) {
+    *out = find_set(handle_g_lagrange);
+    if (!*out) { set_error("%s: unknown base-set handle %llu", who, (unsigned long long)handle_g_lagrange); return H2B_ERR_BAD_ARGUMENT; }
+    if (((size_t)1 << k) > (*out)->n) { set_error("%s: 2^%u points requested from a set of %zu", who, k, (*out)->n); return H2B_ERR_BAD_ARGUMENT; }
     return H2B_OK;
 }
 
@@ -1745,35 +1866,11 @@ int h2b_permutation_build_vk(const uint64_t* const* mapping, uint32_t n_columns,
     static const char* who = "h2b_permutation_build_vk";
     H2B_TRY(keygen_check(who, mapping, n_columns, k, delta, omega));
     if (!out_commitments) { set_error("%s: null output", who); return H2B_ERR_BAD_ARGUMENT; }
-    const size_t n = (size_t)1 << k;
-    SetRef bs = find_set(handle_g_lagrange);
-    if (!bs) { set_error("%s: unknown base-set handle %llu", who, (unsigned long long)handle_g_lagrange); return H2B_ERR_BAD_ARGUMENT; }
-    if (n > bs->n) { set_error("%s: 2^%u points requested from a set of %zu", who, k, bs->n); return H2B_ERR_BAD_ARGUMENT; }
-    std::vector<uint64_t> com((size_t)n_columns * 12);
+    SetRef bs;
+    H2B_TRY(keygen_lookup_set(who, handle_g_lagrange, k, &bs));
     KeygenJob job;
-    job.mapping = mapping; job.n_columns = n_columns; job.k = k; job.delta = delta; job.omega = omega;
-    if (!bs->sharded) {
-        job.commit_set = bs.get();
-        job.commitments = com.data();
-        job.col_begin = 0; job.col_end = n_columns;
-        H2B_TRY(keygen_run(who, job));
-    } else {
-        // a sharded set holds every point on one device only: sigma comes back to the host and each commitment is split by point
-        // range over the devices, as h2b_msm_bn254_g1_batch_registered does with such a set
-        const uint32_t chunk = (uint32_t)ntt_batch_max();
-        std::vector<std::vector<uint64_t>> sigma(chunk, std::vector<uint64_t>(4 * n));
-        std::vector<uint64_t*> ptrs(n_columns, nullptr);
-        job.sigma_out = ptrs.data();
-        for (uint32_t c0 = 0; c0 < n_columns; c0 += chunk) {
-            const uint32_t c1 = n_columns - c0 < chunk ? n_columns : c0 + chunk;
-            for (uint32_t i = c0; i < c1; ++i) ptrs[i] = sigma[i - c0].data();
-            job.col_begin = c0; job.col_end = c1;
-            H2B_TRY(keygen_run(who, job));
-            for (uint32_t i = c0; i < c1; ++i) H2B_TRY(msm_host(ptrs[i], *bs, 0, n, com.data() + 12 * (size_t)i));
-        }
-    }
-    memcpy(out_commitments, com.data(), com.size() * 8);
-    return H2B_OK;
+    job.mapping = mapping; job.n_sigma = n_columns; job.k = k; job.delta = delta; job.omega = omega;
+    return keygen_commit(who, job, *bs, out_commitments);
 }
 
 int h2b_permutation_build_pk(const uint64_t* const* mapping, uint32_t n_columns, uint32_t k, uint32_t extended_k, const uint64_t delta[4],
@@ -1787,7 +1884,7 @@ int h2b_permutation_build_pk(const uint64_t* const* mapping, uint32_t n_columns,
         if (outs)
             for (uint32_t i = 0; i < n_columns; ++i) if (!outs[i]) { set_error("%s: output column %u is null", who, i); return H2B_ERR_BAD_ARGUMENT; }
     KeygenJob job;
-    job.mapping = mapping; job.n_columns = n_columns; job.k = k; job.extended_k = extended_k; job.delta = delta; job.omega = omega;
+    job.mapping = mapping; job.n_sigma = n_columns; job.k = k; job.extended_k = extended_k; job.delta = delta; job.omega = omega;
     job.omega_inv = omega_inv; job.ifft_divisor = ifft_divisor; job.extended_omega = extended_omega; job.zeta_powers = zeta_powers;
     job.col_begin = 0; job.col_end = n_columns;
     // every entry is checked before the first byte of caller memory is written: a pass that only builds sigma, then the real one
@@ -1795,7 +1892,131 @@ int h2b_permutation_build_pk(const uint64_t* const* mapping, uint32_t n_columns,
     H2B_TRY(keygen_run(who, job));
     if (!out_permutations && !out_polys && !out_cosets) return H2B_OK;
     job.validate_only = false;
-    job.sigma_out = out_permutations; job.poly_out = out_polys; job.coset_out = out_cosets;
+    job.values_out = out_permutations; job.poly_out = out_polys; job.coset_out = out_cosets;
+    return keygen_run(who, job);
+}
+
+// ---- key generation: compress_selectors and the fixed columns of keygen_vk / keygen_pk --------------------------------------------
+// ([UP] halo2_proofs/src/plonk/circuit/compress_selectors.rs process, plonk/keygen.rs keygen_vk / keygen_pk)
+static const uint32_t SELECTORS_MAX = 1u << 14;
+
+static int selectors_check(const char* who, const uint8_t* const* activations, uint32_t n_selectors, uint32_t k) {
+    if (k > 28) { set_error("%s: k = %u (need k <= 28)", who, k); return H2B_ERR_BAD_ARGUMENT; }
+    if (n_selectors > SELECTORS_MAX) { set_error("%s: %u selectors (at most %u)", who, n_selectors, SELECTORS_MAX); return H2B_ERR_BAD_ARGUMENT; }
+    if (n_selectors && !activations) { set_error("%s: null activations", who); return H2B_ERR_BAD_ARGUMENT; }
+    for (uint32_t s = 0; s < n_selectors; ++s) if (!activations[s]) { set_error("%s: activations of selector %u are null", who, s); return H2B_ERR_BAD_ARGUMENT; }
+    return H2B_OK;
+}
+
+int h2b_selector_exclusion(const uint8_t* const* activations, uint32_t n_selectors, uint32_t k, uint8_t* out) {
+    static const char* who = "h2b_selector_exclusion";
+    H2B_TRY(require_init());
+    H2B_TRY(selectors_check(who, activations, n_selectors, k));
+    if (!out) { set_error("%s: null output", who); return H2B_ERR_BAD_ARGUMENT; }
+    if (n_selectors == 0) return H2B_OK;
+    const size_t n = (size_t)1 << k, S = n_selectors;
+    std::unique_lock<std::mutex> lk;
+    size_t d = 0;
+    DeviceCtx& c = *pick_device(lk, &d);
+    H2B_CUDA(cudaSetDevice(c.device));
+    const cudaStream_t st = c.stream;
+    KeygenScratch s;
+    s.ctx = &c;
+    for (cudaEvent_t& e : s.ev) H2B_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    void *d_bits, *d_flags;
+    H2B_TRY(s.alloc(S * selector_words(n) * 4, &d_bits));
+    H2B_TRY(s.alloc(S * S * 4, &d_flags));
+    std::vector<uint32_t> all(S);
+    for (uint32_t i = 0; i < S; ++i) all[i] = i;
+    c.prof.mark(PROF_BEGIN, st);
+    H2B_TRY(keygen_pack_selectors(c, s, activations, all, n, d_bits, st));
+    c.prof.mark(PROF_KEYGEN_PACK, st);
+    H2B_TRY(selector_exclusion_run(c, d_bits, n_selectors, n, d_flags, st));
+    c.prof.mark(PROF_KEYGEN_EXCLUSION, st);
+    std::vector<uint32_t> flags(S * S);
+    H2B_CUDA(cudaMemcpyAsync(flags.data(), d_flags, S * S * 4, cudaMemcpyDeviceToHost, st));
+    H2B_CUDA(cudaStreamSynchronize(st));
+    for (size_t i = 0; i < S; ++i)
+        for (size_t j = 0; j < S; ++j) out[i * S + j] = (uint8_t)(i > j ? flags[i * S + j] != 0 : i < j ? flags[j * S + i] != 0 : 0);
+    return H2B_OK;
+}
+
+// the arguments both fixed-column entry points take, checked before any device work; *comb receives the members of each combination
+static int fixed_keygen_check(const char* who, const uint64_t* const* fixed, uint32_t n_fixed, const uint8_t* const* activations, uint32_t n_selectors,
+                              const uint32_t* combination_of, const uint32_t* root_of, uint32_t n_combinations, uint32_t k,
+                              SelectorCombinations* comb) {
+    H2B_TRY(require_init());
+    H2B_TRY(selectors_check(who, activations, n_selectors, k));
+    if ((uint64_t)n_fixed + n_combinations == 0) { set_error("%s: no fixed and no combination columns", who); return H2B_ERR_BAD_ARGUMENT; }
+    if (n_fixed && !fixed) { set_error("%s: null fixed columns", who); return H2B_ERR_BAD_ARGUMENT; }
+    for (uint32_t i = 0; i < n_fixed; ++i) if (!fixed[i]) { set_error("%s: fixed column %u is null", who, i); return H2B_ERR_BAD_ARGUMENT; }
+    if (n_selectors && (!combination_of || !root_of)) { set_error("%s: null assignment", who); return H2B_ERR_BAD_ARGUMENT; }
+    comb->activations = activations;
+    comb->n_selectors = n_selectors;
+    comb->n_combinations = n_combinations;
+    comb->root_of = root_of;
+    comb->members.assign(n_combinations, std::vector<uint32_t>());
+    for (uint32_t s = 0; s < n_selectors; ++s) {
+        if (combination_of[s] >= n_combinations || root_of[s] == 0) {
+            set_error("%s: selector %u: combination %u of %u, root %u (need combination < %u and root > 0)", who, s, combination_of[s], n_combinations,
+                      root_of[s], n_combinations);
+            return H2B_ERR_BAD_ARGUMENT;
+        }
+        comb->members[combination_of[s]].push_back(s);
+    }
+    for (uint32_t c = 0; c < n_combinations; ++c)
+        if (comb->members[c].empty()) { set_error("%s: combination %u has no selector", who, c); return H2B_ERR_BAD_ARGUMENT; }
+    return H2B_OK;
+}
+
+int h2b_keygen_fixed_build_vk(const uint64_t* const* fixed, uint32_t n_fixed, const uint8_t* const* activations, uint32_t n_selectors,
+                              const uint32_t* combination_of, const uint32_t* root_of, uint32_t n_combinations, uint32_t k, uint64_t handle_g_lagrange,
+                              uint64_t* out_commitments) {
+    static const char* who = "h2b_keygen_fixed_build_vk";
+    SelectorCombinations comb;
+    H2B_TRY(fixed_keygen_check(who, fixed, n_fixed, activations, n_selectors, combination_of, root_of, n_combinations, k, &comb));
+    if (!out_commitments) { set_error("%s: null output", who); return H2B_ERR_BAD_ARGUMENT; }
+    SetRef bs;
+    H2B_TRY(keygen_lookup_set(who, handle_g_lagrange, k, &bs));
+    KeygenJob job;
+    job.fixed = fixed; job.n_fixed = n_fixed; job.comb = &comb; job.k = k;
+    return keygen_commit(who, job, *bs, out_commitments);
+}
+
+int h2b_keygen_fixed_build_pk(const uint64_t* const* fixed, uint32_t n_fixed, const uint8_t* const* activations, uint32_t n_selectors,
+                              const uint32_t* combination_of, const uint32_t* root_of, uint32_t n_combinations, uint32_t k, uint32_t extended_k,
+                              const uint64_t omega_inv[4], const uint64_t ifft_divisor[4], const uint64_t extended_omega[4], const uint64_t zeta_powers[12],
+                              uint64_t* const* out_combination_values, uint64_t* const* out_polys, uint64_t* const* out_cosets) {
+    static const char* who = "h2b_keygen_fixed_build_pk";
+    SelectorCombinations comb;
+    H2B_TRY(fixed_keygen_check(who, fixed, n_fixed, activations, n_selectors, combination_of, root_of, n_combinations, k, &comb));
+    if (extended_k > 28 || extended_k < k) { set_error("%s: need k <= extended_k <= 28 (k = %u, extended_k = %u)", who, k, extended_k); return H2B_ERR_BAD_ARGUMENT; }
+    if (!omega_inv || !ifft_divisor || !extended_omega || !zeta_powers) { set_error("%s: null pointer", who); return H2B_ERR_BAD_ARGUMENT; }
+    const uint32_t total = n_fixed + n_combinations;
+    if (out_combination_values)
+        for (uint32_t c = 0; c < n_combinations; ++c)
+            if (!out_combination_values[c]) { set_error("%s: combination output %u is null", who, c); return H2B_ERR_BAD_ARGUMENT; }
+    for (uint64_t* const* outs : {out_polys, out_cosets})
+        if (outs)
+            for (uint32_t i = 0; i < total; ++i) if (!outs[i]) { set_error("%s: output column %u is null", who, i); return H2B_ERR_BAD_ARGUMENT; }
+    KeygenJob job;
+    job.fixed = fixed; job.n_fixed = n_fixed; job.comb = &comb; job.k = k; job.extended_k = extended_k;
+    job.omega_inv = omega_inv; job.ifft_divisor = ifft_divisor; job.extended_omega = extended_omega; job.zeta_powers = zeta_powers;
+    job.col_begin = 0; job.col_end = total;
+    // no caller memory is written before every combination column has been built once and found valid
+    if (n_combinations) {
+        job.validate_only = true;
+        job.col_begin = n_fixed;
+        H2B_TRY(keygen_run(who, job));
+        job.validate_only = false;
+        job.col_begin = 0;
+    }
+    if (!out_combination_values && !out_polys && !out_cosets) return H2B_OK;
+    std::vector<uint64_t*> values(total, nullptr);
+    if (out_combination_values)
+        for (uint32_t c = 0; c < n_combinations; ++c) values[n_fixed + c] = out_combination_values[c];
+    job.values_out = out_combination_values ? values.data() : nullptr;
+    job.poly_out = out_polys; job.coset_out = out_cosets;
     return keygen_run(who, job);
 }
 

@@ -75,7 +75,8 @@ enum ProfTag { PROF_BEGIN = 0, PROF_MSM_DECOMPOSE = 1, PROF_MSM_SCAN = 2, PROF_M
                PROF_SRS_SCALARS = 24, PROF_SRS_FIXED_BASE = 25, PROF_SRS_NORMALISE = 26, PROF_SRS_TABLE = 27,
                PROF_G1NTT_TWIDDLE = 28, PROF_G1NTT_STAGES = 29, PROF_G1NTT_NORMALISE = 30,
                PROF_KEYGEN_UPLOAD = 31, PROF_KEYGEN_SIGMA = 32, PROF_KEYGEN_COMMIT = 33, PROF_KEYGEN_INTT = 34, PROF_KEYGEN_COSET = 35,
-               PROF_KEYGEN_DOWNLOAD = 36 };
+               PROF_KEYGEN_DOWNLOAD = 36, PROF_KEYGEN_PACK = 37, PROF_KEYGEN_EXCLUSION = 38, PROF_KEYGEN_FIXED_UPLOAD = 39,
+               PROF_KEYGEN_COMBINATION = 40 };
 struct Profiler {
     bool enabled = false;
     std::vector<cudaEvent_t> ev;
@@ -216,6 +217,14 @@ int permutation_sigma_tables_run(DeviceCtx& ctx, uint32_t n_columns, uint32_t k,
 // sigma of `count` mapping columns (flat column index col0 + y for the status word), with the tables of the last permutation_sigma_tables_run
 int permutation_sigma_run(DeviceCtx& ctx, const void* const* d_mapping, uint32_t count, uint32_t col0, uint32_t n_columns, uint32_t k,
                           void* const* d_sigma, void* d_status, cudaStream_t stream);
+// selector activations: n bytes (0 / 1) -> selector_words(n) words, bit j of word w = row 32 w + j
+__host__ __device__ __forceinline__ size_t selector_words(size_t n) { return (n + 31) / 32; }
+int selector_pack_run(DeviceCtx& ctx, const void* d_activations, size_t n, void* d_bits, cudaStream_t stream);
+// d_flags (S x S u32, zeroed here): flags[i S + j] = 1 for j < i when bitsets i and j (S consecutive ones in d_bits) share a row
+int selector_exclusion_run(DeviceCtx& ctx, const void* d_bits, uint32_t n_selectors, size_t n, void* d_flags, cudaStream_t stream);
+// one combination column: d_members holds n_members (bitset slot in d_bits, root) u32 pairs; two members on one row raise d_status
+int combination_column_run(DeviceCtx& ctx, const void* d_bits, const void* d_members, uint32_t n_members, uint32_t combination, uint32_t k, void* d_out,
+                           void* d_status, cudaStream_t stream);
 // l0, l_last, l_active_row (d_cols[0..3), 2^extended_k elements each) of keygen_pk
 int keygen_indicators_run(DeviceCtx& ctx, uint32_t k, uint32_t extended_k, uint32_t blinding_factors, const uint64_t omega_inv[4],
                           const uint64_t ifft_divisor[4], const uint64_t extended_omega[4], const uint64_t zeta_powers[12], void* const* d_cols,

@@ -1,5 +1,6 @@
 // Key generation on the device: the σ columns of the permutation argument ([UP] halo2_proofs/src/plonk/permutation/keygen.rs
-// Assembly::build_vk / build_pk @ v2023_02_02) and the l_0 / l_last / l_active_row columns of keygen_pk ([UP] plonk/keygen.rs).
+// Assembly::build_vk / build_pk @ v2023_02_02), the l_0 / l_last / l_active_row columns of keygen_pk ([UP] plonk/keygen.rs), and
+// the exclusion matrix and combination columns of compress_selectors ([UP] plonk/circuit/compress_selectors.rs).
 //
 // σ_i[j] = δ^c · ω^r for (c, r) = mapping[i][j].  Upstream tabulates deltaomega[c][r] for every (c, r), P x n values; here the
 // exponent is split at h = ⌈k/2⌉: ω^r = ω^(r mod 2^h) · ω^(2^h ⌊r / 2^h⌋), and δ^c is folded into the high factor, so that
@@ -118,6 +119,119 @@ int keygen_indicators_run(DeviceCtx& ctx, uint32_t k, uint32_t extended_k, uint3
     H2B_CUDA(cudaGetLastError());
     H2B_TRY(lagrange_to_coeff_batch_run(ctx, d_cols, 3, k, omega_inv, ifft_divisor, stream));
     return coeff_to_extended_batch_run(ctx, d_cols, 3, k, extended_k, extended_omega, zeta_powers, stream);
+}
+
+// ---- selectors: compress_selectors' exclusion matrix and combination columns ([UP] plonk/circuit/compress_selectors.rs) --------
+// A selector's activations (Rust Vec<bool>: n bytes of 0 / 1) are packed into n / 32 words, bit j of word w = row 32 w + j.
+
+__device__ __forceinline__ uint32_t nonzero_bytes(uint32_t y) {
+    return ((y & 0xFFu) ? 1u : 0u) | ((y & 0xFF00u) ? 2u : 0u) | ((y & 0xFF0000u) ? 4u : 0u) | ((y & 0xFF000000u) ? 8u : 0u);
+}
+
+__global__ void __launch_bounds__(256) keygen_selector_pack_kernel(const uint8_t* __restrict__ act, size_t n, uint32_t* __restrict__ bits) {
+    const size_t w = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (w >= selector_words(n)) return;
+    uint32_t x = 0;
+    if (32 * (w + 1) <= n) {
+        const uint4* p = (const uint4*)(act + 32 * w);
+        const uint4 a = p[0], b = p[1];
+        const uint32_t y[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+#pragma unroll
+        for (int i = 0; i < 8; ++i) x |= nonzero_bytes(y[i]) << (4 * i);
+    } else {
+        for (size_t r = 32 * w; r < n; ++r) x |= (act[r] ? 1u : 0u) << (r - 32 * w);
+    }
+    bits[w] = x;
+}
+
+int selector_pack_run(DeviceCtx&, const void* d_activations, size_t n, void* d_bits, cudaStream_t stream) {
+    const size_t W = selector_words(n);
+    H2B_LAUNCH(keygen_selector_pack_kernel, (unsigned)((W + 255) / 256), 256, 0, stream, (const uint8_t*)d_activations, n, (uint32_t*)d_bits);
+    H2B_CUDA(cudaGetLastError());
+    return H2B_OK;
+}
+
+static const uint32_t EXCL_TILE = 64;     // selectors per side of a tile pair
+static const uint32_t EXCL_WORDS = 32;    // bitset words (1024 rows) per block
+
+// One block: a chunk of EXCL_WORDS words of the selectors of tile pair (ti, tj), ti >= tj (blockIdx.y = ti (ti + 1) / 2 + tj).  Each
+// word of every bitset is read from memory once per tile pair -- once in all when S <= 64 -- and thread (i, q) ORs a_i & a_j over the
+// chunk for the 16 selectors j = q, q + 4, ..; a pair that meets sets flags[i S + j] (i > j).
+__global__ void __launch_bounds__(256) keygen_selector_exclusion_kernel(const uint32_t* __restrict__ bits, uint32_t S, size_t W, uint32_t* flags) {
+    __shared__ uint32_t a[EXCL_TILE][EXCL_WORDS + 1], b[EXCL_TILE][EXCL_WORDS + 1];
+    const uint32_t p = blockIdx.y;
+    uint32_t ti = 0;
+    while ((ti + 1) * (ti + 2) / 2 <= p) ++ti;
+    const uint32_t tj = p - ti * (ti + 1) / 2;
+    const size_t w0 = (size_t)blockIdx.x * EXCL_WORDS;
+    for (uint32_t t = threadIdx.x; t < EXCL_TILE * EXCL_WORDS; t += blockDim.x) {
+        const uint32_t s = t / EXCL_WORDS, w = t % EXCL_WORDS;
+        const uint32_t si = ti * EXCL_TILE + s, sj = tj * EXCL_TILE + s;
+        const size_t ww = w0 + w;
+        a[s][w] = (si < S && ww < W) ? bits[(size_t)si * W + ww] : 0u;
+        b[s][w] = (sj < S && ww < W) ? bits[(size_t)sj * W + ww] : 0u;
+    }
+    __syncthreads();
+    const uint32_t i = threadIdx.x >> 2, q = threadIdx.x & 3;
+    uint32_t acc[EXCL_TILE / 4];
+#pragma unroll
+    for (uint32_t u = 0; u < EXCL_TILE / 4; ++u) acc[u] = 0;
+    for (uint32_t w = 0; w < EXCL_WORDS; ++w) {
+        const uint32_t x = a[i][w];
+#pragma unroll
+        for (uint32_t u = 0; u < EXCL_TILE / 4; ++u) acc[u] |= x & b[q + 4 * u][w];
+    }
+    const uint32_t gi = ti * EXCL_TILE + i;
+    if (gi >= S) return;
+#pragma unroll
+    for (uint32_t u = 0; u < EXCL_TILE / 4; ++u) {
+        const uint32_t gj = tj * EXCL_TILE + q + 4 * u;
+        uint32_t* f = flags + (size_t)gi * S + gj;
+        if (gj < gi && acc[u] && !*f) *f = 1;
+    }
+}
+
+int selector_exclusion_run(DeviceCtx&, const void* d_bits, uint32_t n_selectors, size_t n, void* d_flags, cudaStream_t stream) {
+    const size_t W = selector_words(n);
+    const uint32_t tiles = (n_selectors + EXCL_TILE - 1) / EXCL_TILE;
+    H2B_CUDA(cudaMemsetAsync(d_flags, 0, (size_t)n_selectors * n_selectors * 4, stream));
+    const dim3 grid((unsigned)((W + EXCL_WORDS - 1) / EXCL_WORDS), tiles * (tiles + 1) / 2);
+    H2B_LAUNCH(keygen_selector_exclusion_kernel, grid, 256, 0, stream, (const uint32_t*)d_bits, n_selectors, W, (uint32_t*)d_flags);
+    H2B_CUDA(cudaGetLastError());
+    return H2B_OK;
+}
+
+// out[j] = F::from(root_m) (Montgomery) for the member m active on row j, 0 on rows where none is.  Members are (bitset slot, root)
+// pairs.  A row where two members are active raises the status word to 1 + (combination << k) + j (saturated) and writes nothing.
+__global__ void __launch_bounds__(256) keygen_combination_kernel(const uint32_t* __restrict__ bits, size_t W, const uint2* __restrict__ members,
+                                                                 uint32_t n_members, uint32_t combination, uint32_t k, uint4* out, unsigned* status) {
+    const size_t j = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >> k) return;
+    uint32_t root = 0, hits = 0;
+    for (uint32_t m = 0; m < n_members; ++m) {
+        const uint2 e = members[m];
+        if ((bits[(size_t)e.x * W + (j >> 5)] >> (j & 31)) & 1u) { root = e.y; ++hits; }
+    }
+    if (hits > 1) {
+        const uint64_t flat = ((uint64_t)combination << k) + j + 1;
+        atomicMax(status, flat > 0xFFFFFFFFull ? 0xFFFFFFFFu : (unsigned)flat);
+        return;
+    }
+    Fr v = fp_zero<FR>();
+    if (root) {
+        v.l[0] = root;
+        v = fp_to_mont(v);
+    }
+    fp_store<FR>(out + 2 * j, v);
+}
+
+int combination_column_run(DeviceCtx&, const void* d_bits, const void* d_members, uint32_t n_members, uint32_t combination, uint32_t k, void* d_out,
+                           void* d_status, cudaStream_t stream) {
+    const size_t n = (size_t)1 << k;
+    H2B_LAUNCH(keygen_combination_kernel, (unsigned)((n + 255) / 256), 256, 0, stream, (const uint32_t*)d_bits, selector_words(n), (const uint2*)d_members,
+               n_members, combination, k, (uint4*)d_out, (unsigned*)d_status);
+    H2B_CUDA(cudaGetLastError());
+    return H2B_OK;
 }
 
 }  // namespace h2b

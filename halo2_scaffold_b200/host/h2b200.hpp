@@ -694,6 +694,116 @@ inline LagrangeIndicators lagrange_indicators(const poly::EvaluationDomain& doma
     check(h2b_memcpy_d2h(domain.device(), out.l_active_row.data(), d2.get(), en * sizeof(Fr)), "d2h");
     return out;
 }
+
+// compress_selectors (plonk/circuit/compress_selectors.rs process) and the fixed half of keygen_vk / keygen_pk.  A selector's
+// activations are one byte per row (Rust's Vec<bool> layout; std::vector<bool> is bit-packed, so it is not used).
+typedef std::vector<std::vector<uint8_t>> Activations;
+// per selector: its combination, its root and the combination's length -- the substitution is q * prod_{r = 1..len, r != root} (r - q)
+struct SelectorAssignment { std::vector<uint32_t> combination_of, root_of, len_of; uint32_t n_combinations = 0; };
+
+inline std::vector<const uint8_t*> activation_rows(const Activations& acts, size_t n) {
+    std::vector<const uint8_t*> rows;
+    for (const auto& a : acts) {
+        if (a.size() != n) throw Panic("compress_selectors: activations length != 2^k");
+        rows.push_back(a.data());
+    }
+    return rows;
+}
+// process over selectors of these gate degrees (0: in no gate polynomial) against max_degree = cs.degree(); the exclusion matrix comes
+// from the device, the greedy step is upstream's
+inline SelectorAssignment compress_selectors(const Activations& acts, const std::vector<uint32_t>& degrees, uint32_t max_degree, uint32_t k) {
+    ensure_init();
+    const size_t S = acts.size();
+    if (degrees.size() != S) throw Panic("compress_selectors: one degree per selector");
+    SelectorAssignment a;
+    a.combination_of.assign(S, 0); a.root_of.assign(S, 0); a.len_of.assign(S, 0);
+    std::vector<uint32_t> simple;
+    for (uint32_t s = 0; s < S; ++s) {
+        if (degrees[s] != 0) { simple.push_back(s); continue; }
+        a.combination_of[s] = a.n_combinations++; a.root_of[s] = 1; a.len_of[s] = 1;
+    }
+    const auto all_rows = activation_rows(acts, (size_t)1 << k);
+    const size_t m = simple.size();
+    std::vector<uint8_t> excl(m * m);
+    std::vector<const uint8_t*> rows;
+    for (uint32_t s : simple) rows.push_back(all_rows[s]);
+    if (m) check(h2b_selector_exclusion(rows.data(), (uint32_t)m, k, excl.data()), "compress_selectors: exclusion matrix");
+    std::vector<bool> added(m, false);
+    for (size_t i = 0; i < m; ++i) {
+        if (added[i]) continue;
+        added[i] = true;
+        if (degrees[simple[i]] > max_degree) throw Panic("compress_selectors: selector degree above max_degree");
+        size_t d = degrees[simple[i]] - 1;
+        std::vector<size_t> comb{i};
+        for (size_t j = i + 1; j < m; ++j) {
+            if (d + comb.size() == max_degree) break;
+            if (added[j]) continue;
+            bool excluded = false;
+            for (size_t x : comb) excluded = excluded || excl[j * m + x];
+            if (excluded) continue;
+            const size_t new_d = std::max(d, (size_t)degrees[simple[j]] - 1);
+            if (new_d + comb.size() + 1 > max_degree) continue;
+            d = new_d;
+            comb.push_back(j);
+            added[j] = true;
+        }
+        for (size_t t = 0; t < comb.size(); ++t) {
+            const uint32_t s = simple[comb[t]];
+            a.combination_of[s] = a.n_combinations; a.root_of[s] = (uint32_t)(t + 1); a.len_of[s] = (uint32_t)comb.size();
+        }
+        ++a.n_combinations;
+    }
+    return a;
+}
+
+inline std::vector<const uint64_t*> fixed_columns_of(const std::vector<std::vector<Fr>>& fixed, size_t n) {
+    std::vector<const uint64_t*> cols;
+    for (const auto& c : fixed) {
+        if (c.size() != n) throw Panic("keygen: fixed column length != 2^k");
+        cols.push_back(reinterpret_cast<const uint64_t*>(c.data()));
+    }
+    return cols;
+}
+// keygen_vk's fixed_commitments: commit_lagrange of each fixed column, then of each combination column
+inline std::vector<G1> fixed_build_vk(const poly::kzg::ParamsKZG& params, const poly::EvaluationDomain& domain, const std::vector<std::vector<Fr>>& fixed,
+                                      const Activations& acts, const SelectorAssignment& a) {
+    ensure_init();
+    const size_t n = (size_t)1 << domain.k();
+    const auto cols = fixed_columns_of(fixed, n);
+    const auto rows = activation_rows(acts, n);
+    std::vector<G1> out(cols.size() + a.n_combinations);
+    check(h2b_keygen_fixed_build_vk(cols.data(), (uint32_t)cols.size(), rows.data(), (uint32_t)rows.size(), a.combination_of.data(), a.root_of.data(),
+                                    a.n_combinations, domain.k(), params.g_lagrange_handle(), reinterpret_cast<uint64_t*>(out.data())),
+          "keygen::fixed_build_vk");
+    return out;
+}
+// keygen_pk's fixed columns: the combination columns in Lagrange form (fixed_values = fixed ++ these), and fixed_polys / fixed_cosets
+// of every column
+struct FixedProvingKey { std::vector<std::vector<Fr>> combination_values, polys, cosets; };
+inline FixedProvingKey fixed_build_pk(const poly::kzg::ParamsKZG&, const poly::EvaluationDomain& domain, const std::vector<std::vector<Fr>>& fixed,
+                                      const Activations& acts, const SelectorAssignment& a) {
+    ensure_init();
+    const size_t n = (size_t)1 << domain.k();
+    const auto cols = fixed_columns_of(fixed, n);
+    const auto rows = activation_rows(acts, n);
+    FixedProvingKey pk;
+    std::vector<uint64_t*> v, p, e;
+    for (uint32_t c = 0; c < a.n_combinations; ++c) {
+        pk.combination_values.emplace_back(n);
+        v.push_back(reinterpret_cast<uint64_t*>(pk.combination_values.back().data()));
+    }
+    for (size_t i = 0; i < cols.size() + a.n_combinations; ++i) {
+        pk.polys.emplace_back(n); pk.cosets.emplace_back(domain.extended_len());
+        p.push_back(reinterpret_cast<uint64_t*>(pk.polys.back().data()));
+        e.push_back(reinterpret_cast<uint64_t*>(pk.cosets.back().data()));
+    }
+    const Fr z[3] = {fr::one(), domain.get_g_coset(), domain.get_g_coset_inv()};
+    check(h2b_keygen_fixed_build_pk(cols.data(), (uint32_t)cols.size(), rows.data(), (uint32_t)rows.size(), a.combination_of.data(), a.root_of.data(),
+                                    a.n_combinations, domain.k(), domain.extended_k(), domain.get_omega_inv().l, domain.get_ifft_divisor().l,
+                                    domain.get_extended_omega().l, z[0].l, v.data(), p.data(), e.data()),
+          "keygen::fixed_build_pk");
+    return pk;
+}
 }  // namespace keygen
 
 namespace lookup {

@@ -399,6 +399,37 @@ int h2b_permutation_build_pk(const uint64_t* const* mapping, uint32_t n_columns,
                              const uint64_t omega[4], const uint64_t omega_inv[4], const uint64_t ifft_divisor[4], const uint64_t extended_omega[4],
                              const uint64_t zeta_powers[12], uint64_t* const* out_permutations, uint64_t* const* out_polys, uint64_t* const* out_cosets);
 
+/* ---- key generation: compress_selectors and the fixed columns of keygen_vk / keygen_pk -------------------------------------------
+ * [UP] halo2_proofs/src/plonk/circuit/compress_selectors.rs (process) and plonk/keygen.rs.  A selector's activations are upstream's
+ * Vec<bool> as it sits in memory: n = 2^k bytes, a non-zero byte is an active row.  An assignment gives each selector s a combination
+ * combination_of[s] < n_combinations and a root root_of[s] > 0; combination column c holds F::from(root_of[s]) (Montgomery form) on
+ * the rows where its member s is active and zero on every other row -- what process fills -- so no two members of a combination may
+ * be active on one row.  n_selectors is at most 2^14. */
+/* out (n_selectors x n_selectors bytes, row-major): out[i][j] = 1 when selectors i and j are both active on some row, else 0; symmetric,
+ * zero diagonal -- process's exclusion matrix.  activations[s] may be pageable.  Synchronous.  k > 28, more than 2^14 selectors and
+ * null pointers fail with H2B_ERR_BAD_ARGUMENT before anything is written; n_selectors = 0 writes nothing. */
+int h2b_selector_exclusion(const uint8_t* const* activations, uint32_t n_selectors, uint32_t k, uint8_t* out);
+/* keygen_vk's fixed commitments: out_commitments[12 i ..] = commit_lagrange(column i) (Jacobian) over the registered set
+ * handle_g_lagrange (replicated or sharded, at least n points), for the n_fixed caller columns fixed[i] (n x 32 B Montgomery, pageable
+ * is fine) and then the n_combinations combination columns -- upstream's order, fixed.extend(selector_polys).  n_fixed = 0 or
+ * n_selectors = 0 are fine, both n_fixed = n_combinations = 0 is not.  Columns go round-robin over the devices as in
+ * h2b_permutation_build_vk; each device uploads and packs the selectors of its combinations once.  Synchronous.  k > 28, null
+ * pointers, a combination index >= n_combinations, a root of 0, a combination no selector uses, an unknown handle, a set shorter than n
+ * and two members of one combination active on one row fail with H2B_ERR_BAD_ARGUMENT and leave out_commitments untouched. */
+int h2b_keygen_fixed_build_vk(const uint64_t* const* fixed, uint32_t n_fixed, const uint8_t* const* activations, uint32_t n_selectors,
+                              const uint32_t* combination_of, const uint32_t* root_of, uint32_t n_combinations, uint32_t k, uint64_t handle_g_lagrange,
+                              uint64_t* out_commitments);
+/* keygen_pk's fixed columns: out_combination_values[c] = combination column c (n x 32 B; the caller holds its fixed columns), and for
+ * all n_fixed + n_combinations columns i in the order of h2b_keygen_fixed_build_vk out_polys[i] = lagrange_to_coeff(column i) (n x 32 B)
+ * and out_cosets[i] = coeff_to_extended(out_polys[i]) (2^extended_k x 32 B), with the constants of h2b_lagrange_to_coeff_dev_batch /
+ * h2b_coeff_to_extended_dev_batch.  Any of the three arrays may be NULL.  Refuses what h2b_keygen_fixed_build_vk refuses, and
+ * extended_k < k or > 28; every combination column is built and checked before any caller memory is written, so a refused call leaves
+ * every output untouched.  Synchronous. */
+int h2b_keygen_fixed_build_pk(const uint64_t* const* fixed, uint32_t n_fixed, const uint8_t* const* activations, uint32_t n_selectors,
+                              const uint32_t* combination_of, const uint32_t* root_of, uint32_t n_combinations, uint32_t k, uint32_t extended_k,
+                              const uint64_t omega_inv[4], const uint64_t ifft_divisor[4], const uint64_t extended_omega[4], const uint64_t zeta_powers[12],
+                              uint64_t* const* out_combination_values, uint64_t* const* out_polys, uint64_t* const* out_cosets);
+
 /* ---- raw device memory helpers (so that non-CUDA hosts -- ctypes, Rust -- can hold device buffers) --- */
 int h2b_dev_alloc(int device, size_t bytes, void** out);
 int h2b_dev_free(int device, void* p);
@@ -446,7 +477,9 @@ unsigned long long h2b_launch_count(void);
  * k of them), 30 normalisation (batch inversion and the affine finish);  h2b_permutation_build_vk / h2b_permutation_build_pk tags
  * (per column or group of columns): 31 mapping upload, 32 sigma kernel (the first also builds the twiddle tables), 33 commitments,
  * 34 inverse NTTs (lagrange_to_coeff), 35 coset NTTs (coeff_to_extended), 36 downloads; the MSM / NTT tags recorded inside a phase
- * belong to the keygen tag that follows them. */
+ * belong to the keygen tag that follows them;  h2b_selector_exclusion and h2b_keygen_fixed_build_vk / _pk add 37 selector uploads
+ * and packing (all selectors of the call or device at once), 38 exclusion kernel, 39 fixed column upload, 40 combination column
+ * kernel, with 33 - 36 as above. */
 int h2b_profile_enable(int device, int on);
 int h2b_profile_read(int device, int* tags, float* ms, int cap, int* count);
 /* force the MSM window size (0 = automatic) -- tuning / tests only */

@@ -117,6 +117,14 @@ extern "C" {
     pub fn h2b_permutation_build_pk(mapping: *const *const u64, n_columns: u32, k: u32, extended_k: u32, delta: *const u64, omega: *const u64,
                                     omega_inv: *const u64, ifft_divisor: *const u64, extended_omega: *const u64, zeta_powers: *const u64,
                                     out_permutations: *const *mut u64, out_polys: *const *mut u64, out_cosets: *const *mut u64) -> c_int;
+    // compress_selectors' exclusion matrix and the fixed columns of keygen_vk / keygen_pk
+    pub fn h2b_selector_exclusion(activations: *const *const u8, n_selectors: u32, k: u32, out: *mut u8) -> c_int;
+    pub fn h2b_keygen_fixed_build_vk(fixed: *const *const u64, n_fixed: u32, activations: *const *const u8, n_selectors: u32, combination_of: *const u32,
+                                     root_of: *const u32, n_combinations: u32, k: u32, handle_g_lagrange: u64, out_commitments: *mut u64) -> c_int;
+    pub fn h2b_keygen_fixed_build_pk(fixed: *const *const u64, n_fixed: u32, activations: *const *const u8, n_selectors: u32, combination_of: *const u32,
+                                     root_of: *const u32, n_combinations: u32, k: u32, extended_k: u32, omega_inv: *const u64, ifft_divisor: *const u64,
+                                     extended_omega: *const u64, zeta_powers: *const u64, out_combination_values: *const *mut u64,
+                                     out_polys: *const *mut u64, out_cosets: *const *mut u64) -> c_int;
     pub fn h2b_dev_alloc(device: c_int, bytes: usize, out: *mut *mut c_void) -> c_int;
     pub fn h2b_dev_free(device: c_int, p: *mut c_void) -> c_int;
     pub fn h2b_memcpy_h2d(device: c_int, d_dst: *mut c_void, h_src: *const c_void, bytes: usize) -> c_int;
@@ -310,4 +318,82 @@ pub fn keygen_lagrange_indicators(dom: &KeygenDomain, blinding_factors: u32) -> 
         panic!("keygen_pk indicators failed: {}", last_error());
     }
     out
+}
+
+/// compress_selectors' assignment: per selector its combination (the index of the fixed column `process` allocates for it, counted
+/// from the first one) and its root; `n_combinations` columns in all.
+pub struct SelectorAssignment {
+    pub combination_of: Vec<u32>,
+    pub root_of: Vec<u32>,
+    pub n_combinations: u32,
+}
+
+/// Rust's `bool` is one byte, 0 or 1: a `Vec<bool>` goes to the C ABI as it sits in memory.
+fn activation_rows(activations: &[Vec<bool>], n: usize) -> Vec<*const u8> {
+    activations.iter().map(|a| {
+        assert_eq!(a.len(), n, "selector activations length != 2^k");
+        a.as_ptr() as *const u8
+    }).collect()
+}
+
+fn fixed_rows(fixed: &[&[[u64; 4]]], n: usize) -> Vec<*const u64> {
+    fixed.iter().map(|c| {
+        assert_eq!(c.len(), n, "fixed column length != 2^k");
+        c.as_ptr() as *const u64
+    }).collect()
+}
+
+/// `process`'s exclusion matrix: `out[i][j]` is true when selectors i and j are both active on some row (symmetric, false on the
+/// diagonal).
+pub fn selector_exclusion(activations: &[Vec<bool>], k: u32) -> Vec<Vec<bool>> {
+    ensure_init();
+    let s = activations.len();
+    let rows = activation_rows(activations, 1usize << k);
+    let mut out = vec![0u8; s * s];
+    let rc = unsafe { h2b_selector_exclusion(rows.as_ptr(), s as u32, k, out.as_mut_ptr()) };
+    if rc != 0 {
+        panic!("h2b_selector_exclusion failed ({rc}): {}", last_error());
+    }
+    out.chunks(s.max(1)).take(s).map(|r| r.iter().map(|&b| b != 0).collect()).collect()
+}
+
+/// keygen_vk's `fixed_commitments`: `commit_lagrange` (Jacobian, 12 u64) of each fixed column, then of each combination column.
+pub fn keygen_fixed_build_vk(fixed: &[&[[u64; 4]]], activations: &[Vec<bool>], a: &SelectorAssignment, k: u32, handle_g_lagrange: u64) -> Vec<[u64; 12]> {
+    ensure_init();
+    let n = 1usize << k;
+    let (f, rows) = (fixed_rows(fixed, n), activation_rows(activations, n));
+    let mut out = vec![[0u64; 12]; fixed.len() + a.n_combinations as usize];
+    let rc = unsafe {
+        h2b_keygen_fixed_build_vk(f.as_ptr(), f.len() as u32, rows.as_ptr(), rows.len() as u32, a.combination_of.as_ptr(), a.root_of.as_ptr(),
+                                  a.n_combinations, k, handle_g_lagrange, out.as_mut_ptr() as *mut u64)
+    };
+    if rc != 0 {
+        panic!("h2b_keygen_fixed_build_vk failed ({rc}): {}", last_error());
+    }
+    out
+}
+
+/// keygen_pk's fixed columns: the combination columns (Lagrange), and the coefficients and extended cosets of every fixed and
+/// combination column, as Montgomery scalars.
+#[allow(clippy::type_complexity)]
+pub fn keygen_fixed_build_pk(fixed: &[&[[u64; 4]]], activations: &[Vec<bool>], a: &SelectorAssignment, dom: &KeygenDomain)
+    -> (Vec<Vec<[u64; 4]>>, Vec<Vec<[u64; 4]>>, Vec<Vec<[u64; 4]>>) {
+    ensure_init();
+    let n = 1usize << dom.k;
+    let (f, rows) = (fixed_rows(fixed, n), activation_rows(activations, n));
+    let total = fixed.len() + a.n_combinations as usize;
+    let mut values = vec![vec![[0u64; 4]; n]; a.n_combinations as usize];
+    let mut polys = vec![vec![[0u64; 4]; n]; total];
+    let mut cosets = vec![vec![[0u64; 4]; 1usize << dom.extended_k]; total];
+    let outs = |v: &mut Vec<Vec<[u64; 4]>>| v.iter_mut().map(|c| c.as_mut_ptr() as *mut u64).collect::<Vec<_>>();
+    let (v, p, e) = (outs(&mut values), outs(&mut polys), outs(&mut cosets));
+    let rc = unsafe {
+        h2b_keygen_fixed_build_pk(f.as_ptr(), f.len() as u32, rows.as_ptr(), rows.len() as u32, a.combination_of.as_ptr(), a.root_of.as_ptr(),
+                                  a.n_combinations, dom.k, dom.extended_k, dom.omega_inv.as_ptr(), dom.ifft_divisor.as_ptr(), dom.extended_omega.as_ptr(),
+                                  dom.zeta_powers.as_ptr() as *const u64, v.as_ptr(), p.as_ptr(), e.as_ptr())
+    };
+    if rc != 0 {
+        panic!("h2b_keygen_fixed_build_pk failed ({rc}): {}", last_error());
+    }
+    (values, polys, cosets)
 }

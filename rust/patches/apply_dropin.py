@@ -11,6 +11,9 @@ Turns a checkout of halo2_proofs (PSE tag v2023_02_02 or axiom-crypto branch axi
     `Assembly::build_vk` / `build_pk` and around keygen_pk's l0 / l_blind / l_last block, and the defaulted
     `Params::h2b_g_lagrange_handle` that `ParamsKZG<Bn256>` overrides.  Each substitution is asserted, and so is upstream's
     `mapping: Vec<Vec<(usize, usize)>>` layout of `Assembly`;
+  * src/plonk/circuit/compress_selectors.rs, src/plonk/circuit.rs, src/plonk/keygen.rs: the fixed-column keygen drop-in
+    (rust/patches/fixed_keygen_dropin.rs): `process_h2b`, a copy of `ConstraintSystem::compress_selectors` that calls it, and G1Affine
+    dispatches around keygen_vk's fixed commitments and keygen_pk's fixed values / polys / cosets.  Each substitution is asserted;
   * Cargo.toml: `h2b200-sys = { path = ".../rust/h2b200-sys" }` is added to [dependencies].
 Idempotent.  Not run in the build container (no Rust sources of halo2_proofs are available there)."""
 import pathlib
@@ -84,6 +87,46 @@ if "fn h2b_g_lagrange_handle" not in kzg.read_text():
                "\\1\n    fn h2b_g_lagrange_handle(&self) -> Option<u64> {\n"
                "        if TypeId::of::<E>() == TypeId::of::<Bn256>() { Some(self.handle_g_lagrange) } else { None }\n    }",
                "impl Params for ParamsKZG", re.S)
+# compress_selectors and the fixed columns of keygen_vk / keygen_pk (rust/patches/fixed_keygen_dropin.rs, whose header states the mechanism)
+fixed_dropin = (rust / "patches" / "fixed_keygen_dropin.rs").read_text()
+process_part, keygen_part = fixed_dropin.split("// ---- keygen.rs ----", 1)
+compress = crate / "src" / "plonk" / "circuit" / "compress_selectors.rs"
+if "process_h2b" not in compress.read_text():
+    assert re.search(r"\bpub fn process<F: FieldExt, E>\(", compress.read_text()), "compress_selectors::process not found in %s" % compress
+    compress.write_text(compress.read_text() + "\n// ---- libh2b200 drop-in (rust/patches/fixed_keygen_dropin.rs) ----\n" + process_part + "\n")
+circuit = crate / "src" / "plonk" / "circuit.rs"
+if "compress_selectors_h2b" not in circuit.read_text():
+    text = circuit.read_text()
+    m = re.search(r"\n(    pub\(crate\) fn compress_selectors\(mut self, selectors: Vec<Vec<bool>>\) -> \(Self, Vec<Vec<F>>\) \{.*?\n    \})\n", text, re.S)
+    assert m, "ConstraintSystem::compress_selectors not found in %s" % circuit
+    body = m.group(1)
+    assert body.count("compress_selectors::process(") == 1, "compress_selectors does not call process exactly once"
+    copy = body.replace("fn compress_selectors(", "fn compress_selectors_h2b(", 1).replace("-> (Self, Vec<Vec<F>>)", "-> (Self, h2b200_sys::SelectorAssignment)", 1)
+    copy = copy.replace("compress_selectors::process(", "compress_selectors::process_h2b(", 1)
+    circuit.write_text(text[:m.end(1)] + "\n\n    // libh2b200: upstream's body above with process -> process_h2b (rust/patches/fixed_keygen_dropin.rs)\n" + copy + text[m.end(1):])
+if "fixed_keygen_h2b" not in keygen.read_text():
+    # keygen_vk: the assignment instead of the filled columns, and the fixed commitments from the device
+    substitute(keygen, r"(let \(cs, selector_polys\) = cs\.compress_selectors\(assembly\.selectors\);\s*fixed\.extend\(\s*selector_polys\s*\.into_iter\(\)\s*"
+               r"\.map\(\|poly\| domain\.lagrange_from_vec\(poly\)\),?\s*\);)",
+               "let h2b_handle = if TypeId::of::<C>() == TypeId::of::<G1Affine>() { params.h2b_g_lagrange_handle() } else { None };\n"
+               "    let (cs, h2b_fixed_commitments) = if let Some(h) = h2b_handle {\n"
+               "        let (cs, assignment) = cs.compress_selectors_h2b(assembly.selectors.clone());\n"
+               "        let com = fixed_commitments_h2b::<C>(&fixed, &assembly.selectors, &assignment, params.k(), h);\n"
+               "        (cs, Some(com))\n"
+               "    } else {\n    \\1\n    (cs, None)\n    };", "keygen_vk's compress_selectors", re.S)
+    substitute(keygen, r"(let fixed_commitments = )(fixed\s*\.iter\(\)\s*\.map\(\|poly\| params\.commit_lagrange\(poly, Blind::default\(\)\)\.to_affine\(\)\)\s*\.collect\(\));",
+               "\\1h2b_fixed_commitments.unwrap_or_else(|| \\2);", "keygen_vk's fixed_commitments", re.S)
+    # keygen_pk: fixed_values, fixed_polys and fixed_cosets from the device
+    substitute(keygen, r"(let \(cs, selector_polys\) = cs\.compress_selectors\(assembly\.selectors\.clone\(\)\);\s*fixed\.extend\(\s*selector_polys\s*\.into_iter\(\)\s*"
+               r"\.map\(\|poly\| vk\.domain\.lagrange_from_vec\(poly\)\),?\s*\);\s*"
+               r"let fixed_polys: Vec<_> = fixed\s*\.iter\(\)\s*\.map\(\|poly\| vk\.domain\.lagrange_to_coeff\(poly\.clone\(\)\)\)\s*\.collect\(\);\s*"
+               r"let fixed_cosets = fixed_polys\s*\.iter\(\)\s*\.map\(\|poly\| vk\.domain\.coeff_to_extended\(poly\.clone\(\)\)\)\s*\.collect\(\);)",
+               "let (cs, fixed, fixed_polys, fixed_cosets) = if TypeId::of::<C>() == TypeId::of::<G1Affine>() {\n"
+               "        let (cs, assignment) = cs.compress_selectors_h2b(assembly.selectors.clone());\n"
+               "        let (fixed, fixed_polys, fixed_cosets) = fixed_keygen_h2b(fixed, &assembly.selectors, &assignment, &vk.domain);\n"
+               "        (cs, fixed, fixed_polys, fixed_cosets)\n"
+               "    } else {\n    \\1\n    (cs, fixed, fixed_polys, fixed_cosets)\n    };", "keygen_pk's fixed columns", re.S)
+    keygen.write_text(keygen.read_text() + "\n// ---- libh2b200 drop-in (rust/patches/fixed_keygen_dropin.rs) ----\n" + keygen_part + "\n")
 toml = crate / "Cargo.toml"
 t = toml.read_text()
 if "h2b200-sys" not in t:

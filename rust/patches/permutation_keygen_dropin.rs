@@ -24,7 +24,7 @@
 // refuses a halo2_proofs whose Assembly holds another mapping type.  The l0 / l_blind / l_last block of keygen_pk is replaced by
 // `keygen_indicators_h2b` below (plonk/keygen.rs), by the same TypeId dispatch.
 
-fn h2b_domain<F: ff::PrimeField>(domain: &EvaluationDomain<F>) -> h2b200_sys::KeygenDomain {
+pub(crate) fn h2b_domain<F: ff::PrimeField>(domain: &EvaluationDomain<F>) -> h2b200_sys::KeygenDomain {
     // F == halo2curves::bn256::Fr here (checked through TypeId by every caller): Montgomery limbs, plain old data
     let w = |x: &F| unsafe { std::mem::transmute_copy::<F, [u64; 4]>(x) };
     let n = F::from(1u64 << domain.k());
@@ -44,7 +44,7 @@ fn h2b_delta<F: ff::PrimeField>() -> [u64; 4] {
     unsafe { std::mem::transmute_copy::<F, [u64; 4]>(&F::DELTA) }
 }
 
-fn h2b_columns<F: Copy>(v: Vec<[u64; 4]>) -> Vec<F> {
+pub(crate) fn h2b_columns<F: Copy>(v: Vec<[u64; 4]>) -> Vec<F> {
     // F == Fr: 32 bytes of Montgomery limbs per element
     v.iter().map(|x| unsafe { std::mem::transmute_copy::<[u64; 4], F>(x) }).collect()
 }
