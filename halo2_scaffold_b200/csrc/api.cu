@@ -178,6 +178,40 @@ static DeviceCtx* pick_device(std::unique_lock<std::mutex>& lock_out, size_t* in
     return c;
 }
 
+// fn(d) for every device index d in `devs`: on the calling thread when there is one, on one thread per device otherwise.  Returns
+// the first failure in list order, its message prefixed with "device d: ".
+static int on_devices(const std::vector<size_t>& devs, const std::function<int(size_t)>& fn) {
+    const size_t m = devs.size();
+    std::vector<int> rcs(m, 0);
+    std::vector<std::string> errs(m);
+    auto run = [&](size_t i) { rcs[i] = fn(devs[i]); if (rcs[i]) errs[i] = get_error(); };
+    if (m == 1) {
+        run(0);
+    } else {
+        std::vector<std::thread> th;
+        for (size_t i = 0; i < m; ++i) th.emplace_back(run, i);
+        for (auto& t : th) t.join();
+    }
+    for (size_t i = 0; i < m; ++i) if (rcs[i]) { set_error("device %zu: %s", devs[i], errs[i].c_str()); return rcs[i]; }
+    return H2B_OK;
+}
+static std::vector<size_t> first_devices(size_t m) {
+    std::vector<size_t> devs(m);
+    for (size_t d = 0; d < m; ++d) devs[d] = d;
+    return devs;
+}
+
+// every device allocation of this file.  A failed cudaMalloc stays the thread's last error, which the next launch check on this
+// thread would report as its own: it is cleared here.
+static int dev_malloc(void** p, size_t bytes, const char* what) {
+    const cudaError_t e = cudaMalloc(p, bytes);
+    if (e == cudaSuccess) return H2B_OK;
+    cudaGetLastError();
+    *p = nullptr;
+    set_error("cudaMalloc of %zu bytes for %s failed: %s", bytes, what, cudaGetErrorString(e));
+    return H2B_ERR_OOM;
+}
+
 // ---- content digests of host arrays (implicit cache) --------------------------------------------------------------------
 // best_multiexp is a pure function of its arguments: a device copy may only be reused if the caller's array still holds exactly
 // what was uploaded.  Every block of digest_block() points gets a 128-bit digest (multiply-fold over 64-bit words, four
@@ -238,21 +272,39 @@ static bool digest_blocks(const uint64_t* bases, size_t b0, size_t b1, uint64_t*
 }
 
 // ---- building resident sets ------------------------------------------------------------------------------------------------
-static void layout_rows(size_t n, bool sharded, std::vector<size_t>& lo, std::vector<size_t>& rows) {
+// a set of n points laid out over every device, nothing allocated yet
+static SetRef new_set(size_t n, bool sharded) {
     const size_t nd = G.devs.size();
-    lo.assign(nd, 0);
-    rows.assign(nd, n);
-    if (!sharded) return;
-    for (size_t d = 0; d < nd; ++d) { lo[d] = n * d / nd; rows[d] = n * (d + 1) / nd - lo[d]; }
+    SetRef bs(new BaseSet());
+    bs->n = n;
+    bs->sharded = sharded;
+    bs->lo.assign(nd, 0);
+    bs->rows.assign(nd, n);
+    if (sharded)
+        for (size_t d = 0; d < nd; ++d) { bs->lo[d] = n * d / nd; bs->rows[d] = n * (d + 1) / nd - bs->lo[d]; }
+    for (size_t d = 0; d < nd; ++d) bs->ordinal.push_back(G.devs[d]->device);
+    bs->dev.assign(nd, nullptr);
+    return bs;
 }
 
 static SetRef new_set_like(const BaseSet& src) {
-    SetRef bs(new BaseSet());
-    bs->handle = src.handle; bs->implicit = src.implicit; bs->host_ptr = src.host_ptr; bs->n = src.n; bs->digest = src.digest;
-    bs->last_use = src.last_use; bs->uses = src.uses; bs->sharded = src.sharded; bs->refs = src.refs;
-    bs->lo = src.lo; bs->rows = src.rows; bs->ordinal = src.ordinal;
-    bs->dev.assign(src.dev.size(), nullptr);
+    SetRef bs = new_set(src.n, src.sharded);
+    bs->handle = src.handle; bs->implicit = src.implicit; bs->host_ptr = src.host_ptr; bs->digest = src.digest;
+    bs->last_use = src.last_use; bs->uses = src.uses; bs->refs = src.refs;
     return bs;
+}
+
+// device 0's rows of a replicated set -> every other device, one peer copy each
+static int replicate_device0(BaseSet& bs) {
+    for (size_t d = 1; d < G.devs.size(); ++d) {
+        DeviceCtx& c = *G.devs[d];
+        std::lock_guard<std::mutex> lk(c.mu);
+        H2B_CUDA(cudaSetDevice(c.device));
+        H2B_TRY(dev_malloc(&bs.dev[d], bs.n * 64 + 64, "SRS bases"));
+        const cudaError_t e = cudaMemcpyPeer(bs.dev[d], c.device, bs.dev[0], G.devs[0]->device, bs.n * 64);
+        if (e != cudaSuccess) { set_error("device %zu: peer copy of SRS bases: %s", d, cudaGetErrorString(e)); return H2B_ERR_CUDA; }
+    }
+    return H2B_OK;
 }
 
 // The table set of msm.cu step 0 for a resident point set (table 0 = the points themselves) as a NEW set; the source stays
@@ -294,7 +346,7 @@ static SetRef build_tables(const SetRef& src) {
         const size_t R = src->rows[d];
         if (R == 0) continue;
         cudaSetDevice(c.device);
-        if (cudaMalloc(&out->dev[d], (size_t)nt * R * 64 + 64) != cudaSuccess) { cudaGetLastError(); out->dev[d] = nullptr; ok = false; break; }
+        if (dev_malloc(&out->dev[d], (size_t)nt * R * 64 + 64, "window tables") != H2B_OK) { ok = false; break; }
         const size_t r0 = gather ? R * d / nd : 0, r1 = gather ? R * (d + 1) / nd : R;
         c.prof.mark(PROF_BEGIN, c.stream);
         if (cudaMemcpyAsync(out->dev[d], src->dev[d], R * 64, cudaMemcpyDeviceToDevice, c.stream) != cudaSuccess) ok = false;
@@ -332,45 +384,21 @@ static SetRef build_tables(const SetRef& src) {
 
 // upload `bases` (host) as a new resident set
 static int create_set(const uint64_t* bases, size_t n, bool sharded, bool with_tables, SetRef* out) {
-    const size_t nd = G.devs.size();
-    SetRef bs(new BaseSet());
-    bs->n = n;
-    bs->sharded = sharded && nd > 1;
-    layout_rows(n, bs->sharded, bs->lo, bs->rows);
-    bs->dev.assign(nd, nullptr);
-    for (size_t d = 0; d < nd; ++d) bs->ordinal.push_back(G.devs[d]->device);
-    for (size_t d = 0; d < nd; ++d) {
-        if (bs->rows[d] == 0) continue;
-        H2B_CUDA(cudaSetDevice(G.devs[d]->device));
-        cudaError_t e = cudaMalloc(&bs->dev[d], bs->rows[d] * 64 + 64);
-        if (e != cudaSuccess) { cudaGetLastError(); set_error("cudaMalloc of %zu bytes for SRS bases failed: %s", bs->rows[d] * 64, cudaGetErrorString(e)); return H2B_ERR_OOM; }
-    }
-    std::vector<int> rcs(nd, 0);
-    std::vector<std::string> errs(nd);
-    auto upload_one = [&](size_t d) {
+    SetRef bs = new_set(n, sharded && G.devs.size() > 1);
+    // sharded: disjoint slices, one upload per device, concurrently (each over its own PCIe link).  Replicated: one trip over PCIe
+    // to device 0, then peer copies: D concurrent uploads of the same host array only fight for the host's memory
+    std::vector<size_t> devs;
+    for (size_t d = 0; d < (bs->sharded ? G.devs.size() : 1); ++d) if (bs->rows[d]) devs.push_back(d);
+    H2B_TRY(on_devices(devs, [&](size_t d) -> int {
         DeviceCtx& c = *G.devs[d];
         std::lock_guard<std::mutex> lk(c.mu);
-        if (cudaSetDevice(c.device) != cudaSuccess) { rcs[d] = H2B_ERR_CUDA; return; }
-        rcs[d] = host_upload(c, bs->dev[d], bases + 8 * bs->lo[d], bs->rows[d] * 64, c.stream);
-        if (!rcs[d] && cudaStreamSynchronize(c.stream) != cudaSuccess) { set_error("SRS upload: %s", cudaGetErrorString(cudaGetLastError())); rcs[d] = H2B_ERR_CUDA; }
-        if (rcs[d]) errs[d] = get_error();
-    };
-    if (bs->sharded) {
-        // disjoint slices: one upload per device, concurrently (each over its own PCIe link)
-        std::vector<std::thread> th;
-        for (size_t d = 0; d < nd; ++d) if (bs->rows[d]) th.emplace_back(upload_one, d);
-        for (auto& t : th) t.join();
-    } else {
-        // one trip over PCIe, then peer copies: D concurrent uploads of the same host array only fight for the host's memory
-        upload_one(0);
-        for (size_t d = 1; d < nd && !rcs[0]; ++d) {
-            std::lock_guard<std::mutex> lk(G.devs[d]->mu);
-            cudaError_t e = cudaSetDevice(G.devs[d]->device);
-            if (e == cudaSuccess) e = cudaMemcpyPeer(bs->dev[d], G.devs[d]->device, bs->dev[0], G.devs[0]->device, n * 64);
-            if (e != cudaSuccess) { set_error("peer copy of SRS bases: %s", cudaGetErrorString(e)); rcs[d] = H2B_ERR_CUDA; errs[d] = get_error(); }
-        }
-    }
-    for (size_t d = 0; d < nd; ++d) if (rcs[d]) { set_error("device %zu: %s", d, errs[d].c_str()); return rcs[d]; }
+        H2B_CUDA(cudaSetDevice(c.device));
+        H2B_TRY(dev_malloc(&bs->dev[d], bs->rows[d] * 64 + 64, "SRS bases"));
+        H2B_TRY(host_upload(c, bs->dev[d], bases + 8 * bs->lo[d], bs->rows[d] * 64, c.stream));
+        if (cudaStreamSynchronize(c.stream) != cudaSuccess) { set_error("SRS upload: %s", cudaGetErrorString(cudaGetLastError())); return H2B_ERR_CUDA; }
+        return H2B_OK;
+    }));
+    if (!bs->sharded) H2B_TRY(replicate_device0(*bs));
     *out = with_tables ? build_tables(bs) : bs;
     return H2B_OK;
 }
@@ -383,9 +411,12 @@ static SetRef find_set(uint64_t handle) {
     std::lock_guard<std::mutex> lk(G.mu);
     return find_set_locked(handle);
 }
-static void publish_locked(const SetRef& bs) {
-    for (auto& sp : G.sets) if (sp->handle == bs->handle) { sp = bs; return; }
+// hands a new set out under a fresh handle.  Caller holds G.mu.
+static uint64_t publish_new_locked(const SetRef& bs) {
+    bs->handle = G.next_handle++;
+    bs->last_use = ++G.use_counter;
     G.sets.push_back(bs);
+    return bs->handle;
 }
 static void drop_locked(uint64_t handle) {
     for (size_t i = 0; i < G.sets.size(); ++i) if (G.sets[i]->handle == handle) { G.sets.erase(G.sets.begin() + i); return; }
@@ -447,16 +478,14 @@ static int implicit_insert_locked(const uint64_t* bases, size_t n, SetRef* out) 
     }
     SetRef bs;
     H2B_TRY(create_set(bases, n, n >= MULTI_DEVICE_MIN_POINTS, false, &bs));
-    bs->handle = G.next_handle++;
     bs->implicit = true;
     bs->host_ptr = bases;
-    bs->last_use = ++G.use_counter;
     bs->uses = 1;
     bs->refs = 0;
     const size_t nblocks = n / digest_block();
     bs->digest.resize(2 * nblocks);
     digest_blocks(bases, 0, nblocks, bs->digest.data(), nullptr);
-    G.sets.push_back(bs);
+    publish_new_locked(bs);
     G.implicit_uploads++;
     *out = bs;
     return H2B_OK;
@@ -515,20 +544,14 @@ static int msm_host(const uint64_t* scalars, const BaseSet& bs, size_t offset, s
     // point-range sharding: every piece is a complete Pippenger on its device; the partial sums are folded on device 0
     const size_t np = pieces.size();
     std::vector<uint64_t> blocks(28 * np);
-    std::vector<int> rcs(np, 0);
-    std::vector<std::string> errs(np);
-    std::vector<std::thread> th;
-    for (size_t i = 0; i < np; ++i) {
-        th.emplace_back([&, i] {
-            const Piece& p = pieces[i];
-            DeviceCtx& c = *G.devs[p.d];
-            std::lock_guard<std::mutex> lk(c.mu);
-            rcs[i] = msm_on_device(c, scalars + 4 * p.lo, bases_of(bs, p.d, offset + p.lo), p.n, &blocks[28 * i]);
-            if (rcs[i]) errs[i] = get_error();
-        });
-    }
-    for (auto& t : th) t.join();
-    for (size_t i = 0; i < np; ++i) if (rcs[i]) { set_error("device %zu: %s", pieces[i].d, errs[i].c_str()); return rcs[i]; }
+    std::vector<size_t> devs, piece_on(G.devs.size());
+    for (size_t i = 0; i < np; ++i) { devs.push_back(pieces[i].d); piece_on[pieces[i].d] = i; }
+    H2B_TRY(on_devices(devs, [&](size_t d) -> int {
+        const size_t i = piece_on[d];
+        DeviceCtx& c = *G.devs[d];
+        std::lock_guard<std::mutex> lk(c.mu);
+        return msm_on_device(c, scalars + 4 * pieces[i].lo, bases_of(bs, d, offset + pieces[i].lo), pieces[i].n, &blocks[28 * i]);
+    }));
     DeviceCtx& c0 = *G.devs[0];
     std::lock_guard<std::mutex> lk(c0.mu);
     H2B_CUDA(cudaSetDevice(c0.device));
@@ -677,30 +700,22 @@ int h2b_msm_bn254_g1(const uint64_t* scalars, const uint64_t* bases, size_t n, u
     return msm_direct(scalars, bases, n, out_jac);      // unreachable in practice: the array changed twice while we looked at it
 }
 
-int h2b_register_bases(const uint64_t* bases, size_t n, uint64_t* handle) {
+static int register_bases(const char* who, const uint64_t* bases, size_t n, bool sharded, uint64_t* handle) {
     H2B_TRY(require_init());
-    if (!bases || !handle || n == 0) { set_error("h2b_register_bases: bad argument"); return H2B_ERR_BAD_ARGUMENT; }
+    if (!bases || !handle || n == 0) { set_error("%s: bad argument", who); return H2B_ERR_BAD_ARGUMENT; }
     std::lock_guard<std::mutex> lk(G.mu);
     SetRef bs;
-    H2B_TRY(create_set(bases, n, false, true, &bs));
-    bs->handle = G.next_handle++;
-    bs->last_use = ++G.use_counter;
-    *handle = bs->handle;
-    G.sets.push_back(bs);
+    H2B_TRY(create_set(bases, n, sharded, true, &bs));
+    *handle = publish_new_locked(bs);
     return H2B_OK;
 }
 
+int h2b_register_bases(const uint64_t* bases, size_t n, uint64_t* handle) {
+    return register_bases("h2b_register_bases", bases, n, false, handle);
+}
+
 int h2b_register_bases_sharded(const uint64_t* bases, size_t n, uint64_t* handle) {
-    H2B_TRY(require_init());
-    if (!bases || !handle || n == 0) { set_error("h2b_register_bases_sharded: bad argument"); return H2B_ERR_BAD_ARGUMENT; }
-    std::lock_guard<std::mutex> lk(G.mu);
-    SetRef bs;
-    H2B_TRY(create_set(bases, n, true, true, &bs));
-    bs->handle = G.next_handle++;
-    bs->last_use = ++G.use_counter;
-    *handle = bs->handle;
-    G.sets.push_back(bs);
-    return H2B_OK;
+    return register_bases("h2b_register_bases_sharded", bases, n, true, handle);
 }
 
 int h2b_unregister_bases(uint64_t handle) {
@@ -753,16 +768,6 @@ static bool ntt_multi_applicable(uint32_t log_n, uint32_t* log_d) {
     return true;
 }
 
-static int on_all_devices(size_t nd, const std::function<int(size_t)>& fn) {
-    std::vector<int> rcs(nd, 0);
-    std::vector<std::string> errs(nd);
-    std::vector<std::thread> th;
-    for (size_t d = 0; d < nd; ++d) th.emplace_back([&, d] { rcs[d] = fn(d); if (rcs[d]) errs[d] = get_error(); });
-    for (auto& t : th) t.join();
-    for (size_t d = 0; d < nd; ++d) if (rcs[d]) { set_error("device %zu: %s", d, errs[d].c_str()); return rcs[d]; }
-    return H2B_OK;
-}
-
 static int ntt_multi_device(uint64_t* a, const uint64_t omega[4], uint32_t log_n, uint32_t log_d) {
     const size_t D = (size_t)1 << log_d;
     const uint32_t r1 = log_n / 2, r2 = log_n - r1;
@@ -779,7 +784,8 @@ static int ntt_multi_device(uint64_t* a, const uint64_t omega[4], uint32_t log_n
         H2B_CUDA(cudaMemcpyAsync(roots, c0.msm_out.p, 64, cudaMemcpyDeviceToHost, c0.stream));
         H2B_CUDA(cudaStreamSynchronize(c0.stream));
     }
-    H2B_TRY(on_all_devices(D, [&](size_t d) -> int {
+    const std::vector<size_t> devs = first_devices(D);
+    H2B_TRY(on_devices(devs, [&](size_t d) -> int {
         DeviceCtx& c = *G.devs[d];
         H2B_CUDA(cudaSetDevice(c.device));
         H2B_TRY(c.ntt_io.reserve(slice));
@@ -792,7 +798,7 @@ static int ntt_multi_device(uint64_t* a, const uint64_t omega[4], uint32_t log_n
         H2B_CUDA(cudaStreamSynchronize(c.stream));
         return H2B_OK;
     }));
-    return on_all_devices(D, [&](size_t e) -> int {
+    return on_devices(devs, [&](size_t e) -> int {
         DeviceCtx& c = *G.devs[e];
         H2B_CUDA(cudaSetDevice(c.device));
         for (size_t k = 0; k < D; ++k) {                  // C x Rd, rows [d Cd, (d+1) Cd) from device d; every device starts with its own block
@@ -897,22 +903,9 @@ int h2b_msm_bn254_g1_batch_registered(const uint64_t* const* scalars, const size
         }
         return H2B_OK;
     };
-    size_t busy = 0;
-    for (size_t d = 0; d < nd; ++d) busy += dev_groups[d].empty() ? 0 : 1;
-    if (busy <= 1) {
-        for (size_t d = 0; d < nd; ++d) if (!dev_groups[d].empty()) H2B_TRY(run_device(d));
-        return H2B_OK;
-    }
-    std::vector<int> rcs(nd, 0);
-    std::vector<std::string> errs(nd);
-    std::vector<std::thread> th;
-    for (size_t d = 0; d < nd; ++d) {
-        if (dev_groups[d].empty()) continue;
-        th.emplace_back([&, d] { rcs[d] = run_device(d); if (rcs[d]) errs[d] = get_error(); });
-    }
-    for (auto& t : th) t.join();
-    for (size_t d = 0; d < nd; ++d) if (rcs[d]) { set_error("device %zu: %s", d, errs[d].c_str()); return rcs[d]; }
-    return H2B_OK;
+    std::vector<size_t> busy;
+    for (size_t d = 0; d < nd; ++d) if (!dev_groups[d].empty()) busy.push_back(d);
+    return on_devices(busy, run_device);
 }
 
 int h2b_ntt_bn254_fr_batch(uint64_t* const* a, size_t count, const uint64_t omega[4], uint32_t log_n) {
@@ -946,15 +939,7 @@ int h2b_ntt_bn254_fr_batch(uint64_t* const* a, size_t count, const uint64_t omeg
         }
         return H2B_OK;
     };
-    const size_t workers = count < nd ? count : nd;
-    if (workers <= 1) return run_device(0);
-    std::vector<int> rcs(workers, 0);
-    std::vector<std::string> errs(workers);
-    std::vector<std::thread> th;
-    for (size_t d = 0; d < workers; ++d) th.emplace_back([&, d] { rcs[d] = run_device(d); if (rcs[d]) errs[d] = get_error(); });
-    for (auto& t : th) t.join();
-    for (size_t d = 0; d < workers; ++d) if (rcs[d]) { set_error("device %zu: %s", d, errs[d].c_str()); return rcs[d]; }
-    return H2B_OK;
+    return on_devices(first_devices(count < nd ? count : nd), run_device);
 }
 
 int h2b_ntt_bn254_fr_dev_batch(int device, void* const* d_polys, size_t count, const uint64_t omega[4], uint32_t log_n, void* stream) {
@@ -1156,8 +1141,7 @@ int h2b_column_pipeline(int device, const uint64_t* lagrange, uint64_t handle_g_
     H2B_TRY(c->msm_out.reserve(256));
     if (want_ext) {
         if (d_extended) {
-            cudaError_t e = cudaMalloc(&d_ext, en * 32);
-            if (e != cudaSuccess) { cudaGetLastError(); set_error("h2b_column_pipeline: cudaMalloc(%zu): %s", en * 32, cudaGetErrorString(e)); return H2B_ERR_OOM; }
+            H2B_TRY(dev_malloc(&d_ext, en * 32, "h2b_column_pipeline's extended column"));
         } else {
             H2B_TRY(c->col_ext.reserve(en * 32));
             d_ext = c->col_ext.p;
@@ -1287,74 +1271,49 @@ namespace {
 struct FileCloser { FILE* f; ~FileCloser() { if (f) fclose(f); } };
 }  // namespace
 
-// points on device 0 (d_pts, n x 64 B + 64, owned by the new set from here on) -> a registered, replicated base set: peer
-// copies to the other devices, window tables, a handle.  Caller holds G.mu.
-static int adopt_device0_points_locked(void* d_pts, size_t n, const char* caller, const char* what, uint64_t* handle) {
+// One point vector made on device 0: `produce` fills n x 64 B on device 0's stream; the points are downloaded to host_out (may be
+// null), then registered under *handle as a replicated set with window tables (handle may be null: the points are dropped).
+// release_g1gen: the producer runs g1gen.cu kernels whose scratch is given back once they are done.  Errors read "caller: what: ...".
+// Caller holds G.mu.
+static int device0_points_locked(size_t n, const char* caller, const char* what, bool release_g1gen,
+                                 const std::function<int(DeviceCtx&, void*)>& produce, uint64_t* host_out, uint64_t* handle) {
     DeviceCtx& c = *G.devs[0];
-    SetRef bs(new BaseSet());
-    bs->last_use = ++G.use_counter;
-    bs->n = n;
-    layout_rows(n, false, bs->lo, bs->rows);
-    bs->dev.assign(G.devs.size(), nullptr);
-    for (size_t d = 0; d < G.devs.size(); ++d) bs->ordinal.push_back(G.devs[d]->device);
-    bs->dev[0] = d_pts;
-    for (size_t d = 1; d < G.devs.size(); ++d) {        // the other devices take a peer copy of the points
-        std::lock_guard<std::mutex> lk(G.devs[d]->mu);
-        cudaError_t e = cudaSetDevice(G.devs[d]->device);
-        if (e == cudaSuccess) e = cudaMalloc(&bs->dev[d], n * 64 + 64);
-        if (e == cudaSuccess) e = cudaMemcpyPeer(bs->dev[d], G.devs[d]->device, d_pts, c.device, n * 64);
-        if (e != cudaSuccess) { set_error("%s: copy of %s to device %zu: %s", caller, what, d, cudaGetErrorString(e)); return H2B_ERR_CUDA; }
+    SetRef bs = new_set(n, false);      // owns the points from here on: every failure path frees them
+    int rc;
+    {
+        std::lock_guard<std::mutex> lk(c.mu);
+        H2B_CUDA(cudaSetDevice(c.device));
+        const size_t scan_cap = c.scan_scratch.cap;
+        rc = dev_malloc(&bs->dev[0], n * 64 + 64, "SRS bases");
+        if (!rc) rc = produce(c, bs->dev[0]);
+        if (!rc && host_out) rc = host_download(c, host_out, bs->dev[0], n * 64, c.stream);
+        if (!rc && cudaStreamSynchronize(c.stream) != cudaSuccess) { set_error("%s", cudaGetErrorString(cudaGetLastError())); rc = H2B_ERR_CUDA; }
+        if (release_g1gen) g1gen_release_scratch(c, scan_cap);
     }
-    bs = build_tables(bs);
-    bs->handle = G.next_handle++;
-    *handle = bs->handle;
-    G.sets.push_back(bs);
+    if (!rc && handle) rc = replicate_device0(*bs);
+    if (rc) { set_error("%s: %s: %s", caller, what, std::string(get_error()).c_str()); return rc; }
+    if (handle) *handle = publish_new_locked(build_tables(bs));
     return H2B_OK;
 }
 
-// one vector of the file: bytes -> device 0 -> decoded points; optionally downloaded and / or registered on every device
+// one vector of the file: bytes -> device 0 -> decoded points
 static int srs_read_vector(const unsigned char* raw, const char* what, size_t n, int format, uint64_t* host_out, uint64_t* handle) {
     const size_t ps = format == H2B_SERDE_PROCESSED ? 32 : 64;
     std::lock_guard<std::mutex> glk(G.mu);
-    DeviceCtx& c = *G.devs[0];
-    void* d_pts = nullptr;
-    {
-        std::lock_guard<std::mutex> lk(c.mu);
-        H2B_CUDA(cudaSetDevice(c.device));
+    return device0_points_locked(n, "h2b_srs_read", what, false, [&](DeviceCtx& c, void* d_pts) -> int {
         H2B_TRY(c.srs_io.reserve(n * ps));
-        cudaError_t e = cudaMalloc(&d_pts, n * 64 + 64);
-        if (e != cudaSuccess) { set_error("cudaMalloc of %zu bytes for %s failed: %s", n * 64, what, cudaGetErrorString(e)); return H2B_ERR_OOM; }
         // the mapping is pageable memory: the staging threads of stage.cu pull it through the page cache in parallel
-        int rc = host_upload(c, c.srs_io.p, raw, n * ps, c.stream);
+        H2B_TRY(host_upload(c, c.srs_io.p, raw, n * ps, c.stream));
         uint64_t bad = 0;
-        if (!rc) rc = g1_decode_run(c, c.srs_io.p, n, format, d_pts, &bad, c.stream);
-        if (!rc && host_out) rc = host_download(c, host_out, d_pts, n * 64, c.stream);
-        if (!rc && cudaStreamSynchronize(c.stream) != cudaSuccess) { set_error("h2b_srs_read: %s", cudaGetErrorString(cudaGetLastError())); rc = H2B_ERR_CUDA; }
-        if (rc || !handle) { cudaFree(d_pts); if (rc) set_error("%s: %s", what, std::string(get_error()).c_str()); return rc; }
-    }
-    return adopt_device0_points_locked(d_pts, n, "h2b_srs_read", what, handle);
+        return g1_decode_run(c, c.srs_io.p, n, format, d_pts, &bad, c.stream);
+    }, host_out, handle);
 }
 
-// one vector of ParamsKZG::setup (which 0: g, 1: g_lagrange) computed on device 0; optionally downloaded and / or registered
+// one vector of ParamsKZG::setup (which 0: g, 1: g_lagrange)
 static int srs_setup_vector(uint32_t k, const uint64_t s[4], int which, uint64_t* host_out, uint64_t* handle) {
-    const size_t n = (size_t)1 << k;
-    const char* what = which ? "g_lagrange" : "g";
     std::lock_guard<std::mutex> glk(G.mu);
-    DeviceCtx& c = *G.devs[0];
-    void* d_pts = nullptr;
-    {
-        std::lock_guard<std::mutex> lk(c.mu);
-        H2B_CUDA(cudaSetDevice(c.device));
-        cudaError_t e = cudaMalloc(&d_pts, n * 64 + 64);
-        if (e != cudaSuccess) { set_error("cudaMalloc of %zu bytes for %s failed: %s", n * 64, what, cudaGetErrorString(e)); return H2B_ERR_OOM; }
-        const size_t scan_cap = c.scan_scratch.cap;
-        int rc = srs_setup_run(c, k, s, which, d_pts, c.stream);
-        if (!rc && host_out) rc = host_download(c, host_out, d_pts, n * 64, c.stream);
-        if (!rc && cudaStreamSynchronize(c.stream) != cudaSuccess) { set_error("h2b_srs_setup: %s", cudaGetErrorString(cudaGetLastError())); rc = H2B_ERR_CUDA; }
-        if (!rc) g1gen_release_scratch(c, scan_cap);
-        if (rc || !handle) { cudaFree(d_pts); if (rc) set_error("%s: %s", what, std::string(get_error()).c_str()); return rc; }
-    }
-    return adopt_device0_points_locked(d_pts, n, "h2b_srs_setup", what, handle);
+    return device0_points_locked((size_t)1 << k, "h2b_srs_setup", which ? "g_lagrange" : "g", true,
+                                 [&](DeviceCtx& c, void* d_pts) { return srs_setup_run(c, k, s, which, d_pts, c.stream); }, host_out, handle);
 }
 
 namespace {
@@ -1515,40 +1474,16 @@ int h2b_srs_downsize(uint64_t handle_g, uint32_t k, uint64_t* out_g_lagrange, ui
     if (!src || src->implicit) { set_error("h2b_srs_downsize: unknown base-set handle %llu", (unsigned long long)handle_g); return H2B_ERR_BAD_ARGUMENT; }
     if (src->sharded) { set_error("h2b_srs_downsize: handle %llu is a sharded set (g must be whole on device 0)", (unsigned long long)handle_g); return H2B_ERR_BAD_ARGUMENT; }
     if (n > src->n) { set_error("h2b_srs_downsize: 2^%u points requested from a set of %zu", k, src->n); return H2B_ERR_BAD_ARGUMENT; }
-    const bool want_gl = out_g_lagrange || handle_g_lagrange_out;
-    DeviceCtx& c = *G.devs[0];
-    void* d_g = nullptr;
-    void* d_gl = nullptr;
-    {
-        std::lock_guard<std::mutex> lk(c.mu);
-        H2B_CUDA(cudaSetDevice(c.device));
-        int rc = H2B_OK;
-        if (handle_g_out && cudaMalloc(&d_g, n * 64 + 64) != cudaSuccess) rc = H2B_ERR_OOM;
-        if (!rc && want_gl && cudaMalloc(&d_gl, n * 64 + 64) != cudaSuccess) rc = H2B_ERR_OOM;
-        if (rc) set_error("h2b_srs_downsize: cudaMalloc of %zu bytes failed", n * 64);
-        if (!rc && d_g && cudaMemcpyAsync(d_g, src->dev[0], n * 64, cudaMemcpyDeviceToDevice, c.stream) != cudaSuccess) {
-            set_error("h2b_srs_downsize: copy of g: %s", cudaGetErrorString(cudaGetLastError()));
-            rc = H2B_ERR_CUDA;
-        }
-        const size_t scan_cap = c.scan_scratch.cap;
-        if (!rc && d_gl) rc = g1_to_lagrange_run(c, src->dev[0], k, d_gl, c.stream);
-        if (!rc && out_g_lagrange) rc = host_download(c, out_g_lagrange, d_gl, n * 64, c.stream);
-        if (!rc && cudaStreamSynchronize(c.stream) != cudaSuccess) { set_error("h2b_srs_downsize: %s", cudaGetErrorString(cudaGetLastError())); rc = H2B_ERR_CUDA; }
-        g1gen_release_scratch(c, scan_cap);
-        if (rc) {
-            if (d_g) cudaFree(d_g);
-            if (d_gl) cudaFree(d_gl);
-            return rc;
-        }
-        if (d_gl && !handle_g_lagrange_out) { cudaFree(d_gl); d_gl = nullptr; }
-    }
     uint64_t hg = 0, hl = 0;
-    if (d_g) {
-        int rc = adopt_device0_points_locked(d_g, n, "h2b_srs_downsize", "g", &hg);
-        if (rc) { if (d_gl) cudaFree(d_gl); return rc; }
-    }
-    if (d_gl) {
-        int rc = adopt_device0_points_locked(d_gl, n, "h2b_srs_downsize", "g_lagrange", &hl);
+    if (handle_g_out)
+        H2B_TRY(device0_points_locked(n, "h2b_srs_downsize", "g", false, [&](DeviceCtx& c, void* d_g) -> int {
+            H2B_CUDA(cudaMemcpyAsync(d_g, src->dev[0], n * 64, cudaMemcpyDeviceToDevice, c.stream));
+            return H2B_OK;
+        }, nullptr, &hg));
+    if (out_g_lagrange || handle_g_lagrange_out) {
+        const int rc = device0_points_locked(n, "h2b_srs_downsize", "g_lagrange", true,
+                                             [&](DeviceCtx& c, void* d_gl) { return g1_to_lagrange_run(c, src->dev[0], k, d_gl, c.stream); },
+                                             out_g_lagrange, handle_g_lagrange_out ? &hl : nullptr);
         if (rc) {
             if (hg) drop_locked(hg);
             return rc;
@@ -1630,8 +1565,7 @@ struct KeygenScratch {
     cudaEvent_t ev[2] = {nullptr, nullptr};
     DeviceCtx* ctx = nullptr;
     int alloc(size_t bytes, void** out) {
-        cudaError_t e = cudaMalloc(out, bytes);
-        if (e != cudaSuccess) { cudaGetLastError(); set_error("key generation: cudaMalloc(%zu): %s", bytes, cudaGetErrorString(e)); return H2B_ERR_OOM; }
+        H2B_TRY(dev_malloc(out, bytes, "key generation"));
         bufs.push_back(*out);
         return H2B_OK;
     }
@@ -1795,7 +1729,7 @@ static int keygen_device(size_t d, const KeygenJob& job, uint32_t* bad) {
 static int keygen_run(const char* who, const KeygenJob& job) {
     const size_t nd = G.devs.size();
     std::vector<uint32_t> bad(nd, 0);
-    H2B_TRY(on_all_devices(nd, [&](size_t d) { return keygen_device(d, job, &bad[d]); }));
+    H2B_TRY(on_devices(first_devices(nd), [&](size_t d) { return keygen_device(d, job, &bad[d]); }));
     for (size_t d = 0; d < nd; ++d) {
         if (!bad[d]) continue;
         const uint64_t flat = bad[d] - 1, n = (uint64_t)1 << job.k;
@@ -2129,9 +2063,7 @@ int h2b_dev_alloc(int device, size_t bytes, void** out) {
     DeviceCtx* c = nullptr;
     H2B_TRY(get_ctx(device, &c));
     if (!out) { set_error("h2b_dev_alloc: null out"); return H2B_ERR_BAD_ARGUMENT; }
-    cudaError_t e = cudaMalloc(out, bytes ? bytes : 1);
-    if (e != cudaSuccess) { set_error("cudaMalloc(%zu): %s", bytes, cudaGetErrorString(e)); return H2B_ERR_OOM; }
-    return H2B_OK;
+    return dev_malloc(out, bytes ? bytes : 1, "h2b_dev_alloc");
 }
 int h2b_dev_free(int device, void* p) {
     DeviceCtx* c = nullptr;

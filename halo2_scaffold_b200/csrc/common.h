@@ -42,11 +42,14 @@ struct DevBuf {
         if (p) { cudaFree(p); p = nullptr; cap = 0; }
         size_t want = bytes + bytes / 8;
         cudaError_t e = cudaMalloc(&p, want);
+        // a failed allocation stays the thread's last error, which the next launch check would report: clear it
         if (e != cudaSuccess) {
+            cudaGetLastError();
             e = cudaMalloc(&p, bytes);
             want = bytes;
         }
         if (e != cudaSuccess) {
+            cudaGetLastError();
             p = nullptr;
             set_error("cudaMalloc(%zu) failed: %s", bytes, cudaGetErrorString(e));
             return H2B_ERR_OOM;

@@ -171,7 +171,15 @@ static inline void __threadfence() { __atomic_thread_fence(__ATOMIC_SEQ_CST); }
 template <class T> static inline T __ldg(const T* p) { return *p; }
 
 // ---- runtime API subset -------------------------------------------------------------------
-static inline cudaError_t cudaMalloc(void** p, size_t n) { *p = aligned_alloc(256, ((n + 255) / 256) * 256 + 256); return *p ? cudaSuccess : cudaErrorMemoryAllocation; }
+// the runtime's per-thread last error: a failed cudaMalloc leaves it set until cudaGetLastError reads it, so a caller that does
+// not clear it sees its next launch check fail
+namespace emu { inline thread_local cudaError_t last_error = cudaSuccess; }
+static inline cudaError_t cudaMalloc(void** p, size_t n) {
+    *p = aligned_alloc(256, ((n + 255) / 256) * 256 + 256);
+    if (*p) return cudaSuccess;
+    emu::last_error = cudaErrorMemoryAllocation;
+    return cudaErrorMemoryAllocation;
+}
 template <class T> static inline cudaError_t cudaMalloc(T** p, size_t n) { return cudaMalloc((void**)p, n); }
 static inline cudaError_t cudaFree(void* p) { free(p); return cudaSuccess; }
 static inline cudaError_t cudaMallocHost(void** p, size_t n) { return cudaMalloc(p, n); }
@@ -196,8 +204,8 @@ static inline cudaError_t cudaStreamCreate(cudaStream_t* s) { *s = nullptr; retu
 static inline cudaError_t cudaStreamDestroy(cudaStream_t) { return cudaSuccess; }
 static inline cudaError_t cudaStreamSynchronize(cudaStream_t) { return cudaSuccess; }
 static inline cudaError_t cudaDeviceSynchronize() { return cudaSuccess; }
-static inline cudaError_t cudaGetLastError() { return cudaSuccess; }
-static inline cudaError_t cudaPeekAtLastError() { return cudaSuccess; }
+static inline cudaError_t cudaGetLastError() { const cudaError_t e = emu::last_error; emu::last_error = cudaSuccess; return e; }
+static inline cudaError_t cudaPeekAtLastError() { return emu::last_error; }
 static inline const char* cudaGetErrorString(cudaError_t) { return "emu"; }
 static inline cudaError_t cudaSetDevice(int) { return cudaSuccess; }
 static inline cudaError_t cudaGetDevice(int* d) { *d = 0; return cudaSuccess; }
