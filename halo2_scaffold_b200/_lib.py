@@ -42,7 +42,14 @@ _EXPORTS = [
     "h2b_srs_setup", "h2b_g1_generator_mul_dev", "h2b_g1_to_lagrange_dev", "h2b_srs_downsize",
     "h2b_permutation_sigma_dev", "h2b_keygen_lagrange_indicators_dev", "h2b_permutation_build_vk", "h2b_permutation_build_pk",
     "h2b_selector_exclusion", "h2b_keygen_fixed_build_vk", "h2b_keygen_fixed_build_pk",
+    "h2b_pk_create", "h2b_keygen_fixed_build_pk_resident", "h2b_permutation_build_pk_resident", "h2b_keygen_lagrange_indicators_resident",
+    "h2b_pk_put_lagrange", "h2b_pk_column", "h2b_pk_download", "h2b_pk_info", "h2b_pk_release",
 ]
+
+# include/h2b200.h enums of the resident proving key
+PK_FIXED, PK_PERMUTATION, PK_INDICATORS = 0, 1, 2
+PK_VALUES, PK_COEFF, PK_EXTENDED = 0, 1, 2
+PK_REPLICATED, PK_ROW_SHARDED = 0, 1
 
 
 # ---- include/h2b200.h structs of the quotient evaluation ------------------------------------------------
@@ -217,6 +224,15 @@ class Lib:
         L.h2b_selector_exclusion.argtypes = [vp, u32, u32, vp]
         L.h2b_keygen_fixed_build_vk.argtypes = [vp, u32, vp, u32, vp, vp, u32, u32, u64, vp]
         L.h2b_keygen_fixed_build_pk.argtypes = [vp, u32, vp, u32, vp, vp, u32, u32, u32, vp, vp, vp, vp, vp, vp, vp]
+        L.h2b_pk_create.argtypes = [u32, u32, u32, u32, i32, u32, vp, vp, vp, vp, vp, ctypes.POINTER(u64)]
+        L.h2b_keygen_fixed_build_pk_resident.argtypes = [vp, u32, vp, u32, vp, vp, u32, u64, u32]
+        L.h2b_permutation_build_pk_resident.argtypes = [vp, u32, vp, u64]
+        L.h2b_keygen_lagrange_indicators_resident.argtypes = [u64, u32]
+        L.h2b_pk_put_lagrange.argtypes = [u64, i32, u32, u32, vp]
+        L.h2b_pk_column.argtypes = [u64, i32, i32, i32, u32, ctypes.POINTER(vp), vp]
+        L.h2b_pk_download.argtypes = [u64, i32, i32, u32, vp]
+        L.h2b_pk_info.argtypes = [u64, vp]
+        L.h2b_pk_release.argtypes = [u64]
         L.h2b_evaluate_graph_dev.argtypes = [i32, vp, vp, vp, u32, i32, vp]
         L.h2b_evaluate_h_permutation_dev.argtypes = [i32, vp, u32, i32, vp, u32, vp, vp, u32, u32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
         L.h2b_evaluate_h_lookup_dev.argtypes = [i32, vp, vp, vp, u32, i32, vp, vp, vp, vp, vp, vp, vp]
@@ -800,6 +816,55 @@ class Lib:
         self.check(self.L.h2b_keygen_fixed_build_pk(arr(fx), len(fx), arr(acts), len(acts), co.ctypes.data, ro.ctypes.data, n_combinations, k, extended_k,
                                                     *[x.ctypes.data for x in w], zp.ctypes.data, arr(vals), arr(polys), arr(cosets)))
         return dict(combination_values=vals, polys=polys, cosets=cosets)
+
+    # ---- the proving key resident on the devices ---------------------------------------------------------------------------------
+    def pk_create(self, k: int, extended_k: int, n_fixed: int, n_permutation: int, layout: int, halo: int, omega, omega_inv, ifft_divisor,
+                  extended_omega, zeta_powers) -> int:
+        w = [_u64(x).reshape(4) for x in (omega, omega_inv, ifft_divisor, extended_omega)]
+        zp = _u64(zeta_powers).reshape(3, 4)
+        h = ctypes.c_uint64(0)
+        self.check(self.L.h2b_pk_create(k, extended_k, n_fixed, n_permutation, layout, halo, *[x.ctypes.data for x in w], zp.ctypes.data, ctypes.byref(h)))
+        return h.value
+
+    def keygen_fixed_build_pk_resident(self, fixed, activations, combination_of, root_of, n_combinations: int, k: int, pk: int, first_column: int = 0):
+        fx, acts, co, ro = _fixed_args(fixed, activations, combination_of, root_of, k)
+        arr = lambda xs: _ptr_array([x.ctypes.data for x in xs]) if xs else None
+        self.check(self.L.h2b_keygen_fixed_build_pk_resident(arr(fx), len(fx), arr(acts), len(acts), co.ctypes.data, ro.ctypes.data, n_combinations, pk,
+                                                             first_column))
+
+    def permutation_build_pk_resident(self, mapping, k: int, delta, pk: int):
+        cols = _mapping_columns(mapping, k)
+        dl = _u64(delta).reshape(4)
+        self.check(self.L.h2b_permutation_build_pk_resident(_ptr_array([c.ctypes.data for c in cols]), len(cols), dl.ctypes.data, pk))
+
+    def keygen_lagrange_indicators_resident(self, pk: int, blinding_factors: int):
+        self.check(self.L.h2b_keygen_lagrange_indicators_resident(pk, blinding_factors))
+
+    def pk_put_lagrange(self, pk: int, part: int, first: int, values, k: int):
+        cols = [_u64(c).reshape(-1, 4) for c in values]
+        for c in cols:
+            assert c.shape[0] == 1 << k, "column of %d rows, expected 2^%d" % (c.shape[0], k)
+        self.check(self.L.h2b_pk_put_lagrange(pk, part, first, len(cols), _ptr_array([c.ctypes.data for c in cols]) if cols else None))
+
+    def pk_column(self, pk: int, device: int, part: int, form: int, index: int):
+        """-> (device pointer, (row0, rows, halo)) of one column on `device`"""
+        p, sh = ctypes.c_void_p(0), ShardStruct()
+        self.check(self.L.h2b_pk_column(pk, device, part, form, index, ctypes.byref(p), ctypes.addressof(sh)))
+        return p.value or 0, (sh.row0, sh.rows, sh.halo)
+
+    def pk_download(self, pk: int, part: int, form: int, index: int, rows: int) -> np.ndarray:
+        out = np.empty((rows, 4), dtype=np.uint64)
+        self.check(self.L.h2b_pk_download(pk, part, form, index, out.ctypes.data))
+        return out
+
+    def pk_info(self, pk: int) -> list:
+        """-> bytes the pk holds on each device"""
+        out = np.zeros(max(self.device_count(), 1), dtype=np.uint64)
+        self.check(self.L.h2b_pk_info(pk, out.ctypes.data))
+        return [int(x) for x in out]
+
+    def pk_release(self, pk: int):
+        self.check(self.L.h2b_pk_release(pk))
 
     # ---- quotient evaluation (evaluate_h) on device-resident extended-coset columns ------------------
     def evaluate_graph_dev(self, device: int, graph: GraphArrays, cols: EvalColumns, d_values: int, size: int, rot_scale: int, stream: int = 0,

@@ -12,6 +12,8 @@
 #include "../../include/h2b200.h"
 #include "common.h"
 
+struct ResidentPk;   // a proving key held on the devices (h2b_pk_create)
+
 namespace h2b {
 
 unsigned long long g_launch_count = 0;
@@ -71,6 +73,7 @@ struct Global {
     std::mutex mu;
     std::vector<std::unique_ptr<DeviceCtx>> devs;
     std::vector<SetRef> sets;
+    std::vector<std::shared_ptr<::ResidentPk>> pks;
     std::vector<SrsCacheEntry> srs_cache;
     uint64_t next_handle = 1;
     uint64_t use_counter = 0;
@@ -623,6 +626,7 @@ int h2b_init_device(int device) {
 void h2b_shutdown(void) {
     std::lock_guard<std::mutex> lk(G.mu);
     G.sets.clear();      // device memory goes when the last holder lets go (now, unless a call is still in flight)
+    G.pks.clear();
     G.srs_cache.clear();
     for (auto& c : G.devs) {
         cudaSetDevice(c->device);
@@ -1539,6 +1543,83 @@ struct SelectorCombinations {
     const uint32_t* root_of = nullptr;
 };
 
+// A proving key resident on the devices (h2b_pk_create): one allocation per device, holding per part and form a block of columns.
+// Device d's block order is FIXED VALUES | FIXED COEFF | FIXED EXTENDED | PERMUTATION (the same three) | INDICATORS EXTENDED; an
+// EXTENDED column there has ext_rows[d] rows (E replicated, the device's slice with its halo sharded).  Immutable in shape once created;
+// builds write the columns under `build` and mark them filled.
+struct ResidentPk {
+    uint64_t handle = 0;
+    uint32_t k = 0, extended_k = 0, halo = 0;
+    uint32_t count[3] = {0, 0, 3};              // columns per part
+    bool sharded = false;
+    uint64_t omega[4], omega_inv[4], ifft_divisor[4], extended_omega[4], zeta_powers[12];
+    std::vector<int> ordinal;
+    std::vector<void*> dev;
+    std::vector<size_t> row0, rows, ext_rows;   // per device: the owned extended rows and the slice length with halo
+    std::vector<uint8_t> filled[3];             // per part and column: every form written by a completed build
+    std::mutex build;                           // one build at a time
+    mutable std::mutex filled_mu;               // guards filled[] for the readers
+    ~ResidentPk() {
+        for (size_t d = 0; d < dev.size(); ++d) {
+            if (!dev[d]) continue;
+            cudaSetDevice(ordinal[d]);
+            cudaDeviceSynchronize();            // work already queued on the device may still read the columns
+            cudaFree(dev[d]);
+        }
+        cudaGetLastError();
+    }
+    static bool holds(int part, int form) { return part != H2B_PK_INDICATORS || form == H2B_PK_EXTENDED; }
+    size_t col_rows(size_t d, int form) const { return form == H2B_PK_EXTENDED ? ext_rows[d] : (size_t)1 << k; }
+    size_t bytes_on(size_t d) const {
+        size_t b = 0;
+        for (int p = 0; p < 3; ++p)
+            for (int f = 0; f < 3; ++f) if (holds(p, f)) b += (size_t)count[p] * col_rows(d, f) * 32;
+        return b;
+    }
+    char* ptr(size_t d, int part, int form, uint32_t index) const {
+        size_t off = 0;
+        for (int p = 0; p < 3; ++p)
+            for (int f = 0; f < 3; ++f) {
+                if (!holds(p, f)) continue;
+                if (p == part && f == form) return (char*)dev[d] + off + (size_t)index * col_rows(d, f) * 32;
+                off += (size_t)count[p] * col_rows(d, f) * 32;
+            }
+        return nullptr;
+    }
+    // first global row of device d's extended slice
+    size_t slice_start(size_t d) const {
+        const size_t E = (size_t)1 << extended_k;
+        return sharded ? (row0[d] + E - halo) % E : 0;
+    }
+};
+typedef std::shared_ptr<ResidentPk> PkRef;
+
+// Column `index` of (part, form), whole on device d at `src`, into the pk's storage of every device: a plain copy on d, a peer copy
+// over NVLink elsewhere; of a sharded EXTENDED column each device receives its slice, in two pieces when it wraps past row E - 1.
+// Enqueued on d's stream `st` (the caller synchronises it).
+static int pk_place(const ResidentPk& pk, size_t d, cudaStream_t st, const void* src, int part, int form, uint32_t index) {
+    DeviceCtx& c = *G.devs[d];
+    const size_t E = (size_t)1 << pk.extended_k;
+    for (size_t e = 0; e < pk.dev.size(); ++e) {
+        char* dst = pk.ptr(e, part, form, index);
+        auto copy = [&](char* to, const char* from, size_t bytes) -> int {
+            if (to == from || bytes == 0) return H2B_OK;
+            if (e == d) H2B_CUDA(cudaMemcpyAsync(to, from, bytes, cudaMemcpyDeviceToDevice, st));
+            else H2B_CUDA(cudaMemcpyPeerAsync(to, pk.ordinal[e], from, pk.ordinal[d], bytes, st));
+            return H2B_OK;
+        };
+        if (form != H2B_PK_EXTENDED || !pk.sharded) {
+            H2B_TRY(copy(dst, (const char*)src, pk.col_rows(e, form) * 32));
+        } else {
+            const size_t s = pk.slice_start(e), len = pk.ext_rows[e], head = len < E - s ? len : E - s;
+            H2B_TRY(copy(dst, (const char*)src + s * 32, head * 32));
+            H2B_TRY(copy(dst + head * 32, (const char*)src, (len - head) * 32));
+        }
+        c.prof.mark(e == d ? PROF_PK_FORM_COPY : PROF_PK_PLACE, st);
+    }
+    return H2B_OK;
+}
+
 // One build_vk / build_pk pass over the columns [col_begin, col_end); column i runs on device i mod D.  Column i's Lagrange values
 // come from, in this order: sigma of mapping[i] for i < n_sigma, the caller's fixed[i - n_sigma] for the next n_fixed, and the
 // combination columns of `comb` after those.
@@ -1556,6 +1637,9 @@ struct KeygenJob {
     uint64_t* const* values_out = nullptr;      // per column (indexed by column; an entry may be null), or null
     uint64_t* const* poly_out = nullptr;
     uint64_t* const* coset_out = nullptr;
+    const ResidentPk* resident = nullptr;       // every form of column i goes to column resident_first + i of resident_part
+    int resident_part = 0;
+    uint32_t resident_first = 0;
     uint32_t n_columns() const { return n_sigma + n_fixed + (comb ? comb->n_combinations : 0); }
 };
 
@@ -1614,8 +1698,9 @@ static int keygen_device(size_t d, const KeygenJob& job, uint32_t* bad) {
     const uint32_t k = job.k;
     const size_t n = (size_t)1 << k;
     const uint32_t comb0 = job.n_sigma + job.n_fixed;
-    const bool pk = job.poly_out || job.coset_out;
-    const size_t col_bytes = (job.coset_out && !job.validate_only ? (size_t)1 << job.extended_k : n) * 32;
+    const bool want_coset = job.coset_out || job.resident;
+    const bool pk = job.poly_out || want_coset;
+    const size_t col_bytes = (want_coset && !job.validate_only ? (size_t)1 << job.extended_k : n) * 32;
     size_t group = ntt_batch_max();
     while (group > 1 && group * col_bytes > KEYGEN_GROUP_BYTES) group >>= 1;
     if (job.commit_set && group > msm_batch_max()) group = msm_batch_max();
@@ -1708,6 +1793,12 @@ static int keygen_device(size_t d, const KeygenJob& job, uint32_t* bad) {
                 if (job.values_out[mine[g0 + t]]) H2B_TRY(host_download(c, job.values_out[mine[g0 + t]], cols[t], n * 32, st));
             c.prof.mark(PROF_KEYGEN_DOWNLOAD, st);
         }
+        // the resident pk takes each form off the group buffer before the next in-place transform
+        auto store = [&](int form) -> int {
+            for (size_t t = 0; t < m; ++t) H2B_TRY(pk_place(*job.resident, d, st, cols[t], job.resident_part, form, job.resident_first + mine[g0 + t]));
+            return H2B_OK;
+        };
+        if (job.resident) H2B_TRY(store(H2B_PK_VALUES));
         if (!pk) continue;
         H2B_TRY(lagrange_to_coeff_batch_run(c, cols.data(), m, k, job.omega_inv, job.ifft_divisor, st));
         c.prof.mark(PROF_KEYGEN_INTT, st);
@@ -1715,12 +1806,18 @@ static int keygen_device(size_t d, const KeygenJob& job, uint32_t* bad) {
             for (size_t t = 0; t < m; ++t) H2B_TRY(host_download(c, job.poly_out[mine[g0 + t]], cols[t], n * 32, st));
             c.prof.mark(PROF_KEYGEN_DOWNLOAD, st);
         }
-        if (job.coset_out) {
+        if (job.resident) H2B_TRY(store(H2B_PK_COEFF));
+        if (want_coset) {
             H2B_TRY(coeff_to_extended_batch_run(c, cols.data(), m, k, job.extended_k, job.extended_omega, job.zeta_powers, st));
             c.prof.mark(PROF_KEYGEN_COSET, st);
-            for (size_t t = 0; t < m; ++t) H2B_TRY(host_download(c, job.coset_out[mine[g0 + t]], cols[t], col_bytes, st));
-            c.prof.mark(PROF_KEYGEN_DOWNLOAD, st);
+            if (job.coset_out) {
+                for (size_t t = 0; t < m; ++t) H2B_TRY(host_download(c, job.coset_out[mine[g0 + t]], cols[t], col_bytes, st));
+                c.prof.mark(PROF_KEYGEN_DOWNLOAD, st);
+            }
+            if (job.resident) H2B_TRY(store(H2B_PK_EXTENDED));
         }
+        // the next group's uploads into the group buffer must not overtake the copies out of it
+        if (job.resident) H2B_CUDA(cudaStreamSynchronize(st));
     }
     return H2B_OK;
 }
@@ -1952,6 +2049,242 @@ int h2b_keygen_fixed_build_pk(const uint64_t* const* fixed, uint32_t n_fixed, co
     job.values_out = out_combination_values ? values.data() : nullptr;
     job.poly_out = out_polys; job.coset_out = out_cosets;
     return keygen_run(who, job);
+}
+
+// ---- the proving key resident on the devices ---------------------------------------------------------------------------------------
+static int pk_lookup(const char* who, uint64_t handle, PkRef* out) {
+    H2B_TRY(require_init());
+    std::lock_guard<std::mutex> lk(G.mu);
+    for (auto& p : G.pks) if (p->handle == handle) { *out = p; return H2B_OK; }
+    set_error("%s: unknown proving-key handle %llu", who, (unsigned long long)handle);
+    return H2B_ERR_BAD_ARGUMENT;
+}
+
+// a keygen job over the pk's domain, writing into it
+static KeygenJob pk_job(const ResidentPk& pk, int part, uint32_t first) {
+    KeygenJob job;
+    job.k = pk.k; job.extended_k = pk.extended_k; job.omega = pk.omega; job.omega_inv = pk.omega_inv; job.ifft_divisor = pk.ifft_divisor;
+    job.extended_omega = pk.extended_omega; job.zeta_powers = pk.zeta_powers;
+    job.resident = &pk; job.resident_part = part; job.resident_first = first;
+    return job;
+}
+
+// after the writing pass over columns [first, first + count) of `part`: filled when it succeeded, no longer trusted when it failed midway
+static int pk_mark(ResidentPk& pk, int part, uint32_t first, uint32_t count, int rc) {
+    std::lock_guard<std::mutex> lk(pk.filled_mu);
+    for (uint32_t i = first; i < first + count; ++i) pk.filled[part][i] = rc == H2B_OK;
+    return rc;
+}
+
+static int pk_range_check(const char* who, const ResidentPk& pk, int part, uint64_t first, uint64_t count) {
+    if (first + count > pk.count[part]) {
+        set_error("%s: columns %llu .. %llu of a part of %u columns", who, (unsigned long long)first, (unsigned long long)(first + count), pk.count[part]);
+        return H2B_ERR_BAD_ARGUMENT;
+    }
+    return H2B_OK;
+}
+
+int h2b_pk_create(uint32_t k, uint32_t extended_k, uint32_t n_fixed, uint32_t n_permutation, int layout, uint32_t halo, const uint64_t omega[4],
+                  const uint64_t omega_inv[4], const uint64_t ifft_divisor[4], const uint64_t extended_omega[4], const uint64_t zeta_powers[12],
+                  uint64_t* handle) {
+    static const char* who = "h2b_pk_create";
+    H2B_TRY(require_init());
+    if (k > 28 || extended_k < k || extended_k > 28) { set_error("%s: need k <= extended_k <= 28 (k = %u, extended_k = %u)", who, k, extended_k); return H2B_ERR_BAD_ARGUMENT; }
+    if (layout != H2B_PK_REPLICATED && layout != H2B_PK_ROW_SHARDED) { set_error("%s: unknown layout %d", who, layout); return H2B_ERR_BAD_ARGUMENT; }
+    if (!omega || !omega_inv || !ifft_divisor || !extended_omega || !zeta_powers || !handle) { set_error("%s: null pointer", who); return H2B_ERR_BAD_ARGUMENT; }
+    const size_t nd = G.devs.size(), E = (size_t)1 << extended_k;
+    PkRef pk(new ResidentPk());
+    pk->k = k; pk->extended_k = extended_k;
+    pk->count[H2B_PK_FIXED] = n_fixed; pk->count[H2B_PK_PERMUTATION] = n_permutation;
+    pk->sharded = layout == H2B_PK_ROW_SHARDED;
+    pk->halo = pk->sharded ? halo : 0;
+    memcpy(pk->omega, omega, 32); memcpy(pk->omega_inv, omega_inv, 32); memcpy(pk->ifft_divisor, ifft_divisor, 32);
+    memcpy(pk->extended_omega, extended_omega, 32); memcpy(pk->zeta_powers, zeta_powers, 96);
+    for (size_t d = 0; d < nd; ++d) {
+        const size_t r0 = pk->sharded ? E * d / nd : 0, r1 = pk->sharded ? E * (d + 1) / nd : E;
+        pk->row0.push_back(r0);
+        pk->rows.push_back(r1 - r0);
+        pk->ext_rows.push_back(r1 - r0 + 2 * (size_t)pk->halo);
+        if (pk->ext_rows[d] > E) {
+            set_error("%s: device %zu holds %zu rows + 2 x %u halo rows of a 2^%u-row coset", who, d, r1 - r0, pk->halo, extended_k);
+            return H2B_ERR_BAD_ARGUMENT;
+        }
+        pk->ordinal.push_back(G.devs[d]->device);
+    }
+    for (int p = 0; p < 3; ++p) pk->filled[p].assign(pk->count[p], 0);
+    pk->dev.assign(nd, nullptr);
+    for (size_t d = 0; d < nd; ++d) {
+        H2B_CUDA(cudaSetDevice(pk->ordinal[d]));
+        H2B_TRY(dev_malloc(&pk->dev[d], pk->bytes_on(d), "the resident proving key"));     // pk's destructor frees what was reserved
+    }
+    std::lock_guard<std::mutex> lk(G.mu);
+    pk->handle = G.next_handle++;
+    G.pks.push_back(pk);
+    *handle = pk->handle;
+    return H2B_OK;
+}
+
+int h2b_keygen_fixed_build_pk_resident(const uint64_t* const* fixed, uint32_t n_fixed, const uint8_t* const* activations, uint32_t n_selectors,
+                                       const uint32_t* combination_of, const uint32_t* root_of, uint32_t n_combinations, uint64_t handle, uint32_t first_column) {
+    static const char* who = "h2b_keygen_fixed_build_pk_resident";
+    PkRef pk;
+    H2B_TRY(pk_lookup(who, handle, &pk));
+    SelectorCombinations comb;
+    H2B_TRY(fixed_keygen_check(who, fixed, n_fixed, activations, n_selectors, combination_of, root_of, n_combinations, pk->k, &comb));
+    const uint32_t total = n_fixed + n_combinations;
+    H2B_TRY(pk_range_check(who, *pk, H2B_PK_FIXED, first_column, total));
+    std::lock_guard<std::mutex> lk(pk->build);
+    KeygenJob job = pk_job(*pk, H2B_PK_FIXED, first_column);
+    job.fixed = fixed; job.n_fixed = n_fixed; job.comb = &comb;
+    job.col_begin = 0; job.col_end = total;
+    // nothing is stored before every combination column has been built once and found valid
+    if (n_combinations) {
+        job.validate_only = true;
+        job.col_begin = n_fixed;
+        H2B_TRY(keygen_run(who, job));
+        job.validate_only = false;
+        job.col_begin = 0;
+    }
+    return pk_mark(*pk, H2B_PK_FIXED, first_column, total, keygen_run(who, job));
+}
+
+int h2b_permutation_build_pk_resident(const uint64_t* const* mapping, uint32_t n_columns, const uint64_t delta[4], uint64_t handle) {
+    static const char* who = "h2b_permutation_build_pk_resident";
+    PkRef pk;
+    H2B_TRY(pk_lookup(who, handle, &pk));
+    H2B_TRY(keygen_check(who, mapping, n_columns, pk->k, delta, pk->omega));
+    if (n_columns != pk->count[H2B_PK_PERMUTATION]) {
+        set_error("%s: %u mapping columns for a pk of %u permutation columns", who, n_columns, pk->count[H2B_PK_PERMUTATION]);
+        return H2B_ERR_BAD_ARGUMENT;
+    }
+    std::lock_guard<std::mutex> lk(pk->build);
+    KeygenJob job = pk_job(*pk, H2B_PK_PERMUTATION, 0);
+    job.mapping = mapping; job.n_sigma = n_columns; job.delta = delta;
+    job.col_begin = 0; job.col_end = n_columns;
+    // every entry is checked before the first column is stored: a pass that only builds sigma, then the real one
+    job.validate_only = true;
+    H2B_TRY(keygen_run(who, job));
+    job.validate_only = false;
+    return pk_mark(*pk, H2B_PK_PERMUTATION, 0, n_columns, keygen_run(who, job));
+}
+
+int h2b_keygen_lagrange_indicators_resident(uint64_t handle, uint32_t blinding_factors) {
+    static const char* who = "h2b_keygen_lagrange_indicators_resident";
+    PkRef pk;
+    H2B_TRY(pk_lookup(who, handle, &pk));
+    if ((uint64_t)blinding_factors + 1 >= ((uint64_t)1 << pk->k)) {
+        set_error("%s: k = %u, %u blinding factors (need bf + 1 < 2^k)", who, pk->k, blinding_factors);
+        return H2B_ERR_BAD_ARGUMENT;
+    }
+    std::lock_guard<std::mutex> lk(pk->build);
+    auto run = [&]() -> int {
+        DeviceCtx& c = *G.devs[0];
+        std::lock_guard<std::mutex> dlk(c.mu);
+        H2B_CUDA(cudaSetDevice(c.device));
+        const cudaStream_t st = c.stream;
+        KeygenScratch s;
+        s.ctx = &c;
+        // replicated: straight into device 0's columns, then peer copies; sharded: the whole cosets in scratch, then the slices
+        void* cols[3];
+        for (uint32_t i = 0; i < 3; ++i) {
+            if (pk->sharded) H2B_TRY(s.alloc(((size_t)1 << pk->extended_k) * 32, &cols[i]));
+            else cols[i] = pk->ptr(0, H2B_PK_INDICATORS, H2B_PK_EXTENDED, i);
+        }
+        c.prof.mark(PROF_BEGIN, st);
+        H2B_TRY(keygen_indicators_run(c, pk->k, pk->extended_k, blinding_factors, pk->omega_inv, pk->ifft_divisor, pk->extended_omega, pk->zeta_powers, cols,
+                                      st));
+        for (uint32_t i = 0; i < 3; ++i) H2B_TRY(pk_place(*pk, 0, st, cols[i], H2B_PK_INDICATORS, H2B_PK_EXTENDED, i));
+        H2B_CUDA(cudaStreamSynchronize(st));
+        return H2B_OK;
+    };
+    return pk_mark(*pk, H2B_PK_INDICATORS, 0, 3, run());
+}
+
+int h2b_pk_put_lagrange(uint64_t handle, int part, uint32_t first, uint32_t count, const uint64_t* const* values) {
+    static const char* who = "h2b_pk_put_lagrange";
+    PkRef pk;
+    H2B_TRY(pk_lookup(who, handle, &pk));
+    if (part != H2B_PK_FIXED && part != H2B_PK_PERMUTATION) {
+        set_error("%s: part %d (FIXED or PERMUTATION; the indicators come from h2b_keygen_lagrange_indicators_resident)", who, part);
+        return H2B_ERR_BAD_ARGUMENT;
+    }
+    H2B_TRY(pk_range_check(who, *pk, part, first, count));
+    if (count == 0) return H2B_OK;
+    if (!values) { set_error("%s: null values", who); return H2B_ERR_BAD_ARGUMENT; }
+    for (uint32_t j = 0; j < count; ++j) if (!values[j]) { set_error("%s: values[%u] is null", who, j); return H2B_ERR_BAD_ARGUMENT; }
+    std::lock_guard<std::mutex> lk(pk->build);
+    KeygenJob job = pk_job(*pk, part, first);
+    job.fixed = values; job.n_fixed = count;
+    job.col_begin = 0; job.col_end = count;
+    return pk_mark(*pk, part, first, count, keygen_run(who, job));
+}
+
+// the checks every reader of one column makes
+static int pk_column_check(const char* who, const ResidentPk& pk, int part, int form, uint32_t index) {
+    if (part < 0 || part > 2 || form < 0 || form > 2 || !ResidentPk::holds(part, form)) {
+        set_error("%s: part %d does not hold form %d", who, part, form);
+        return H2B_ERR_BAD_ARGUMENT;
+    }
+    if (index >= pk.count[part]) { set_error("%s: column %u of a part of %u columns", who, index, pk.count[part]); return H2B_ERR_BAD_ARGUMENT; }
+    std::lock_guard<std::mutex> lk(pk.filled_mu);
+    if (!pk.filled[part][index]) { set_error("%s: column %u of part %d was never filled", who, index, part); return H2B_ERR_BAD_ARGUMENT; }
+    return H2B_OK;
+}
+
+int h2b_pk_column(uint64_t handle, int device, int part, int form, uint32_t index, void** d_ptr, h2b_eval_shard* shard) {
+    static const char* who = "h2b_pk_column";
+    PkRef pk;
+    H2B_TRY(pk_lookup(who, handle, &pk));
+    if (device < 0 || (size_t)device >= pk->dev.size()) { set_error("%s: device index %d out of range (have %zu)", who, device, pk->dev.size()); return H2B_ERR_BAD_ARGUMENT; }
+    if (!d_ptr) { set_error("%s: null output", who); return H2B_ERR_BAD_ARGUMENT; }
+    H2B_TRY(pk_column_check(who, *pk, part, form, index));
+    *d_ptr = pk->ptr(device, part, form, index);
+    if (shard) {
+        const bool slice = form == H2B_PK_EXTENDED && pk->sharded;
+        shard->row0 = slice ? (uint32_t)pk->row0[device] : 0;
+        shard->rows = (uint32_t)(slice ? pk->rows[device] : pk->col_rows(device, form));
+        shard->halo = slice ? pk->halo : 0;
+    }
+    return H2B_OK;
+}
+
+int h2b_pk_download(uint64_t handle, int part, int form, uint32_t index, uint64_t* host_out) {
+    static const char* who = "h2b_pk_download";
+    PkRef pk;
+    H2B_TRY(pk_lookup(who, handle, &pk));
+    if (!host_out) { set_error("%s: null output", who); return H2B_ERR_BAD_ARGUMENT; }
+    H2B_TRY(pk_column_check(who, *pk, part, form, index));
+    const bool slices = form == H2B_PK_EXTENDED && pk->sharded;
+    for (size_t d = 0; d < (slices ? pk->dev.size() : 1); ++d) {
+        DeviceCtx& c = *G.devs[d];
+        std::lock_guard<std::mutex> lk(c.mu);
+        H2B_CUDA(cudaSetDevice(c.device));
+        // a sharded coset: the rows this device owns sit after its leading halo
+        const char* src = pk->ptr(d, part, form, index) + (slices ? (size_t)pk->halo * 32 : 0);
+        const size_t row = slices ? pk->row0[d] : 0, rows = slices ? pk->rows[d] : pk->col_rows(d, form);
+        H2B_TRY(host_download(c, host_out + 4 * row, src, rows * 32, c.stream));
+        H2B_CUDA(cudaStreamSynchronize(c.stream));
+    }
+    return H2B_OK;
+}
+
+int h2b_pk_info(uint64_t handle, uint64_t* per_device_bytes) {
+    PkRef pk;
+    H2B_TRY(pk_lookup("h2b_pk_info", handle, &pk));
+    if (per_device_bytes)
+        for (size_t d = 0; d < pk->dev.size(); ++d) per_device_bytes[d] = pk->bytes_on(d);
+    return H2B_OK;
+}
+
+int h2b_pk_release(uint64_t handle) {
+    PkRef drop;      // freed after G.mu is let go (the destructor waits for the devices)
+    {
+        std::lock_guard<std::mutex> lk(G.mu);
+        for (size_t i = 0; i < G.pks.size(); ++i)
+            if (G.pks[i]->handle == handle) { drop = G.pks[i]; G.pks.erase(G.pks.begin() + i); break; }
+    }
+    if (!drop) { set_error("h2b_pk_release: unknown proving-key handle %llu", (unsigned long long)handle); return H2B_ERR_BAD_ARGUMENT; }
+    return H2B_OK;
 }
 
 int h2b_srs_cache_clear(void) {

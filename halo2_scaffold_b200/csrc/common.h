@@ -79,7 +79,7 @@ enum ProfTag { PROF_BEGIN = 0, PROF_MSM_DECOMPOSE = 1, PROF_MSM_SCAN = 2, PROF_M
                PROF_G1NTT_TWIDDLE = 28, PROF_G1NTT_STAGES = 29, PROF_G1NTT_NORMALISE = 30,
                PROF_KEYGEN_UPLOAD = 31, PROF_KEYGEN_SIGMA = 32, PROF_KEYGEN_COMMIT = 33, PROF_KEYGEN_INTT = 34, PROF_KEYGEN_COSET = 35,
                PROF_KEYGEN_DOWNLOAD = 36, PROF_KEYGEN_PACK = 37, PROF_KEYGEN_EXCLUSION = 38, PROF_KEYGEN_FIXED_UPLOAD = 39,
-               PROF_KEYGEN_COMBINATION = 40 };
+               PROF_KEYGEN_COMBINATION = 40, PROF_PK_FORM_COPY = 41, PROF_PK_PLACE = 42 };
 struct Profiler {
     bool enabled = false;
     std::vector<cudaEvent_t> ev;

@@ -806,6 +806,69 @@ inline FixedProvingKey fixed_build_pk(const poly::kzg::ParamsKZG&, const poly::E
 }
 }  // namespace keygen
 
+// ProvingKey's fixed, permutation and indicator columns held on the devices from keygen to the last proof (h2b_pk_*): built there by
+// the keygen kernels, or registered from a key built elsewhere, and read by the device steps of create_proof through column().  RAII:
+// the destructor releases the handle (freeing waits for the work queued on the devices).
+class ProvingKeyOnDevice {
+  public:
+    ProvingKeyOnDevice(const poly::EvaluationDomain& domain, uint32_t n_fixed, uint32_t n_permutation, int layout = H2B_PK_REPLICATED,
+                       uint32_t halo = 0)
+        : k_(domain.k()), extended_k_(domain.extended_k()) {
+        ensure_init();
+        const Fr z[3] = {fr::one(), domain.get_g_coset(), domain.get_g_coset_inv()};
+        check(h2b_pk_create(k_, extended_k_, n_fixed, n_permutation, layout, halo, domain.get_omega().l, domain.get_omega_inv().l,
+                            domain.get_ifft_divisor().l, domain.get_extended_omega().l, z[0].l, &handle_),
+              "ProvingKeyOnDevice: create");
+    }
+    ~ProvingKeyOnDevice() { if (handle_) h2b_pk_release(handle_); }
+    ProvingKeyOnDevice(const ProvingKeyOnDevice&) = delete;
+    ProvingKeyOnDevice& operator=(const ProvingKeyOnDevice&) = delete;
+
+    void build_fixed(const std::vector<std::vector<Fr>>& fixed, const keygen::Activations& acts, const keygen::SelectorAssignment& a,
+                     uint32_t first_column = 0) {
+        const size_t n = (size_t)1 << k_;
+        const auto cols = keygen::fixed_columns_of(fixed, n);
+        const auto rows = keygen::activation_rows(acts, n);
+        check(h2b_keygen_fixed_build_pk_resident(cols.data(), (uint32_t)cols.size(), rows.data(), (uint32_t)rows.size(), a.combination_of.data(),
+                                                 a.root_of.data(), a.n_combinations, handle_, first_column),
+              "ProvingKeyOnDevice::build_fixed");
+    }
+    void build_permutation(const permutation::keygen::Mapping& mapping) {
+        const auto cols = permutation::keygen::columns_of(mapping, (size_t)1 << k_);
+        check(h2b_permutation_build_pk_resident(cols.data(), (uint32_t)cols.size(), permutation::keygen::delta().l, handle_),
+              "ProvingKeyOnDevice::build_permutation");
+    }
+    void build_indicators(uint32_t blinding_factors) {
+        check(h2b_keygen_lagrange_indicators_resident(handle_, blinding_factors), "ProvingKeyOnDevice::build_indicators");
+    }
+    // columns of a ProvingKey built elsewhere (the CPU keygen, ProvingKey::read), in Lagrange form
+    void put_lagrange(int part, uint32_t first, const std::vector<std::vector<Fr>>& values) {
+        const auto cols = keygen::fixed_columns_of(values, (size_t)1 << k_);
+        check(h2b_pk_put_lagrange(handle_, part, first, (uint32_t)cols.size(), cols.data()), "ProvingKeyOnDevice::put_lagrange");
+    }
+    // the column on `device`, valid while this object lives; *shard (optional) receives its slice
+    const void* column(int device, int part, int form, uint32_t index, h2b_eval_shard* shard = nullptr) const {
+        void* p = nullptr;
+        check(h2b_pk_column(handle_, device, part, form, index, &p, shard), "ProvingKeyOnDevice::column");
+        return p;
+    }
+    std::vector<Fr> download(int part, int form, uint32_t index) const {
+        std::vector<Fr> out((size_t)1 << (form == H2B_PK_EXTENDED ? extended_k_ : k_));
+        check(h2b_pk_download(handle_, part, form, index, reinterpret_cast<uint64_t*>(out.data())), "ProvingKeyOnDevice::download");
+        return out;
+    }
+    std::vector<uint64_t> info() const {
+        std::vector<uint64_t> bytes((size_t)h2b_device_count());
+        check(h2b_pk_info(handle_, bytes.data()), "ProvingKeyOnDevice::info");
+        return bytes;
+    }
+    uint64_t handle() const { return handle_; }
+
+  private:
+    uint32_t k_, extended_k_;
+    uint64_t handle_ = 0;
+};
+
 namespace lookup {
 // fn permute_expression_pair(..) -> Result<(Vec<F>, Vec<F>), Error>: the first usable_rows rows of (A', S')
 inline std::pair<std::vector<Fr>, std::vector<Fr>> permute_expression_pair(const std::vector<Fr>& input_expression, const std::vector<Fr>& table_expression,

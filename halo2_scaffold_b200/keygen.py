@@ -8,11 +8,15 @@ runs on the device: sigma, its commitments, its coefficient and extended-coset f
 The fixed half of keygen_vk / keygen_pk ([UP] plonk/circuit/compress_selectors.rs, plonk/keygen.rs) runs here too: compress_selectors
 takes process's exclusion matrix from the device and keeps upstream's greedy step on the host, and the fixed and combination columns
 get their commitments, coefficients and extended cosets on the device.  batch_invert_assigned stays with the caller.
+
+ResidentProvingKey keeps those columns on the devices as one handle (h2b_pk_*), built there by the same kernels, so that the prover's
+device steps read them instead of uploading them for every proof.
 """
 from __future__ import annotations
 
 import numpy as np
 
+from . import _lib
 from .domain import FR_MODULUS, FR_S, fr_to_words
 
 FR_GENERATOR = 7
@@ -108,3 +112,83 @@ def fixed_build_pk(params, domain, fixed, activations, assignment) -> dict:
     return params.lib.keygen_fixed_build_pk(fixed, activations, assignment["combination_of"], assignment["root_of"], assignment["n_combinations"],
                                             domain.k, domain.extended_k, fr_to_words(domain.omega_inv), fr_to_words(domain.ifft_divisor),
                                             fr_to_words(domain.extended_omega), _zeta_powers(domain))
+
+
+# ---- the proving key resident on the devices (include/h2b200.h h2b_pk_*) ------------------------------------------------------------
+_PARTS = {"fixed": _lib.PK_FIXED, "permutation": _lib.PK_PERMUTATION, "indicators": _lib.PK_INDICATORS}
+_FORMS = {"values": _lib.PK_VALUES, "coeff": _lib.PK_COEFF, "extended": _lib.PK_EXTENDED}
+_LAYOUTS = {"replicated": _lib.PK_REPLICATED, "row_sharded": _lib.PK_ROW_SHARDED}
+
+
+def _code(table, x):
+    return table[x] if isinstance(x, str) else int(x)
+
+
+class ResidentProvingKey:
+    """A ProvingKey's fixed, permutation and indicator columns held on the devices of the library from keygen to the last proof.
+
+    Fixed and permutation columns keep three forms each (values: Lagrange, coeff: lagrange_to_coeff, extended: coeff_to_extended), the
+    indicators l0 / l_last / l_active_row their extended form.  layout "replicated" puts every column on every device; "row_sharded"
+    keeps the n-row forms on every device and gives device d of D only its rows of each extended column plus `halo` rows on each side
+    -- the slice the row-sharded evaluate_h reads.  A context manager: the handle is released on exit."""
+
+    def __init__(self, domain, n_fixed: int, n_permutation: int, layout="replicated", halo: int = 0, lib=None):
+        self.lib = lib or domain.lib
+        self.domain = domain
+        self.n_fixed, self.n_permutation = int(n_fixed), int(n_permutation)
+        self.layout = _code(_LAYOUTS, layout)
+        d = domain
+        self.handle = self.lib.pk_create(d.k, d.extended_k, self.n_fixed, self.n_permutation, self.layout, halo, fr_to_words(d.omega),
+                                         fr_to_words(d.omega_inv), fr_to_words(d.ifft_divisor), fr_to_words(d.extended_omega), _zeta_powers(d))
+
+    def close(self):
+        if self.handle:
+            h, self.handle = self.handle, 0
+            self.lib.pk_release(h)
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    # ---- building ----
+    def build_fixed(self, fixed, activations, assignment, first_column: int = 0):
+        """keygen_pk's fixed columns (the caller's, then compress_selectors' combination columns) into FIXED columns first_column .."""
+        self.lib.keygen_fixed_build_pk_resident(fixed, activations, assignment["combination_of"], assignment["root_of"], assignment["n_combinations"],
+                                                self.domain.k, self.handle, first_column)
+
+    def build_permutation(self, mapping):
+        """Assembly::build_pk's sigma columns from the mapping ((P, 2^k, 2) (column, row) pairs)"""
+        self.lib.permutation_build_pk_resident(mapping, self.domain.k, fr_to_words(FR_DELTA), self.handle)
+
+    def build_indicators(self, blinding_factors: int):
+        """keygen_pk's l0, l_last, l_active_row"""
+        self.lib.keygen_lagrange_indicators_resident(self.handle, blinding_factors)
+
+    def put_lagrange(self, part, values, first: int = 0):
+        """columns of a ProvingKey built elsewhere, in Lagrange form; the other forms are derived on the device"""
+        self.lib.pk_put_lagrange(self.handle, _code(_PARTS, part), first, list(values), self.domain.k)
+
+    # ---- reading ----
+    def column(self, part, form, index: int, device: int = 0):
+        """-> (device pointer, (row0, rows, halo)) of one column on `device`"""
+        return self.lib.pk_column(self.handle, device, _code(_PARTS, part), _code(_FORMS, form), index)
+
+    def download(self, part, form, index: int) -> np.ndarray:
+        rows = 1 << (self.domain.extended_k if _code(_FORMS, form) == _lib.PK_EXTENDED else self.domain.k)
+        return self.lib.pk_download(self.handle, _code(_PARTS, part), _code(_FORMS, form), index, rows)
+
+    def info(self) -> list:
+        """bytes held on each device"""
+        return self.lib.pk_info(self.handle)
+
+    def eval_columns(self, device: int = 0) -> dict:
+        """what the h2b_evaluate_* entry points take from the pk on `device`: dict(fixed, permutation: lists of extended-coset pointers,
+        l0, l_last, l_active_row, shard: (row0, rows, halo) for the row-sharded entry points, None in the replicated layout)"""
+        ext = lambda part, i: self.column(part, "extended", i, device)
+        fixed = [ext("fixed", i) for i in range(self.n_fixed)]
+        perm = [ext("permutation", i) for i in range(self.n_permutation)]
+        ind = [ext("indicators", i) for i in range(3)]
+        return dict(fixed=[p for p, _ in fixed], permutation=[p for p, _ in perm], l0=ind[0][0], l_last=ind[1][0], l_active_row=ind[2][0],
+                    shard=ind[0][1] if self.layout == _lib.PK_ROW_SHARDED else None)

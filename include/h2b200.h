@@ -430,6 +430,56 @@ int h2b_keygen_fixed_build_pk(const uint64_t* const* fixed, uint32_t n_fixed, co
                               const uint64_t omega_inv[4], const uint64_t ifft_divisor[4], const uint64_t extended_omega[4], const uint64_t zeta_powers[12],
                               uint64_t* const* out_combination_values, uint64_t* const* out_polys, uint64_t* const* out_cosets);
 
+/* ---- the proving key resident on the devices ----------------------------------------------------------------------------------------
+ * [UP] halo2_proofs/src/plonk.rs ProvingKey: fixed_values / fixed_polys / fixed_cosets, permutation.{permutations, polys, cosets} and
+ * l0 / l_last / l_active_row, held on the devices of h2b_init from keygen to the last proof, so that create_proof's device steps read
+ * them instead of uploading them again for every proof.  A pk is a reference-counted object behind a handle, like a registered base set:
+ * a call holds it while it runs, h2b_pk_release drops the handle's reference, and device memory goes when the last holder lets go.
+ *   parts : FIXED       n_fixed columns -- the caller's fixed columns, then the combination columns (upstream's fixed.extend(selector_polys))
+ *           PERMUTATION n_permutation sigma columns
+ *           INDICATORS  l0, l_last, l_active_row (in that order)
+ *   forms : VALUES (Lagrange, 2^k rows), COEFF (2^k), EXTENDED (2^extended_k); FIXED and PERMUTATION hold all three, INDICATORS EXTENDED only
+ *   layout: REPLICATED  every device holds every form of every column
+ *           ROW_SHARDED every device holds the 2^k-row forms; of every EXTENDED column, device d of D holds its rows
+ *                       [floor(d E / D), floor((d + 1) E / D)) plus `halo` rows on each side, wrap-around included, starting at global row
+ *                       (row0 - halo) mod E (E = 2^extended_k): the slice h2b_evaluate_*_shard_dev takes, halo its largest rotated read. */
+enum h2b_pk_part { H2B_PK_FIXED = 0, H2B_PK_PERMUTATION = 1, H2B_PK_INDICATORS = 2 };
+enum h2b_pk_form { H2B_PK_VALUES = 0, H2B_PK_COEFF = 1, H2B_PK_EXTENDED = 2 };
+enum h2b_pk_layout { H2B_PK_REPLICATED = 0, H2B_PK_ROW_SHARDED = 1 };
+/* An empty pk with every byte of its storage reserved on every device now (H2B_ERR_OOM if it does not fit, before any key generation).
+ * The domain constants (those of h2b_lagrange_to_coeff_dev_batch / h2b_coeff_to_extended_dev_batch, plus omega) are stored with it and
+ * used by every later build.  k > 28, extended_k < k or > 28, an unknown layout, a null pointer and, in the sharded layout,
+ * rows + 2 halo > 2^extended_k for some device fail with H2B_ERR_BAD_ARGUMENT.  halo is ignored in the replicated layout. */
+int h2b_pk_create(uint32_t k, uint32_t extended_k, uint32_t n_fixed, uint32_t n_permutation, int layout, uint32_t halo, const uint64_t omega[4],
+                  const uint64_t omega_inv[4], const uint64_t ifft_divisor[4], const uint64_t extended_omega[4], const uint64_t zeta_powers[12],
+                  uint64_t* handle);
+/* h2b_keygen_fixed_build_pk with the pk as its destination: the n_fixed + n_combinations columns go to FIXED columns first_column ..,
+ * all three forms.  Refuses what h2b_keygen_fixed_build_pk refuses (k and the constants are the pk's), an unknown handle and columns past
+ * the pk's n_fixed; every combination column is checked before anything is stored, so a refused call leaves the pk as it was.  Nothing
+ * passes through the host: forms are copied off the group buffers on the device and placed on the other devices by peer copies.
+ * Synchronous. */
+int h2b_keygen_fixed_build_pk_resident(const uint64_t* const* fixed, uint32_t n_fixed, const uint8_t* const* activations, uint32_t n_selectors,
+                                       const uint32_t* combination_of, const uint32_t* root_of, uint32_t n_combinations, uint64_t pk, uint32_t first_column);
+/* h2b_permutation_build_pk into the pk's PERMUTATION part (n_columns must equal its n_permutation); every mapping entry is checked first. */
+int h2b_permutation_build_pk_resident(const uint64_t* const* mapping, uint32_t n_columns, const uint64_t delta[4], uint64_t pk);
+/* h2b_keygen_lagrange_indicators_dev into the pk's INDICATORS (computed on device 0, placed on the others).  bf + 1 >= 2^k fails. */
+int h2b_keygen_lagrange_indicators_resident(uint64_t pk, uint32_t blinding_factors);
+/* Registers a proving key built elsewhere (the CPU keygen, ProvingKey::read): values[j] (2^k x 32 B Lagrange form, pageable is fine)
+ * becomes column first + j of `part` (FIXED or PERMUTATION), and COEFF / EXTENDED are derived on the device by the conversions keygen
+ * uses -- the pk then equals what the device keygen stores.  INDICATORS are built with h2b_keygen_lagrange_indicators_resident. */
+int h2b_pk_put_lagrange(uint64_t pk, int part, uint32_t first, uint32_t count, const uint64_t* const* values);
+/* *d_ptr = the column on `device` (an index into the devices of h2b_init), valid while the handle is held.  shard (may be NULL) receives
+ * {row0, rows, halo} of the slice: of a sharded EXTENDED column, this device's; of any other column {0, its length, 0}.  A column never
+ * filled, a form the part does not hold, an index out of range, a device outside h2b_init and an unknown handle fail with
+ * H2B_ERR_BAD_ARGUMENT. */
+int h2b_pk_column(uint64_t pk, int device, int part, int form, uint32_t index, void** d_ptr, h2b_eval_shard* shard);
+/* a host copy of one column (2^k or 2^extended_k x 32 B) -- a sharded EXTENDED column is assembled from the devices' slices */
+int h2b_pk_download(uint64_t pk, int part, int form, uint32_t index, uint64_t* host_out);
+/* per_device_bytes[d] (h2b_device_count() entries, may be NULL): the storage the pk holds on device d */
+int h2b_pk_info(uint64_t pk, uint64_t* per_device_bytes);
+/* drops the handle; freeing waits for the work queued on the pk's devices.  An unknown or already released handle fails. */
+int h2b_pk_release(uint64_t pk);
+
 /* ---- raw device memory helpers (so that non-CUDA hosts -- ctypes, Rust -- can hold device buffers) --- */
 int h2b_dev_alloc(int device, size_t bytes, void** out);
 int h2b_dev_free(int device, void* p);
@@ -479,7 +529,8 @@ unsigned long long h2b_launch_count(void);
  * 34 inverse NTTs (lagrange_to_coeff), 35 coset NTTs (coeff_to_extended), 36 downloads; the MSM / NTT tags recorded inside a phase
  * belong to the keygen tag that follows them;  h2b_selector_exclusion and h2b_keygen_fixed_build_vk / _pk add 37 selector uploads
  * and packing (all selectors of the call or device at once), 38 exclusion kernel, 39 fixed column upload, 40 combination column
- * kernel, with 33 - 36 as above. */
+ * kernel, with 33 - 36 as above;  the resident pk builds (h2b_*_resident, h2b_pk_put_lagrange) add 41 form copies into the pk's storage on
+ * the computing device and 42 placement on the other devices (peer copies, sharded slices), in place of 36. */
 int h2b_profile_enable(int device, int on);
 int h2b_profile_read(int device, int* tags, float* ms, int cap, int* count);
 /* force the MSM window size (0 = automatic) -- tuning / tests only */

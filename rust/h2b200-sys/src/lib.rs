@@ -125,6 +125,18 @@ extern "C" {
                                      root_of: *const u32, n_combinations: u32, k: u32, extended_k: u32, omega_inv: *const u64, ifft_divisor: *const u64,
                                      extended_omega: *const u64, zeta_powers: *const u64, out_combination_values: *const *mut u64,
                                      out_polys: *const *mut u64, out_cosets: *const *mut u64) -> c_int;
+    // the proving key resident on the devices (h2b_pk_*)
+    pub fn h2b_pk_create(k: u32, extended_k: u32, n_fixed: u32, n_permutation: u32, layout: c_int, halo: u32, omega: *const u64, omega_inv: *const u64,
+                         ifft_divisor: *const u64, extended_omega: *const u64, zeta_powers: *const u64, handle: *mut u64) -> c_int;
+    pub fn h2b_keygen_fixed_build_pk_resident(fixed: *const *const u64, n_fixed: u32, activations: *const *const u8, n_selectors: u32,
+                                              combination_of: *const u32, root_of: *const u32, n_combinations: u32, pk: u64, first_column: u32) -> c_int;
+    pub fn h2b_permutation_build_pk_resident(mapping: *const *const u64, n_columns: u32, delta: *const u64, pk: u64) -> c_int;
+    pub fn h2b_keygen_lagrange_indicators_resident(pk: u64, blinding_factors: u32) -> c_int;
+    pub fn h2b_pk_put_lagrange(pk: u64, part: c_int, first: u32, count: u32, values: *const *const u64) -> c_int;
+    pub fn h2b_pk_column(pk: u64, device: c_int, part: c_int, form: c_int, index: u32, d_ptr: *mut *mut c_void, shard: *mut h2b_eval_shard) -> c_int;
+    pub fn h2b_pk_download(pk: u64, part: c_int, form: c_int, index: u32, host_out: *mut u64) -> c_int;
+    pub fn h2b_pk_info(pk: u64, per_device_bytes: *mut u64) -> c_int;
+    pub fn h2b_pk_release(pk: u64) -> c_int;
     pub fn h2b_dev_alloc(device: c_int, bytes: usize, out: *mut *mut c_void) -> c_int;
     pub fn h2b_dev_free(device: c_int, p: *mut c_void) -> c_int;
     pub fn h2b_memcpy_h2d(device: c_int, d_dst: *mut c_void, h_src: *const c_void, bytes: usize) -> c_int;
@@ -396,4 +408,92 @@ pub fn keygen_fixed_build_pk(fixed: &[&[[u64; 4]]], activations: &[Vec<bool>], a
         panic!("h2b_keygen_fixed_build_pk failed ({rc}): {}", last_error());
     }
     (values, polys, cosets)
+}
+
+// ---- the proving key resident on the devices ------------------------------------------------------------------------------------
+pub const PK_FIXED: c_int = 0;
+pub const PK_PERMUTATION: c_int = 1;
+pub const PK_INDICATORS: c_int = 2;
+pub const PK_VALUES: c_int = 0;
+pub const PK_COEFF: c_int = 1;
+pub const PK_EXTENDED: c_int = 2;
+pub const PK_REPLICATED: c_int = 0;
+pub const PK_ROW_SHARDED: c_int = 1;
+
+/// A `ProvingKey`'s fixed, permutation and indicator columns held on the devices (`h2b_pk_*`).  Every call panics on a non-zero
+/// return code, as the upstream functions' asserts do; `Drop` releases the handle.
+pub struct ResidentProvingKey {
+    pub handle: u64,
+    pub k: u32,
+    pub extended_k: u32,
+}
+
+impl ResidentProvingKey {
+    pub fn new(dom: &KeygenDomain, n_fixed: u32, n_permutation: u32, layout: c_int, halo: u32) -> Self {
+        ensure_init();
+        let mut handle = 0u64;
+        let rc = unsafe {
+            h2b_pk_create(dom.k, dom.extended_k, n_fixed, n_permutation, layout, halo, dom.omega.as_ptr(), dom.omega_inv.as_ptr(), dom.ifft_divisor.as_ptr(),
+                          dom.extended_omega.as_ptr(), dom.zeta_powers.as_ptr() as *const u64, &mut handle)
+        };
+        if rc != 0 {
+            panic!("h2b_pk_create failed ({rc}): {}", last_error());
+        }
+        ResidentProvingKey { handle, k: dom.k, extended_k: dom.extended_k }
+    }
+
+    fn check(rc: c_int, what: &str) {
+        if rc != 0 {
+            panic!("{what} failed ({rc}): {}", last_error());
+        }
+    }
+
+    /// keygen_pk's fixed columns (the caller's, then the combination columns) into FIXED columns `first_column ..`
+    pub fn build_fixed(&self, fixed: &[&[[u64; 4]]], activations: &[Vec<bool>], a: &SelectorAssignment, first_column: u32) {
+        let n = 1usize << self.k;
+        let (f, rows) = (fixed_rows(fixed, n), activation_rows(activations, n));
+        Self::check(unsafe {
+            h2b_keygen_fixed_build_pk_resident(f.as_ptr(), f.len() as u32, rows.as_ptr(), rows.len() as u32, a.combination_of.as_ptr(), a.root_of.as_ptr(),
+                                               a.n_combinations, self.handle, first_column)
+        }, "h2b_keygen_fixed_build_pk_resident");
+    }
+
+    /// `Assembly::build_pk` into the PERMUTATION part; panics like upstream's out-of-range index on an invalid mapping entry
+    pub fn build_permutation(&self, mapping: &[Vec<(usize, usize)>], delta: &[u64; 4]) {
+        let (_owned, ptrs) = mapping_columns(mapping, 1usize << self.k);
+        Self::check(unsafe { h2b_permutation_build_pk_resident(ptrs.as_ptr(), ptrs.len() as u32, delta.as_ptr(), self.handle) },
+                    "h2b_permutation_build_pk_resident");
+    }
+
+    pub fn build_indicators(&self, blinding_factors: u32) {
+        Self::check(unsafe { h2b_keygen_lagrange_indicators_resident(self.handle, blinding_factors) }, "h2b_keygen_lagrange_indicators_resident");
+    }
+
+    /// columns of a `ProvingKey` built elsewhere, in Lagrange form
+    pub fn put_lagrange(&self, part: c_int, first: u32, values: &[&[[u64; 4]]]) {
+        let v = fixed_rows(values, 1usize << self.k);
+        Self::check(unsafe { h2b_pk_put_lagrange(self.handle, part, first, v.len() as u32, v.as_ptr()) }, "h2b_pk_put_lagrange");
+    }
+
+    /// the column on `device` and its slice (row0, rows, halo); the pointer is valid while `self` lives
+    pub fn column(&self, device: c_int, part: c_int, form: c_int, index: u32) -> (*mut c_void, h2b_eval_shard) {
+        let mut p = std::ptr::null_mut();
+        let mut shard = h2b_eval_shard { row0: 0, rows: 0, halo: 0 };
+        Self::check(unsafe { h2b_pk_column(self.handle, device, part, form, index, &mut p, &mut shard) }, "h2b_pk_column");
+        (p, shard)
+    }
+
+    /// a host copy of one column, for `ProvingKey`'s host fields and `pk.write`
+    pub fn download(&self, part: c_int, form: c_int, index: u32) -> Vec<[u64; 4]> {
+        let rows = 1usize << if form == PK_EXTENDED { self.extended_k } else { self.k };
+        let mut out = vec![[0u64; 4]; rows];
+        Self::check(unsafe { h2b_pk_download(self.handle, part, form, index, out.as_mut_ptr() as *mut u64) }, "h2b_pk_download");
+        out
+    }
+}
+
+impl Drop for ResidentProvingKey {
+    fn drop(&mut self) {
+        unsafe { h2b_pk_release(self.handle) };
+    }
 }
