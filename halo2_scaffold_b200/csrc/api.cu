@@ -1515,20 +1515,23 @@ int h2b_permutation_sigma_dev(int device, const void* const* d_mapping, uint32_t
     return permutation_sigma_run(*c, d_mapping, n_columns, 0, n_columns, k, d_sigma, d_status, st);
 }
 
+// the domain arguments of the keygen_pk entry points: the sizes and the constants of the iNTT and the coset NTT
+static int domain_check(const char* who, uint32_t k, uint32_t extended_k, const uint64_t* omega_inv, const uint64_t* ifft_divisor,
+                        const uint64_t* extended_omega, const uint64_t* zeta_powers) {
+    if (extended_k > 28 || extended_k < k) { set_error("%s: need k <= extended_k <= 28 (k = %u, extended_k = %u)", who, k, extended_k); return H2B_ERR_BAD_ARGUMENT; }
+    if (!omega_inv || !ifft_divisor || !extended_omega || !zeta_powers) { set_error("%s: null pointer", who); return H2B_ERR_BAD_ARGUMENT; }
+    return H2B_OK;
+}
+
 int h2b_keygen_lagrange_indicators_dev(int device, uint32_t k, uint32_t extended_k, uint32_t blinding_factors, const uint64_t omega_inv[4],
                                        const uint64_t ifft_divisor[4], const uint64_t extended_omega[4], const uint64_t zeta_powers[12], void* d_l0,
                                        void* d_l_last, void* d_l_active_row, void* stream) {
     DeviceCtx* c = nullptr;
     H2B_TRY(get_ctx(device, &c));
-    if (extended_k > 28 || extended_k < k || (uint64_t)blinding_factors + 1 >= ((uint64_t)1 << k)) {
-        set_error("h2b_keygen_lagrange_indicators_dev: k = %u, extended_k = %u, %u blinding factors (need k <= extended_k <= 28 and bf + 1 < 2^k)", k,
-                  extended_k, blinding_factors);
-        return H2B_ERR_BAD_ARGUMENT;
-    }
-    if (!omega_inv || !ifft_divisor || !extended_omega || !zeta_powers || !d_l0 || !d_l_last || !d_l_active_row) {
-        set_error("h2b_keygen_lagrange_indicators_dev: null pointer");
-        return H2B_ERR_BAD_ARGUMENT;
-    }
+    static const char* who = "h2b_keygen_lagrange_indicators_dev";
+    H2B_TRY(domain_check(who, k, extended_k, omega_inv, ifft_divisor, extended_omega, zeta_powers));
+    if ((uint64_t)blinding_factors + 1 >= ((uint64_t)1 << k)) { set_error("%s: k = %u, %u blinding factors (need bf + 1 < 2^k)", who, k, blinding_factors); return H2B_ERR_BAD_ARGUMENT; }
+    if (!d_l0 || !d_l_last || !d_l_active_row) { set_error("%s: null pointer", who); return H2B_ERR_BAD_ARGUMENT; }
     std::lock_guard<std::mutex> lk(c->mu);
     void* cols[3] = {d_l0, d_l_last, d_l_active_row};
     return keygen_indicators_run(*c, k, extended_k, blinding_factors, omega_inv, ifft_divisor, extended_omega, zeta_powers, cols, (cudaStream_t)stream);
@@ -1620,6 +1623,13 @@ static int pk_place(const ResidentPk& pk, size_t d, cudaStream_t st, const void*
     return H2B_OK;
 }
 
+// after the writing pass over columns [first, first + count) of `part`: filled when it succeeded, no longer trusted when it failed midway
+static int pk_mark(ResidentPk& pk, int part, uint32_t first, uint32_t count, int rc) {
+    std::lock_guard<std::mutex> lk(pk.filled_mu);
+    for (uint32_t i = first; i < first + count; ++i) pk.filled[part][i] = rc == H2B_OK;
+    return rc;
+}
+
 // One build_vk / build_pk pass over the columns [col_begin, col_end); column i runs on device i mod D.  Column i's Lagrange values
 // come from, in this order: sigma of mapping[i] for i < n_sigma, the caller's fixed[i - n_sigma] for the next n_fixed, and the
 // combination columns of `comb` after those.
@@ -1637,7 +1647,7 @@ struct KeygenJob {
     uint64_t* const* values_out = nullptr;      // per column (indexed by column; an entry may be null), or null
     uint64_t* const* poly_out = nullptr;
     uint64_t* const* coset_out = nullptr;
-    const ResidentPk* resident = nullptr;       // every form of column i goes to column resident_first + i of resident_part
+    ResidentPk* resident = nullptr;             // every form of column i goes to column resident_first + i of resident_part
     int resident_part = 0;
     uint32_t resident_first = 0;
     uint32_t n_columns() const { return n_sigma + n_fixed + (comb ? comb->n_combinations : 0); }
@@ -1788,33 +1798,27 @@ static int keygen_device(size_t d, const KeygenJob& job, uint32_t* bad) {
             H2B_CUDA(cudaStreamSynchronize(st));
             for (size_t t = 0; t < m; ++t) memcpy(job.commitments + 12 * (size_t)mine[g0 + t], &blocks[28 * t], 96);
         }
-        if (job.values_out) {
-            for (size_t t = 0; t < m; ++t)
-                if (job.values_out[mine[g0 + t]]) H2B_TRY(host_download(c, job.values_out[mine[g0 + t]], cols[t], n * 32, st));
-            c.prof.mark(PROF_KEYGEN_DOWNLOAD, st);
-        }
-        // the resident pk takes each form off the group buffer before the next in-place transform
-        auto store = [&](int form) -> int {
-            for (size_t t = 0; t < m; ++t) H2B_TRY(pk_place(*job.resident, d, st, cols[t], job.resident_part, form, job.resident_first + mine[g0 + t]));
+        // each form goes to the caller's arrays and into the resident pk before the next in-place transform
+        auto emit = [&](int form) -> int {
+            uint64_t* const* out = form == H2B_PK_VALUES ? job.values_out : form == H2B_PK_COEFF ? job.poly_out : job.coset_out;
+            if (out) {
+                for (size_t t = 0; t < m; ++t)
+                    if (out[mine[g0 + t]]) H2B_TRY(host_download(c, out[mine[g0 + t]], cols[t], form == H2B_PK_EXTENDED ? col_bytes : n * 32, st));
+                c.prof.mark(PROF_KEYGEN_DOWNLOAD, st);
+            }
+            if (job.resident)
+                for (size_t t = 0; t < m; ++t) H2B_TRY(pk_place(*job.resident, d, st, cols[t], job.resident_part, form, job.resident_first + mine[g0 + t]));
             return H2B_OK;
         };
-        if (job.resident) H2B_TRY(store(H2B_PK_VALUES));
+        H2B_TRY(emit(H2B_PK_VALUES));
         if (!pk) continue;
         H2B_TRY(lagrange_to_coeff_batch_run(c, cols.data(), m, k, job.omega_inv, job.ifft_divisor, st));
         c.prof.mark(PROF_KEYGEN_INTT, st);
-        if (job.poly_out) {
-            for (size_t t = 0; t < m; ++t) H2B_TRY(host_download(c, job.poly_out[mine[g0 + t]], cols[t], n * 32, st));
-            c.prof.mark(PROF_KEYGEN_DOWNLOAD, st);
-        }
-        if (job.resident) H2B_TRY(store(H2B_PK_COEFF));
+        H2B_TRY(emit(H2B_PK_COEFF));
         if (want_coset) {
             H2B_TRY(coeff_to_extended_batch_run(c, cols.data(), m, k, job.extended_k, job.extended_omega, job.zeta_powers, st));
             c.prof.mark(PROF_KEYGEN_COSET, st);
-            if (job.coset_out) {
-                for (size_t t = 0; t < m; ++t) H2B_TRY(host_download(c, job.coset_out[mine[g0 + t]], cols[t], col_bytes, st));
-                c.prof.mark(PROF_KEYGEN_DOWNLOAD, st);
-            }
-            if (job.resident) H2B_TRY(store(H2B_PK_EXTENDED));
+            H2B_TRY(emit(H2B_PK_EXTENDED));
         }
         // the next group's uploads into the group buffer must not overtake the copies out of it
         if (job.resident) H2B_CUDA(cudaStreamSynchronize(st));
@@ -1842,6 +1846,24 @@ static int keygen_run(const char* who, const KeygenJob& job) {
         return H2B_ERR_BAD_ARGUMENT;
     }
     return H2B_OK;
+}
+
+// The build_pk of every column of `job`: a pass that only builds and checks the columns [first_checked, end) -- the ones that can be
+// invalid -- then, when the job has an output, the pass that writes it.  So no caller memory and no resident column is written before
+// every sigma entry and combination column has been found valid.  The resident columns are marked after the writing pass only: a
+// refused build leaves what the pk held readable.
+static int keygen_build(const char* who, KeygenJob job, uint32_t first_checked) {
+    job.col_begin = 0;
+    job.col_end = job.n_columns();
+    if (first_checked < job.col_end) {
+        KeygenJob check = job;
+        check.validate_only = true;
+        check.col_begin = first_checked;
+        H2B_TRY(keygen_run(who, check));
+    }
+    if (!job.values_out && !job.poly_out && !job.coset_out && !job.resident) return H2B_OK;
+    const int rc = keygen_run(who, job);
+    return job.resident ? pk_mark(*job.resident, job.resident_part, job.resident_first, job.col_end, rc) : rc;
 }
 
 // commitments of every column of `job` over a registered g_lagrange set (the caller has checked that it holds at least n points)
@@ -1909,22 +1931,15 @@ int h2b_permutation_build_pk(const uint64_t* const* mapping, uint32_t n_columns,
                              const uint64_t zeta_powers[12], uint64_t* const* out_permutations, uint64_t* const* out_polys, uint64_t* const* out_cosets) {
     static const char* who = "h2b_permutation_build_pk";
     H2B_TRY(keygen_check(who, mapping, n_columns, k, delta, omega));
-    if (extended_k > 28 || extended_k < k) { set_error("%s: need k <= extended_k <= 28 (k = %u, extended_k = %u)", who, k, extended_k); return H2B_ERR_BAD_ARGUMENT; }
-    if (!omega_inv || !ifft_divisor || !extended_omega || !zeta_powers) { set_error("%s: null pointer", who); return H2B_ERR_BAD_ARGUMENT; }
+    H2B_TRY(domain_check(who, k, extended_k, omega_inv, ifft_divisor, extended_omega, zeta_powers));
     for (uint64_t* const* outs : {out_permutations, out_polys, out_cosets})
         if (outs)
             for (uint32_t i = 0; i < n_columns; ++i) if (!outs[i]) { set_error("%s: output column %u is null", who, i); return H2B_ERR_BAD_ARGUMENT; }
     KeygenJob job;
     job.mapping = mapping; job.n_sigma = n_columns; job.k = k; job.extended_k = extended_k; job.delta = delta; job.omega = omega;
     job.omega_inv = omega_inv; job.ifft_divisor = ifft_divisor; job.extended_omega = extended_omega; job.zeta_powers = zeta_powers;
-    job.col_begin = 0; job.col_end = n_columns;
-    // every entry is checked before the first byte of caller memory is written: a pass that only builds sigma, then the real one
-    job.validate_only = true;
-    H2B_TRY(keygen_run(who, job));
-    if (!out_permutations && !out_polys && !out_cosets) return H2B_OK;
-    job.validate_only = false;
     job.values_out = out_permutations; job.poly_out = out_polys; job.coset_out = out_cosets;
-    return keygen_run(who, job);
+    return keygen_build(who, job, 0);
 }
 
 // ---- key generation: compress_selectors and the fixed columns of keygen_vk / keygen_pk --------------------------------------------
@@ -2021,8 +2036,7 @@ int h2b_keygen_fixed_build_pk(const uint64_t* const* fixed, uint32_t n_fixed, co
     static const char* who = "h2b_keygen_fixed_build_pk";
     SelectorCombinations comb;
     H2B_TRY(fixed_keygen_check(who, fixed, n_fixed, activations, n_selectors, combination_of, root_of, n_combinations, k, &comb));
-    if (extended_k > 28 || extended_k < k) { set_error("%s: need k <= extended_k <= 28 (k = %u, extended_k = %u)", who, k, extended_k); return H2B_ERR_BAD_ARGUMENT; }
-    if (!omega_inv || !ifft_divisor || !extended_omega || !zeta_powers) { set_error("%s: null pointer", who); return H2B_ERR_BAD_ARGUMENT; }
+    H2B_TRY(domain_check(who, k, extended_k, omega_inv, ifft_divisor, extended_omega, zeta_powers));
     const uint32_t total = n_fixed + n_combinations;
     if (out_combination_values)
         for (uint32_t c = 0; c < n_combinations; ++c)
@@ -2030,25 +2044,15 @@ int h2b_keygen_fixed_build_pk(const uint64_t* const* fixed, uint32_t n_fixed, co
     for (uint64_t* const* outs : {out_polys, out_cosets})
         if (outs)
             for (uint32_t i = 0; i < total; ++i) if (!outs[i]) { set_error("%s: output column %u is null", who, i); return H2B_ERR_BAD_ARGUMENT; }
-    KeygenJob job;
-    job.fixed = fixed; job.n_fixed = n_fixed; job.comb = &comb; job.k = k; job.extended_k = extended_k;
-    job.omega_inv = omega_inv; job.ifft_divisor = ifft_divisor; job.extended_omega = extended_omega; job.zeta_powers = zeta_powers;
-    job.col_begin = 0; job.col_end = total;
-    // no caller memory is written before every combination column has been built once and found valid
-    if (n_combinations) {
-        job.validate_only = true;
-        job.col_begin = n_fixed;
-        H2B_TRY(keygen_run(who, job));
-        job.validate_only = false;
-        job.col_begin = 0;
-    }
-    if (!out_combination_values && !out_polys && !out_cosets) return H2B_OK;
     std::vector<uint64_t*> values(total, nullptr);
     if (out_combination_values)
         for (uint32_t c = 0; c < n_combinations; ++c) values[n_fixed + c] = out_combination_values[c];
+    KeygenJob job;
+    job.fixed = fixed; job.n_fixed = n_fixed; job.comb = &comb; job.k = k; job.extended_k = extended_k;
+    job.omega_inv = omega_inv; job.ifft_divisor = ifft_divisor; job.extended_omega = extended_omega; job.zeta_powers = zeta_powers;
     job.values_out = out_combination_values ? values.data() : nullptr;
     job.poly_out = out_polys; job.coset_out = out_cosets;
-    return keygen_run(who, job);
+    return keygen_build(who, job, n_fixed);
 }
 
 // ---- the proving key resident on the devices ---------------------------------------------------------------------------------------
@@ -2061,19 +2065,12 @@ static int pk_lookup(const char* who, uint64_t handle, PkRef* out) {
 }
 
 // a keygen job over the pk's domain, writing into it
-static KeygenJob pk_job(const ResidentPk& pk, int part, uint32_t first) {
+static KeygenJob pk_job(ResidentPk& pk, int part, uint32_t first) {
     KeygenJob job;
     job.k = pk.k; job.extended_k = pk.extended_k; job.omega = pk.omega; job.omega_inv = pk.omega_inv; job.ifft_divisor = pk.ifft_divisor;
     job.extended_omega = pk.extended_omega; job.zeta_powers = pk.zeta_powers;
     job.resident = &pk; job.resident_part = part; job.resident_first = first;
     return job;
-}
-
-// after the writing pass over columns [first, first + count) of `part`: filled when it succeeded, no longer trusted when it failed midway
-static int pk_mark(ResidentPk& pk, int part, uint32_t first, uint32_t count, int rc) {
-    std::lock_guard<std::mutex> lk(pk.filled_mu);
-    for (uint32_t i = first; i < first + count; ++i) pk.filled[part][i] = rc == H2B_OK;
-    return rc;
 }
 
 static int pk_range_check(const char* who, const ResidentPk& pk, int part, uint64_t first, uint64_t count) {
@@ -2089,9 +2086,9 @@ int h2b_pk_create(uint32_t k, uint32_t extended_k, uint32_t n_fixed, uint32_t n_
                   uint64_t* handle) {
     static const char* who = "h2b_pk_create";
     H2B_TRY(require_init());
-    if (k > 28 || extended_k < k || extended_k > 28) { set_error("%s: need k <= extended_k <= 28 (k = %u, extended_k = %u)", who, k, extended_k); return H2B_ERR_BAD_ARGUMENT; }
+    H2B_TRY(domain_check(who, k, extended_k, omega_inv, ifft_divisor, extended_omega, zeta_powers));
     if (layout != H2B_PK_REPLICATED && layout != H2B_PK_ROW_SHARDED) { set_error("%s: unknown layout %d", who, layout); return H2B_ERR_BAD_ARGUMENT; }
-    if (!omega || !omega_inv || !ifft_divisor || !extended_omega || !zeta_powers || !handle) { set_error("%s: null pointer", who); return H2B_ERR_BAD_ARGUMENT; }
+    if (!omega || !handle) { set_error("%s: null pointer", who); return H2B_ERR_BAD_ARGUMENT; }
     const size_t nd = G.devs.size(), E = (size_t)1 << extended_k;
     PkRef pk(new ResidentPk());
     pk->k = k; pk->extended_k = extended_k;
@@ -2136,16 +2133,7 @@ int h2b_keygen_fixed_build_pk_resident(const uint64_t* const* fixed, uint32_t n_
     std::lock_guard<std::mutex> lk(pk->build);
     KeygenJob job = pk_job(*pk, H2B_PK_FIXED, first_column);
     job.fixed = fixed; job.n_fixed = n_fixed; job.comb = &comb;
-    job.col_begin = 0; job.col_end = total;
-    // nothing is stored before every combination column has been built once and found valid
-    if (n_combinations) {
-        job.validate_only = true;
-        job.col_begin = n_fixed;
-        H2B_TRY(keygen_run(who, job));
-        job.validate_only = false;
-        job.col_begin = 0;
-    }
-    return pk_mark(*pk, H2B_PK_FIXED, first_column, total, keygen_run(who, job));
+    return keygen_build(who, job, n_fixed);
 }
 
 int h2b_permutation_build_pk_resident(const uint64_t* const* mapping, uint32_t n_columns, const uint64_t delta[4], uint64_t handle) {
@@ -2160,12 +2148,7 @@ int h2b_permutation_build_pk_resident(const uint64_t* const* mapping, uint32_t n
     std::lock_guard<std::mutex> lk(pk->build);
     KeygenJob job = pk_job(*pk, H2B_PK_PERMUTATION, 0);
     job.mapping = mapping; job.n_sigma = n_columns; job.delta = delta;
-    job.col_begin = 0; job.col_end = n_columns;
-    // every entry is checked before the first column is stored: a pass that only builds sigma, then the real one
-    job.validate_only = true;
-    H2B_TRY(keygen_run(who, job));
-    job.validate_only = false;
-    return pk_mark(*pk, H2B_PK_PERMUTATION, 0, n_columns, keygen_run(who, job));
+    return keygen_build(who, job, 0);
 }
 
 int h2b_keygen_lagrange_indicators_resident(uint64_t handle, uint32_t blinding_factors) {
@@ -2215,8 +2198,7 @@ int h2b_pk_put_lagrange(uint64_t handle, int part, uint32_t first, uint32_t coun
     std::lock_guard<std::mutex> lk(pk->build);
     KeygenJob job = pk_job(*pk, part, first);
     job.fixed = values; job.n_fixed = count;
-    job.col_begin = 0; job.col_end = count;
-    return pk_mark(*pk, part, first, count, keygen_run(who, job));
+    return keygen_build(who, job, count);
 }
 
 // the checks every reader of one column makes

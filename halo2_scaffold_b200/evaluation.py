@@ -278,28 +278,37 @@ class Evaluator:
         lookups[n]  = dict(product_coset=, permuted_input_coset=, permuted_table_coset=)
         pk = a keygen.ResidentProvingKey: the fixed cosets, the permutation's sigma cosets and l0 / l_last / l_active_row are then read
         from it on `device` and not uploaded (fixed, permutation["cosets"] and the indicators are not needed); a row-sharded pk gives the
-        shard of `device`."""
+        shard of `device`.
+        shard = (row0, rows, halo): rows [row0, row0 + rows) only; every column is cut to its slice with `halo` rows on both sides
+        (wrap-around included) before it is uploaded -- what each device of a row-sharded evaluate_h holds (a row-sharded pk holds its
+        columns that way already).  -> the `rows` values of the shard"""
         L = lib or _lib.load()
         pk_cols = pk.eval_columns(device) if pk is not None else None
         if pk_cols is not None:
             assert shard is None or pk_cols["shard"] is not None, "a replicated pk feeds the unsharded evaluate_h"
             assert shard is None or tuple(shard) == tuple(pk_cols["shard"]), "this device's shard of the pk is %r" % (pk_cols["shard"],)
             shard = pk_cols["shard"]
-        if shard is not None:
-            return self._evaluate_h_shard(L, device, shard, size=size, rot_scale=rot_scale, fixed=fixed, advice=advice, instance=instance,
-                                          challenges=challenges, y=y, beta=beta, gamma=gamma, theta=theta, l0=l0, l_last=l_last, l_active_row=l_active_row,
-                                          permutation=permutation, lookups=lookups, values=values, pk_cols=pk_cols)
-        with _Device(L, device, size) as dev:
-            up = dev.up
+        assert len(lookups) == len(self.lookups)
+        row0, rows, halo = shard if shard is not None else (0, size, 0)
+        if values is None:
+            values = np.zeros((rows, 4), dtype=np.uint64)
+        elif shard is not None:
+            values = np.ascontiguousarray(values, dtype=np.uint64).reshape(-1, 4)[row0:row0 + rows]
+        with _Device(L, device, rows + 2 * halo) as dev, _Device(L, device, rows) as vdev:
+            if shard is None:
+                up = dev.up
+            else:
+                take = np.arange(row0 - halo, row0 + rows + halo) % size
+                up = lambda a: dev.up(np.ascontiguousarray(a, dtype=np.uint64).reshape(-1, 4)[take])
             d_advice, d_instance = [up(c) for c in advice], [up(c) for c in instance]
             if pk_cols is None:
                 d_fixed, d_l0, d_l_last, d_l_active = [up(c) for c in fixed], up(l0), up(l_last), up(l_active_row)
             else:
                 d_fixed, d_l0, d_l_last, d_l_active = pk_cols["fixed"], pk_cols["l0"], pk_cols["l_last"], pk_cols["l_active_row"]
-            d_values = up(values if values is not None else np.zeros((size, 4), dtype=np.uint64))
+            d_values = vdev.up(values)
             cols = _lib.EvalColumns(d_fixed, d_advice, d_instance, challenges, beta, gamma, theta, y)
             # Custom gates
-            L.evaluate_graph_dev(device, self.custom_gates.arrays(), cols, d_values, size, rot_scale)
+            L.evaluate_graph_dev(device, self.custom_gates.arrays(), cols, d_values, size, rot_scale, shard=shard)
             # Permutations
             if permutation is not None and permutation["product_cosets"]:
                 by_type = {"advice": d_advice, "fixed": d_fixed, "instance": d_instance}
@@ -307,42 +316,8 @@ class Evaluator:
                 L.evaluate_h_permutation_dev(device, d_values, size, rot_scale, [up(c) for c in permutation["product_cosets"]],
                                              [by_type[t][i] for t, i in permutation["columns"]], d_sigma,
                                              permutation["chunk_len"], permutation["last_rotation"], d_l0, d_l_last, d_l_active, beta, gamma, y,
-                                             permutation["delta"], permutation["zeta"], permutation["extended_omega"])
-            # Lookups
-            assert len(lookups) == len(self.lookups)
-            for graph, lk in zip(self.lookups, lookups):
-                L.evaluate_h_lookup_dev(device, graph.arrays(), cols, d_values, size, rot_scale, up(lk["product_coset"]),
-                                        up(lk["permuted_input_coset"]), up(lk["permuted_table_coset"]), d_l0, d_l_last, d_l_active)
-            return dev.down(d_values)
-
-    def _evaluate_h_shard(self, L, device, shard, *, size, rot_scale, fixed, advice, instance, challenges, y, beta, gamma, theta, l0, l_last, l_active_row,
-                          permutation, lookups, values, pk_cols=None):
-        """rows [row0, row0 + rows) only: every column is cut to its slice with `halo` rows on both sides (wrap-around included) before it is
-        uploaded -- what each device of a row-sharded evaluate_h holds (a row-sharded pk holds its columns that way already).  -> the `rows`
-        values of the shard"""
-        row0, rows, halo = shard
-        take = (np.arange(row0 - halo, row0 + rows + halo) % size)
-
-        def cut(a):
-            return np.ascontiguousarray(np.ascontiguousarray(a, dtype=np.uint64).reshape(-1, 4)[take])
-        with _Device(L, device, rows + 2 * halo) as dev, _Device(L, device, rows) as vdev:
-            up = lambda a: dev.up(cut(a))
-            d_advice, d_instance = [up(c) for c in advice], [up(c) for c in instance]
-            if pk_cols is None:
-                d_fixed, d_l0, d_l_last, d_l_active = [up(c) for c in fixed], up(l0), up(l_last), up(l_active_row)
-            else:
-                d_fixed, d_l0, d_l_last, d_l_active = pk_cols["fixed"], pk_cols["l0"], pk_cols["l_last"], pk_cols["l_active_row"]
-            v0 = np.zeros((rows, 4), dtype=np.uint64) if values is None else np.ascontiguousarray(values, dtype=np.uint64).reshape(-1, 4)[row0:row0 + rows]
-            d_values = vdev.up(v0)
-            cols = _lib.EvalColumns(d_fixed, d_advice, d_instance, challenges, beta, gamma, theta, y)
-            L.evaluate_graph_dev(device, self.custom_gates.arrays(), cols, d_values, size, rot_scale, shard=shard)
-            if permutation is not None and permutation["product_cosets"]:
-                by_type = {"advice": d_advice, "fixed": d_fixed, "instance": d_instance}
-                d_sigma = [up(c) for c in permutation["cosets"]] if pk_cols is None else pk_cols["permutation"]
-                L.evaluate_h_permutation_dev(device, d_values, size, rot_scale, [up(c) for c in permutation["product_cosets"]],
-                                             [by_type[t][i] for t, i in permutation["columns"]], d_sigma,
-                                             permutation["chunk_len"], permutation["last_rotation"], d_l0, d_l_last, d_l_active, beta, gamma, y,
                                              permutation["delta"], permutation["zeta"], permutation["extended_omega"], shard=shard)
+            # Lookups
             for graph, lk in zip(self.lookups, lookups):
                 L.evaluate_h_lookup_dev(device, graph.arrays(), cols, d_values, size, rot_scale, up(lk["product_coset"]),
                                         up(lk["permuted_input_coset"]), up(lk["permuted_table_coset"]), d_l0, d_l_last, d_l_active, shard=shard)

@@ -1,22 +1,17 @@
 """Builds tests/cpp/host_mirror_test.cpp against a given libh2b200 build, runs it on seeded inputs and checks every
 output file against the oracle (shared by the CPU emulator test and the GPU test)."""
-import os
 import subprocess
 
 import numpy as np
 
 import bn254 as o
 import parity_cases as pc
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+from harness import build_mirror
 
 
 def run_host_mirror(oc, lib_path, tmp_path, k=6, j=4):
     n = 1 << k
-    exe = str(tmp_path / "host_mirror_test")
-    libdir, libfile = os.path.split(lib_path)
-    subprocess.check_call(["g++", "-O2", "-std=c++17", "-Wall", "-o", exe, os.path.join(ROOT, "tests", "cpp", "host_mirror_test.cpp"),
-                           "-L" + libdir, "-l:" + libfile, "-Wl,-rpath," + libdir])
+    exe = build_mirror("host_mirror_test", lib_path, tmp_path)
     s, P, lag = oc.random_fr(0xC0 + k, n), oc.gen_points(0xC1 + k, n), oc.random_fr(0xC2 + k, n)
     s[1] = 0
     P[2] = 0

@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 import parity_cases as pc
+from harness import run_on_emulated_devices
 
 
 def test_field_arithmetic(emu, oc):
@@ -515,44 +516,32 @@ def test_lookup_compress_expressions(emu, oc):
     assert (got == want).all()
 
 
-def _emu_subprocess(emu, body, env_extra, timeout=900):
-    import os, subprocess, sys
-    root = pc.__file__.rsplit('/tests/', 1)[0]
-    code = ("import sys; sys.path[:0]=[%r,%r,%r]\n"
-            "import numpy as np, oracle_c as oc, parity_cases as pc\n"
-            "from halo2_scaffold_b200._lib import Lib\n"
-            "L=Lib(%r, allow_emulator=True); L.init(0)\n" % (root, root + '/oracle', root + '/tests', emu.path)) + body + "\nprint('ok')\n"
-    out = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, **env_extra), capture_output=True, text=True, timeout=timeout)
-    assert out.returncode == 0 and "ok" in out.stdout, (out.stdout[-1000:], out.stderr[-3000:])
-
-
 def test_implicit_cache_is_content_addressed(emu):
     # digest blocks of 16 points, arrays from 64 points on are cached: the logic of the 1024 / 4096 production values at CPU sizes
-    _emu_subprocess(emu, "pc.check_implicit_cache_is_content_addressed(L, oc, 320, 16)\n"
-                         "pc.check_implicit_cache_under_threads(L, oc, 256, threads=8, rounds=2)",
-                    dict(H2B_DIGEST_BLOCK_LOG="4", H2B_IMPLICIT_MIN_LOG="6"))
+    run_on_emulated_devices(None, "pc.check_implicit_cache_is_content_addressed(L, oc, 320, 16)\n"
+                                  "pc.check_implicit_cache_under_threads(L, oc, 256, threads=8, rounds=2)", None,
+                            dict(H2B_DIGEST_BLOCK_LOG="4", H2B_IMPLICIT_MIN_LOG="6"), timeout=900)
 
 
 def test_implicit_cache_can_be_disabled(emu):
-    _emu_subprocess(emu, "s, P = oc.random_fr(1, 256), oc.gen_points(2, 256)\n"
-                         "w = pc.affine_of(oc, oc.best_multiexp(s, P))\n"
-                         "assert all((pc.affine_of(oc, L.msm(s, P)) == w).all() for _ in range(2))\n"
-                         "st = L.implicit_cache_stats(); assert st['uploads'] == 0 and st['direct'] == 2, st",
-                    dict(H2B_DIGEST_BLOCK_LOG="4", H2B_IMPLICIT_MIN_LOG="6", H2B_IMPLICIT_CACHE="0"))
+    run_on_emulated_devices(None, "s, P = oc.random_fr(1, 256), oc.gen_points(2, 256)\n"
+                                  "w = pc.affine_of(oc, oc.best_multiexp(s, P))\n"
+                                  "assert all((pc.affine_of(oc, L.msm(s, P)) == w).all() for _ in range(2))\n"
+                                  "st = L.implicit_cache_stats(); assert st['uploads'] == 0 and st['direct'] == 2, st", None,
+                            dict(H2B_DIGEST_BLOCK_LOG="4", H2B_IMPLICIT_MIN_LOG="6", H2B_IMPLICIT_CACHE="0"), timeout=900)
 
 
 @pytest.mark.parametrize("devices", ["2", "3"])
 def test_multi_device_host_logic_on_emulated_devices(emu, devices):
-    # H2B_EMU_DEVICES: the emulator reports several devices, so point-range sharding, sharded base sets (tables per slice),
+    # the emulator reports several devices, so point-range sharding, sharded base sets (tables per slice),
     # the table all-gather of replicated sets, round-robin + batched columns and the implicit cache's sharded copies all run here
-    _emu_subprocess(emu, "assert L.device_count() == %s\n"
-                         "pc.check_sharded_base_set(L, oc, 700, spacing=8)\n"
-                         "pc.check_sharded_base_set(L, oc, 333, spacing=0, kind=1)\n"
-                         "pc.check_msm_tables(L, oc, 600, 8, kind=0, ranges=[(0, 600), (100, 450)])\n"
-                         "pc.check_msm(L, oc, 500, kind=1)\n"
-                         "pc.check_implicit_cache_is_content_addressed(L, oc, 320, 16)\n"
-                         "pc.check_batched_columns(L, oc, 300, 7, spacing=8)" % devices,
-                    dict(H2B_EMU_DEVICES=devices, H2B_MULTI_DEVICE_MIN_LOG="7", H2B_DIGEST_BLOCK_LOG="4", H2B_IMPLICIT_MIN_LOG="6"))
+    run_on_emulated_devices(None, "pc.check_sharded_base_set(L, oc, 700, spacing=8)\n"
+                                  "pc.check_sharded_base_set(L, oc, 333, spacing=0, kind=1)\n"
+                                  "pc.check_msm_tables(L, oc, 600, 8, kind=0, ranges=[(0, 600), (100, 450)])\n"
+                                  "pc.check_msm(L, oc, 500, kind=1)\n"
+                                  "pc.check_implicit_cache_is_content_addressed(L, oc, 320, 16)\n"
+                                  "pc.check_batched_columns(L, oc, 300, 7, spacing=8)", devices,
+                            dict(H2B_MULTI_DEVICE_MIN_LOG="7", H2B_DIGEST_BLOCK_LOG="4", H2B_IMPLICIT_MIN_LOG="6"), timeout=900)
 
 
 def test_fr_transpose(emu, oc):
@@ -564,14 +553,13 @@ def test_one_ntt_across_emulated_devices(emu, devices):
     # SURVEY.md 8e "one NTT across GPUs": the four-step split of h2b_ntt_bn254_fr (strided uploads of column blocks, transposes,
     # strided-batch transforms, twiddles, 2-D peer copies, strided downloads) against best_fft, both directions, odd and even log_n,
     # pageable host arrays through the staging threads with 1 KiB pieces (several rows per piece, several pieces per thread)
-    _emu_subprocess(emu, "assert L.device_count() == %s\n"
-                         "for k in (4, 5, 8, 11, 12, 13):\n"
-                         "    pc.check_ntt(L, oc, k)\n" % devices,
-                    dict(H2B_EMU_DEVICES=devices, H2B_NTT_MULTI_MIN_LOG="4", H2B_STAGE_PIECE_LOG="10", H2B_STAGE_THREADS="3"))
+    run_on_emulated_devices(None, "for k in (4, 5, 8, 11, 12, 13):\n"
+                                  "    pc.check_ntt(L, oc, k)\n", devices,
+                            dict(H2B_NTT_MULTI_MIN_LOG="4", H2B_STAGE_PIECE_LOG="10", H2B_STAGE_THREADS="3"), timeout=900)
     # the strided-batch mode of the multi-pass plans (2, 3 and 4 passes per row / column transform)
-    _emu_subprocess(emu, "for k in (12, 14, 15):\n"
-                         "    pc.check_ntt(L, oc, k)\n",
-                    dict(H2B_EMU_DEVICES=devices, H2B_NTT_MULTI_MIN_LOG="4", H2B_NTT_BMAX="2"))
+    run_on_emulated_devices(None, "for k in (12, 14, 15):\n"
+                                  "    pc.check_ntt(L, oc, k)\n", devices,
+                            dict(H2B_NTT_MULTI_MIN_LOG="4", H2B_NTT_BMAX="2"), timeout=900)
 
 
 @pytest.mark.parametrize("n,ncols,spacing,window", [(600, 6, 8, 0), (600, 5, 8, 4), (257, 9, 0, 0), (1200, 4, 12, 6), (40, 33, 6, 0), (300, 4, -1, 0)])
@@ -602,15 +590,15 @@ def test_msm_partitioned_sort(emu):
     # section 2c of msm.cu (two-level sort: partition histogram in shared memory, contiguous runs per partition, chunked placement
     # with shared-memory cursors) forced at CPU sizes -- it needs W <= 16 windows, i.e. 16-bit windows or wider: uniform /
     # witness-like / one-bucket columns (hot partitions), table and plain mode, ragged batches, chunked uploads, tiny chunks
-    _emu_subprocess(emu, "pc.check_msm_tables(L, oc, 3000, 16, kind=0, windows=(16,), ranges=[(0, 3000), (100, 2500)])\n"
-                         "pc.check_msm_tables(L, oc, 2500, 16, kind=1, windows=(16,))\n"
-                         "pc.check_msm_tables(L, oc, 1500, 18, kind=0, windows=(18,))\n"
-                         "pc.check_msm_single_bucket(L, oc, 20000, scalar=1, tables=True)\n"
-                         "pc.check_batched_columns(L, oc, 300, 3, spacing=16, window=16)",
-                    dict(H2B_MSM_SORT2_MIN_LOG="8", H2B_MSM_SORT2_CHUNK_LOG="7", H2B_MSM_PRECOMP="16"), timeout=2400)
-    _emu_subprocess(emu, "pc.check_msm_tables(L, oc, 4097, 16, kind=1, windows=(16,), ranges=[(0, 4097)])",
-                    dict(H2B_MSM_SORT2_MIN_LOG="8", H2B_MSM_UPLOAD_CHUNK_LOG="10"), timeout=2400)
+    run_on_emulated_devices(None, "pc.check_msm_tables(L, oc, 3000, 16, kind=0, windows=(16,), ranges=[(0, 3000), (100, 2500)])\n"
+                                  "pc.check_msm_tables(L, oc, 2500, 16, kind=1, windows=(16,))\n"
+                                  "pc.check_msm_tables(L, oc, 1500, 18, kind=0, windows=(18,))\n"
+                                  "pc.check_msm_single_bucket(L, oc, 20000, scalar=1, tables=True)\n"
+                                  "pc.check_batched_columns(L, oc, 300, 3, spacing=16, window=16)", None,
+                            dict(H2B_MSM_SORT2_MIN_LOG="8", H2B_MSM_SORT2_CHUNK_LOG="7", H2B_MSM_PRECOMP="16"), timeout=2400)
+    run_on_emulated_devices(None, "pc.check_msm_tables(L, oc, 4097, 16, kind=1, windows=(16,), ranges=[(0, 4097)])", None,
+                            dict(H2B_MSM_SORT2_MIN_LOG="8", H2B_MSM_UPLOAD_CHUNK_LOG="10"), timeout=2400)
     # the bucket scan of a partition in several passes of blockDim buckets (the 4096-bucket partitions of 22-bit tables)
-    _emu_subprocess(emu, "pc.check_msm_tables(L, oc, 3000, 16, kind=0, windows=(16,), ranges=[(0, 3000), (100, 2500)])\n"
-                         "pc.check_msm_tables(L, oc, 2500, 18, kind=1, windows=(18,))",
-                    dict(H2B_MSM_SORT2_MIN_LOG="8", H2B_MSM_SORT2_CHUNK_LOG="7", H2B_MSM_PLACE_SCAN_THREADS="32"), timeout=2400)
+    run_on_emulated_devices(None, "pc.check_msm_tables(L, oc, 3000, 16, kind=0, windows=(16,), ranges=[(0, 3000), (100, 2500)])\n"
+                                  "pc.check_msm_tables(L, oc, 2500, 18, kind=1, windows=(18,))", None,
+                            dict(H2B_MSM_SORT2_MIN_LOG="8", H2B_MSM_SORT2_CHUNK_LOG="7", H2B_MSM_PLACE_SCAN_THREADS="32"), timeout=2400)

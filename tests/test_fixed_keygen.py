@@ -7,41 +7,26 @@ no recollection of upstream: the exclusion matrix is np.any(a_i & a_j), no two m
 combination keeps max(deg - 1) + len <= max_degree, each substitution expression is non-zero exactly on its selector's rows, and
 commit_lagrange(column) = commit(poly) with extended_to_coeff(coset) = poly padded with zeros."""
 import ctypes
-import os
 import subprocess
-import sys
-import tempfile
 
 import numpy as np
 import pytest
 
 import bn254 as o
-import test_permutation_keygen as tp
-import test_srs_setup as ts
+from harness import (Consts, W, affine, build_mirror, build_oracle, disjoint, ints, orc_srs_setup, run_on_emulated_devices, sparse,
+                     threads)
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 H2B_ERR_BAD_ARGUMENT = -2
 R = o.R_MOD
-_ORACLE = None
 
 
 # ---- helpers ---------------------------------------------------------------------------------------------------------
 def oracle():
-    """tests/cpp/fixed_keygen_oracle.cpp, built once per process into a temporary directory"""
-    global _ORACLE
-    if _ORACLE is None:
-        d = tempfile.mkdtemp(prefix="fixed_keygen_oracle_")
-        so = os.path.join(d, "libfixed_keygen_oracle.so")
-        subprocess.check_call(["g++", "-O3", "-march=x86-64-v3", "-std=c++17", "-fPIC", "-shared", "-pthread", "-Wno-unused-function", "-o", so,
-                               os.path.join(ROOT, "tests", "cpp", "fixed_keygen_oracle.cpp")])
-        L = ctypes.CDLL(so)
-        vp, u32, i32 = ctypes.c_void_p, ctypes.c_uint32, ctypes.c_int
-        L.orc_selector_exclusion.argtypes = [vp, u32, u32, vp]
-        L.orc_compress_selectors.argtypes = [vp, vp, u32, u32, u32, vp, vp, vp, vp]
-        L.orc_compress_selectors.restype = u32
-        L.orc_fixed_build.argtypes = [vp, u32, u32, u32, vp, vp, vp, vp, vp, i32, vp, vp, vp]
-        _ORACLE = L
-    return _ORACLE
+    """tests/cpp/fixed_keygen_oracle.cpp"""
+    vp, u32, i32 = ctypes.c_void_p, ctypes.c_uint32, ctypes.c_int
+    return build_oracle("fixed_keygen_oracle", dict(orc_selector_exclusion=[vp, u32, u32, vp], orc_compress_selectors=[vp, vp, u32, u32, u32, vp, vp, vp, vp],
+                                                    orc_fixed_build=[vp, u32, u32, u32, vp, vp, vp, vp, vp, i32, vp, vp, vp]),
+                        restypes=dict(orc_compress_selectors=u32))
 
 
 def acts_array(acts, n):
@@ -76,21 +61,8 @@ def orc_fixed_build(columns, c, g_lagrange=None, want_pk=True):
     gl = np.ascontiguousarray(g_lagrange, dtype=np.uint64) if g_lagrange is not None else None
     p = lambda x: x.ctypes.data if x is not None else None
     oracle().orc_fixed_build(cols.ctypes.data, m, c.k, c.ek, c.omega_inv.ctypes.data, c.ifft.ctypes.data, c.ext_omega.ctypes.data, c.zeta.ctypes.data,
-                             p(gl), tp.threads(), p(jac), p(polys), p(cosets))
+                             p(gl), threads(), p(jac), p(polys), p(cosets))
     return jac, polys, cosets
-
-
-def sparse(rng, S, n, density):
-    return rng.random((S, n)) < density
-
-
-def disjoint(S, n, stride=None):
-    """selector s active on the rows r = s mod stride"""
-    stride = stride or S
-    a = np.zeros((S, n), dtype=bool)
-    for s in range(S):
-        a[s, s::stride] = True
-    return a
 
 
 def cases(oc, k, seed):
@@ -122,7 +94,7 @@ def device_assignment(L, acts, degrees, max_degree):
 
 
 def check_against_oracle(L, oc, k, seed, which=None):
-    c = tp.Consts(L, k)
+    c = Consts(L, k)
     pts = oc.gen_points(seed, c.n)
     h = L.register_bases(pts)
     try:
@@ -142,7 +114,7 @@ def check_against_oracle(L, oc, k, seed, which=None):
             assert (np.stack(r["polys"]) == polys).all(), (k, name)
             assert (np.stack(r["cosets"]) == cosets).all(), (k, name)
             vk = L.keygen_fixed_build_vk(list(fixed), list(acts), co, ro, C, k, h)
-            assert (tp.affine(oc, vk) == tp.affine(oc, jac)).all(), (k, name)
+            assert (affine(oc, vk) == affine(oc, jac)).all(), (k, name)
     finally:
         L.unregister_bases(h)
 
@@ -162,7 +134,7 @@ def check_exclusion(L, k, S, seed, density):
 def check_pins(L, oc, k, fixed, acts, degrees, max_degree, seed):
     import halo2_scaffold_b200 as h2
     from halo2_scaffold_b200 import keygen as kg
-    c = tp.Consts(L, k)
+    c = Consts(L, k)
     n, S = c.n, len(acts)
     a = kg.compress_selectors(list(acts), degrees, max_degree, lib=L)
     simple = [s for s in range(S) if degrees[s] > 0]
@@ -175,8 +147,8 @@ def check_pins(L, oc, k, fixed, acts, degrees, max_degree, seed):
         vk = kg.fixed_build_vk(params, c.dom, list(fixed), list(acts), a)
         pk = kg.fixed_build_pk(params, c.dom, list(fixed), list(acts), a)
         cols = list(fixed) + pk["combination_values"]
-        assert (tp.affine(oc, vk) == tp.affine(oc, params.commit_lagrange_many(cols))).all()
-        assert (tp.affine(oc, vk) == tp.affine(oc, params.commit_many(pk["polys"]))).all()
+        assert (affine(oc, vk) == affine(oc, params.commit_lagrange_many(cols))).all()
+        assert (affine(oc, vk) == affine(oc, params.commit_many(pk["polys"]))).all()
     finally:
         params.close()
     for poly, coset in zip(pk["polys"], pk["cosets"]):
@@ -192,7 +164,7 @@ def check_pins(L, oc, k, fixed, acts, degrees, max_degree, seed):
         col = pk["combination_values"][comb]
         q = np.full(n, -1, dtype=np.int64)
         for t in range(len(members) + 1):
-            q[(col == tp.W(t)).all(axis=1)] = t
+            q[(col == W(t)).all(axis=1)] = t
         assert (q >= 0).all(), comb
         for s in members:
             comb_s, root, ln = a["expressions"][s]
@@ -216,7 +188,7 @@ def pins_shapes(oc, k, seed, A=8):
 
 # ---- refused inputs --------------------------------------------------------------------------------------------------------
 def check_refused(L, oc, k=4):
-    c = tp.Consts(L, k)
+    c = Consts(L, k)
     n = c.n
     fixed = [oc.random_fr(3 + i, n) for i in range(2)]
     acts = [np.ascontiguousarray(x, dtype=np.uint8) for x in disjoint(4, n)]
@@ -281,10 +253,7 @@ def check_refused(L, oc, k=4):
 
 # ---- the C++ mirror, and every device ----------------------------------------------------------------------------------------
 def check_cpp_mirror(oc, lib_path, tmp_path, k):
-    exe = str(tmp_path / "fixed_keygen_mirror")
-    libdir, libfile = os.path.split(lib_path)
-    subprocess.check_call(["g++", "-O2", "-std=c++17", "-Wall", "-o", exe, os.path.join(ROOT, "tests", "cpp", "fixed_keygen_mirror.cpp"),
-                           "-L" + libdir, "-l:" + libfile, "-Wl,-rpath," + libdir])
+    exe = build_mirror("fixed_keygen_mirror", lib_path, tmp_path)
     n = 1 << k
     s = oc.random_fr(950 + k, 1)[0]
     s.tofile(str(tmp_path / "s.bin"))
@@ -298,29 +267,18 @@ def check_cpp_mirror(oc, lib_path, tmp_path, k):
     C = len(comb_cols)
     rd = lambda name, shape, dt=np.uint64: np.fromfile(str(tmp_path / name), dtype=dt).reshape(shape)
     assert (rd("assignment.bin", (3, len(acts)), np.uint32) == np.stack([co, ro, lo])).all()
-    c = tp.Consts.__new__(tp.Consts)
-    import halo2_scaffold_b200.domain as dm
-    ek = k + 2
-    w = dm.FR_ROOT_OF_UNITY
-    for _ in range(ek, dm.FR_S):
-        w = w * w % R
-    ext_omega = w
-    for _ in range(k, ek):
-        w = w * w % R
-    c.k, c.ek, c.n = k, ek, n
-    c.omega_inv, c.ifft, c.ext_omega = tp.W(pow(w, -1, R)), tp.W(pow(n, -1, R)), tp.W(ext_omega)
-    c.zeta = np.stack([tp.W(1), tp.W(dm.FR_ZETA), tp.W(dm.FR_ZETA * dm.FR_ZETA % R)])
-    _, gl = ts.orc_srs_setup(k, s)
+    c = Consts.on_host(k)
+    _, gl = orc_srs_setup(k, s)
     jac, polys, cosets = orc_fixed_build(np.concatenate([fixed, comb_cols]), c, gl)
     assert (rd("values.bin", comb_cols.shape) == comb_cols).all()
     assert (rd("polys.bin", polys.shape) == polys).all()
     assert (rd("cosets.bin", cosets.shape) == cosets).all()
-    assert (tp.affine(oc, rd("vk.bin", (len(fixed) + C, 12))) == tp.affine(oc, jac)).all()
+    assert (affine(oc, rd("vk.bin", (len(fixed) + C, 12))) == affine(oc, jac)).all()
 
 
 def check_every_device(L, oc, k, seed):
     """the host entries with columns dealt over every device, with a replicated and a sharded g_lagrange set"""
-    c = tp.Consts(L, k)
+    c = Consts(L, k)
     _, fixed, acts, degrees, max_degree = cases(oc, k, seed)[5]
     co, ro, lo, comb_cols = orc_compress(acts, degrees, max_degree, k)
     pts = oc.gen_points(seed, c.n)
@@ -332,7 +290,7 @@ def check_every_device(L, oc, k, seed):
         h = register(pts)
         try:
             vk = L.keygen_fixed_build_vk(list(fixed), list(acts), co, ro, len(comb_cols), k, h)
-            assert (tp.affine(oc, vk) == tp.affine(oc, jac)).all(), register.__name__
+            assert (affine(oc, vk) == affine(oc, jac)).all(), register.__name__
         finally:
             L.unregister_bases(h)
 
@@ -340,7 +298,7 @@ def check_every_device(L, oc, k, seed):
 # ---- the restatement itself, against big-int arithmetic ------------------------------------------------------------------
 @pytest.mark.parametrize("k", [2, 3, 4])
 def test_oracle_matches_bigint_definition(emu, oc, k):
-    c = tp.Consts(emu, k)
+    c = Consts(emu, k)
     n, ek = c.n, c.ek
     rng = np.random.default_rng(k)
     acts = sparse(rng, 6, n, 0.3)
@@ -354,17 +312,17 @@ def test_oracle_matches_bigint_definition(emu, oc, k):
                 for r in range(n):
                     if acts[s, r]:
                         want[r] = int(ro[s])
-        assert tp.ints(cols[comb]) == want
+        assert ints(cols[comb]) == want
     assert (orc_exclusion(acts, k) == np.array([[i != j and bool(np.any(acts[i] & acts[j])) for j in range(6)] for i in range(6)])).all()
     fixed = np.stack([oc.random_fr(k * 5 + i, n) for i in range(2)])
     all_cols = np.concatenate([fixed, cols])
     _, polys, cosets = orc_fixed_build(all_cols, c)
     w, we, z = c.dom.omega, c.dom.extended_omega, c.dom.g_coset
     for i in range(len(all_cols)):
-        v = tp.ints(all_cols[i])
+        v = ints(all_cols[i])
         co_ = [pow(n, -1, R) * sum(v[j] * pow(w, -t * j % n, R) for j in range(n)) % R for t in range(n)]
-        assert tp.ints(polys[i]) == co_
-        assert tp.ints(cosets[i]) == [sum(co_[t] * pow(z * pow(we, e, R), t, R) for t in range(n)) % R for e in range(1 << ek)]
+        assert ints(polys[i]) == co_
+        assert ints(cosets[i]) == [sum(co_[t] * pow(z * pow(we, e, R), t, R) for t in range(n)) % R for e in range(1 << ek)]
 
 
 # ---- CPU: the kernel sources through the emulator ----------------------------------------------------------------------
@@ -394,18 +352,9 @@ def test_cpp_mirror_emu(emu, oc, tmp_path):
 
 @pytest.mark.parametrize("devices", ["2", "3"])
 def test_fixed_keygen_on_emulated_devices(emu, devices):
-    code = ("import sys; sys.path[:0]=[%r,%r,%r]\n"
-            "import oracle_c as oc, test_fixed_keygen as t\n"
-            "from halo2_scaffold_b200._lib import Lib\n"
-            "L=Lib(%r, allow_emulator=True); L.init(0)\n"
-            "assert L.device_count() == %s\n"
-            "t.check_every_device(L, oc, 4, 530)\n"
-            "t.check_against_oracle(L, oc, 3, 531, which=('random mixed degrees', 'fixed only', 'selectors only'))\n"
-            "t.check_refused(L, oc)\n"
-            "print('ok')\n") % (ROOT, os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests"), emu.path, devices)
-    env = dict(os.environ, H2B_EMU_DEVICES=devices)
-    out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=1200)
-    assert out.returncode == 0 and "ok" in out.stdout, out.stderr[-3000:]
+    run_on_emulated_devices("test_fixed_keygen", "t.check_every_device(L, oc, 4, 530)\n"
+                                                 "t.check_against_oracle(L, oc, 3, 531, which=('random mixed degrees', 'fixed only', 'selectors only'))\n"
+                                                 "t.check_refused(L, oc)", devices)
 
 
 # ---- GPU ------------------------------------------------------------------------------------------------------------------

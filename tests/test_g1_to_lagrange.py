@@ -8,36 +8,23 @@ shares no code with the G1 NTT."""
 import ctypes
 import os
 import subprocess
-import sys
-import tempfile
 
 import numpy as np
 import pytest
 
 import bn254 as o
 import parity_cases as pc
-import test_srs_setup as ts
+from harness import affine_ints, build_mirror, build_oracle, mont, orc_srs_setup, run_on_emulated_devices
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 H2B_ERR_BAD_ARGUMENT = -2
-_ORACLE = None
 
 
 # ---- helpers ---------------------------------------------------------------------------------------------------------
 def oracle():
-    """tests/cpp/g1_to_lagrange_oracle.cpp, built once per process into a temporary directory"""
-    global _ORACLE
-    if _ORACLE is None:
-        d = tempfile.mkdtemp(prefix="g1_to_lagrange_oracle_")
-        so = os.path.join(d, "libg1_to_lagrange_oracle.so")
-        subprocess.check_call(["g++", "-O3", "-march=x86-64-v3", "-std=c++17", "-fPIC", "-shared", "-pthread", "-Wno-unused-function", "-o", so,
-                               os.path.join(ROOT, "tests", "cpp", "g1_to_lagrange_oracle.cpp")])
-        L = ctypes.CDLL(so)
-        vp = ctypes.c_void_p
-        L.orc_g1_to_lagrange.argtypes = [vp, ctypes.c_uint32, ctypes.c_int, vp]
-        L.orc_g1_mul_points.argtypes = [vp, vp, ctypes.c_size_t, ctypes.c_int, vp]
-        _ORACLE = L
-    return _ORACLE
+    """tests/cpp/g1_to_lagrange_oracle.cpp"""
+    vp = ctypes.c_void_p
+    return build_oracle("g1_to_lagrange_oracle", dict(orc_g1_to_lagrange=[vp, ctypes.c_uint32, ctypes.c_int, vp],
+                                                      orc_g1_mul_points=[vp, vp, ctypes.c_size_t, ctypes.c_int, vp]))
 
 
 def orc_g1_to_lagrange(points, k, threads=0):
@@ -62,7 +49,7 @@ def random_points(oc, seed, n):
 def neg(oc, points):
     """-P for affine Montgomery points (the identity stays (0, 0))"""
     ints = []
-    for p in ts.affine_ints(oc, points):
+    for p in affine_ints(oc, points):
         ints += [0, 0] if p is None else [o.to_mont(p[0], o.P_MOD), o.to_mont(-p[1] % o.P_MOD, o.P_MOD)]
     return oc.ints_to_words(ints).reshape(-1, 8)
 
@@ -115,7 +102,7 @@ def check_known_answers(L, oc, k):
 
 
 def check_scalar_mul_edges(L, oc, n_random=0):
-    e = ts.mont(oc, edge_scalars())
+    e = mont(oc, edge_scalars())
     if n_random:
         e = np.concatenate([e, oc.random_fr(61, n_random)])
     P = random_points(oc, 62, e.shape[0])
@@ -188,7 +175,7 @@ def check_params_downsize(L, oc, K, k, seed):
             with pytest.raises(RuntimeError):
                 L.base_set_info(h)
         e = oc.random_fr(seed + 1, n)
-        coeff = oc.fr_scale(oc.best_fft(e, pc.omega_words(oc, k, inverse=True), k), ts.mont(oc, [pow(n, -1, o.R_MOD)])[0])
+        coeff = oc.fr_scale(oc.best_fft(e, pc.omega_words(oc, k, inverse=True), k), mont(oc, [pow(n, -1, o.R_MOD)])[0])
         assert (pc.affine_of(oc, params.commit_lagrange(e)) == pc.affine_of(oc, params.commit(coeff))).all()
     finally:
         params.close()
@@ -226,17 +213,14 @@ def check_handles_on_every_device(L, oc, K, k, seed):
 
 def check_cpp_mirror(oc, lib_path, tmp_path, K, k):
     """tests/cpp/srs_downsize_mirror.cpp: ParamsKZG::setup(K, s) then downsize(k) of the C++ host mirror"""
-    exe = str(tmp_path / "srs_downsize_mirror")
-    libdir, libfile = os.path.split(lib_path)
-    subprocess.check_call(["g++", "-O2", "-std=c++17", "-Wall", "-o", exe, os.path.join(ROOT, "tests", "cpp", "srs_downsize_mirror.cpp"),
-                           "-L" + libdir, "-l:" + libfile, "-Wl,-rpath," + libdir])
+    exe = build_mirror("srs_downsize_mirror", lib_path, tmp_path)
     s = oc.random_fr(800 + k, 1)[0]
     s.tofile(str(tmp_path / "s.bin"))
     out = subprocess.run([exe, str(tmp_path), str(K), str(k)], capture_output=True, text=True, timeout=1200)
     assert out.returncode == 0 and "SRS_DOWNSIZE_MIRROR_OK" in out.stdout, (out.stdout, out.stderr)
     g = np.fromfile(str(tmp_path / "g.bin"), dtype=np.uint64).reshape(-1, 8)
     gl = np.fromfile(str(tmp_path / "g_lagrange.bin"), dtype=np.uint64).reshape(-1, 8)
-    wg, wgl = ts.orc_srs_setup(k, s)
+    wg, wgl = orc_srs_setup(k, s)
     assert (g == wg).all() and (gl == wgl).all()
 
 
@@ -245,8 +229,8 @@ def check_cpp_mirror(oc, lib_path, tmp_path, K, k):
 def test_restatement_matches_naive_dft(oc, k):
     n = 1 << k
     pts = with_scattered_identities(oc, k, 90 + k) if k >= 2 else random_points(oc, 90 + k, n)
-    got = ts.affine_ints(oc, orc_g1_to_lagrange(pts, k, threads=3))
-    g = ts.affine_ints(oc, pts)
+    got = affine_ints(oc, orc_g1_to_lagrange(pts, k, threads=3))
+    g = affine_ints(oc, pts)
     w_inv = pow(o.omega_for(k), -1, o.R_MOD)
     n_inv = pow(n, -1, o.R_MOD)
     want = []
@@ -259,7 +243,7 @@ def test_restatement_matches_naive_dft(oc, k):
     assert got == want
     e = [0, 1, o.R_MOD - 1, 0x1234567890ABCDEF1122334455667788]
     P = random_points(oc, 95, len(e))
-    assert ts.affine_ints(oc, orc_g1_mul_points(P, ts.mont(oc, e))) == [o.g1_mul(p, v) for p, v in zip(ts.affine_ints(oc, P), e)]
+    assert affine_ints(oc, orc_g1_mul_points(P, mont(oc, e))) == [o.g1_mul(p, v) for p, v in zip(affine_ints(oc, P), e)]
 
 
 # ---- CPU: the kernel sources through the emulator ----------------------------------------------------------------------
@@ -296,17 +280,8 @@ def test_cpp_mirror_downsize_emu(emu, oc, tmp_path):
 
 @pytest.mark.parametrize("devices", ["2", "3"])
 def test_downsize_handles_on_emulated_devices(emu, devices):
-    code = ("import sys; sys.path[:0]=[%r,%r,%r]\n"
-            "import oracle_c as oc, test_g1_to_lagrange as t\n"
-            "from halo2_scaffold_b200._lib import Lib\n"
-            "L=Lib(%r, allow_emulator=True); L.init(0)\n"
-            "assert L.device_count() == %s\n"
-            "t.check_handles_on_every_device(L, oc, 5, 4, 140)\n"
-            "t.check_refused(L, oc)\n"
-            "print('ok')\n") % (ROOT, os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests"), emu.path, devices)
-    env = dict(os.environ, H2B_EMU_DEVICES=devices)
-    out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=1200)
-    assert out.returncode == 0 and "ok" in out.stdout, out.stderr[-3000:]
+    run_on_emulated_devices("test_g1_to_lagrange", "t.check_handles_on_every_device(L, oc, 5, 4, 140)\n"
+                                                   "t.check_refused(L, oc)", devices)
 
 
 # ---- GPU ------------------------------------------------------------------------------------------------------------------

@@ -6,7 +6,7 @@ CPU: the kernel sources through the emulator, which keeps that per-thread last e
 import pytest
 
 import parity_cases as pc
-import test_srs_setup as srs
+from harness import orc_srs_setup
 from halo2_scaffold_b200._lib import H2BError
 
 H2B_ERR_OOM = -4
@@ -32,7 +32,7 @@ def check_launches_after_a_refused_allocation(L, oc, k):
     s = oc.random_fr(13, 1)[0]
     params = h2.ParamsKZG.setup(k, s, lib=L)
     try:
-        g, gl = srs.orc_srs_setup(k, s)
+        g, gl = orc_srs_setup(k, s)
         assert (params.g == g).all() and (params.g_lagrange == gl).all()
     finally:
         params.close()

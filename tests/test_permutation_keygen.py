@@ -7,78 +7,27 @@ that need no recollection of upstream: sigma's cycles are the connected componen
 them closes the permutation product, the toy circuit of parity_cases' quotient check gets its hand-built sigma,
 commit_lagrange(sigma) = commit(coefficients), and l_active_row + l_last + l_blind = 1 with l0 = (1/n) sum X^i."""
 import ctypes
-import os
 import subprocess
-import sys
-import tempfile
 
 import numpy as np
 import pytest
 
 import bn254 as o
-import parity_cases as pc
-import test_srs_setup as ts
+from harness import (Consts, W, affine, build_mirror, build_oracle, ints, orc_mapping, orc_srs_setup, random_copies, run_on_emulated_devices,
+                     threads)
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 H2B_ERR_BAD_ARGUMENT = -2
 R = o.R_MOD
-_ORACLE = None
 
 
 # ---- helpers ---------------------------------------------------------------------------------------------------------
 def oracle():
-    """tests/cpp/permutation_keygen_oracle.cpp, built once per process into a temporary directory"""
-    global _ORACLE
-    if _ORACLE is None:
-        d = tempfile.mkdtemp(prefix="permutation_keygen_oracle_")
-        so = os.path.join(d, "libpermutation_keygen_oracle.so")
-        subprocess.check_call(["g++", "-O3", "-march=x86-64-v3", "-std=c++17", "-fPIC", "-shared", "-pthread", "-Wno-unused-function", "-o", so,
-                               os.path.join(ROOT, "tests", "cpp", "permutation_keygen_oracle.cpp")])
-        L = ctypes.CDLL(so)
-        vp, u32, sz, i32 = ctypes.c_void_p, ctypes.c_uint32, ctypes.c_size_t, ctypes.c_int
-        L.orc_assembly_mapping.argtypes = [u32, u32, vp, sz, vp]
-        L.orc_permutation_sigma.argtypes = [vp, u32, u32, vp, vp, i32, vp]
-        L.orc_permutation_build_vk.argtypes = [vp, u32, u32, vp, vp, vp, i32, vp]
-        L.orc_permutation_build_pk.argtypes = [vp, u32, u32, u32, vp, vp, vp, vp, vp, vp, i32, vp, vp, vp]
-        L.orc_lagrange_indicators.argtypes = [u32, u32, u32, vp, vp, vp, vp, i32, vp, vp, vp]
-        _ORACLE = L
-    return _ORACLE
-
-
-def threads():
-    return os.cpu_count() or 1
-
-
-def W(x):
-    from halo2_scaffold_b200.domain import fr_to_words
-    return fr_to_words(int(x))
-
-
-def ints(words):
-    """Montgomery words -> canonical integers"""
-    import oracle_c
-    return [o.from_mont(v, R) for v in oracle_c.words_to_ints(np.ascontiguousarray(words, dtype=np.uint64).reshape(-1, 4))]
-
-
-class Consts:
-    """the domain constants of EvaluationDomain::new(5, k) (extended_k = k + 2), as words"""
-
-    def __init__(self, L, k):
-        import halo2_scaffold_b200 as h2
-        from halo2_scaffold_b200 import keygen as kg
-        self.dom = h2.EvaluationDomain(5, k, lib=L)
-        d = self.dom
-        self.k, self.ek, self.n = k, d.extended_k, 1 << k
-        self.delta, self.omega, self.omega_inv = W(kg.FR_DELTA), W(d.omega), W(d.omega_inv)
-        self.ifft, self.ext_omega = W(d.ifft_divisor), W(d.extended_omega)
-        self.zeta = np.stack([W(1), W(d.g_coset), W(d.g_coset_inv)])
-
-
-def orc_mapping(P, k, copies):
-    c = np.ascontiguousarray(np.array(copies, dtype=np.uint64).reshape(-1, 4))
-    out = np.empty((P, 1 << k, 2), dtype=np.uint64)
-    oracle().orc_assembly_mapping(P, k, c.ctypes.data, c.shape[0], out.ctypes.data)
-    return out
+    """tests/cpp/permutation_keygen_oracle.cpp"""
+    vp, u32, i32 = ctypes.c_void_p, ctypes.c_uint32, ctypes.c_int
+    return build_oracle("permutation_keygen_oracle", dict(orc_permutation_sigma=[vp, u32, u32, vp, vp, i32, vp],
+                                                          orc_permutation_build_vk=[vp, u32, u32, vp, vp, vp, i32, vp],
+                                                          orc_permutation_build_pk=[vp, u32, u32, u32, vp, vp, vp, vp, vp, vp, i32, vp, vp, vp],
+                                                          orc_lagrange_indicators=[u32, u32, u32, vp, vp, vp, vp, i32, vp, vp, vp]))
 
 
 def orc_build_pk(mapping, c):
@@ -109,21 +58,6 @@ def orc_indicators(c, bf):
 def device_pk(L, mapping, c):
     r = L.permutation_build_pk(mapping, c.k, c.ek, c.delta, c.omega, c.omega_inv, c.ifft, c.ext_omega, c.zeta)
     return np.stack(r["permutations"]), np.stack(r["polys"]), np.stack(r["cosets"])
-
-
-def affine(oc, jacs):
-    return np.stack([pc.affine_of(oc, j) for j in np.asarray(jacs).reshape(-1, 12)])
-
-
-def random_copies(rng, P, n, count, rows=None):
-    """copies between random cells (rows < `rows`), with repeated and reversed (redundant) copies mixed in"""
-    rows = rows or n
-    cs = [(int(rng.integers(P)), int(rng.integers(rows)), int(rng.integers(P)), int(rng.integers(rows))) for _ in range(count)]
-    extra = [cs[int(rng.integers(len(cs)))] for _ in range(count // 4)]
-    extra += [(d, e, a, b) for (a, b, d, e) in (cs[int(rng.integers(len(cs)))] for _ in range(count // 4))]
-    cs += extra
-    rng.shuffle(cs)
-    return cs
 
 
 def one_cycle(P, n):
@@ -378,10 +312,7 @@ def check_commitment_and_indicator_pins(L, oc, k, P, seed, bf=5):
 
 
 def check_cpp_mirror(oc, lib_path, tmp_path, k, P, bf=3):
-    exe = str(tmp_path / "permutation_keygen_mirror")
-    libdir, libfile = os.path.split(lib_path)
-    subprocess.check_call(["g++", "-O2", "-std=c++17", "-Wall", "-o", exe, os.path.join(ROOT, "tests", "cpp", "permutation_keygen_mirror.cpp"),
-                           "-L" + libdir, "-l:" + libfile, "-Wl,-rpath," + libdir])
+    exe = build_mirror("permutation_keygen_mirror", lib_path, tmp_path)
     n = 1 << k
     s = oc.random_fr(900 + k, 1)[0]
     s.tofile(str(tmp_path / "s.bin"))
@@ -389,29 +320,13 @@ def check_cpp_mirror(oc, lib_path, tmp_path, k, P, bf=3):
     mapping.tofile(str(tmp_path / "mapping.bin"))
     out = subprocess.run([exe, str(tmp_path), str(k), str(P), str(bf)], capture_output=True, text=True, timeout=1200)
     assert out.returncode == 0 and "PERMUTATION_KEYGEN_MIRROR_OK" in out.stdout, (out.stdout, out.stderr)
-
-    class C:
-        pass
-    c = C()
-    import halo2_scaffold_b200.domain as dm
-    from halo2_scaffold_b200 import keygen as kg
-    # the domain constants on the host only (no device needed for them)
-    ek = k + 2
-    w = dm.FR_ROOT_OF_UNITY
-    for _ in range(ek, dm.FR_S):
-        w = w * w % R
-    ext_omega = w
-    for _ in range(k, ek):
-        w = w * w % R
-    c.k, c.ek, c.n = k, ek, n
-    c.delta, c.omega, c.omega_inv, c.ifft, c.ext_omega = W(kg.FR_DELTA), W(w), W(pow(w, -1, R)), W(pow(n, -1, R)), W(ext_omega)
-    c.zeta = np.stack([W(1), W(dm.FR_ZETA), W(dm.FR_ZETA * dm.FR_ZETA % R)])
+    c = Consts.on_host(k)
     perm, polys, cosets = orc_build_pk(mapping, c)
     rd = lambda name, shape: np.fromfile(str(tmp_path / name), dtype=np.uint64).reshape(shape)
     assert (rd("permutations.bin", perm.shape) == perm).all()
     assert (rd("polys.bin", polys.shape) == polys).all()
     assert (rd("cosets.bin", cosets.shape) == cosets).all()
-    _, gl = ts.orc_srs_setup(k, s)
+    _, gl = orc_srs_setup(k, s)
     assert (affine(oc, rd("vk.bin", (P, 12))) == affine(oc, orc_build_vk(mapping, c, gl))).all()
     for name, want in zip(("l0.bin", "l_last.bin", "l_active.bin"), orc_indicators(c, bf)):
         assert (rd(name, want.shape) == want).all(), name
@@ -493,18 +408,9 @@ def test_cpp_mirror_emu(emu, oc, tmp_path):
 
 @pytest.mark.parametrize("devices", ["2", "3"])
 def test_keygen_on_emulated_devices(emu, devices):
-    code = ("import sys; sys.path[:0]=[%r,%r,%r]\n"
-            "import oracle_c as oc, test_permutation_keygen as t\n"
-            "from halo2_scaffold_b200._lib import Lib\n"
-            "L=Lib(%r, allow_emulator=True); L.init(0)\n"
-            "assert L.device_count() == %s\n"
-            "t.check_every_device(L, oc, 4, 5, 330)\n"
-            "t.check_against_oracle(L, oc, 3, 331, which=('random', 'P = 1'))\n"
-            "t.check_refused(L, oc)\n"
-            "print('ok')\n") % (ROOT, os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests"), emu.path, devices)
-    env = dict(os.environ, H2B_EMU_DEVICES=devices)
-    out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=1200)
-    assert out.returncode == 0 and "ok" in out.stdout, out.stderr[-3000:]
+    run_on_emulated_devices("test_permutation_keygen", "t.check_every_device(L, oc, 4, 5, 330)\n"
+                                                       "t.check_against_oracle(L, oc, 3, 331, which=('random', 'P = 1'))\n"
+                                                       "t.check_refused(L, oc)", devices)
 
 
 # ---- GPU ------------------------------------------------------------------------------------------------------------------

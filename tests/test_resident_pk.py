@@ -8,18 +8,13 @@ resident builders, and evaluate_h reading it through the handle gives the host p
 
 CPU: the kernel sources through the emulator on 1, 2 and 3 emulated devices.  GPU: the product library on every visible B200."""
 import ctypes
-import os
-import subprocess
-import sys
 
 import numpy as np
 import pytest
 
 import bn254 as o
-import test_fixed_keygen as tf
-import test_permutation_keygen as tp
+from harness import Consts, disjoint, orc_mapping, random_copies, run_on_emulated_devices, sparse
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 H2B_ERR_BAD_ARGUMENT = -2
 R = o.R_MOD
 FIXED, PERMUTATION, INDICATORS = 0, 1, 2
@@ -34,15 +29,15 @@ def inputs(L, oc, k, seed, shape):
     rng = np.random.default_rng(seed)
     fixed = np.stack([oc.random_fr(seed * 13 + i, n) for i in range(2)])
     if shape == "overlapping":
-        acts = tf.sparse(rng, 4, n, 0.25)
+        acts = sparse(rng, 4, n, 0.25)
         acts[:, 0] = True
         degrees, max_degree = [2, 2, 2, 2], 5
     else:
-        acts = tf.disjoint(6, n)
+        acts = disjoint(6, n)
         degrees, max_degree = [3, 2, 3, 1, 2, 3], 5
     assignment = kg.compress_selectors(list(acts), degrees, max_degree, lib=L)
     P = 3
-    mapping = tp.orc_mapping(P, k, tp.random_copies(rng, P, n, max(4, n // 4)))
+    mapping = orc_mapping(P, k, random_copies(rng, P, n, max(4, n // 4)))
     return fixed, acts, assignment, mapping
 
 
@@ -101,7 +96,7 @@ def check_matches(L, c, pk, ref):
 
 def check_contents(L, oc, k, seed, layout, halo=0, shapes=("overlapping", "disjoint")):
     from halo2_scaffold_b200 import keygen as kg
-    c = tp.Consts(L, k)
+    c = Consts(L, k)
     for shape in shapes:
         fixed, acts, assignment, mapping = inputs(L, oc, k, seed, shape)
         ref = host_reference(L, c, fixed, acts, assignment, mapping)
@@ -122,7 +117,7 @@ def check_contents(L, oc, k, seed, layout, halo=0, shapes=("overlapping", "disjo
 def check_info(L, k, F, P, halo):
     """bytes per device: 2n-row forms of F + P columns everywhere, extended columns whole or as the device's slice"""
     from halo2_scaffold_b200 import keygen as kg
-    c = tp.Consts(L, k)
+    c = Consts(L, k)
     n, E, D = 1 << k, 1 << c.ek, L.device_count()
     with kg.ResidentProvingKey(c.dom, F, P, "replicated", lib=L) as pk:
         assert pk.info() == [32 * (2 * n * (F + P) + E * (F + P + 3))] * D
@@ -134,7 +129,7 @@ def check_info(L, k, F, P, halo):
 # ---- refusals and lifetime ---------------------------------------------------------------------------------------------------------
 def check_refused(L, oc, k=4):
     from halo2_scaffold_b200 import keygen as kg
-    c = tp.Consts(L, k)
+    c = Consts(L, k)
     n, E, D = c.n, 1 << c.ek, L.device_count()
     Lr = L.L
     vp = ctypes.c_void_p
@@ -310,22 +305,13 @@ def test_quotient_pin_emu(emu, oc):
 @pytest.mark.parametrize("devices", ["2", "3"])
 def test_resident_pk_on_emulated_devices(emu, devices):
     # 2 devices: the slices wrap at the start (device 0) and at the end (device 1); 3 devices: D does not divide E
-    code = ("import sys; sys.path[:0]=[%r,%r,%r]\n"
-            "import oracle_c as oc, test_resident_pk as t\n"
-            "oc.build()\n"
-            "from halo2_scaffold_b200._lib import Lib\n"
-            "L=Lib(%r, allow_emulator=True); L.init(0)\n"
-            "assert L.device_count() == %s\n"
-            "t.check_contents(L, oc, 4, 730, 'row_sharded', 5)\n"
-            "t.check_contents(L, oc, 3, 731, 'row_sharded', 3, shapes=('overlapping',))\n"
-            "t.check_contents(L, oc, 4, 732, 'replicated', shapes=('disjoint',))\n"
-            "t.check_info(L, 4, 3, 2, 7)\n"
-            "t.check_refused(L, oc)\n"
-            "t.check_pin(L, oc, 5, 733)\n"
-            "print('ok')\n") % (ROOT, os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests"), emu.path, devices)
-    env = dict(os.environ, H2B_EMU_DEVICES=devices)
-    out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=1200)
-    assert out.returncode == 0 and "ok" in out.stdout, out.stderr[-3000:]
+    run_on_emulated_devices("test_resident_pk", "oc.build()\n"
+                                                "t.check_contents(L, oc, 4, 730, 'row_sharded', 5)\n"
+                                                "t.check_contents(L, oc, 3, 731, 'row_sharded', 3, shapes=('overlapping',))\n"
+                                                "t.check_contents(L, oc, 4, 732, 'replicated', shapes=('disjoint',))\n"
+                                                "t.check_info(L, 4, 3, 2, 7)\n"
+                                                "t.check_refused(L, oc)\n"
+                                                "t.check_pin(L, oc, 5, 733)", devices)
 
 
 # ---- GPU -------------------------------------------------------------------------------------------------------------------------
@@ -367,7 +353,7 @@ def test_device_memory_returns_after_release(gpu):
 
     def free_bytes():
         return [torch.cuda.mem_get_info(d)[0] for d in range(gpu.device_count())]
-    c = tp.Consts(gpu, 20)
+    c = Consts(gpu, 20)
     slack = 64 << 20
     before = free_bytes()
     pk = kg.ResidentProvingKey(c.dom, 6, 6, lib=gpu)

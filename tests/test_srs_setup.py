@@ -6,35 +6,22 @@ identities at k = 20 and 24 that share no code with the setup."""
 import ctypes
 import os
 import subprocess
-import sys
-import tempfile
 
 import numpy as np
 import pytest
 
 import bn254 as o
 import parity_cases as pc
+from harness import affine_ints, build_mirror, build_oracle, mont, orc_srs_setup, run_on_emulated_devices
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 H2B_ERR_BAD_ARGUMENT = -2
-_SETUP_ORACLE = None
 
 
 # ---- helpers ---------------------------------------------------------------------------------------------------------
 def setup_oracle():
-    """tests/cpp/srs_setup_oracle.cpp (on oracle/h2_oracle.cpp), built once per process into a temporary directory"""
-    global _SETUP_ORACLE
-    if _SETUP_ORACLE is None:
-        d = tempfile.mkdtemp(prefix="srs_setup_oracle_")
-        so = os.path.join(d, "libsrs_setup_oracle.so")
-        subprocess.check_call(["g++", "-O3", "-march=x86-64-v3", "-std=c++17", "-fPIC", "-shared", "-pthread", "-Wno-unused-function", "-o", so,
-                               os.path.join(ROOT, "tests", "cpp", "srs_setup_oracle.cpp")])
-        L = ctypes.CDLL(so)
-        vp = ctypes.c_void_p
-        L.orc_g1_generator_mul.argtypes = [vp, ctypes.c_size_t, ctypes.c_int, vp]
-        L.orc_srs_setup.argtypes = [ctypes.c_uint32, vp, ctypes.c_int, vp, vp]
-        _SETUP_ORACLE = L
-    return _SETUP_ORACLE
+    """tests/cpp/srs_setup_oracle.cpp"""
+    vp = ctypes.c_void_p
+    return build_oracle("srs_setup_oracle", dict(orc_g1_generator_mul=[vp, ctypes.c_size_t, ctypes.c_int, vp]))
 
 
 def orc_g1_generator_mul(scalars, threads=0):
@@ -42,17 +29,6 @@ def orc_g1_generator_mul(scalars, threads=0):
     out = np.empty((s.shape[0], 8), dtype=np.uint64)
     setup_oracle().orc_g1_generator_mul(s.ctypes.data, s.shape[0], threads or os.cpu_count() or 1, out.ctypes.data)
     return out
-
-
-def orc_srs_setup(k, s, threads=0):
-    s = np.ascontiguousarray(s, dtype=np.uint64).reshape(4)
-    g, gl = np.empty((1 << k, 8), dtype=np.uint64), np.empty((1 << k, 8), dtype=np.uint64)
-    setup_oracle().orc_srs_setup(k, s.ctypes.data, threads or os.cpu_count() or 1, g.ctypes.data, gl.ctypes.data)
-    return g, gl
-
-
-def mont(oc, vals):
-    return oc.ints_to_words([o.to_mont(v % o.R_MOD, o.R_MOD) for v in vals])
 
 
 def edge_scalars():
@@ -67,12 +43,6 @@ def edge_scalars():
             vals.append((1 << (W * m)) - sum(1 << (W * i) for i in range(m)))            # digits -1, ..., -1, 1
             vals.append(sum((1 << (W - 1)) << (W * i) for i in range(m)))                  # digits 2^(W-1)
     return [v % r for v in vals]
-
-
-def affine_ints(oc, pts):
-    v = oc.words_to_ints(np.ascontiguousarray(pts).reshape(-1, 4))
-    return [None if v[2 * i] == 0 and v[2 * i + 1] == 0 else (o.from_mont(v[2 * i], o.P_MOD), o.from_mont(v[2 * i + 1], o.P_MOD))
-            for i in range(len(v) // 2)]
 
 
 def omega_int(k):
@@ -163,11 +133,8 @@ def check_handles_on_every_device(L, oc, k, s):
 
 
 def check_cpp_mirror(oc, lib_path, tmp_path, k):
-    """tests/cpp/srs_setup_mirror.cpp (built as tests/host_mirror_case.py builds its program) against the restatement"""
-    exe = str(tmp_path / "srs_setup_mirror")
-    libdir, libfile = os.path.split(lib_path)
-    subprocess.check_call(["g++", "-O2", "-std=c++17", "-Wall", "-o", exe, os.path.join(ROOT, "tests", "cpp", "srs_setup_mirror.cpp"),
-                           "-L" + libdir, "-l:" + libfile, "-Wl,-rpath," + libdir])
+    """tests/cpp/srs_setup_mirror.cpp against the restatement"""
+    exe = build_mirror("srs_setup_mirror", lib_path, tmp_path)
     n = 1 << k
     s, poly = oc.random_fr(500 + k, 1)[0], oc.random_fr(501 + k, n)
     s.tofile(str(tmp_path / "s.bin"))
@@ -227,16 +194,7 @@ def test_cpp_mirror_setup_emu(emu, oc, tmp_path):
 
 @pytest.mark.parametrize("devices", ["2", "3"])
 def test_setup_handles_on_emulated_devices(emu, devices):
-    code = ("import sys; sys.path[:0]=[%r,%r,%r]\n"
-            "import oracle_c as oc, test_srs_setup as t\n"
-            "from halo2_scaffold_b200._lib import Lib\n"
-            "L=Lib(%r, allow_emulator=True); L.init(0)\n"
-            "assert L.device_count() == %s\n"
-            "t.check_handles_on_every_device(L, oc, 6, oc.random_fr(9, 1)[0])\n"
-            "print('ok')\n") % (ROOT, os.path.join(ROOT, "oracle"), os.path.join(ROOT, "tests"), emu.path, devices)
-    env = dict(os.environ, H2B_EMU_DEVICES=devices)
-    out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=1200)
-    assert out.returncode == 0 and "ok" in out.stdout, out.stderr[-3000:]
+    run_on_emulated_devices("test_srs_setup", "t.check_handles_on_every_device(L, oc, 6, oc.random_fr(9, 1)[0])", devices)
 
 
 # ---- GPU ------------------------------------------------------------------------------------------------------------------
