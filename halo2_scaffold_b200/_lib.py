@@ -44,6 +44,7 @@ _EXPORTS = [
     "h2b_selector_exclusion", "h2b_keygen_fixed_build_vk", "h2b_keygen_fixed_build_pk",
     "h2b_pk_create", "h2b_keygen_fixed_build_pk_resident", "h2b_permutation_build_pk_resident", "h2b_keygen_lagrange_indicators_resident",
     "h2b_pk_put_lagrange", "h2b_pk_column", "h2b_pk_download", "h2b_pk_info", "h2b_pk_release",
+    "h2b_fr_eval_queries_dev", "h2b_shplonk_begin", "h2b_shplonk_finish", "h2b_shplonk_release",
 ]
 
 # include/h2b200.h enums of the resident proving key
@@ -76,6 +77,19 @@ class EvalColumnsStruct(ctypes.Structure):
                 ("instance", ctypes.c_void_p), ("n_instance", ctypes.c_uint32),
                 ("challenges", ctypes.c_void_p), ("n_challenges", ctypes.c_uint32),
                 ("beta", ctypes.c_void_p), ("gamma", ctypes.c_void_p), ("theta", ctypes.c_void_p), ("y", ctypes.c_void_p)]
+
+
+class OpeningQueryStruct(ctypes.Structure):
+    _fields_ = [("poly", ctypes.c_uint32), ("reserved", ctypes.c_uint32), ("point", ctypes.c_uint64 * 4)]
+
+
+def _queries(queries):
+    """[(poly index, point words)] -> a ctypes array of h2b_opening_query"""
+    arr = (OpeningQueryStruct * max(len(queries), 1))()
+    for i, (poly, point) in enumerate(queries):
+        arr[i].poly = int(poly)
+        arr[i].point[:] = [int(w) for w in np.asarray(point, dtype=np.uint64).reshape(4)]
+    return arr
 
 
 class ShardStruct(ctypes.Structure):
@@ -233,6 +247,10 @@ class Lib:
         L.h2b_pk_download.argtypes = [u64, i32, i32, u32, vp]
         L.h2b_pk_info.argtypes = [u64, vp]
         L.h2b_pk_release.argtypes = [u64]
+        L.h2b_fr_eval_queries_dev.argtypes = [i32, vp, u32, sz, vp, u32, vp, vp]
+        L.h2b_shplonk_begin.argtypes = [i32, vp, i32, u32, sz, vp, u32, u64, vp, vp, vp, ctypes.POINTER(u64)]
+        L.h2b_shplonk_finish.argtypes = [u64, vp, vp]
+        L.h2b_shplonk_release.argtypes = [u64]
         L.h2b_evaluate_graph_dev.argtypes = [i32, vp, vp, vp, u32, i32, vp]
         L.h2b_evaluate_h_permutation_dev.argtypes = [i32, vp, u32, i32, vp, u32, vp, vp, u32, u32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
         L.h2b_evaluate_h_lookup_dev.argtypes = [i32, vp, vp, vp, u32, i32, vp, vp, vp, vp, vp, vp, vp]
@@ -865,6 +883,33 @@ class Lib:
 
     def pk_release(self, pk: int):
         self.check(self.L.h2b_pk_release(pk))
+
+    # ---- the multi-point opening (SHPLONK) ---------------------------------------------------------------
+    def eval_queries_dev(self, device: int, d_polys, n: int, queries, d_out: int, stream: int = 0):
+        """eval_polynomial of every query (poly index into d_polys, point words) -> d_out, one Fr per query"""
+        ptrs = _ptr_array(list(d_polys))
+        q = _queries(queries)
+        self.check(self.L.h2b_fr_eval_queries_dev(device, ptrs, len(d_polys), n, q, len(queries), d_out, stream))
+
+    def shplonk_begin(self, device: int, polys, on_host: bool, n: int, queries, handle_g: int, y, v):
+        """polys: host arrays (on_host) or device pointers -> (h1 Jacobian, session handle)"""
+        ptrs = _ptr_array([p.ctypes.data for p in polys] if on_host else list(polys))
+        q = _queries(queries)
+        y, v = _u64(y).reshape(4), _u64(v).reshape(4)
+        out = np.zeros(12, dtype=np.uint64)
+        h = ctypes.c_uint64(0)
+        self.check(self.L.h2b_shplonk_begin(device, ptrs, 1 if on_host else 0, len(polys), n, q, len(queries), handle_g, y.ctypes.data, v.ctypes.data,
+                                            out.ctypes.data, ctypes.byref(h)))
+        return out, h.value
+
+    def shplonk_finish(self, session: int, u) -> np.ndarray:
+        u = _u64(u).reshape(4)
+        out = np.zeros(12, dtype=np.uint64)
+        self.check(self.L.h2b_shplonk_finish(session, u.ctypes.data, out.ctypes.data))
+        return out
+
+    def shplonk_release(self, session: int):
+        self.check(self.L.h2b_shplonk_release(session))
 
     # ---- quotient evaluation (evaluate_h) on device-resident extended-coset columns ------------------
     def evaluate_graph_dev(self, device: int, graph: GraphArrays, cols: EvalColumns, d_values: int, size: int, rot_scale: int, stream: int = 0,

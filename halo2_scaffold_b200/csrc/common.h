@@ -79,7 +79,9 @@ enum ProfTag { PROF_BEGIN = 0, PROF_MSM_DECOMPOSE = 1, PROF_MSM_SCAN = 2, PROF_M
                PROF_G1NTT_TWIDDLE = 28, PROF_G1NTT_STAGES = 29, PROF_G1NTT_NORMALISE = 30,
                PROF_KEYGEN_UPLOAD = 31, PROF_KEYGEN_SIGMA = 32, PROF_KEYGEN_COMMIT = 33, PROF_KEYGEN_INTT = 34, PROF_KEYGEN_COSET = 35,
                PROF_KEYGEN_DOWNLOAD = 36, PROF_KEYGEN_PACK = 37, PROF_KEYGEN_EXCLUSION = 38, PROF_KEYGEN_FIXED_UPLOAD = 39,
-               PROF_KEYGEN_COMBINATION = 40, PROF_PK_FORM_COPY = 41, PROF_PK_PLACE = 42 };
+               PROF_KEYGEN_COMBINATION = 40, PROF_PK_FORM_COPY = 41, PROF_PK_PLACE = 42,
+               PROF_OPEN_UPLOAD = 43, PROF_OPEN_EVAL = 44, PROF_OPEN_SCALARS = 45, PROF_OPEN_NUMERATORS = 46, PROF_OPEN_MSM = 47,
+               PROF_OPEN_LINEARISE = 48 };
 struct Profiler {
     bool enabled = false;
     std::vector<cudaEvent_t> ev;
@@ -121,6 +123,8 @@ struct DeviceCtx {
     DevBuf gen_table;                  // fixed-base table of the G1 generator, built on first use (g1gen.cu)
     DevBuf gen_scratch;                // normalisation denominators and SRS scalars of one chunk; the G1 NTT work buffer (g1gen.cu)
     DevBuf keygen_tables;              // the two-level delta^c omega^r tables of the sigma kernel (keygen.cu)
+    DevBuf open_scratch;               // point powers and level values of the query evaluation (multiopen.cu)
+    DevBuf open_tables;                // plan tables and pair values of h2b_fr_eval_queries_dev (api.cu)
     EvalScratch* eval = nullptr;       // compiled-program ring of the quotient evaluation (evaluate.cu)
     std::vector<NttTwiddles*> twiddles;  // small LRU cache keyed by (omega, log_n)
     MsmScratch* msm = nullptr;
@@ -144,6 +148,8 @@ int fq_batch_invert_run(DeviceCtx& ctx, void* d_a, size_t n, cudaStream_t stream
 int fr_prefix_product_run(DeviceCtx& ctx, const void* d_in, void* d_out, size_t n, cudaStream_t stream);
 int fr_eval_polynomial_run(DeviceCtx& ctx, const void* d_coeffs, size_t n, const uint64_t x[4], void* d_out, cudaStream_t stream);
 int fr_kate_division_run(DeviceCtx& ctx, const void* d_a, size_t n, const uint64_t b[4], void* d_q, cudaStream_t stream);
+// the same with the point b already on the device (d_b: one Fr, outside ctx.scan_scratch)
+int fr_kate_division_at_run(DeviceCtx& ctx, const void* d_a, size_t n, const void* d_b, void* d_q, cudaStream_t stream);
 int fr_lincomb_run(DeviceCtx& ctx, const void* const* d_cols, const uint64_t* coeffs, uint32_t m, size_t n, void* d_out, cudaStream_t stream);
 int permutation_product_run(DeviceCtx& ctx, const void* const* d_values, const void* const* d_sigma, uint32_t m, size_t n, const uint64_t* beta,
                             const uint64_t* gamma, const uint64_t* delta, const uint64_t* deltaomega, const uint64_t* omega, const uint64_t* last_z,
@@ -232,6 +238,36 @@ int combination_column_run(DeviceCtx& ctx, const void* d_bits, const void* d_mem
 int keygen_indicators_run(DeviceCtx& ctx, uint32_t k, uint32_t extended_k, uint32_t blinding_factors, const uint64_t omega_inv[4],
                           const uint64_t ifft_divisor[4], const uint64_t extended_omega[4], const uint64_t zeta_powers[12], void* const* d_cols,
                           cudaStream_t stream);
+// ---- multiopen.cu ----
+// construct_intermediate_sets of a list of queries over n_polys polynomials: slots are the polynomials in first-appearance order,
+// pairs the distinct (slot, point) queries grouped by slot, T the distinct points in first-appearance order; a set holds the slots
+// of one point set (points in its first slot's order).  Only index and byte comparisons: no field arithmetic on the host.
+static const uint32_t SHPLONK_MAX_POINTS = 16;
+struct ShplonkPlan {
+    std::vector<uint32_t> used;                   // caller's polynomial index of each slot
+    std::vector<const void*> d_polys;             // device coefficients of each slot (filled by the caller of the plan)
+    std::vector<uint64_t> points;                 // T, 4 Montgomery words per point
+    std::vector<uint32_t> pair_point;             // T index of each pair
+    std::vector<uint32_t> slot_first, slot_count; // the pairs of each slot
+    std::vector<uint32_t> query_pair;             // pair of each query
+    std::vector<uint32_t> slot_set, slot_member;  // set of each slot and its place j in the set
+    std::vector<std::vector<uint32_t>> set_slots, set_points;
+    uint32_t n_points() const { return (uint32_t)(points.size() / 4); }
+};
+bool fr_canonical(const uint64_t w[4]);
+// need_every_poly: a polynomial that no query names is refused
+int shplonk_plan_build(const char* who, const h2b_opening_query* queries, uint32_t n_queries, uint32_t n_polys, bool need_every_poly, ShplonkPlan* out);
+size_t shplonk_tables_bytes(const ShplonkPlan& p);
+size_t shplonk_scalars_count(const ShplonkPlan& p);
+int shplonk_tables_upload(const ShplonkPlan& p, const void* const* d_polys_by_slot, void* d_tables, cudaStream_t stream);
+const void* shplonk_tables_status(const ShplonkPlan& p, const void* d_tables);      // u32, 1 when z_0 = 0
+const void* shplonk_tables_jac(const ShplonkPlan& p, const void* d_tables);         // 96 B for an MSM result
+int shplonk_eval_pairs_run(DeviceCtx& ctx, const ShplonkPlan& p, const void* d_tables, size_t n, void* d_evals, cudaStream_t stream);
+int shplonk_eval_queries_run(DeviceCtx& ctx, const ShplonkPlan& p, const void* d_tables, size_t n, void* d_pair_evals, void* d_out, cudaStream_t stream);
+int shplonk_begin_run(DeviceCtx& ctx, const ShplonkPlan& p, const void* d_tables, size_t n, const uint64_t y[4], const uint64_t v[4], void* d_evals,
+                      void* d_scal, void* d_hx, void* d_a, void* d_b, cudaStream_t stream);
+int shplonk_finish_run(DeviceCtx& ctx, const ShplonkPlan& p, const void* d_tables, size_t n, const uint64_t u[4], const void* d_evals, void* d_scal,
+                       const void* d_hx, void* d_a, void* d_b, cudaStream_t stream);
 // ---- testgen.cu ----
 int msm_checksum_run(DeviceCtx& ctx, const void* d_scalars, uint64_t seed, uint64_t first, size_t n, void* d_out, cudaStream_t stream);
 int gen_scalars_run(DeviceCtx& ctx, uint64_t seed, size_t n, int kind, void* d_out, cudaStream_t stream);

@@ -229,18 +229,25 @@ static int kate_carries(DeviceCtx& ctx, const uint4* s, uint32_t chunks, const u
     return kate_level(ctx, s, chunks, pts, level + 1, carry, scratch, stream);
 }
 
-int fr_kate_division_run(DeviceCtx& ctx, const void* d_a, size_t n, const uint64_t b[4], void* d_q, cudaStream_t stream) {
+// b on the host (kind = cudaMemcpyHostToDevice) or on the device (cudaMemcpyDeviceToDevice)
+static int kate_division(DeviceCtx& ctx, const void* d_a, size_t n, const void* b, cudaMemcpyKind kind, void* d_q, cudaStream_t stream) {
     if (!b || (n && (!d_a || !d_q))) { set_error("kate_division: null pointer"); return H2B_ERR_BAD_ARGUMENT; }
     if (n <= 1) return H2B_OK;                 // the quotient of a constant is empty
     if (n > ((size_t)1 << 31)) { set_error("kate_division: at most 2^31 coefficients"); return H2B_ERR_BAD_ARGUMENT; }
     H2B_TRY(ctx.scan_scratch.reserve((n / 7 + 256) * 32));
     uint4* pts = (uint4*)ctx.scan_scratch.p;
     uint4* buf = pts + 2 * (POLY_LEVELS_MAX + 1);
-    H2B_CUDA(cudaMemcpyAsync(pts + 2 * POLY_LEVELS_MAX, b, 32, cudaMemcpyHostToDevice, stream));
+    H2B_CUDA(cudaMemcpyAsync(pts + 2 * POLY_LEVELS_MAX, b, 32, kind, stream));
     H2B_LAUNCH(fr_point_powers_kernel, 1, 32, 0, stream, (const uint4*)(pts + 2 * POLY_LEVELS_MAX), POLY_LEVELS_MAX, pts);
     H2B_TRY(kate_level(ctx, (const uint4*)d_a, n, pts, 0, (uint4*)d_q, buf, stream));
     H2B_CUDA(cudaGetLastError());
     return H2B_OK;
+}
+int fr_kate_division_run(DeviceCtx& ctx, const void* d_a, size_t n, const uint64_t b[4], void* d_q, cudaStream_t stream) {
+    return kate_division(ctx, d_a, n, b, cudaMemcpyHostToDevice, d_q, stream);
+}
+int fr_kate_division_at_run(DeviceCtx& ctx, const void* d_a, size_t n, const void* d_b, void* d_q, cudaStream_t stream) {
+    return kate_division(ctx, d_a, n, d_b, cudaMemcpyDeviceToDevice, d_q, stream);
 }
 
 // ---- the grand products themselves --------------------------------------------------------------------------------------

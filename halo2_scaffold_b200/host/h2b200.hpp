@@ -283,6 +283,8 @@ namespace kzg {
 enum class SerdeFormat : int { Processed = H2B_SERDE_PROCESSED, RawBytes = H2B_SERDE_RAW_BYTES, RawBytesUnchecked = H2B_SERDE_RAW_BYTES_UNCHECKED };
 
 class ParamsKZG {
+    friend class ProverSHPLONK;
+
   public:
     ParamsKZG(uint32_t k, const std::vector<G1Affine>& g, const std::vector<G1Affine>& g_lagrange, std::vector<uint8_t> g2_bytes = {})
         : k_(k), n_((uint64_t)1 << k), host_g_(g), host_g_lagrange_(g_lagrange), g2_bytes_(std::move(g2_bytes)) {
@@ -404,6 +406,37 @@ class ParamsKZG {
     std::vector<G1Affine> host_g_, host_g_lagrange_;
     std::vector<uint8_t> g2_bytes_;           // g2 | s_g2 as stored: G2 arithmetic is the verifier's (host) business
     uint64_t g_ = 0, g_lagrange_ = 0;
+};
+
+// ProverSHPLONK::create_proof ([UP] poly/kzg/multiopen/shplonk/prover.rs): queries are (polynomial, point) with the polynomial an
+// index into `polys` (upstream compares PolynomialPointers by address; a caller maps them to indices the same way).  y and v are the
+// challenges the caller squeezed; squeeze_u(h1) writes h1 to the transcript and returns u.  The session is released on every path.
+struct Query { uint32_t poly; Fr point; };
+class ProverSHPLONK {
+  public:
+    explicit ProverSHPLONK(const ParamsKZG& params, int device = 0) : params_(params), device_(device) {}
+    template <class SqueezeU>
+    std::pair<G1, G1> create_proof(const std::vector<std::vector<Fr>>& polys, const std::vector<Query>& queries, const Fr& y, const Fr& v,
+                                   SqueezeU squeeze_u) const {
+        std::vector<const void*> ptrs;
+        for (const auto& p : polys) ptrs.push_back(p.data());
+        std::vector<h2b_opening_query> q(queries.size());
+        for (size_t i = 0; i < queries.size(); ++i) { q[i].poly = queries[i].poly; q[i].reserved = 0; memcpy(q[i].point, queries[i].point.l, 32); }
+        const size_t n = polys.empty() ? 0 : polys[0].size();
+        for (const auto& p : polys) if (p.size() != n) throw Panic("ProverSHPLONK::create_proof: polynomials of different lengths");
+        G1 h1, h2;
+        uint64_t session = 0;
+        check(h2b_shplonk_begin(device_, ptrs.data(), 1, (uint32_t)polys.size(), n, q.data(), (uint32_t)q.size(), params_.g_, y.l, v.l,
+                                reinterpret_cast<uint64_t*>(&h1), &session), "ProverSHPLONK::create_proof (h1)");
+        struct Release { uint64_t s; ~Release() { h2b_shplonk_release(s); } } release{session};
+        const Fr u = squeeze_u(h1);
+        check(h2b_shplonk_finish(session, u.l, reinterpret_cast<uint64_t*>(&h2)), "ProverSHPLONK::create_proof (h2)");
+        return {h1, h2};
+    }
+
+  private:
+    const ParamsKZG& params_;
+    int device_;
 };
 
 }  // namespace kzg

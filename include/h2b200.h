@@ -480,6 +480,34 @@ int h2b_pk_info(uint64_t pk, uint64_t* per_device_bytes);
 /* drops the handle; freeing waits for the work queued on the pk's devices.  An unknown or already released handle fails. */
 int h2b_pk_release(uint64_t pk);
 
+/* ---- the multi-point opening: [UP] halo2_proofs/src/poly/kzg/multiopen/shplonk/prover.rs ProverSHPLONK::create_proof ----------
+ * A query opens polynomial `poly` (an index into the caller's list; polynomials are identified by index, as upstream identifies them
+ * by pointer) at `point` (Montgomery form).  Every polynomial has n coefficients.  Refused with H2B_ERR_BAD_ARGUMENT, every output
+ * untouched: no queries, a poly index >= n_polys, a polynomial that no query opens, a point >= r, more than 16 distinct points for one
+ * polynomial, n < 2 or n > 2^28. */
+typedef struct h2b_opening_query { uint32_t poly; uint32_t reserved; uint64_t point[4]; } h2b_opening_query;
+/* eval_polynomial(poly, point) of every query -> d_out (one Fr per query, in query order).  d_polys: n_polys device pointers.
+ * Each coefficient is read from device memory once per polynomial however many points open it.  Asynchronous on `stream`; its
+ * tables and scratch stay reserved on the device until h2b_shutdown. */
+int h2b_fr_eval_queries_dev(int device, const void* const* d_polys, uint32_t n_polys, size_t n, const h2b_opening_query* queries, uint32_t n_queries,
+                            void* d_out, void* stream);
+/* Steps 1-6 of create_proof: construct_intermediate_sets, the evaluations, interpolants, numerators, quotients and h_x, and
+ * h1 = commit(h_x) over the registered set handle_g (Jacobian, out_h1_jac) -- for the y and v the caller squeezed.  With
+ * polys_on_host, polys[i] are host arrays (pageable is fine), uploaded once into the session; otherwise they are device pointers on
+ * `device`, borrowed: they must stay unchanged until h2b_shplonk_finish returns.  Synchronous.  Besides the refusals above, a
+ * challenge >= r, an unknown handle_g and one that does not hold rows [0, n) on `device` are refused.  The session is a
+ * reference-counted handle like a proving key.  The scratch of the evaluations (about n / 15 Fr per (polynomial, point) pair) is
+ * shared with h2b_fr_eval_queries_dev and stays reserved on the device until h2b_shutdown, so that later openings allocate nothing
+ * but their session. */
+int h2b_shplonk_begin(int device, const void* const* polys, int polys_on_host, uint32_t n_polys, size_t n, const h2b_opening_query* queries,
+                      uint32_t n_queries, uint64_t handle_g, const uint64_t y[4], const uint64_t v[4], uint64_t out_h1_jac[12], uint64_t* session);
+/* Step 7 for the u the caller squeezed after writing h1: h2 = commit(kate_division(L, u) / z_0) (Jacobian, out_h2_jac).  Synchronous.
+ * u >= r and u in T \ S_0 (z_0 = 0, where upstream panics in invert().unwrap()) are refused, output untouched, and the session can
+ * be finished with another u; after a successful finish every further call on the session is refused. */
+int h2b_shplonk_finish(uint64_t session, const uint64_t u[4], uint64_t out_h2_jac[12]);
+/* drops the handle; device memory goes when the last call holding the session returns.  An unknown or released handle fails. */
+int h2b_shplonk_release(uint64_t session);
+
 /* ---- raw device memory helpers (so that non-CUDA hosts -- ctypes, Rust -- can hold device buffers) --- */
 int h2b_dev_alloc(int device, size_t bytes, void** out);
 int h2b_dev_free(int device, void* p);

@@ -137,6 +137,12 @@ extern "C" {
     pub fn h2b_pk_download(pk: u64, part: c_int, form: c_int, index: u32, host_out: *mut u64) -> c_int;
     pub fn h2b_pk_info(pk: u64, per_device_bytes: *mut u64) -> c_int;
     pub fn h2b_pk_release(pk: u64) -> c_int;
+    pub fn h2b_fr_eval_queries_dev(device: c_int, d_polys: *const *const c_void, n_polys: u32, n: usize, queries: *const h2b_opening_query, n_queries: u32,
+                                   d_out: *mut c_void, stream: *mut c_void) -> c_int;
+    pub fn h2b_shplonk_begin(device: c_int, polys: *const *const c_void, polys_on_host: c_int, n_polys: u32, n: usize, queries: *const h2b_opening_query,
+                             n_queries: u32, handle_g: u64, y: *const u64, v: *const u64, out_h1_jac: *mut u64, session: *mut u64) -> c_int;
+    pub fn h2b_shplonk_finish(session: u64, u: *const u64, out_h2_jac: *mut u64) -> c_int;
+    pub fn h2b_shplonk_release(session: u64) -> c_int;
     pub fn h2b_dev_alloc(device: c_int, bytes: usize, out: *mut *mut c_void) -> c_int;
     pub fn h2b_dev_free(device: c_int, p: *mut c_void) -> c_int;
     pub fn h2b_memcpy_h2d(device: c_int, d_dst: *mut c_void, h_src: *const c_void, bytes: usize) -> c_int;
@@ -495,5 +501,55 @@ impl ResidentProvingKey {
 impl Drop for ResidentProvingKey {
     fn drop(&mut self) {
         unsafe { h2b_pk_release(self.handle) };
+    }
+}
+
+/// `h2b_opening_query`: polynomial index and point (Montgomery limbs)
+#[repr(C)]
+#[derive(Clone, Copy)]
+pub struct h2b_opening_query {
+    pub poly: u32,
+    pub reserved: u32,
+    pub point: [u64; 4],
+}
+
+/// One SHPLONK opening between its two commitments (`h2b_shplonk_*`): `begin` returns h1, `finish` h2; `Drop` releases the session on
+/// every path, a panic included.  Polynomials are host slices of n Fr limbs, uploaded once by `begin`.
+pub struct ShplonkSession {
+    handle: u64,
+}
+
+impl ShplonkSession {
+    pub fn begin(polys: &[&[[u64; 4]]], queries: &[h2b_opening_query], handle_g: u64, y: &[u64; 4], v: &[u64; 4]) -> (Self, [u64; 12]) {
+        ensure_init();
+        let n = polys.first().map(|p| p.len()).unwrap_or(0);
+        assert!(polys.iter().all(|p| p.len() == n), "ProverSHPLONK: polynomials of different lengths");
+        let ptrs: Vec<*const c_void> = polys.iter().map(|p| p.as_ptr() as *const c_void).collect();
+        let mut h1 = [0u64; 12];
+        let mut handle = 0u64;
+        let rc = unsafe {
+            h2b_shplonk_begin(0, ptrs.as_ptr(), 1, ptrs.len() as u32, n, queries.as_ptr(), queries.len() as u32, handle_g, y.as_ptr(), v.as_ptr(),
+                              h1.as_mut_ptr(), &mut handle)
+        };
+        if rc != 0 {
+            panic!("h2b_shplonk_begin failed ({rc}): {}", last_error());
+        }
+        (ShplonkSession { handle }, h1)
+    }
+
+    pub fn finish(&self, u: &[u64; 4]) -> [u64; 12] {
+        let mut h2 = [0u64; 12];
+        let rc = unsafe { h2b_shplonk_finish(self.handle, u.as_ptr(), h2.as_mut_ptr()) };
+        if rc != 0 {
+            // upstream: z_0.invert().unwrap() panics when u is a point of T outside S_0
+            panic!("h2b_shplonk_finish failed ({rc}): {}", last_error());
+        }
+        h2
+    }
+}
+
+impl Drop for ShplonkSession {
+    fn drop(&mut self) {
+        unsafe { h2b_shplonk_release(self.handle) };
     }
 }

@@ -127,6 +127,16 @@ if "fixed_keygen_h2b" not in keygen.read_text():
                "        (cs, fixed, fixed_polys, fixed_cosets)\n"
                "    } else {\n    \\1\n    (cs, fixed, fixed_polys, fixed_cosets)\n    };", "keygen_pk's fixed columns", re.S)
     keygen.write_text(keygen.read_text() + "\n// ---- libh2b200 drop-in (rust/patches/fixed_keygen_dropin.rs) ----\n" + keygen_part + "\n")
+# ProverSHPLONK::create_proof (rust/patches/shplonk_dropin.rs, whose header states the mechanism)
+shplonk = crate / "src" / "poly" / "kzg" / "multiopen" / "shplonk" / "prover.rs"
+if "create_proof_h2b" not in shplonk.read_text():
+    m = re.search(r"(\n    fn create_proof<'com, Ch: EncodedChallenge<E::G1Affine>, T: TranscriptWrite<E::G1Affine, Ch>, R, I>\((.*?)\)\s*->\s*io::Result<\(\)>(.*?)\{)",
+                  shplonk.read_text(), re.S)
+    assert m, "ProverSHPLONK::create_proof not found in %s" % shplonk
+    substitute(shplonk, re.escape(m.group(1)), lambda _: m.group(1) + "\n        if TypeId::of::<E>() == TypeId::of::<Bn256>() { return self.create_proof_h2b(transcript, queries); }",
+               "ProverSHPLONK::create_proof", re.S)
+    add_uses(shplonk, ["use std::any::TypeId;", "use halo2curves::bn256::Bn256;", "use crate::poly::{Coeff, Polynomial};"])
+    shplonk.write_text(shplonk.read_text() + "\n// ---- libh2b200 drop-in (rust/patches/shplonk_dropin.rs) ----\n" + (rust / "patches" / "shplonk_dropin.rs").read_text() + "\n")
 toml = crate / "Cargo.toml"
 t = toml.read_text()
 if "h2b200-sys" not in t:
