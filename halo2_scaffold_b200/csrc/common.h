@@ -97,7 +97,6 @@ struct Profiler {
 struct Stager;        // stage.cu
 struct NttTwiddles;   // ntt.cu
 struct MsmScratch;    // msm.cu
-struct BaseSet;       // api.cu
 struct EvalScratch;   // evaluate.cu
 
 struct DeviceCtx {
@@ -111,7 +110,7 @@ struct DeviceCtx {
     bool ntt_attr_set = false;
     bool msm_attr_set = false;
     DevBuf ntt_io;                     // staging for the host-pointer NTT entry point
-    DevBuf ntt_fs[2];                  // the two other matrices of the multi-device four-step NTT (api.cu: ntt_multi_device)
+    DevBuf ntt_fs[2];                  // the two other matrices of the multi-device four-step NTT (api_sets.cu: ntt_multi_device)
     DevBuf col_ext;                    // extended form of h2b_column_pipeline when the caller only wants it on the host
     DevBuf scale_table;                // factor table of h2b_fr_scale_dev with more than 8 factors
     DevBuf msm_scalars;                // staging for host-pointer MSM scalars
@@ -124,7 +123,7 @@ struct DeviceCtx {
     DevBuf gen_scratch;                // normalisation denominators and SRS scalars of one chunk; the G1 NTT work buffer (g1gen.cu)
     DevBuf keygen_tables;              // the two-level delta^c omega^r tables of the sigma kernel (keygen.cu)
     DevBuf open_scratch;               // point powers and level values of the query evaluation (multiopen.cu)
-    DevBuf open_tables;                // plan tables and pair values of h2b_fr_eval_queries_dev (api.cu)
+    DevBuf open_tables;                // plan tables and pair values of h2b_fr_eval_queries_dev (api_open.cu)
     EvalScratch* eval = nullptr;       // compiled-program ring of the quotient evaluation (evaluate.cu)
     std::vector<NttTwiddles*> twiddles;  // small LRU cache keyed by (omega, log_n)
     MsmScratch* msm = nullptr;

@@ -535,7 +535,7 @@ int ntt_run_strided(DeviceCtx& ctx, void* d_base, size_t count, size_t stride_el
     return H2B_OK;
 }
 
-// ---- pieces of the four-step NTT across the devices of one process (api.cu: ntt_multi_device) ------------------------------------
+// ---- pieces of the four-step NTT across the devices of one process (api_sets.cu: ntt_multi_device) ------------------------------------
 // out[c * rows + r] = in[r * cols + c] for a rows x cols matrix of Fr elements (32-byte tiles through shared memory: both sides coalesced)
 __global__ void __launch_bounds__(256) fr_transpose_kernel(const uint4* __restrict__ in, uint4* __restrict__ out, uint32_t rows, uint32_t cols) {
     __shared__ uint4 tile[2][32][33];

@@ -17,7 +17,7 @@ fn main() {
         return;
     }
 
-    let sources = ["api.cu", "ntt.cu", "msm.cu", "testgen.cu", "g1gen.cu", "stage.cu", "scan.cu", "evaluate.cu", "srs.cu", "lookup.cu", "keygen.cu", "multiopen.cu"];
+    let sources = ["api.cu", "api_sets.cu", "api_srs.cu", "api_keygen.cu", "api_open.cu", "ntt.cu", "msm.cu", "testgen.cu", "g1gen.cu", "stage.cu", "scan.cu", "evaluate.cu", "srs.cu", "lookup.cu", "keygen.cu", "multiopen.cu"];
     let mut objects = Vec::new();
     for src in sources {
         let obj = out.join(src.replace(".cu", ".o"));
