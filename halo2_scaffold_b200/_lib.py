@@ -45,6 +45,7 @@ _EXPORTS = [
     "h2b_pk_create", "h2b_keygen_fixed_build_pk_resident", "h2b_permutation_build_pk_resident", "h2b_keygen_lagrange_indicators_resident",
     "h2b_pk_put_lagrange", "h2b_pk_column", "h2b_pk_download", "h2b_pk_info", "h2b_pk_release",
     "h2b_fr_eval_queries_dev", "h2b_shplonk_begin", "h2b_shplonk_finish", "h2b_shplonk_release",
+    "h2b_mock_verify",
 ]
 
 # include/h2b200.h enums of the resident proving key
@@ -97,6 +98,30 @@ class ShardStruct(ctypes.Structure):
 
 
 assert ctypes.sizeof(CalculationStruct) == 40
+
+
+# ---- include/h2b200.h structs of h2b_mock_verify -----------------------------------------------------------
+MOCK_CONSTRAINT_NOT_SATISFIED, MOCK_CONSTRAINT_POISONED, MOCK_LOOKUP, MOCK_PERMUTATION = range(4)
+MOCK_MAX_LOOKUP_WIDTH = 16
+
+
+class MockRootStruct(ctypes.Structure):
+    _fields_ = [("gate", ctypes.c_uint32), ("poly", ctypes.c_uint32), ("value", ValueSourceStruct)]
+
+
+class MockLookupStruct(ctypes.Structure):
+    _fields_ = [("graph", GraphStruct), ("inputs", ctypes.c_void_p), ("tables", ctypes.c_void_p), ("m", ctypes.c_uint32)]
+
+
+class MockCircuitStruct(ctypes.Structure):
+    _fields_ = [("k", ctypes.c_uint32), ("blinding_factors", ctypes.c_uint32),
+                ("fixed", ctypes.c_void_p), ("fixed_assigned", ctypes.c_void_p), ("n_fixed", ctypes.c_uint32),
+                ("advice", ctypes.c_void_p), ("advice_assigned", ctypes.c_void_p), ("n_advice", ctypes.c_uint32),
+                ("instance", ctypes.c_void_p), ("n_instance", ctypes.c_uint32),
+                ("challenges", ctypes.c_void_p), ("n_challenges", ctypes.c_uint32),
+                ("gates", ctypes.c_void_p), ("roots", ctypes.c_void_p), ("n_roots", ctypes.c_uint32),
+                ("lookups", ctypes.c_void_p), ("n_lookups", ctypes.c_uint32),
+                ("permutation", ctypes.c_void_p), ("mapping", ctypes.c_void_p), ("n_permutation", ctypes.c_uint32)]
 
 
 class GraphArrays:
@@ -231,6 +256,7 @@ class Lib:
         L.h2b_g1_generator_mul_dev.argtypes = [i32, vp, sz, vp, vp]
         L.h2b_g1_to_lagrange_dev.argtypes = [i32, vp, u32, vp, vp]
         L.h2b_srs_downsize.argtypes = [u64, u32, vp, ctypes.POINTER(u64), ctypes.POINTER(u64)]
+        L.h2b_mock_verify.argtypes = [i32, vp, vp, u64, ctypes.POINTER(u64)]
         L.h2b_permutation_sigma_dev.argtypes = [i32, vp, u32, u32, vp, vp, vp, vp, vp]
         L.h2b_keygen_lagrange_indicators_dev.argtypes = [i32, u32, u32, u32, vp, vp, vp, vp, vp, vp, vp, vp]
         L.h2b_permutation_build_vk.argtypes = [vp, u32, u32, vp, vp, u64, vp]
@@ -947,6 +973,51 @@ class Lib:
         else:
             sh = ShardStruct(*shard)
             self.check(self.L.h2b_evaluate_h_lookup_shard_dev(*args, ctypes.addressof(sh), stream))
+
+    def mock_verify(self, device: int, k: int, blinding_factors: int, fixed, fixed_assigned, advice, advice_assigned, instance, challenges,
+                    gates, roots, lookups, permutation, mapping, capacity: int, circuit_hook=None):
+        """h2b_mock_verify.  Columns: host arrays of 2^k x 4 u64 (Montgomery); *_assigned: (2^k + 7) // 8 bitmap bytes per column;
+        gates: GraphArrays (or None without roots); roots: [(gate, poly, value source)]; lookups: [(GraphArrays, input value sources,
+        table value sources)]; permutation: [(kind, index)] (H2B_VS_FIXED / ADVICE / INSTANCE); mapping: per permutation column 2^k x 2
+        u64.  circuit_hook(struct) may edit the circuit struct before the call (tests of the refusals).
+        -> (total count, the first min(count, capacity) records as (kind, index, poly, row) rows of a uint32 array)"""
+        keep = []
+
+        def cols(arrs, dtype, shape):
+            arrs = [np.ascontiguousarray(a, dtype=dtype).reshape(shape) for a in arrs]
+            keep.append(arrs)
+            return _ptr_array([a.ctypes.data for a in arrs]) if arrs else None, len(arrs)
+
+        n = 1 << k
+        fx, nf = cols(fixed, np.uint64, (-1, 4))
+        fa, _ = cols(fixed_assigned, np.uint8, (-1,))
+        ad, na = cols(advice, np.uint64, (-1, 4))
+        aa, _ = cols(advice_assigned, np.uint8, (-1,))
+        ins, ni = cols(instance, np.uint64, (-1, 4))
+        mp, npm = cols(mapping, np.uint64, (-1, 2))
+        ch = np.ascontiguousarray(challenges, dtype=np.uint64).reshape(-1, 4)
+        rt = (MockRootStruct * max(len(roots), 1))(*[MockRootStruct(g, p, ValueSourceStruct(*v)) for g, p, v in roots])
+        gs = gates.struct() if gates is not None else None
+        lks = (MockLookupStruct * max(len(lookups), 1))()
+        for i, (graph, ins_, tbs) in enumerate(lookups):
+            a = (ValueSourceStruct * max(len(ins_), 1))(*[ValueSourceStruct(*v) for v in ins_])
+            b = (ValueSourceStruct * max(len(tbs), 1))(*[ValueSourceStruct(*v) for v in tbs])
+            keep.append((graph, a, b))
+            lks[i] = MockLookupStruct(graph.struct(), ctypes.addressof(a), ctypes.addressof(b), len(ins_))
+        pm = np.ascontiguousarray(np.asarray(permutation, dtype=np.uint32).reshape(-1, 2))
+        c = MockCircuitStruct(k, blinding_factors, ctypes.addressof(fx) if fx else None, ctypes.addressof(fa) if fa else None, nf,
+                              ctypes.addressof(ad) if ad else None, ctypes.addressof(aa) if aa else None, na, ctypes.addressof(ins) if ins else None,
+                              ni, ch.ctypes.data, ch.shape[0], ctypes.addressof(gs) if gs is not None else None, ctypes.addressof(rt), len(roots),
+                              ctypes.addressof(lks), len(lookups), pm.ctypes.data, ctypes.addressof(mp) if mp else None, npm)
+        assert npm == pm.shape[0], "one mapping column per permutation column"
+        assert all(a.shape[0] == n for i in (0, 2, 4, 5) for a in keep[i]), "every column has 2^k rows"
+        assert all(a.shape[0] == (n + 7) // 8 for i in (1, 3) for a in keep[i]), "every bitmap has (2^k + 7) / 8 bytes"
+        if circuit_hook is not None:
+            circuit_hook(c)
+        out = np.zeros((max(int(capacity), 1), 4), dtype=np.uint32)
+        count = ctypes.c_uint64(0)
+        self.check(self.L.h2b_mock_verify(device, ctypes.addressof(c), out.ctypes.data if capacity else None, int(capacity), ctypes.byref(count)))
+        return count.value, out[:min(count.value, int(capacity))]
 
     def evaluate_graph_info(self):
         """-> (live-value slots, micro-operations) of the graph this thread compiled last"""

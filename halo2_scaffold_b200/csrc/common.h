@@ -81,7 +81,8 @@ enum ProfTag { PROF_BEGIN = 0, PROF_MSM_DECOMPOSE = 1, PROF_MSM_SCAN = 2, PROF_M
                PROF_KEYGEN_DOWNLOAD = 36, PROF_KEYGEN_PACK = 37, PROF_KEYGEN_EXCLUSION = 38, PROF_KEYGEN_FIXED_UPLOAD = 39,
                PROF_KEYGEN_COMBINATION = 40, PROF_PK_FORM_COPY = 41, PROF_PK_PLACE = 42,
                PROF_OPEN_UPLOAD = 43, PROF_OPEN_EVAL = 44, PROF_OPEN_SCALARS = 45, PROF_OPEN_NUMERATORS = 46, PROF_OPEN_MSM = 47,
-               PROF_OPEN_LINEARISE = 48 };
+               PROF_OPEN_LINEARISE = 48, PROF_MOCK_UPLOAD = 49, PROF_MOCK_GATES = 50, PROF_MOCK_LOOKUPS = 51, PROF_MOCK_PERMUTATION = 52,
+               PROF_MOCK_RECORDS = 53 };
 struct Profiler {
     bool enabled = false;
     std::vector<cudaEvent_t> ev;
@@ -267,6 +268,11 @@ int shplonk_begin_run(DeviceCtx& ctx, const ShplonkPlan& p, const void* d_tables
                       void* d_scal, void* d_hx, void* d_a, void* d_b, cudaStream_t stream);
 int shplonk_finish_run(DeviceCtx& ctx, const ShplonkPlan& p, const void* d_tables, size_t n, const uint64_t u[4], const void* d_evals, void* d_scal,
                        const void* d_hx, void* d_a, void* d_b, cudaStream_t stream);
+// ---- mock.cu ----
+// the refusals that need the compiler (graph and root contents); the caller has checked pointers, sizes and indices
+int mock_verify_check(const h2b_mock_circuit* c);
+// h2b_mock_verify on one device after every check: synchronous, the call's device memory given back before it returns
+int mock_verify_run(DeviceCtx& ctx, const h2b_mock_circuit* c, h2b_mock_record* records, uint64_t capacity, uint64_t* count);
 // ---- testgen.cu ----
 int msm_checksum_run(DeviceCtx& ctx, const void* d_scalars, uint64_t seed, uint64_t first, size_t n, void* d_out, cudaStream_t stream);
 int gen_scalars_run(DeviceCtx& ctx, uint64_t seed, size_t n, int kind, void* d_out, cudaStream_t stream);

@@ -15,47 +15,15 @@
 #include <algorithm>
 #include <cstdlib>
 
-#include "common.h"
+#include "evaluate.cuh"
 
 namespace h2b {
-
-enum MicroOp : uint32_t { MOP_ADD = 0, MOP_SUB = 1, MOP_MUL = 2, MOP_SQR = 3, MOP_DBL = 4, MOP_NEG = 5, MOP_FMA = 6, MOP_MOV = 7 };
-// operand encoding: kind in the top two bits
-static const uint32_t OPK_SLOT = 0u << 30, OPK_CONST = 1u << 30, OPK_COL = 2u << 30, OPK_PREV = 3u << 30, OPK_MASK = 3u << 30;
-static const uint32_t MOP_NOSTORE = 0x80;       // flag in the op word: the result is only consumed through OPK_PREV
-static const uint32_t MAX_ROT = 1024, MAX_COLS = 1u << 20, MAX_SLOTS = 64;
-
-struct EvalProgram {            // device view of a compiled graph
-    const uint4* ops;
-    const uint4* consts;        // Fr table: graph constants, challenges, beta, gamma, theta, y, zero
-    const uint32_t* rot_off;    // (rot * rot_scale).rem_euclid(size) per rotation index; last entry 0
-    const void* const* cols;    // fixed..., advice..., instance..., values
-    uint32_t n_ops;
-    uint32_t size;
-    // row shard: this launch evaluates rows [row0, row0 + rows) of the domain; every column pointer is a slice that starts at global row
-    // `base` = row0 - halo (mod size) and holds rows + 2 * halo rows.  The whole domain is row0 = base = 0, rows = size.
-    uint32_t row0, rows, base;
-};
-
-__device__ __forceinline__ uint32_t shard_local(uint32_t row, uint32_t base, uint32_t size) { return row >= base ? row - base : row + (size - base); }
 
 struct LookupTerms {            // the lookup argument's extra columns
     const uint4 *product, *permuted_input, *permuted_table, *l0, *l_last, *l_active_row;
     uint32_t off_next, off_prev;    // rot_scale and -rot_scale, reduced mod size
     uint32_t beta, gamma, y;        // indices into the constants table
 };
-
-__device__ __forceinline__ Fr eval_fetch(const EvalProgram& p, uint32_t enc, uint32_t idx, const Fr* slots, const Fr& prev) {
-    const uint32_t kind = enc & OPK_MASK, v = enc & ~OPK_MASK;
-    if (kind == OPK_PREV) return prev;
-    if (kind == OPK_SLOT) return slots[v];
-    if (kind == OPK_CONST) return fp_load<FR>(p.consts + 2 * (size_t)v);
-    uint32_t row = idx + __ldg(p.rot_off + (v & (MAX_ROT - 1)));
-    if (row >= p.size) row -= p.size;
-    row = shard_local(row, p.base, p.size);
-    const uint4* col = reinterpret_cast<const uint4*>(__ldg(reinterpret_cast<const unsigned long long*>(p.cols) + (v >> 10)));
-    return fp_load<FR>(col + 2 * (size_t)row);
-}
 
 template <int S>
 __device__ __forceinline__ Fr eval_row(const EvalProgram& p, uint32_t idx, Fr* slots) {
@@ -139,18 +107,8 @@ struct Ref {            // a resolved operand: either an external source (alread
     uint32_t enc = 0;
 };
 
-struct Compiled {
-    std::vector<uint4> ops;
-    std::vector<uint64_t> consts;       // 4 words per entry
-    std::vector<uint32_t> rot_off;
-    std::vector<const void*> cols;
-    uint32_t n_slots = 0;
-    uint32_t c_beta = 0, c_gamma = 0, c_theta = 0, c_y = 0, c_zero = 0;
-};
-
 thread_local uint32_t t_last_slots = 0, t_last_ops = 0;
 
-struct Shard { uint32_t row0, rows, halo, base; };
 // whole domain when `sh` is null; otherwise rows [row0, row0 + rows) with `halo` rows of every column on both sides
 static int make_shard(const h2b_eval_shard* sh, uint32_t size, Shard& out) {
     if (!sh) { out = Shard{0, size, 0, 0}; return H2B_OK; }
@@ -174,8 +132,11 @@ static uint32_t rem_euclid_u32(int64_t v, uint32_t size) {
     return (uint32_t)m;
 }
 
-static int compile_graph(const h2b_graph* g, const h2b_eval_columns* cols, const void* d_values, uint32_t size, int32_t rot_scale, bool previous_is_zero,
-                         const Shard& shard, Compiled& out) {
+}  // namespace
+
+int compile_graph(const h2b_graph* g, const h2b_eval_columns* cols, const void* d_values, uint32_t size, int32_t rot_scale, bool previous_is_zero,
+                  const Shard& shard, const h2b_value_source* roots, uint32_t n_roots, Compiled& out) {
+    if (n_roots && !roots) { set_error("evaluate: null root list"); return H2B_ERR_BAD_ARGUMENT; }
     if (!g || !cols) { set_error("evaluate: null graph / columns"); return H2B_ERR_BAD_ARGUMENT; }
     if (size == 0 || size > (1u << 30)) { set_error("evaluate: size must be in [1, 2^30]"); return H2B_ERR_BAD_ARGUMENT; }
     if ((g->n_constants && !g->constants) || (g->n_rotations && !g->rotations) || (g->n_calculations && !g->calculations) || (g->n_parts && !g->parts) ||
@@ -216,7 +177,7 @@ static int compile_graph(const h2b_graph* g, const h2b_eval_columns* cols, const
     const uint32_t n = g->n_calculations;
     out.ops.clear();
     out.n_slots = 0;
-    if (n == 0) return H2B_OK;
+    if (n == 0 && n_roots == 0) return H2B_OK;
 
     // 1. resolve operands: intermediates become references to the calculation that defined them, Stores are forwarded
     std::vector<int32_t> cur_def(g->n_intermediates, -1);
@@ -278,10 +239,15 @@ static int compile_graph(const h2b_graph* g, const h2b_eval_columns* cols, const
         cur_def[k.target] = (int32_t)c;
     }
     first[n] = (uint32_t)refs.size();
+    std::vector<Ref> root_refs(n_roots);
+    for (uint32_t i = 0; i < n_roots; ++i) {
+        root_refs[i] = resolve(roots[i], n);
+        if (bad) { set_error("evaluate: root %u: out-of-range or unwritten value source", i); return H2B_ERR_BAD_ARGUMENT; }
+    }
 
-    // 2. the result is the last calculation's value; count the uses of every reachable calculation
-    const uint32_t root = n - 1;
-    const bool root_is_store = g->calculations[root].op == H2B_CALC_STORE;
+    // 2. the result is the last calculation's value, or every root; count the uses of every reachable calculation
+    const uint32_t root = n ? n - 1 : 0;
+    const bool root_is_store = n_roots == 0 && g->calculations[root].op == H2B_CALC_STORE;
     std::vector<uint32_t> uses(n, 0);
     std::vector<uint8_t> reach(n, 0);
     std::vector<uint32_t> stack;
@@ -290,7 +256,9 @@ static int compile_graph(const h2b_graph* g, const h2b_eval_columns* cols, const
         ++uses[r.def];
         if (!reach[r.def]) { reach[r.def] = 1; stack.push_back((uint32_t)r.def); }
     };
-    if (root_is_store) visit(alias[root]); else { reach[root] = 1; stack.push_back(root); }
+    if (n_roots) for (const Ref& r : root_refs) visit(r);
+    else if (root_is_store) visit(alias[root]);
+    else { reach[root] = 1; stack.push_back(root); }
     while (!stack.empty()) {
         const uint32_t c = stack.back();
         stack.pop_back();
@@ -314,67 +282,80 @@ static int compile_graph(const h2b_graph* g, const h2b_eval_columns* cols, const
     std::vector<Frame> frames;
     std::vector<uint8_t> done(n, 0);
     auto push = [&](uint32_t c) { frames.push_back(Frame{c, 0, -1}); };
-    if (root_is_store) { if (alias[root].def >= 0) push((uint32_t)alias[root].def); } else push(root);
-    while (!frames.empty()) {
-        Frame& f = frames.back();
-        const uint32_t c = f.c;
-        if (done[c]) { frames.pop_back(); continue; }
-        const h2b_calculation& k = g->calculations[c];
-        const uint32_t lo = first[c], cnt = first[c + 1] - lo;
-        if (k.op != H2B_CALC_HORNER) {
-            // make sure every operand exists, then emit
-            bool pushed = false;
-            for (uint32_t i = f.stage; i < cnt; ++i) {
-                const Ref& r = refs[lo + i];
-                if (r.def >= 0 && !done[r.def]) { f.stage = i; push((uint32_t)r.def); pushed = true; break; }
+    auto drain = [&]() {
+        while (!frames.empty()) {
+            Frame& f = frames.back();
+            const uint32_t c = f.c;
+            if (done[c]) { frames.pop_back(); continue; }
+            const h2b_calculation& k = g->calculations[c];
+            const uint32_t lo = first[c], cnt = first[c + 1] - lo;
+            if (k.op != H2B_CALC_HORNER) {
+                // make sure every operand exists, then emit
+                bool pushed = false;
+                for (uint32_t i = f.stage; i < cnt; ++i) {
+                    const Ref& r = refs[lo + i];
+                    if (r.def >= 0 && !done[r.def]) { f.stage = i; push((uint32_t)r.def); pushed = true; break; }
+                }
+                if (pushed) continue;
+                const uint32_t a = enc_of(refs[lo]), b = cnt > 1 ? enc_of(refs[lo + 1]) : 0;
+                for (uint32_t i = 0; i < cnt; ++i) release(refs[lo + i]);
+                const uint32_t dst = alloc_slot();
+                static const uint32_t code_of[8] = {MOP_ADD, MOP_SUB, MOP_MUL, MOP_SQR, MOP_DBL, MOP_NEG, MOP_FMA, MOP_MOV};
+                emit(code_of[k.op], dst, a, b, 0);
+                slot_of[c] = (int32_t)dst;
+                done[c] = 1;
+                frames.pop_back();
+                continue;
             }
-            if (pushed) continue;
-            const uint32_t a = enc_of(refs[lo]), b = cnt > 1 ? enc_of(refs[lo + 1]) : 0;
-            for (uint32_t i = 0; i < cnt; ++i) release(refs[lo + i]);
-            const uint32_t dst = alloc_slot();
-            static const uint32_t code_of[8] = {MOP_ADD, MOP_SUB, MOP_MUL, MOP_SQR, MOP_DBL, MOP_NEG, MOP_FMA, MOP_MOV};
-            emit(code_of[k.op], dst, a, b, 0);
-            slot_of[c] = (int32_t)dst;
-            done[c] = 1;
-            frames.pop_back();
-            continue;
+            // Horner(start = refs[lo], factor = refs[lo+1], parts = refs[lo+2 ..]): value = start; value = value * factor + part
+            // stage 0/1: ensure start and factor; stage 2 + j: part j
+            if (f.stage < 2) {
+                const Ref& r = refs[lo + f.stage];
+                ++f.stage;
+                if (r.def >= 0 && !done[r.def]) { push((uint32_t)r.def); continue; }
+                continue;
+            }
+            const uint32_t parts = cnt - 2;
+            const uint32_t j = f.stage - 2;
+            if (parts == 0) {
+                const uint32_t a = enc_of(refs[lo]);
+                release(refs[lo]); release(refs[lo + 1]);
+                const uint32_t dst = alloc_slot();
+                emit(MOP_MOV, dst, a, 0, 0);
+                slot_of[c] = (int32_t)dst; done[c] = 1; frames.pop_back();
+                continue;
+            }
+            const Ref& part = refs[lo + 2 + j];
+            if (part.def >= 0 && !done[part.def]) { push((uint32_t)part.def); continue; }      // same stage again afterwards
+            {
+                const uint32_t acc = f.acc < 0 ? enc_of(refs[lo]) : (OPK_SLOT | (uint32_t)f.acc);
+                const uint32_t fac = enc_of(refs[lo + 1]), pe = enc_of(part);
+                if (f.acc < 0) release(refs[lo]); else free_slots.push_back((uint32_t)f.acc);
+                release(part);
+                if (j + 1 == parts) release(refs[lo + 1]);
+                const uint32_t dst = alloc_slot();
+                emit(MOP_FMA, dst, acc, fac, pe);
+                f.acc = (int32_t)dst;
+                ++f.stage;
+                if (j + 1 == parts) { slot_of[c] = (int32_t)dst; done[c] = 1; frames.pop_back(); }
+            }
         }
-        // Horner(start = refs[lo], factor = refs[lo+1], parts = refs[lo+2 ..]): value = start; value = value * factor + part
-        // stage 0/1: ensure start and factor; stage 2 + j: part j
-        if (f.stage < 2) {
-            const Ref& r = refs[lo + f.stage];
-            ++f.stage;
-            if (r.def >= 0 && !done[r.def]) { push((uint32_t)r.def); continue; }
-            continue;
+    };
+    if (n_roots) {
+        // each root right after what it needs, then its check; a root shared with a later one keeps its slot until then
+        for (uint32_t i = 0; i < n_roots; ++i) {
+            const Ref& r = root_refs[i];
+            if (r.def >= 0 && !done[r.def]) { push((uint32_t)r.def); drain(); }
+            emit(MOP_CHECK | MOP_NOSTORE, 0, enc_of(r), i, 0);
+            release(r);
         }
-        const uint32_t parts = cnt - 2;
-        const uint32_t j = f.stage - 2;
-        if (parts == 0) {
-            const uint32_t a = enc_of(refs[lo]);
-            release(refs[lo]); release(refs[lo + 1]);
-            const uint32_t dst = alloc_slot();
-            emit(MOP_MOV, dst, a, 0, 0);
-            slot_of[c] = (int32_t)dst; done[c] = 1; frames.pop_back();
-            continue;
+    } else {
+        if (root_is_store) { if (alias[root].def >= 0) push((uint32_t)alias[root].def); } else push(root);
+        drain();
+        if (root_is_store || out.ops.empty()) {
+            const Ref& r = alias[root];
+            emit(MOP_MOV, alloc_slot(), enc_of(r), 0, 0);
         }
-        const Ref& part = refs[lo + 2 + j];
-        if (part.def >= 0 && !done[part.def]) { push((uint32_t)part.def); continue; }      // same stage again afterwards
-        {
-            const uint32_t acc = f.acc < 0 ? enc_of(refs[lo]) : (OPK_SLOT | (uint32_t)f.acc);
-            const uint32_t fac = enc_of(refs[lo + 1]), pe = enc_of(part);
-            if (f.acc < 0) release(refs[lo]); else free_slots.push_back((uint32_t)f.acc);
-            release(part);
-            if (j + 1 == parts) release(refs[lo + 1]);
-            const uint32_t dst = alloc_slot();
-            emit(MOP_FMA, dst, acc, fac, pe);
-            f.acc = (int32_t)dst;
-            ++f.stage;
-            if (j + 1 == parts) { slot_of[c] = (int32_t)dst; done[c] = 1; frames.pop_back(); }
-        }
-    }
-    if (root_is_store || out.ops.empty()) {
-        const Ref& r = alias[root];
-        emit(MOP_MOV, alloc_slot(), enc_of(r), 0, 0);
     }
     if (n_slots > MAX_SLOTS) { set_error("evaluate: graph needs %u live values per row (limit %u)", n_slots, MAX_SLOTS); return H2B_ERR_BAD_ARGUMENT; }
 
@@ -383,6 +364,7 @@ static int compile_graph(const h2b_graph* g, const h2b_eval_columns* cols, const
     std::vector<uint4>& ops = out.ops;
     auto n_operands = [](uint32_t code) { return code == MOP_FMA ? 3u : (code == MOP_ADD || code == MOP_SUB || code == MOP_MUL) ? 2u : 1u; };
     for (size_t i = 1; i < ops.size(); ++i) {
+        if ((ops[i - 1].x & 0x7f) == MOP_CHECK) continue;          // a check writes no slot
         const uint32_t prev_dst = OPK_SLOT | (ops[i - 1].x >> 8);
         uint32_t* e[3] = {&ops[i].y, &ops[i].z, &ops[i].w};
         for (uint32_t q = 0; q < n_operands(ops[i].x & 0x7f); ++q) if (*e[q] == prev_dst) *e[q] = OPK_PREV;
@@ -390,8 +372,10 @@ static int compile_graph(const h2b_graph* g, const h2b_eval_columns* cols, const
     std::vector<uint8_t> live(n_slots ? n_slots : 1, 0);
     for (size_t i = ops.size(); i-- > 0;) {
         const uint32_t dst = ops[i].x >> 8;
-        if (!live[dst]) ops[i].x |= MOP_NOSTORE;
-        live[dst] = 0;
+        if ((ops[i].x & 0x7f) != MOP_CHECK) {
+            if (!live[dst]) ops[i].x |= MOP_NOSTORE;
+            live[dst] = 0;
+        }
         const uint32_t e[3] = {ops[i].y, ops[i].z, ops[i].w};
         for (uint32_t q = 0; q < n_operands(ops[i].x & 0x7f); ++q) if ((e[q] & OPK_MASK) == OPK_SLOT) live[e[q] & ~OPK_MASK] = 1;
     }
@@ -399,11 +383,6 @@ static int compile_graph(const h2b_graph* g, const h2b_eval_columns* cols, const
     return H2B_OK;
 }
 
-// device copy of a compiled program: a small ring of buffers per device so that calls on different streams do not
-// overwrite a program a running kernel still reads
-struct ProgramBuf { DevBuf buf; cudaEvent_t done = nullptr; };
-
-}  // namespace
 
 struct EvalScratch {
     ProgramBuf ring[4];
@@ -424,7 +403,7 @@ static uint32_t eval_ctas_per_sm(uint32_t dflt) {
     return forced ? (uint32_t)forced : dflt;
 }
 
-static int upload_program(DeviceCtx& ctx, const Compiled& c, uint32_t size, const Shard& shard, cudaStream_t stream, EvalProgram& dev, ProgramBuf** used) {
+int upload_program(DeviceCtx& ctx, const Compiled& c, uint32_t size, const Shard& shard, cudaStream_t stream, EvalProgram& dev, ProgramBuf** used) {
     if (!ctx.eval) ctx.eval = new EvalScratch();
     ProgramBuf& pb = ctx.eval->ring[ctx.eval->next++ & 3];
     const size_t o_ops = 0, o_consts = align16(o_ops + c.ops.size() * 16), o_rot = align16(o_consts + c.consts.size() * 8),
@@ -470,7 +449,7 @@ int evaluate_graph_run(DeviceCtx& ctx, const h2b_graph* g, const h2b_eval_column
     Shard shard;
     H2B_TRY(make_shard(sh, size, shard));
     Compiled c;
-    H2B_TRY(compile_graph(g, cols, d_values, size, rot_scale, false, shard, c));
+    H2B_TRY(compile_graph(g, cols, d_values, size, rot_scale, false, shard, nullptr, 0, c));
     t_last_slots = c.n_slots;
     t_last_ops = (uint32_t)c.ops.size();
     if (c.ops.empty()) {        // no calculations: upstream returns zero for every row
@@ -499,7 +478,7 @@ int evaluate_h_lookup_run(DeviceCtx& ctx, const h2b_graph* g, const h2b_eval_col
     H2B_TRY(make_shard(sh, size, shard));
     if (!offset_within_halo(rem_euclid_u32((int64_t)rot_scale, size), size, shard)) { set_error("evaluate_h_lookup: rot_scale exceeds the shard's halo"); return H2B_ERR_BAD_ARGUMENT; }
     Compiled c;
-    H2B_TRY(compile_graph(g, cols, d_values, size, rot_scale, true, shard, c));
+    H2B_TRY(compile_graph(g, cols, d_values, size, rot_scale, true, shard, nullptr, 0, c));
     if (c.ops.empty()) c.ops.push_back(make_uint4(MOP_MOV | MOP_NOSTORE, OPK_CONST | c.c_zero, 0, 0));      // table_value = 0
     t_last_slots = c.n_slots;
     t_last_ops = (uint32_t)c.ops.size();

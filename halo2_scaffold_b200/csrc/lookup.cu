@@ -14,36 +14,9 @@
 //     are elementwise kernels.  The order of the fill is exactly upstream's: the i-th smallest leftover value goes to the
 //     i-th repeated row counted from the end.
 // Rows at and beyond usable_rows (the blinding rows) are the caller's.
-#include "common.h"
+#include "keys.cuh"
 
 namespace h2b {
-
-static const uint32_t SORT_TILE_LOG = 10, SORT_TILE = 1u << SORT_TILE_LOG;       // elements per CTA in the shared-memory phases
-
-struct Key { uint32_t l[8]; };
-__device__ __forceinline__ bool key_less(const Key& a, const Key& b) {
-#pragma unroll
-    for (int i = 7; i >= 0; --i) {
-        if (a.l[i] != b.l[i]) return a.l[i] < b.l[i];
-    }
-    return false;
-}
-__device__ __forceinline__ bool key_eq(const Key& a, const Key& b) {
-    uint32_t o = 0;
-#pragma unroll
-    for (int i = 0; i < 8; ++i) o |= a.l[i] ^ b.l[i];
-    return o == 0;
-}
-__device__ __forceinline__ Key key_load(const uint4* p, size_t i) {
-    const uint4 a = p[2 * i], b = p[2 * i + 1];
-    Key k;
-    k.l[0] = a.x; k.l[1] = a.y; k.l[2] = a.z; k.l[3] = a.w; k.l[4] = b.x; k.l[5] = b.y; k.l[6] = b.z; k.l[7] = b.w;
-    return k;
-}
-__device__ __forceinline__ void key_store(uint4* p, size_t i, const Key& k) {
-    p[2 * i] = make_uint4(k.l[0], k.l[1], k.l[2], k.l[3]);
-    p[2 * i + 1] = make_uint4(k.l[4], k.l[5], k.l[6], k.l[7]);
-}
 
 // canonical keys of the first `usable` rows, all-ones padding up to `padded`
 __global__ void __launch_bounds__(256) lookup_keys_kernel(const uint4* __restrict__ in, uint32_t usable, uint32_t padded, uint4* __restrict__ keys) {
@@ -153,7 +126,7 @@ __global__ void __launch_bounds__(512) bitonic_shared_kernel(uint4* __restrict__
     }
 }
 
-static int bitonic_sort(uint4* keys, uint32_t padded, cudaStream_t stream) {      // padded: a power of two
+int bitonic_sort(uint4* keys, uint32_t padded, cudaStream_t stream) {      // padded: a power of two
     const uint32_t tiles = (padded + SORT_TILE - 1) / SORT_TILE;
     H2B_LAUNCH(bitonic_shared_kernel, tiles, 512, 0, stream, keys, padded, 0u);
     for (uint32_t k = SORT_TILE << 1; k != 0 && k <= padded; k <<= 1) {
@@ -172,7 +145,6 @@ static int bitonic_sort(uint4* keys, uint32_t padded, cudaStream_t stream) {    
 }
 
 // ---- exclusive scan of 32-bit flags (out[count] = total) -----------------------------------------------------------------
-static const uint32_t FLAG_SCAN_BLOCK = 1024;
 __global__ void __launch_bounds__(256) flag_scan_sums_kernel(const uint32_t* __restrict__ in, uint32_t count, uint32_t* __restrict__ sums) {
     __shared__ uint32_t ws[8];
     const uint32_t base = blockIdx.x * FLAG_SCAN_BLOCK + threadIdx.x * 4;
@@ -216,7 +188,7 @@ __global__ void __launch_bounds__(256) flag_scan_apply_kernel(const uint32_t* __
     }
     if (blockIdx.x == gridDim.x - 1 && threadIdx.x == 255) out[count] = sums[gridDim.x];
 }
-static int flag_scan(const uint32_t* in, uint32_t count, uint32_t* out, uint32_t* sums, cudaStream_t stream) {
+int flag_scan(const uint32_t* in, uint32_t count, uint32_t* out, uint32_t* sums, cudaStream_t stream) {
     const uint32_t nblocks = (count + FLAG_SCAN_BLOCK - 1) / FLAG_SCAN_BLOCK;
     H2B_LAUNCH(flag_scan_sums_kernel, nblocks, 256, 0, stream, in, count, sums);
     H2B_LAUNCH(flag_scan_top_kernel, 1, 32, 0, stream, sums, nblocks);

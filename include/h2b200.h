@@ -508,6 +508,54 @@ int h2b_shplonk_finish(uint64_t session, const uint64_t u[4], uint64_t out_h2_ja
 /* drops the handle; device memory goes when the last call holding the session returns.  An unknown or released handle fails. */
 int h2b_shplonk_release(uint64_t session);
 
+/* ---- MockProver::verify: [UP] halo2_proofs/src/dev.rs, the gate, lookup and permutation loops of verify_par ---------------------
+ * n = 2^k rows, usable_rows = n - (blinding_factors + 1).  Cells follow upstream's CellValue: a fixed or advice cell is Assigned
+ * when bit r of its column's bitmap is set (byte r / 8, bit r % 8) and Unassigned otherwise, whatever its value word holds; advice
+ * rows >= usable_rows are Poison(row) (their bits are ignored); instance cells are Assigned(value).  In an expression an Unassigned
+ * cell reads Real(0) and a Poison cell Poison, with upstream's Value arithmetic (Poison * Real(0) = Real(0), Poison otherwise).
+ *   gates   : one graph, its roots in (gate, poly) order, gates ascending.  A root that is Real(!= 0) at row r in [0, n) is
+ *             CONSTRAINT_NOT_SATISFIED, a Poison one CONSTRAINT_POISONED.  Records in (gate, row, poly) order.
+ *   lookups : per lookup a graph with m input roots and m table roots (1 <= m <= H2B_MOCK_MAX_LOOKUP_WIDTH).  fill_row = the table
+ *             tuple at row usable_rows - 1; an input tuple at a usable row that differs from fill_row and from every table tuple of the
+ *             usable rows is a LOOKUP record (index = lookup, poly = 0).  Tuples compare exactly (Real < Poison, Reals by their
+ *             canonical integers).  Records in (lookup, row) order; upstream reports them in (tuple, row) order, which the caller
+ *             restores by sorting the few failures.
+ *   copies  : per permutation column c and row r, (column, row) = mapping[c][2 r], mapping[c][2 r + 1] -- the layout of
+ *             h2b_permutation_sigma_dev.  A cell unequal to its mapped cell (CellValue equality: Unassigned != Assigned(0),
+ *             Poison(i) == Poison(j) only for i = j) is a PERMUTATION record (index = c, poly = 0).  Records in (c, row) order.
+ * The output holds the gate records, then the lookup records, then the permutation records: *count is their total and the first
+ * min(total, capacity) are written to `records`.  A caller that sees *count > capacity calls again with a larger buffer.
+ * Synchronous, on one device.  Host columns may be pageable.  Device memory is allocated for the call and given back before it
+ * returns.  Refused with H2B_ERR_BAD_ARGUMENT before any output is written: null pointers, k = 0 or k > 28, blinding_factors + 1 >= n,
+ * a column, challenge, constant or rotation index out of range, a graph or root that reads an intermediate no calculation wrote, roots
+ * out of gate order, more than H2B_MOCK_MAX_LOOKUP_WIDTH expressions per lookup side, a graph needing more than 64 live values per row,
+ * a permutation column of another kind than fixed / advice / instance and a mapping entry outside the permutation's columns and n
+ * rows.  Profiling tags: 49 uploads, 50 gate check, 51 lookups, 52 copy constraints, 53 scans and records. */
+#define H2B_MOCK_MAX_LOOKUP_WIDTH 16
+enum h2b_mock_failure {
+    H2B_MOCK_CONSTRAINT_NOT_SATISFIED = 0, H2B_MOCK_CONSTRAINT_POISONED = 1, H2B_MOCK_LOOKUP = 2, H2B_MOCK_PERMUTATION = 3
+};
+typedef struct h2b_mock_record { uint32_t kind, index, poly, row; } h2b_mock_record;
+typedef struct h2b_mock_root { uint32_t gate, poly; h2b_value_source value; } h2b_mock_root;
+typedef struct h2b_mock_lookup {
+    h2b_graph graph;                     /* over the circuit's columns and challenges */
+    const h2b_value_source* inputs;      /* m roots: the input expressions */
+    const h2b_value_source* tables;      /* m roots: the table expressions */
+    uint32_t m;
+} h2b_mock_lookup;
+typedef struct h2b_mock_column { uint32_t kind, index; } h2b_mock_column;      /* kind: H2B_VS_FIXED, H2B_VS_ADVICE or H2B_VS_INSTANCE */
+typedef struct h2b_mock_circuit {
+    uint32_t k, blinding_factors;
+    const uint64_t* const* fixed; const uint8_t* const* fixed_assigned; uint32_t n_fixed;        /* host: n x 4 words, n / 8 bytes */
+    const uint64_t* const* advice; const uint8_t* const* advice_assigned; uint32_t n_advice;
+    const uint64_t* const* instance; uint32_t n_instance;
+    const uint64_t* challenges; uint32_t n_challenges;                                             /* n_challenges x 4 words */
+    const h2b_graph* gates; const h2b_mock_root* roots; uint32_t n_roots;                          /* gates may be NULL when n_roots = 0 */
+    const h2b_mock_lookup* lookups; uint32_t n_lookups;
+    const h2b_mock_column* permutation; const uint64_t* const* mapping; uint32_t n_permutation;    /* mapping: host, n x 2 words each */
+} h2b_mock_circuit;
+int h2b_mock_verify(int device, const h2b_mock_circuit* circuit, h2b_mock_record* records, uint64_t capacity, uint64_t* count);
+
 /* ---- raw device memory helpers (so that non-CUDA hosts -- ctypes, Rust -- can hold device buffers) --- */
 int h2b_dev_alloc(int device, size_t bytes, void** out);
 int h2b_dev_free(int device, void* p);

@@ -17,7 +17,7 @@ fn main() {
         return;
     }
 
-    let sources = ["api.cu", "api_sets.cu", "api_srs.cu", "api_keygen.cu", "api_open.cu", "ntt.cu", "msm.cu", "testgen.cu", "g1gen.cu", "stage.cu", "scan.cu", "evaluate.cu", "srs.cu", "lookup.cu", "keygen.cu", "multiopen.cu"];
+    let sources = ["api.cu", "api_sets.cu", "api_srs.cu", "api_keygen.cu", "api_open.cu", "api_mock.cu", "ntt.cu", "msm.cu", "testgen.cu", "g1gen.cu", "stage.cu", "scan.cu", "evaluate.cu", "srs.cu", "lookup.cu", "keygen.cu", "multiopen.cu", "mock.cu"];
     let mut objects = Vec::new();
     for src in sources {
         let obj = out.join(src.replace(".cu", ".o"));
@@ -32,7 +32,7 @@ fn main() {
         objects.push(obj);
         println!("cargo:rerun-if-changed={}", csrc.join(src).display());
     }
-    for hdr in ["common.h", "field.cuh", "ec.cuh", "field_asm.inc"] {
+    for hdr in ["common.h", "evaluate.cuh", "keys.cuh", "field.cuh", "ec.cuh", "field_asm.inc"] {
         println!("cargo:rerun-if-changed={}", csrc.join(hdr).display());
     }
     let lib = out.join("libh2b200.a");

@@ -553,3 +553,54 @@ impl Drop for ShplonkSession {
         unsafe { h2b_shplonk_release(self.handle) };
     }
 }
+
+// ---- MockProver::verify's row loops (h2b_mock_verify) --------------------------------------------------------------------------
+pub const H2B_MOCK_CONSTRAINT_NOT_SATISFIED: u32 = 0;
+pub const H2B_MOCK_CONSTRAINT_POISONED: u32 = 1;
+pub const H2B_MOCK_LOOKUP: u32 = 2;
+pub const H2B_MOCK_PERMUTATION: u32 = 3;
+#[repr(C)]
+#[derive(Clone, Copy, Default, Debug)]
+pub struct h2b_mock_record { pub kind: u32, pub index: u32, pub poly: u32, pub row: u32 }
+#[repr(C)]
+#[derive(Clone, Copy)]
+pub struct h2b_mock_root { pub gate: u32, pub poly: u32, pub value: h2b_value_source }
+#[repr(C)]
+pub struct h2b_mock_lookup { pub graph: h2b_graph, pub inputs: *const h2b_value_source, pub tables: *const h2b_value_source, pub m: u32 }
+#[repr(C)]
+#[derive(Clone, Copy)]
+pub struct h2b_mock_column { pub kind: u32, pub index: u32 }
+#[repr(C)]
+pub struct h2b_mock_circuit {
+    pub k: u32, pub blinding_factors: u32,
+    pub fixed: *const *const u64, pub fixed_assigned: *const *const u8, pub n_fixed: u32,
+    pub advice: *const *const u64, pub advice_assigned: *const *const u8, pub n_advice: u32,
+    pub instance: *const *const u64, pub n_instance: u32,
+    pub challenges: *const u64, pub n_challenges: u32,
+    pub gates: *const h2b_graph, pub roots: *const h2b_mock_root, pub n_roots: u32,
+    pub lookups: *const h2b_mock_lookup, pub n_lookups: u32,
+    pub permutation: *const h2b_mock_column, pub mapping: *const *const u64, pub n_permutation: u32,
+}
+extern "C" {
+    pub fn h2b_mock_verify(device: c_int, circuit: *const h2b_mock_circuit, records: *mut h2b_mock_record, capacity: u64, count: *mut u64) -> c_int;
+}
+
+/// Every record of h2b_mock_verify on device 0: asks once with room for `first_capacity` records and again with room for all when
+/// there are more.  Panics on a refused circuit, as upstream's index arithmetic would.
+pub fn mock_verify(circuit: &h2b_mock_circuit, first_capacity: usize) -> Vec<h2b_mock_record> {
+    ensure_init();
+    let mut cap = first_capacity.max(1);
+    loop {
+        let mut records = vec![h2b_mock_record::default(); cap];
+        let mut count = 0u64;
+        let rc = unsafe { h2b_mock_verify(0, circuit, records.as_mut_ptr(), cap as u64, &mut count) };
+        if rc != 0 {
+            panic!("h2b_mock_verify failed ({rc}): {}", last_error());
+        }
+        if count as usize <= cap {
+            records.truncate(count as usize);
+            return records;
+        }
+        cap = count as usize;
+    }
+}

@@ -14,6 +14,9 @@ Turns a checkout of halo2_proofs (PSE tag v2023_02_02 or axiom-crypto branch axi
   * src/plonk/circuit/compress_selectors.rs, src/plonk/circuit.rs, src/plonk/keygen.rs: the fixed-column keygen drop-in
     (rust/patches/fixed_keygen_dropin.rs): `process_h2b`, a copy of `ConstraintSystem::compress_selectors` that calls it, and G1Affine
     dispatches around keygen_vk's fixed commitments and keygen_pk's fixed values / polys / cosets.  Each substitution is asserted;
+  * src/plonk.rs, src/plonk/evaluation.rs, src/dev.rs: `MockProver::verify_par` dispatches to rust/patches/mock_prover_dropin.rs
+    for Fr; evaluation.rs gains `encode_source` / `FlatGraph` and the `evaluation` module becomes visible in the crate
+    (rust/patches/mock_prover_patch.py, whose functions assert every pattern they rely on);
   * Cargo.toml: `h2b200-sys = { path = ".../rust/h2b200-sys" }` is added to [dependencies].
 Idempotent.  Not run in the build container (no Rust sources of halo2_proofs are available there)."""
 import pathlib
@@ -137,6 +140,14 @@ if "create_proof_h2b" not in shplonk.read_text():
                "ProverSHPLONK::create_proof", re.S)
     add_uses(shplonk, ["use std::any::TypeId;", "use halo2curves::bn256::Bn256;", "use crate::poly::{Coeff, Polynomial};"])
     shplonk.write_text(shplonk.read_text() + "\n// ---- libh2b200 drop-in (rust/patches/shplonk_dropin.rs) ----\n" + (rust / "patches" / "shplonk_dropin.rs").read_text() + "\n")
+# MockProver::verify_par's gate, lookup and permutation loops (rust/patches/mock_prover_dropin.rs, whose header states the mechanism;
+# the text transforms are rust/patches/mock_prover_patch.py)
+sys.path.insert(0, str(rust / "patches"))
+import mock_prover_patch as mpp  # noqa: E402
+for path, transform in ((crate / "src" / "plonk.rs", mpp.patch_plonk),
+                        (crate / "src" / "plonk" / "evaluation.rs", lambda t: mpp.patch_evaluation(t, (rust / "patches" / "evaluation_dropin.rs").read_text())),
+                        (crate / "src" / "dev.rs", lambda t: mpp.patch_dev(t, (rust / "patches" / "mock_prover_dropin.rs").read_text()))):
+    path.write_text(transform(path.read_text()))
 toml = crate / "Cargo.toml"
 t = toml.read_text()
 if "h2b200-sys" not in t:

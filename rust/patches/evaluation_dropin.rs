@@ -6,7 +6,7 @@
 // `GraphEvaluator` already is a flat program; the shim only re-encodes its enums as the repr(C) structs of h2b200-sys.
 use h2b200_sys::{h2b_calculation, h2b_eval_columns, h2b_graph, h2b_value_source};
 
-fn encode_source(s: &ValueSource) -> h2b_value_source {
+pub(crate) fn encode_source(s: &ValueSource) -> h2b_value_source {
     let (kind, index, rotation) = match *s {
         ValueSource::Constant(i) => (0, i, 0),
         ValueSource::Intermediate(i) => (1, i, 0),
