@@ -45,7 +45,7 @@ _EXPORTS = [
     "h2b_pk_create", "h2b_keygen_fixed_build_pk_resident", "h2b_permutation_build_pk_resident", "h2b_keygen_lagrange_indicators_resident",
     "h2b_pk_put_lagrange", "h2b_pk_column", "h2b_pk_download", "h2b_pk_info", "h2b_pk_release",
     "h2b_fr_eval_queries_dev", "h2b_shplonk_begin", "h2b_shplonk_finish", "h2b_shplonk_release",
-    "h2b_mock_verify",
+    "h2b_mock_verify", "h2b_fr_kate_division_batch_dev", "h2b_gwc_create_proof",
 ]
 
 # include/h2b200.h enums of the resident proving key
@@ -277,6 +277,8 @@ class Lib:
         L.h2b_shplonk_begin.argtypes = [i32, vp, i32, u32, sz, vp, u32, u64, vp, vp, vp, ctypes.POINTER(u64)]
         L.h2b_shplonk_finish.argtypes = [u64, vp, vp]
         L.h2b_shplonk_release.argtypes = [u64]
+        L.h2b_fr_kate_division_batch_dev.argtypes = [i32, vp, sz, vp, u32, vp, vp]
+        L.h2b_gwc_create_proof.argtypes = [i32, vp, i32, u32, sz, vp, u32, u64, vp, vp, u32, ctypes.POINTER(u32)]
         L.h2b_evaluate_graph_dev.argtypes = [i32, vp, vp, vp, u32, i32, vp]
         L.h2b_evaluate_h_permutation_dev.argtypes = [i32, vp, u32, i32, vp, u32, vp, vp, u32, u32, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
         L.h2b_evaluate_h_lookup_dev.argtypes = [i32, vp, vp, vp, u32, i32, vp, vp, vp, vp, vp, vp, vp]
@@ -545,6 +547,10 @@ class Lib:
             self.dev_free(device, d)
             self.dev_free(device, d_q)
         return q
+
+    def fr_kate_division_batch_dev(self, device: int, d_a: int, n: int, d_points: int, count: int, d_q: int, stream: int = 0):
+        """count kate_divisions in one launch sequence: d_a count x n Fr, d_points count Fr -> quotient d (n - 1 Fr) at d_q + 32 n d"""
+        self.check(self.L.h2b_fr_kate_division_batch_dev(device, d_a, n, d_points, count, d_q, stream))
 
     # ---- grand products (permutation / lookup z polynomials) -------------------------------------------
     def permutation_product_dev(self, device: int, d_values, d_permutations, n: int, beta, gamma, delta, deltaomega, omega, last_z, d_z: int,
@@ -936,6 +942,19 @@ class Lib:
 
     def shplonk_release(self, session: int):
         self.check(self.L.h2b_shplonk_release(session))
+
+    # ---- the multi-point opening (GWC) -------------------------------------------------------------------
+    def gwc_create_proof(self, device: int, polys, on_host: bool, n: int, queries, handle_g: int, v) -> np.ndarray:
+        """polys: host arrays (on_host) or device pointers -> W of every distinct point, (points, 12) Jacobian, first-appearance order"""
+        ptrs = _ptr_array([p.ctypes.data for p in polys] if on_host else list(polys))
+        q = _queries(queries)
+        v = _u64(v).reshape(4)
+        cap = len(queries)
+        out = np.zeros((cap, 12), dtype=np.uint64)
+        count = ctypes.c_uint32(0)
+        self.check(self.L.h2b_gwc_create_proof(device, ptrs, 1 if on_host else 0, len(polys), n, q, len(queries), handle_g, v.ctypes.data,
+                                               out.ctypes.data, cap, ctypes.byref(count)))
+        return out[:count.value].copy()
 
     # ---- quotient evaluation (evaluate_h) on device-resident extended-coset columns ------------------
     def evaluate_graph_dev(self, device: int, graph: GraphArrays, cols: EvalColumns, d_values: int, size: int, rot_scale: int, stream: int = 0,

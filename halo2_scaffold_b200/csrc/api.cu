@@ -373,6 +373,12 @@ int h2b_fr_kate_division_dev(int device, const void* d_a, size_t n, const uint64
     return on_device(device, [&](DeviceCtx& c) { return fr_kate_division_run(c, d_a, n, b, d_q, (cudaStream_t)stream); });
 }
 
+int h2b_fr_kate_division_batch_dev(int device, const void* d_a, size_t n, const void* d_points, uint32_t count, void* d_q, void* stream) {
+    return on_device(device, [&](DeviceCtx& c) {
+        return fr_kate_division_batch_run(c, d_a, n, d_points, count, d_q, (cudaStream_t)stream);
+    });
+}
+
 int h2b_fr_lincomb_dev(int device, const void* const* d_cols, const uint64_t* coeffs, uint32_t m, size_t n, void* d_out, void* stream) {
     return on_device(device, [&](DeviceCtx& c) { return fr_lincomb_run(c, d_cols, coeffs, m, n, d_out, (cudaStream_t)stream); });
 }

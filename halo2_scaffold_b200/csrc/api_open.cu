@@ -1,4 +1,5 @@
-// C ABI of libh2b200, the multi-point opening (SHPLONK): h2b_fr_eval_queries_dev and the h2b_shplonk_* session.
+// C ABI of libh2b200, the multi-point openings: SHPLONK (h2b_fr_eval_queries_dev and the h2b_shplonk_* session) and GWC
+// (h2b_gwc_create_proof).
 #include "host.h"
 
 namespace h2b {
@@ -153,6 +154,53 @@ int h2b_shplonk_finish(uint64_t session, const uint64_t u[4], uint64_t out_h2_ja
 int h2b_shplonk_release(uint64_t session) {
     SessionRef drop = G.sessions.take(session);      // freed after G.mu is let go (the destructor waits for the device)
     if (!drop) { set_error("h2b_shplonk_release: unknown session handle %llu", (unsigned long long)session); return H2B_ERR_BAD_ARGUMENT; }
+    return H2B_OK;
+}
+
+int h2b_gwc_create_proof(int device, const void* const* polys, int polys_on_host, uint32_t n_polys, size_t n, const h2b_opening_query* queries,
+                         uint32_t n_queries, uint64_t handle_g, const uint64_t v[4], uint64_t* out_w_jac, uint32_t capacity, uint32_t* out_points) {
+    static const char* who = "h2b_gwc_create_proof";
+    GwcPlan plan;
+    SetRef g;      // declared before the device lock: released after it
+    H2B_TRY(on_device(device, [&]() -> int {
+        if (!polys || !v || !out_w_jac || !out_points) { set_error("%s: null pointer", who); return H2B_ERR_BAD_ARGUMENT; }
+        H2B_TRY(shplonk_n_check(who, n));
+        if (!fr_canonical(v)) { set_error("%s: v is not below the scalar field modulus", who); return H2B_ERR_BAD_ARGUMENT; }
+        H2B_TRY(gwc_plan_build(who, queries, n_queries, n_polys, &plan));
+        for (uint32_t i = 0; i < n_polys; ++i) if (!polys[i]) { set_error("%s: polynomial %u is a null pointer", who, i); return H2B_ERR_BAD_ARGUMENT; }
+        g = G.sets.find(handle_g);
+        if (!g) { set_error("%s: unknown base-set handle %llu", who, (unsigned long long)handle_g); return H2B_ERR_BAD_ARGUMENT; }
+        if (g->lo[(size_t)device] != 0 || g->rows[(size_t)device] < n - 1) {
+            set_error("%s: device %d does not hold rows [0, %zu) of the set", who, device, n - 1);
+            return H2B_ERR_BAD_ARGUMENT;
+        }
+        if (capacity < plan.n_points()) { set_error("%s: capacity %u < %u distinct points", who, capacity, plan.n_points()); return H2B_ERR_BAD_ARGUMENT; }
+        return H2B_OK;
+    }, [&](DeviceCtx& c) -> int {
+        // the call's block: the work of gwc_run | the uploaded polynomials of a host-pointer call
+        const size_t work = gwc_work_bytes(plan, n), upload = polys_on_host ? 32 * n * n_polys : 0;
+        struct Block {
+            void* p = nullptr;
+            ~Block() { if (p) { cudaDeviceSynchronize(); cudaFree(p); cudaGetLastError(); } }
+        } mem;
+        H2B_TRY(dev_malloc(&mem.p, work + upload, "the GWC opening"));
+        const cudaStream_t st = c.stream;
+        c.prof.mark(PROF_BEGIN, st);
+        std::vector<const void*> d_polys(polys, polys + n_polys);
+        if (polys_on_host) {
+            for (uint32_t i = 0; i < n_polys; ++i) {
+                void* dst = (char*)mem.p + work + 32 * n * i;
+                H2B_TRY(host_upload(c, dst, polys[i], 32 * n, st));
+                d_polys[i] = dst;
+            }
+            c.prof.mark(PROF_GWC_UPLOAD, st);
+        }
+        std::vector<uint64_t> w(12 * (size_t)plan.n_points());
+        H2B_TRY(gwc_run(c, plan, d_polys.data(), n, v, bases_of(*g, (size_t)device, 0), mem.p, w.data(), st));
+        memcpy(out_w_jac, w.data(), 8 * w.size());
+        *out_points = plan.n_points();
+        return H2B_OK;
+    }));
     return H2B_OK;
 }
 

@@ -82,7 +82,8 @@ enum ProfTag { PROF_BEGIN = 0, PROF_MSM_DECOMPOSE = 1, PROF_MSM_SCAN = 2, PROF_M
                PROF_KEYGEN_COMBINATION = 40, PROF_PK_FORM_COPY = 41, PROF_PK_PLACE = 42,
                PROF_OPEN_UPLOAD = 43, PROF_OPEN_EVAL = 44, PROF_OPEN_SCALARS = 45, PROF_OPEN_NUMERATORS = 46, PROF_OPEN_MSM = 47,
                PROF_OPEN_LINEARISE = 48, PROF_MOCK_UPLOAD = 49, PROF_MOCK_GATES = 50, PROF_MOCK_LOOKUPS = 51, PROF_MOCK_PERMUTATION = 52,
-               PROF_MOCK_RECORDS = 53 };
+               PROF_MOCK_RECORDS = 53, PROF_GWC_UPLOAD = 54, PROF_GWC_SCALARS = 55, PROF_GWC_NUMERATORS = 56, PROF_GWC_DIVISIONS = 57,
+               PROF_GWC_MSM = 58 };
 struct Profiler {
     bool enabled = false;
     std::vector<cudaEvent_t> ev;
@@ -150,6 +151,9 @@ int fr_eval_polynomial_run(DeviceCtx& ctx, const void* d_coeffs, size_t n, const
 int fr_kate_division_run(DeviceCtx& ctx, const void* d_a, size_t n, const uint64_t b[4], void* d_q, cudaStream_t stream);
 // the same with the point b already on the device (d_b: one Fr, outside ctx.scan_scratch)
 int fr_kate_division_at_run(DeviceCtx& ctx, const void* d_a, size_t n, const void* d_b, void* d_q, cudaStream_t stream);
+// `count` divisions of length n in one launch sequence: division d divides the n Fr at d_a + d n by (X - d_b[d]) into d_q + d n (n - 1
+// coefficients; d_b: count consecutive Fr on the device, outside ctx.scan_scratch).  count = 1 is fr_kate_division_at_run.
+int fr_kate_division_batch_run(DeviceCtx& ctx, const void* d_a, size_t n, const void* d_b, uint32_t count, void* d_q, cudaStream_t stream);
 int fr_lincomb_run(DeviceCtx& ctx, const void* const* d_cols, const uint64_t* coeffs, uint32_t m, size_t n, void* d_out, cudaStream_t stream);
 int permutation_product_run(DeviceCtx& ctx, const void* const* d_values, const void* const* d_sigma, uint32_t m, size_t n, const uint64_t* beta,
                             const uint64_t* gamma, const uint64_t* delta, const uint64_t* deltaomega, const uint64_t* omega, const uint64_t* last_z,
@@ -268,6 +272,20 @@ int shplonk_begin_run(DeviceCtx& ctx, const ShplonkPlan& p, const void* d_tables
                       void* d_scal, void* d_hx, void* d_a, void* d_b, cudaStream_t stream);
 int shplonk_finish_run(DeviceCtx& ctx, const ShplonkPlan& p, const void* d_tables, size_t n, const uint64_t u[4], const void* d_evals, void* d_scal,
                        const void* d_hx, void* d_a, void* d_b, cudaStream_t stream);
+// GWC's construct_intermediate_sets: the distinct points in first-appearance order, each with the polynomial of every query there in
+// query order (the j-th is weighted by v^j; a query listed twice is there twice).  The refusals of shplonk_plan_build, no point cap.
+struct GwcPlan {
+    std::vector<uint64_t> points;                    // 4 Montgomery words per point
+    std::vector<std::vector<uint32_t>> polys_at;
+    uint32_t max_queries = 0;                        // the longest list of polys_at
+    uint32_t n_points() const { return (uint32_t)(points.size() / 4); }
+};
+int gwc_plan_build(const char* who, const h2b_opening_query* queries, uint32_t n_queries, uint32_t n_polys, GwcPlan* out);
+// device bytes of one call's work block
+size_t gwc_work_bytes(const GwcPlan& p, size_t n);
+// every W_i (Jacobian, 12 words each) into the host array out_jac, over rows [0, n - 1) of g; d_polys by the caller's index.  Synchronous.
+int gwc_run(DeviceCtx& ctx, const GwcPlan& p, const void* const* d_polys, size_t n, const uint64_t v[4], const MsmBases& g, void* d_work,
+            uint64_t* out_jac, cudaStream_t stream);
 // ---- mock.cu ----
 // the refusals that need the compiler (graph and root contents); the caller has checked pointers, sizes and indices
 int mock_verify_check(const h2b_mock_circuit* c);

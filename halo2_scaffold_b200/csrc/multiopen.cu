@@ -15,6 +15,8 @@
 //     of S_i, ping-ponging between two buffers, then h_x += v^i Q_i;
 //   * linearisation: one combination of every polynomial and h_x with the constant at coefficient 0, already scaled by z_0^-1, and
 //     one division by (X - u): h' = kate_division(L, u) / z_0.
+// The GWC opening ([UP] .../multiopen/gwc/prover.rs, ProverGWC::create_proof) shares the query checks, the combination kernel and
+// scan.cu's kate levels, which divide all of a group's numerators in one launch sequence; see the section at the end.
 #include <algorithm>
 
 #include "common.h"
@@ -38,20 +40,40 @@ static bool fr_words_canonical(const uint64_t* w) {
 }
 bool fr_canonical(const uint64_t w[4]) { return fr_words_canonical(w); }
 
-int shplonk_plan_build(const char* who, const h2b_opening_query* queries, uint32_t n_queries, uint32_t n_polys, bool need_every_poly, ShplonkPlan* out) {
+// the refusals every opening makes of its queries, and the distinct points in first-appearance order (compared as words): *points
+// (4 words each), (*query_point)[q] = the point index of query q
+static int opening_points(const char* who, const h2b_opening_query* queries, uint32_t n_queries, uint32_t n_polys, bool need_every_poly,
+                          std::vector<uint64_t>* points, std::vector<uint32_t>* query_point) {
     if (!queries || n_queries == 0) { set_error("%s: no queries", who); return H2B_ERR_BAD_ARGUMENT; }
-    ShplonkPlan p;
-    std::vector<uint32_t> slot_of(n_polys, UINT32_MAX);
-    std::vector<std::vector<uint32_t>> slot_points;          // T indices, first-appearance order, no repeats
-    p.query_pair.resize(n_queries);
-    std::vector<uint32_t> query_slot(n_queries), query_point(n_queries);
+    std::vector<char> opened(n_polys, 0);
+    query_point->resize(n_queries);
     for (uint32_t q = 0; q < n_queries; ++q) {
         const uint32_t poly = queries[q].poly;
         if (poly >= n_polys) { set_error("%s: query %u names polynomial %u of %u", who, q, poly, n_polys); return H2B_ERR_BAD_ARGUMENT; }
         if (!fr_words_canonical(queries[q].point)) { set_error("%s: the point of query %u is not below the scalar field modulus", who, q); return H2B_ERR_BAD_ARGUMENT; }
+        const size_t count = points->size() / 4;
         uint32_t t = 0;
-        while (t < p.n_points() && memcmp(&p.points[4 * (size_t)t], queries[q].point, 32) != 0) ++t;
-        if (t == p.n_points()) p.points.insert(p.points.end(), queries[q].point, queries[q].point + 4);
+        while (t < count && memcmp(&(*points)[4 * (size_t)t], queries[q].point, 32) != 0) ++t;
+        if (t == count) points->insert(points->end(), queries[q].point, queries[q].point + 4);
+        (*query_point)[q] = t;
+        opened[poly] = 1;
+    }
+    if (need_every_poly)
+        for (uint32_t i = 0; i < n_polys; ++i)
+            if (!opened[i]) { set_error("%s: no query opens polynomial %u", who, i); return H2B_ERR_BAD_ARGUMENT; }
+    return H2B_OK;
+}
+
+int shplonk_plan_build(const char* who, const h2b_opening_query* queries, uint32_t n_queries, uint32_t n_polys, bool need_every_poly, ShplonkPlan* out) {
+    ShplonkPlan p;
+    std::vector<uint32_t> query_point;
+    H2B_TRY(opening_points(who, queries, n_queries, n_polys, need_every_poly, &p.points, &query_point));
+    std::vector<uint32_t> slot_of(n_polys, UINT32_MAX);
+    std::vector<std::vector<uint32_t>> slot_points;          // T indices, first-appearance order, no repeats
+    p.query_pair.resize(n_queries);
+    std::vector<uint32_t> query_slot(n_queries);
+    for (uint32_t q = 0; q < n_queries; ++q) {
+        const uint32_t poly = queries[q].poly, t = query_point[q];
         if (slot_of[poly] == UINT32_MAX) { slot_of[poly] = (uint32_t)p.used.size(); p.used.push_back(poly); slot_points.emplace_back(); }
         std::vector<uint32_t>& sp = slot_points[slot_of[poly]];
         if (std::find(sp.begin(), sp.end(), t) == sp.end()) {
@@ -59,11 +81,6 @@ int shplonk_plan_build(const char* who, const h2b_opening_query* queries, uint32
             sp.push_back(t);
         }
         query_slot[q] = slot_of[poly];
-        query_point[q] = t;
-    }
-    if (need_every_poly && p.used.size() != n_polys) {
-        for (uint32_t i = 0; i < n_polys; ++i)
-            if (slot_of[i] == UINT32_MAX) { set_error("%s: no query opens polynomial %u", who, i); return H2B_ERR_BAD_ARGUMENT; }
     }
     const uint32_t P = (uint32_t)p.used.size();
     // pairs grouped by slot, in the slot's point order
@@ -496,6 +513,80 @@ int shplonk_finish_run(DeviceCtx& ctx, const ShplonkPlan& p, const void* d_table
     H2B_TRY(mo_combine(cols, coef, false, a.F0 + a.P + 1, 1, (const uint4*)d_scal, n, d_a, stream));
     H2B_TRY(fr_kate_division_at_run(ctx, d_a, n, uslot, d_b, stream));
     ctx.prof.mark(PROF_OPEN_LINEARISE, stream);
+    return H2B_OK;
+}
+
+// ---- GWC ([UP] halo2_proofs/src/poly/kzg/multiopen/gwc/prover.rs ProverGWC::create_proof) -------------------------------------
+// For each distinct point z_i: W_i = commit(kate_division(sum_j v^j p_ij, z_i)).  Upstream first subtracts sum_j v^j p_ij(z_i) at
+// coefficient 0, which kate_division never reads (q[i-1] = a[i] + z q[i] for i >= 1), so no evaluation is computed here.  Per group of
+// up to msm_batch_max() points: one combination launch per point and 32 columns, the divisions of every point of the group in one
+// launch sequence, and one batched MSM.
+int gwc_plan_build(const char* who, const h2b_opening_query* queries, uint32_t n_queries, uint32_t n_polys, GwcPlan* out) {
+    GwcPlan p;
+    std::vector<uint32_t> query_point;
+    H2B_TRY(opening_points(who, queries, n_queries, n_polys, true, &p.points, &query_point));
+    p.polys_at.resize(p.n_points());
+    for (uint32_t q = 0; q < n_queries; ++q) p.polys_at[query_point[q]].push_back(queries[q].poly);
+    for (auto& at : p.polys_at) p.max_queries = at.size() > p.max_queries ? (uint32_t)at.size() : p.max_queries;
+    *out = std::move(p);
+    return H2B_OK;
+}
+
+static uint32_t gwc_group(const GwcPlan& p) { return p.n_points() < msm_batch_max() ? p.n_points() : msm_batch_max(); }
+
+// points | v powers | MSM result blocks | numerators | quotients (n Fr each, one group of points)
+size_t gwc_work_bytes(const GwcPlan& p, size_t n) {
+    const size_t m = gwc_group(p);
+    return 32 * (size_t)p.n_points() + 32 * (size_t)p.max_queries + 224 * m + 2 * m * n * 32;
+}
+
+// out[j] = v^j, j < count
+__global__ void __launch_bounds__(128) gwc_powers_kernel(Fr v, uint32_t count, uint4* __restrict__ out) {
+    const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= count) return;
+    fp_store<FR>(out + 2 * (size_t)j, fp_pow_u32<FR>(v, j));
+}
+
+int gwc_run(DeviceCtx& ctx, const GwcPlan& p, const void* const* d_polys, size_t n, const uint64_t v[4], const MsmBases& g, void* d_work,
+            uint64_t* out_jac, cudaStream_t stream) {
+    const uint32_t T = p.n_points(), J = p.max_queries, group = gwc_group(p);
+    char* w = (char*)d_work;
+    uint4* pts = (uint4*)w;    w += 32 * (size_t)T;
+    uint4* vpow = (uint4*)w;   w += 32 * (size_t)J;
+    char* blocks = w;          w += 224 * (size_t)group;
+    char* nums = w;            w += 32 * n * group;
+    char* quots = w;
+    H2B_CUDA(cudaMemcpyAsync(pts, p.points.data(), 32 * (size_t)T, cudaMemcpyHostToDevice, stream));
+    Fr vv;
+    memcpy(vv.l, v, 32);
+    H2B_LAUNCH(gwc_powers_kernel, (J + 127) / 128, 128, 0, stream, vv, J, vpow);
+    ctx.prof.mark(PROF_GWC_SCALARS, stream);
+    std::vector<uint64_t> res(28 * (size_t)group);
+    for (uint32_t g0 = 0; g0 < T; g0 += group) {
+        const uint32_t m = T - g0 < group ? T - g0 : group;
+        for (uint32_t i = 0; i < m; ++i) {
+            const std::vector<uint32_t>& at = p.polys_at[g0 + i];
+            std::vector<const void*> cols;
+            std::vector<uint32_t> coef;
+            for (uint32_t j = 0; j < at.size(); ++j) { cols.push_back(d_polys[at[j]]); coef.push_back(j); }
+            H2B_TRY(mo_combine(cols, coef, false, 0, 0, vpow, n, nums + 32 * n * i, stream));
+        }
+        ctx.prof.mark(PROF_GWC_NUMERATORS, stream);
+        H2B_TRY(fr_kate_division_batch_run(ctx, nums, n, pts + 2 * (size_t)g0, m, quots, stream));
+        ctx.prof.mark(PROF_GWC_DIVISIONS, stream);
+        std::vector<const void*> qs(m);
+        std::vector<size_t> lens(m, n - 1);
+        for (uint32_t i = 0; i < m; ++i) qs[i] = quots + 32 * n * i;
+        if (n - 1 <= ((size_t)1 << 26)) {
+            H2B_TRY(msm_run_batch(ctx, qs.data(), lens.data(), m, g, blocks, stream));
+        } else {                                  // beyond the batched MSM's column length: one by one
+            for (uint32_t i = 0; i < m; ++i) H2B_TRY(msm_run(ctx, qs[i], g, n - 1, blocks + 224 * (size_t)i, false, stream));
+        }
+        ctx.prof.mark(PROF_GWC_MSM, stream);
+        H2B_CUDA(cudaMemcpyAsync(res.data(), blocks, 224 * (size_t)m, cudaMemcpyDeviceToHost, stream));
+        H2B_CUDA(cudaStreamSynchronize(stream));
+        for (uint32_t i = 0; i < m; ++i) memcpy(out_jac + 12 * (size_t)(g0 + i), &res[28 * (size_t)i], 96);
+    }
     return H2B_OK;
 }
 

@@ -134,9 +134,21 @@ int fr_prefix_product_run(DeviceCtx& ctx, const void* d_in, void* d_out, size_t 
 static const uint32_t POLY_K = 16;
 static const uint32_t POLY_LEVELS_MAX = 9;          // 16^8 > 2^31
 
+// The kernels of the kate levels also run a batch of divisions of one length, division d = blockIdx.y: a level's vectors, quotients,
+// chunk sums and carries lie back to back, each as long as the level's vector (n) or its chunk count, and the point powers of
+// division d at pts + d * POLY_PTS.  The offsets follow from arguments every form already has, and only the BATCH forms compute them,
+// so a single division runs the code it ran before batches existed (with the offsets, SHPLONK's per-point divisions measured 2 %
+// slower on a B200).
+static const uint32_t POLY_PTS = POLY_LEVELS_MAX + 1;      // the powers of one point and the point itself
+
 // pts[l] = x^(16^l), l < levels (one thread; a handful of squarings)
+template <bool BATCH>
 __global__ void fr_point_powers_kernel(const uint4* __restrict__ x, uint32_t levels, uint4* __restrict__ pts) {
     if (blockIdx.x != 0 || threadIdx.x != 0) return;
+    if (BATCH) {
+        x += 2 * (size_t)blockIdx.y;
+        pts += 2 * (size_t)blockIdx.y * POLY_PTS;
+    }
     Fr p = fp_load<FR>(x);
     for (uint32_t l = 0; l < levels; ++l) {
         fp_store<FR>(pts + 2 * l, p);
@@ -145,9 +157,15 @@ __global__ void fr_point_powers_kernel(const uint4* __restrict__ x, uint32_t lev
 }
 
 // out[t] = sum_{i < 16} in[16 t + i] * x^i
+template <bool BATCH>
 __global__ void __launch_bounds__(128) fr_horner_chunk_kernel(const uint4* __restrict__ in, size_t n, const uint4* __restrict__ x, uint4* __restrict__ out, uint32_t chunks) {
     const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= chunks) return;
+    if (BATCH) {
+        in += 2 * (size_t)blockIdx.y * n;
+        x += 2 * (size_t)blockIdx.y * POLY_PTS;
+        out += 2 * (size_t)blockIdx.y * chunks;
+    }
     const size_t lo = (size_t)t * POLY_K;
     const size_t hi = lo + POLY_K < n ? lo + POLY_K : n;
     const Fr xx = fp_load<FR>(x);
@@ -165,13 +183,13 @@ int fr_eval_polynomial_run(DeviceCtx& ctx, const void* d_coeffs, size_t n, const
     uint4* pts = (uint4*)ctx.scan_scratch.p;
     uint4* buf = pts + 2 * (POLY_LEVELS_MAX + 1);
     H2B_CUDA(cudaMemcpyAsync(pts + 2 * POLY_LEVELS_MAX, x, 32, cudaMemcpyHostToDevice, stream));
-    H2B_LAUNCH(fr_point_powers_kernel, 1, 32, 0, stream, (const uint4*)(pts + 2 * POLY_LEVELS_MAX), POLY_LEVELS_MAX, pts);
+    H2B_LAUNCH(fr_point_powers_kernel<false>, 1, 32, 0, stream, (const uint4*)(pts + 2 * POLY_LEVELS_MAX), POLY_LEVELS_MAX, pts);
     const uint4* in = (const uint4*)d_coeffs;
     size_t m = n;
     for (uint32_t l = 0;; ++l) {
         const uint32_t chunks = (uint32_t)((m + POLY_K - 1) / POLY_K);
         uint4* out = chunks == 1 ? (uint4*)d_out : buf;
-        H2B_LAUNCH(fr_horner_chunk_kernel, (chunks + 127) / 128, 128, 0, stream, in, m, (const uint4*)(pts + 2 * l), out, chunks);
+        H2B_LAUNCH(fr_horner_chunk_kernel<false>, (chunks + 127) / 128, 128, 0, stream, in, m, (const uint4*)(pts + 2 * l), out, chunks);
         if (chunks == 1) break;
         in = buf;
         buf += 2 * (size_t)chunks;
@@ -185,10 +203,17 @@ int fr_eval_polynomial_run(DeviceCtx& ctx, const void* d_coeffs, size_t n, const
 // carry[t] = s[t+1] + b^16 * carry[t+1] solved recursively, then the replay:
 //   q[i-1] = a[i] + b * q[i] inside chunk t, starting from q[hi-1] = carry[t]
 // `q` has n - 1 coefficients (q[i-1] for i = 1 .. n-1); a[0] only enters the remainder, which the caller does not need.
+template <bool BATCH>
 __global__ void __launch_bounds__(128) fr_kate_replay_kernel(const uint4* __restrict__ a, size_t n, const uint4* __restrict__ b, const uint4* __restrict__ carry,
                                                            uint4* __restrict__ q, uint32_t chunks) {
     const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= chunks) return;
+    if (BATCH) {
+        a += 2 * (size_t)blockIdx.y * n;
+        q += 2 * (size_t)blockIdx.y * n;
+        b += 2 * (size_t)blockIdx.y * POLY_PTS;
+        if (carry) carry += 2 * (size_t)blockIdx.y * chunks;
+    }
     const size_t lo = (size_t)t * POLY_K;
     const size_t hi = lo + POLY_K < n ? lo + POLY_K : n;
     const Fr bb = fp_load<FR>(b);
@@ -203,30 +228,54 @@ __global__ void __launch_bounds__(128) fr_kate_replay_kernel(const uint4* __rest
 
 // carry-in of every chunk at one level: c[t] = value the recurrence has reached when it enters chunk t from above,
 // i.e. c[chunks-1] = 0 and c[t] = s[t+1] + m * c[t+1] with m = b^(16^(level+1)).  Solved by recursion on {s[t+1]}.
-static int kate_carries(DeviceCtx& ctx, const uint4* s, uint32_t chunks, const uint4* pts, uint32_t level, uint4* carry, uint4* scratch, cudaStream_t stream);
+static int kate_carries(DeviceCtx& ctx, const uint4* s, uint32_t chunks, const uint4* pts, uint32_t level, uint4* carry, uint4* scratch, uint32_t count,
+                        cudaStream_t stream);
 
 // q_out[i-1] = a[i] + m * q[i] for a vector a of length n with multiplier pts[level]; writes n - 1 values ... as a reusable
-// step: solve the recurrence for `a` (length n) at `level`, producing q (length n - 1, q[n-1] taken as 0)
-static int kate_level(DeviceCtx& ctx, const uint4* a, size_t n, const uint4* pts, uint32_t level, uint4* q, uint4* scratch, cudaStream_t stream) {
+// step: solve the recurrence for `a` (length n) at `level`, producing q (length n - 1, q[n-1] taken as 0); `count` divisions
+// of a batch (vectors and quotients n elements apart)
+static int kate_level(DeviceCtx& ctx, const uint4* a, size_t n, const uint4* pts, uint32_t level, uint4* q, uint4* scratch, uint32_t count,
+                      cudaStream_t stream) {
     const uint32_t chunks = (uint32_t)((n + POLY_K - 1) / POLY_K);
+    const bool batch = count > 1;
     if (chunks == 1) {
-        H2B_LAUNCH(fr_kate_replay_kernel, 1, 128, 0, stream, a, n, pts + 2 * level, (const uint4*)nullptr, q, 1u);
+        H2B_LAUNCH((batch ? fr_kate_replay_kernel<true> : fr_kate_replay_kernel<false>), dim3(1, count), 128, 0, stream, a, n, pts + 2 * level,
+                   (const uint4*)nullptr, q, 1u);
         return H2B_OK;
     }
-    uint4* s = scratch;                     // chunk sums
-    uint4* carry = s + 2 * (size_t)chunks;  // carry-ins
-    uint4* rest = carry + 2 * (size_t)chunks;
-    H2B_LAUNCH(fr_horner_chunk_kernel, (chunks + 127) / 128, 128, 0, stream, a, n, pts + 2 * level, s, chunks);
-    H2B_TRY(kate_carries(ctx, s, chunks, pts, level, carry, rest, stream));
-    H2B_LAUNCH(fr_kate_replay_kernel, (chunks + 127) / 128, 128, 0, stream, a, n, pts + 2 * level, (const uint4*)carry, q, chunks);
+    uint4* s = scratch;                                  // chunk sums of every division
+    uint4* carry = s + 2 * (size_t)chunks * count;       // carry-ins
+    uint4* rest = carry + 2 * (size_t)chunks * count;
+    const dim3 grid((chunks + 127) / 128, count);
+    H2B_LAUNCH((batch ? fr_horner_chunk_kernel<true> : fr_horner_chunk_kernel<false>), grid, 128, 0, stream, a, n, pts + 2 * level, s, chunks);
+    H2B_TRY(kate_carries(ctx, s, chunks, pts, level, carry, rest, count, stream));
+    H2B_LAUNCH((batch ? fr_kate_replay_kernel<true> : fr_kate_replay_kernel<false>), grid, 128, 0, stream, a, n, pts + 2 * level, (const uint4*)carry, q,
+               chunks);
     return H2B_OK;
 }
 
-static int kate_carries(DeviceCtx& ctx, const uint4* s, uint32_t chunks, const uint4* pts, uint32_t level, uint4* carry, uint4* scratch, cudaStream_t stream) {
+static int kate_carries(DeviceCtx& ctx, const uint4* s, uint32_t chunks, const uint4* pts, uint32_t level, uint4* carry, uint4* scratch, uint32_t count,
+                        cudaStream_t stream) {
     // c[t-1] = s[t] + m * c[t] for t = chunks-1 .. 1, c[chunks-1] = 0: exactly the kate recurrence on the vector s with
     // multiplier m = pts[level + 1]; its solution q has q[t-1] = c[t-1], and c[chunks-1] = 0 completes it
-    H2B_CUDA(cudaMemsetAsync(carry + 2 * (size_t)(chunks - 1), 0, 32, stream));
-    return kate_level(ctx, s, chunks, pts, level + 1, carry, scratch, stream);
+    if (count == 1) H2B_CUDA(cudaMemsetAsync(carry + 2 * (size_t)(chunks - 1), 0, 32, stream));
+    else H2B_CUDA(cudaMemset2DAsync(carry + 2 * (size_t)(chunks - 1), (size_t)chunks * 32, 0, 32, count, stream));
+    return kate_level(ctx, s, chunks, pts, level + 1, carry, scratch, count, stream);
+}
+
+// scratch of `count` divisions of length n: the point powers, and the chunk sums and carries of every level (< 2 n / 15 per division)
+static int kate_reserve(DeviceCtx& ctx, size_t n, uint32_t count) {
+    return ctx.scan_scratch.reserve(((n / 7 + 256) * count + (size_t)POLY_PTS * (count - 1)) * 32);
+}
+
+// x: the `count` points on the device, back to back (for one division it may be the scratch's own point slot)
+static int kate_divisions(DeviceCtx& ctx, const void* d_a, size_t n, const uint4* x, uint32_t count, void* d_q, cudaStream_t stream) {
+    uint4* pts = (uint4*)ctx.scan_scratch.p;
+    uint4* buf = pts + 2 * (size_t)POLY_PTS * count;
+    H2B_LAUNCH((count > 1 ? fr_point_powers_kernel<true> : fr_point_powers_kernel<false>), dim3(1, count), 32, 0, stream, x, POLY_LEVELS_MAX, pts);
+    H2B_TRY(kate_level(ctx, (const uint4*)d_a, n, pts, 0, (uint4*)d_q, buf, count, stream));
+    H2B_CUDA(cudaGetLastError());
+    return H2B_OK;
 }
 
 // b on the host (kind = cudaMemcpyHostToDevice) or on the device (cudaMemcpyDeviceToDevice)
@@ -234,20 +283,24 @@ static int kate_division(DeviceCtx& ctx, const void* d_a, size_t n, const void* 
     if (!b || (n && (!d_a || !d_q))) { set_error("kate_division: null pointer"); return H2B_ERR_BAD_ARGUMENT; }
     if (n <= 1) return H2B_OK;                 // the quotient of a constant is empty
     if (n > ((size_t)1 << 31)) { set_error("kate_division: at most 2^31 coefficients"); return H2B_ERR_BAD_ARGUMENT; }
-    H2B_TRY(ctx.scan_scratch.reserve((n / 7 + 256) * 32));
-    uint4* pts = (uint4*)ctx.scan_scratch.p;
-    uint4* buf = pts + 2 * (POLY_LEVELS_MAX + 1);
-    H2B_CUDA(cudaMemcpyAsync(pts + 2 * POLY_LEVELS_MAX, b, 32, kind, stream));
-    H2B_LAUNCH(fr_point_powers_kernel, 1, 32, 0, stream, (const uint4*)(pts + 2 * POLY_LEVELS_MAX), POLY_LEVELS_MAX, pts);
-    H2B_TRY(kate_level(ctx, (const uint4*)d_a, n, pts, 0, (uint4*)d_q, buf, stream));
-    H2B_CUDA(cudaGetLastError());
-    return H2B_OK;
+    H2B_TRY(kate_reserve(ctx, n, 1));
+    uint4* x = (uint4*)ctx.scan_scratch.p + 2 * POLY_LEVELS_MAX;
+    H2B_CUDA(cudaMemcpyAsync(x, b, 32, kind, stream));
+    return kate_divisions(ctx, d_a, n, x, 1, d_q, stream);
 }
 int fr_kate_division_run(DeviceCtx& ctx, const void* d_a, size_t n, const uint64_t b[4], void* d_q, cudaStream_t stream) {
     return kate_division(ctx, d_a, n, b, cudaMemcpyHostToDevice, d_q, stream);
 }
 int fr_kate_division_at_run(DeviceCtx& ctx, const void* d_a, size_t n, const void* d_b, void* d_q, cudaStream_t stream) {
     return kate_division(ctx, d_a, n, d_b, cudaMemcpyDeviceToDevice, d_q, stream);
+}
+int fr_kate_division_batch_run(DeviceCtx& ctx, const void* d_a, size_t n, const void* d_b, uint32_t count, void* d_q, cudaStream_t stream) {
+    if (count == 0 || n <= 1) return H2B_OK;
+    if (!d_a || !d_b || !d_q) { set_error("kate_division: null pointer"); return H2B_ERR_BAD_ARGUMENT; }
+    if (n > ((size_t)1 << 31)) { set_error("kate_division: at most 2^31 coefficients"); return H2B_ERR_BAD_ARGUMENT; }
+    if (count > 65535) { set_error("kate_division: at most 65535 divisions per batch"); return H2B_ERR_BAD_ARGUMENT; }
+    H2B_TRY(kate_reserve(ctx, n, count));
+    return kate_divisions(ctx, d_a, n, (const uint4*)d_b, count, d_q, stream);
 }
 
 // ---- the grand products themselves --------------------------------------------------------------------------------------

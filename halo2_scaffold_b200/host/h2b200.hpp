@@ -284,6 +284,7 @@ enum class SerdeFormat : int { Processed = H2B_SERDE_PROCESSED, RawBytes = H2B_S
 
 class ParamsKZG {
     friend class ProverSHPLONK;
+    friend class ProverGWC;
 
   public:
     ParamsKZG(uint32_t k, const std::vector<G1Affine>& g, const std::vector<G1Affine>& g_lagrange, std::vector<uint8_t> g2_bytes = {})
@@ -432,6 +433,31 @@ class ProverSHPLONK {
         const Fr u = squeeze_u(h1);
         check(h2b_shplonk_finish(session, u.l, reinterpret_cast<uint64_t*>(&h2)), "ProverSHPLONK::create_proof (h2)");
         return {h1, h2};
+    }
+
+  private:
+    const ParamsKZG& params_;
+    int device_;
+};
+
+// ProverGWC::create_proof ([UP] poly/kzg/multiopen/gwc/prover.rs): queries as for ProverSHPLONK, v the challenge the caller squeezed.
+// Returns W for every distinct point in first-appearance order, which upstream writes to the transcript in that order.
+class ProverGWC {
+  public:
+    explicit ProverGWC(const ParamsKZG& params, int device = 0) : params_(params), device_(device) {}
+    std::vector<G1> create_proof(const std::vector<std::vector<Fr>>& polys, const std::vector<Query>& queries, const Fr& v) const {
+        std::vector<const void*> ptrs;
+        for (const auto& p : polys) ptrs.push_back(p.data());
+        std::vector<h2b_opening_query> q(queries.size());
+        for (size_t i = 0; i < queries.size(); ++i) { q[i].poly = queries[i].poly; q[i].reserved = 0; memcpy(q[i].point, queries[i].point.l, 32); }
+        const size_t n = polys.empty() ? 0 : polys[0].size();
+        for (const auto& p : polys) if (p.size() != n) throw Panic("ProverGWC::create_proof: polynomials of different lengths");
+        std::vector<G1> w(queries.size());
+        uint32_t points = 0;
+        check(h2b_gwc_create_proof(device_, ptrs.data(), 1, (uint32_t)polys.size(), n, q.data(), (uint32_t)q.size(), params_.g_, v.l,
+                                   reinterpret_cast<uint64_t*>(w.data()), (uint32_t)w.size(), &points), "ProverGWC::create_proof");
+        w.resize(points);
+        return w;
     }
 
   private:

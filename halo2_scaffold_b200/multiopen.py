@@ -1,6 +1,7 @@
 """
-The SHPLONK multi-point opening ([UP] halo2_proofs/src/poly/kzg/multiopen/shplonk/prover.rs, ProverSHPLONK::create_proof) and the
-query evaluation of plonk/prover.rs, on the device through h2b_shplonk_* / h2b_fr_eval_queries_dev.
+The multi-point openings of KZG on the device: SHPLONK ([UP] halo2_proofs/src/poly/kzg/multiopen/shplonk/prover.rs,
+ProverSHPLONK::create_proof) through h2b_shplonk_*, GWC (.../multiopen/gwc/prover.rs, ProverGWC::create_proof) through
+h2b_gwc_create_proof, and the query evaluation of plonk/prover.rs through h2b_fr_eval_queries_dev.
 
 A query is (poly, point): poly is a host array of n Fr (n x 4 uint64, Montgomery) or a device pointer (int) on the session's device,
 point 4 Montgomery words.  Polynomials are identified the way upstream identifies them, by object (pointer) identity: two distinct
@@ -28,6 +29,19 @@ def eval_queries(lib, device: int, d_polys, n: int, queries, d_out: int, stream:
     lib.eval_queries_dev(device, d_polys, n, queries, d_out, stream)
 
 
+def _polys_and_n(polys, params):
+    on_host = not isinstance(polys[0], int)
+    if any(isinstance(p, int) == on_host for p in polys):
+        raise ValueError("create_proof: polynomials are either all host arrays or all device pointers")
+    if not on_host:
+        return polys, on_host, params.n
+    polys = [np.ascontiguousarray(p, dtype=np.uint64).reshape(-1, 4) for p in polys]
+    n = polys[0].shape[0]
+    if any(p.shape[0] != n for p in polys):
+        raise ValueError("create_proof: polynomials of different lengths")
+    return polys, on_host, n
+
+
 class ProverSHPLONK:
     """ProverSHPLONK::new(params): create_proof over the params' registered g on one device"""
 
@@ -40,16 +54,7 @@ class ProverSHPLONK:
         """queries [(poly, point)] in the prover's order; y and v the challenges the caller squeezed (upstream squeezes y, then v);
         squeeze_u(h1) is called after h1 (Jacobian) is written and returns u.  Returns (h1, h2), Jacobian."""
         polys, indexed = _index_queries(queries)
-        on_host = not isinstance(polys[0], int)
-        if any(isinstance(p, int) == on_host for p in polys):
-            raise ValueError("create_proof: polynomials are either all host arrays or all device pointers")
-        if on_host:
-            polys = [np.ascontiguousarray(p, dtype=np.uint64).reshape(-1, 4) for p in polys]
-            n = polys[0].shape[0]
-            if any(p.shape[0] != n for p in polys):
-                raise ValueError("create_proof: polynomials of different lengths")
-        else:
-            n = self.params.n
+        polys, on_host, n = _polys_and_n(polys, self.params)
         h1, session = self.lib.shplonk_begin(self.device, polys, on_host, n, indexed, self.params._g, y, v)
         try:
             u = squeeze_u(h1)
@@ -59,4 +64,20 @@ class ProverSHPLONK:
         return h1, h2
 
 
-__all__ = ["ProverSHPLONK", "eval_queries"]
+class ProverGWC:
+    """ProverGWC::new(params): create_proof over the params' registered g on one device"""
+
+    def __init__(self, params, device: int = 0):
+        self.params = params
+        self.lib = params.lib
+        self.device = device
+
+    def create_proof(self, queries, v):
+        """queries [(poly, point)] in the prover's order; v the challenge the caller squeezed.  Returns [W, ...] (Jacobian), one per
+        distinct point in first-appearance order, which upstream writes to the transcript in that order."""
+        polys, indexed = _index_queries(queries)
+        polys, on_host, n = _polys_and_n(polys, self.params)
+        return list(self.lib.gwc_create_proof(self.device, polys, on_host, n, indexed, self.params._g, v))
+
+
+__all__ = ["ProverGWC", "ProverSHPLONK", "eval_queries"]

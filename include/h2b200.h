@@ -184,6 +184,10 @@ int h2b_fr_prefix_product_dev(int device, const void* d_in, void* d_out, size_t 
  * [UP] halo2_proofs::arithmetic::kate_division(a, b): the n - 1 coefficients of a(X) / (X - b) -> d_q (must not alias d_a) */
 int h2b_fr_eval_polynomial_dev(int device, const void* d_coeffs, size_t n, const uint64_t x[4], void* d_out, void* stream);
 int h2b_fr_kate_division_dev(int device, const void* d_a, size_t n, const uint64_t b[4], void* d_q, void* stream);
+/* `count` kate_divisions in one launch sequence: d_a holds count polynomials of n coefficients back to back, d_points count points
+ * (device, Fr); quotient d (n - 1 coefficients) goes to d_q + d n Fr, so d_q holds count x n Fr and must not alias d_a.  Each equals
+ * h2b_fr_kate_division_dev of its polynomial and point.  count <= 65535. */
+int h2b_fr_kate_division_batch_dev(int device, const void* d_a, size_t n, const void* d_points, uint32_t count, void* d_q, void* stream);
 
 /* out[i] = sum_j coeffs[j] * cols[j][i] (m columns of n elements; out may alias none of them): the y- / v-weighted sums of
  * the multi-open argument ([UP] poly/kzg/multiopen/shplonk/prover.rs) and the theta-compression of lookup expressions
@@ -507,6 +511,23 @@ int h2b_shplonk_begin(int device, const void* const* polys, int polys_on_host, u
 int h2b_shplonk_finish(uint64_t session, const uint64_t u[4], uint64_t out_h2_jac[12]);
 /* drops the handle; device memory goes when the last call holding the session returns.  An unknown or released handle fails. */
 int h2b_shplonk_release(uint64_t session);
+
+/* ---- the multi-point opening: [UP] halo2_proofs/src/poly/kzg/multiopen/gwc/prover.rs ProverGWC::create_proof -------------------
+ * Queries and polynomials as for SHPLONK above.  For each distinct point z_i (first-appearance order; points compare as words) with
+ * the queries p_i0, p_i1, ... there in query order (a query listed twice counts twice): W_i = commit(kate_division(sum_j v^j p_ij, z_i))
+ * over rows [0, n - 1) of the registered set handle_g, Jacobian, 12 words at out_w_jac + 12 i; *out_points = the number of points.
+ * Upstream subtracts sum_j v^j p_ij(z_i) at coefficient 0 first, which kate_division never reads, so no evaluation is computed.
+ * A zero quotient gives the identity (z = 0).  With polys_on_host, polys[i] are host arrays (pageable is fine) uploaded for the call;
+ * otherwise device pointers on `device`.  Synchronous; needs no session, since GWC squeezes no challenge between its commitments.
+ * Device memory is allocated for the call and given back before it returns: m numerators and m quotients of n Fr, with m the
+ * number of points or 32 (the batched MSM's width), whichever is smaller, plus the uploaded polynomials of a host-pointer call.
+ * Refused with H2B_ERR_BAD_ARGUMENT, every output untouched: no queries, a poly index >= n_polys, a polynomial that no query opens,
+ * a point or v >= r, n < 2 or n > 2^28, a null pointer, an unknown handle_g or one that does not hold rows [0, n - 1) on `device`,
+ * capacity below the number of points.  There is no limit on points per polynomial.  Profiling tags: 54 upload, 55 v powers,
+ * 56 numerators, 57 divisions, 58 MSMs. */
+int h2b_gwc_create_proof(int device, const void* const* polys, int polys_on_host, uint32_t n_polys, size_t n, const h2b_opening_query* queries,
+                         uint32_t n_queries, uint64_t handle_g, const uint64_t v[4], uint64_t* out_w_jac /* capacity x 12 */, uint32_t capacity,
+                         uint32_t* out_points);
 
 /* ---- MockProver::verify: [UP] halo2_proofs/src/dev.rs, the gate, lookup and permutation loops of verify_par ---------------------
  * n = 2^k rows, usable_rows = n - (blinding_factors + 1).  Cells follow upstream's CellValue: a fixed or advice cell is Assigned

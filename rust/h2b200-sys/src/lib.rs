@@ -143,6 +143,9 @@ extern "C" {
                              n_queries: u32, handle_g: u64, y: *const u64, v: *const u64, out_h1_jac: *mut u64, session: *mut u64) -> c_int;
     pub fn h2b_shplonk_finish(session: u64, u: *const u64, out_h2_jac: *mut u64) -> c_int;
     pub fn h2b_shplonk_release(session: u64) -> c_int;
+    pub fn h2b_gwc_create_proof(device: c_int, polys: *const *const c_void, polys_on_host: c_int, n_polys: u32, n: usize,
+                                queries: *const h2b_opening_query, n_queries: u32, handle_g: u64, v: *const u64, out_w_jac: *mut u64, capacity: u32,
+                                out_points: *mut u32) -> c_int;
     pub fn h2b_dev_alloc(device: c_int, bytes: usize, out: *mut *mut c_void) -> c_int;
     pub fn h2b_dev_free(device: c_int, p: *mut c_void) -> c_int;
     pub fn h2b_memcpy_h2d(device: c_int, d_dst: *mut c_void, h_src: *const c_void, bytes: usize) -> c_int;
@@ -552,6 +555,26 @@ impl Drop for ShplonkSession {
     fn drop(&mut self) {
         unsafe { h2b_shplonk_release(self.handle) };
     }
+}
+
+/// The GWC opening (`h2b_gwc_create_proof`) on device 0: W of every distinct point (Jacobian limbs) in first-appearance order.  Polynomials
+/// are host slices of n Fr limbs, uploaded for the call.
+pub fn gwc_create_proof(polys: &[&[[u64; 4]]], queries: &[h2b_opening_query], handle_g: u64, v: &[u64; 4]) -> Vec<[u64; 12]> {
+    ensure_init();
+    let n = polys.first().map(|p| p.len()).unwrap_or(0);
+    assert!(polys.iter().all(|p| p.len() == n), "ProverGWC: polynomials of different lengths");
+    let ptrs: Vec<*const c_void> = polys.iter().map(|p| p.as_ptr() as *const c_void).collect();
+    let mut w = vec![[0u64; 12]; queries.len()];
+    let mut points = 0u32;
+    let rc = unsafe {
+        h2b_gwc_create_proof(0, ptrs.as_ptr(), 1, ptrs.len() as u32, n, queries.as_ptr(), queries.len() as u32, handle_g, v.as_ptr(),
+                             w.as_mut_ptr() as *mut u64, w.len() as u32, &mut points)
+    };
+    if rc != 0 {
+        panic!("h2b_gwc_create_proof failed ({rc}): {}", last_error());
+    }
+    w.truncate(points as usize);
+    w
 }
 
 // ---- MockProver::verify's row loops (h2b_mock_verify) --------------------------------------------------------------------------

@@ -39,7 +39,7 @@ build_arm cpu
 build_arm gpu
 
 OUT="$HERE/proofs"; mkdir -p "$OUT"; status=0
-for case in standard_plonk halo2_lib; do
+for case in standard_plonk standard_plonk_gwc halo2_lib; do
     for arm in cpu gpu; do
         DEGREE=16 "$HERE/target-$arm/release/proof_bytes" "$case" "$SEED" "$OUT/$case.$arm.proof"
     done

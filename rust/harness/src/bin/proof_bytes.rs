@@ -5,6 +5,7 @@
 //! Run once per arm (stock halo2_proofs / forks patched with libh2b200) and compare the files: scripts/proof_parity.sh.
 //!
 //! Cases (BASELINE.json configs):  standard_plonk  -- /root/reference/examples/standard_plonk.rs:25-64 (PSE prover, k = 5)
+//!                                 standard_plonk_gwc -- the same circuit opened with ProverGWC / VerifierGWC instead of SHPLONK
 //!                                 halo2_lib       -- /root/reference/examples/halo2_lib.rs through the scaffold::prove flow
 //!                                                    (/root/reference/src/scaffold.rs:246-365; Axiom prover; DEGREE / LOOKUP_BITS env)
 //! The circuits themselves are the reference's own types (halo2_scaffold::circuits / ::scaffold); only the rng differs: every call
@@ -27,25 +28,35 @@ mod pse {
         poly::commitment::ParamsProver,
         poly::kzg::{
             commitment::{KZGCommitmentScheme, ParamsKZG},
-            multiopen::{ProverSHPLONK, VerifierSHPLONK},
+            multiopen::{ProverGWC, ProverSHPLONK, VerifierGWC, VerifierSHPLONK},
             strategy::SingleStrategy,
         },
         transcript::{Blake2bRead, Blake2bWrite, Challenge255, TranscriptReadBuffer, TranscriptWriterBuffer},
     };
 
-    pub fn prove<C: Circuit<Fr>>(k: u32, seed: u64, keygen: C, proving: impl FnOnce(&mut ChaCha20Rng) -> C, instances: &[&[Fr]]) -> Vec<u8> {
+    /// gwc: open with ProverGWC / VerifierGWC instead of ProverSHPLONK / VerifierSHPLONK
+    pub fn prove<C: Circuit<Fr>>(k: u32, seed: u64, keygen: C, proving: impl FnOnce(&mut ChaCha20Rng) -> C, instances: &[&[Fr]], gwc: bool) -> Vec<u8> {
         let mut rng = ChaCha20Rng::seed_from_u64(seed);
         let params = ParamsKZG::<Bn256>::setup(k, &mut rng);
         let pk = keygen_pk(&params, keygen_vk(&params, &keygen).expect("vk"), &keygen).expect("pk");
         let circuit = proving(&mut rng);
         let mut w = Blake2bWrite::<_, G1Affine, Challenge255<_>>::init(vec![]);
-        create_proof::<KZGCommitmentScheme<Bn256>, ProverSHPLONK<'_, Bn256>, _, _, _, _>(&params, &pk, &[circuit], &[instances], &mut rng, &mut w)
-            .expect("create_proof");
+        if gwc {
+            create_proof::<KZGCommitmentScheme<Bn256>, ProverGWC<'_, Bn256>, _, _, _, _>(&params, &pk, &[circuit], &[instances], &mut rng, &mut w)
+        } else {
+            create_proof::<KZGCommitmentScheme<Bn256>, ProverSHPLONK<'_, Bn256>, _, _, _, _>(&params, &pk, &[circuit], &[instances], &mut rng, &mut w)
+        }
+        .expect("create_proof");
         let proof = w.finalize();
         let mut r = Blake2bRead::<_, G1Affine, Challenge255<_>>::init(&proof[..]);
-        verify_proof::<KZGCommitmentScheme<Bn256>, VerifierSHPLONK<'_, Bn256>, _, _, SingleStrategy<'_, Bn256>>(
-            params.verifier_params(), pk.get_vk(), SingleStrategy::new(&params), &[instances], &mut r)
-            .expect("the reference verifier rejected the proof");
+        if gwc {
+            verify_proof::<KZGCommitmentScheme<Bn256>, VerifierGWC<'_, Bn256>, _, _, SingleStrategy<'_, Bn256>>(
+                params.verifier_params(), pk.get_vk(), SingleStrategy::new(&params), &[instances], &mut r)
+        } else {
+            verify_proof::<KZGCommitmentScheme<Bn256>, VerifierSHPLONK<'_, Bn256>, _, _, SingleStrategy<'_, Bn256>>(
+                params.verifier_params(), pk.get_vk(), SingleStrategy::new(&params), &[instances], &mut r)
+        }
+        .expect("the reference verifier rejected the proof");
         proof
     }
 }
@@ -124,15 +135,16 @@ mod axiom {
 fn main() {
     let args: Vec<String> = env::args().collect();
     if args.len() != 4 {
-        eprintln!("usage: proof_bytes <standard_plonk|halo2_lib> <seed> <out-file>");
+        eprintln!("usage: proof_bytes <standard_plonk|standard_plonk_gwc|halo2_lib> <seed> <out-file>");
         std::process::exit(2);
     }
     let seed: u64 = args[2].parse().expect("seed");
     let proof = match args[1].as_str() {
-        "standard_plonk" => {
+        case @ ("standard_plonk" | "standard_plonk_gwc") => {
             use halo2_proofs::{circuit::Value, halo2curves::bn256::Fr};
             use halo2_scaffold::circuits::standard_plonk::StandardPlonk;
-            pse::prove(5, seed, StandardPlonk { x: Value::unknown() }, |rng| StandardPlonk { x: Value::known(<Fr as ff::Field>::random(rng)) }, &[])
+            pse::prove(5, seed, StandardPlonk { x: Value::unknown() }, |rng| StandardPlonk { x: Value::known(<Fr as ff::Field>::random(rng)) }, &[],
+                       case == "standard_plonk_gwc")
         }
         "halo2_lib" => axiom::prove(seed),
         other => panic!("unknown case {other}"),

@@ -17,6 +17,8 @@ Turns a checkout of halo2_proofs (PSE tag v2023_02_02 or axiom-crypto branch axi
   * src/plonk.rs, src/plonk/evaluation.rs, src/dev.rs: `MockProver::verify_par` dispatches to rust/patches/mock_prover_dropin.rs
     for Fr; evaluation.rs gains `encode_source` / `FlatGraph` and the `evaluation` module becomes visible in the crate
     (rust/patches/mock_prover_patch.py, whose functions assert every pattern they rely on);
+  * src/poly/kzg/multiopen/shplonk/prover.rs and gwc/prover.rs: `ProverSHPLONK::create_proof` and `ProverGWC::create_proof` dispatch
+    to rust/patches/shplonk_dropin.rs and gwc_dropin.rs for Bn256 (the latter through rust/patches/gwc_patch.py);
   * Cargo.toml: `h2b200-sys = { path = ".../rust/h2b200-sys" }` is added to [dependencies].
 Idempotent.  Not run in the build container (no Rust sources of halo2_proofs are available there)."""
 import pathlib
@@ -140,9 +142,13 @@ if "create_proof_h2b" not in shplonk.read_text():
                "ProverSHPLONK::create_proof", re.S)
     add_uses(shplonk, ["use std::any::TypeId;", "use halo2curves::bn256::Bn256;", "use crate::poly::{Coeff, Polynomial};"])
     shplonk.write_text(shplonk.read_text() + "\n// ---- libh2b200 drop-in (rust/patches/shplonk_dropin.rs) ----\n" + (rust / "patches" / "shplonk_dropin.rs").read_text() + "\n")
+# ProverGWC::create_proof (rust/patches/gwc_dropin.rs, whose header states the mechanism; the text transform is rust/patches/gwc_patch.py)
+sys.path.insert(0, str(rust / "patches"))
+import gwc_patch  # noqa: E402
+gwc = crate / "src" / "poly" / "kzg" / "multiopen" / "gwc" / "prover.rs"
+gwc.write_text(gwc_patch.patch_gwc_prover(gwc.read_text(), (rust / "patches" / "gwc_dropin.rs").read_text()))
 # MockProver::verify_par's gate, lookup and permutation loops (rust/patches/mock_prover_dropin.rs, whose header states the mechanism;
 # the text transforms are rust/patches/mock_prover_patch.py)
-sys.path.insert(0, str(rust / "patches"))
 import mock_prover_patch as mpp  # noqa: E402
 for path, transform in ((crate / "src" / "plonk.rs", mpp.patch_plonk),
                         (crate / "src" / "plonk" / "evaluation.rs", lambda t: mpp.patch_evaluation(t, (rust / "patches" / "evaluation_dropin.rs").read_text())),

@@ -199,6 +199,10 @@ static inline cudaError_t cudaDeviceCanAccessPeer(int* can, int, int) { *can = 1
 static inline cudaError_t cudaDeviceEnablePeerAccess(int, unsigned) { return cudaSuccess; }
 static inline cudaError_t cudaMemset(void* d, int v, size_t n) { memset(d, v, n); return cudaSuccess; }
 static inline cudaError_t cudaMemsetAsync(void* d, int v, size_t n, cudaStream_t = 0) { memset(d, v, n); return cudaSuccess; }
+static inline cudaError_t cudaMemset2DAsync(void* d, size_t pitch, int v, size_t width, size_t height, cudaStream_t = 0) {
+    for (size_t r = 0; r < height; ++r) memset((char*)d + r * pitch, v, width);
+    return cudaSuccess;
+}
 static inline cudaError_t cudaStreamCreateWithFlags(cudaStream_t* s, unsigned) { *s = nullptr; return cudaSuccess; }
 static inline cudaError_t cudaStreamCreate(cudaStream_t* s) { *s = nullptr; return cudaSuccess; }
 static inline cudaError_t cudaStreamDestroy(cudaStream_t) { return cudaSuccess; }
