@@ -1104,7 +1104,8 @@ class Lib:
         b = a if b is None else _u64(b)
         out = np.empty_like(a)
         ops = {"add": 0, "sub": 1, "mul": 2, "sqr": 3, "inv": 4, "from_mont": 5, "to_mont": 6,
-               "mul_lazy": 7, "sqr_lazy": 8, "add_lazy": 9, "sub_lazy": 10, "canon": 11, "is_zero_lazy": 12}
+               "mul_lazy": 7, "sqr_lazy": 8, "add_lazy": 9, "sub_lazy": 10, "canon": 11, "is_zero_lazy": 12,
+               "mul2_lazy": 13}
         self.check(self.L.h2b_field_op({"fr": 0, "fq": 1}[field], ops[op], a.ctypes.data, b.ctypes.data, a.size // 4, out.ctypes.data))
         return out
 

@@ -565,7 +565,7 @@ int h2b_msm_checksum_dev(int device, const void* d_scalars, uint64_t seed, uint6
 }
 
 int h2b_field_op(int field, int op, const uint64_t* a, const uint64_t* b, size_t n, uint64_t* out) {
-    if (field < 0 || field > 1 || op < 0 || op > 12) { set_error("h2b_field_op: bad field/op"); return H2B_ERR_BAD_ARGUMENT; }
+    if (field < 0 || field > 1 || op < 0 || op > 13) { set_error("h2b_field_op: bad field/op"); return H2B_ERR_BAD_ARGUMENT; }
     return elementwise_host(0, field, op, a, b, n, out, 32);
 }
 int h2b_ec_op(int op, const uint64_t* p, const uint64_t* q, size_t n, uint64_t* out) {

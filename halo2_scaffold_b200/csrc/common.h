@@ -33,6 +33,23 @@ const char* get_error();
         if (_r != 0) return _r;   \
     } while (0)
 
+// 16-byte global -> shared copy that does not pass through registers (LDGSTS): a thread issues its copies back to
+// back and waits once, so a tile load costs one memory latency instead of one per element (NTT), and a gathered point
+// waits in shared memory instead of registers (MSM accumulation).
+__device__ __forceinline__ void copy16_async(uint4* smem_dst, const uint4* gmem_src) {
+#ifdef H2B_EMU
+    *smem_dst = *gmem_src;
+#else
+    unsigned sa = (unsigned)__cvta_generic_to_shared(smem_dst);
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sa), "l"(gmem_src) : "memory");
+#endif
+}
+__device__ __forceinline__ void copy_async_wait_all() {
+#ifndef H2B_EMU
+    asm volatile("cp.async.commit_group;\n\tcp.async.wait_group 0;" ::: "memory");
+#endif
+}
+
 // A grow-only device buffer (scratch space reused across calls on one device).
 struct DevBuf {
     void* p = nullptr;

@@ -125,15 +125,7 @@ __device__ __forceinline__ void xyzz_add_affine(XYZZ& acc, const Affine& q_in, b
     Fq ppp = fp_mul(p, pp);
     Fq qq = fp_mul(acc.x, pp);
     Fq x3 = fp_sub(fp_sub(fp_sqr(r), ppp), fp_dbl(qq));
-    // Y3 = R*(Q - X3) - Y1*PPP.  fp_mul2 (two products, one Montgomery reduction) saves 72 of this addition's 1260
-    // FMA-pipe instructions, but measured 2 % SLOWER here (profiles/r01_field_primitives.jsonl): at the 16 warps per
-    // SM this kernel's 126 registers allow, the longer dependency chains of the separated product/reduction form
-    // cost more than the saved dispatch cycles.  Kept behind a switch for kernels with more resident warps.
-#ifdef H2B_MADD_MUL2
-    Fq y3 = fp_mul2(r, fp_sub(qq, x3), fp_neg(acc.y), ppp);
-#else
     Fq y3 = fp_sub(fp_mul(r, fp_sub(qq, x3)), fp_mul(acc.y, ppp));
-#endif
     acc.x = x3;
     acc.y = y3;
     acc.zz = fp_mul(acc.zz, pp);
@@ -163,14 +155,16 @@ __device__ __forceinline__ void xyzz_add_affine_lazy(XYZZ& acc, const Affine& q_
     }
     Fq pp = fp_sqr_lazy(p);
     Fq ppp = fp_mul_lazy(p, pp);
+    // Y3 = R*(Q - X3) + Y1*(p - PPP) with one Montgomery reduction (72 fewer wide multiply-adds than two products); the
+    // second factor of each product is canonicalised, which fp_mul2_lazy needs to stay below 2p.  ZZ3 and ZZZ3 before X3:
+    // of the orders tried this one issues the fewest instructions within the accumulate kernel's 128 registers.
+    Fq nppp = fp_neg_lazy(fp_canon(ppp));
     Fq qq = fp_mul_lazy(acc.x, pp);
-    Fq yppp = fp_mul_lazy(acc.y, ppp);      // before X3: in the order of xyzz_add_affine this kernel spills at 128 registers
-    Fq x3 = fp_sub_lazy(fp_sub_lazy(fp_sqr_lazy(r), ppp), fp_add_lazy(qq, qq));
-    Fq y3 = fp_sub_lazy(fp_mul_lazy(r, fp_sub_lazy(qq, x3)), yppp);
-    acc.x = x3;
-    acc.y = y3;
     acc.zz = fp_mul_lazy(acc.zz, pp);
     acc.zzz = fp_mul_lazy(acc.zzz, ppp);
+    Fq x3 = fp_sub_lazy(fp_sub_lazy(fp_sqr_lazy(r), ppp), fp_add_lazy(qq, qq));
+    acc.y = fp_mul2_lazy(r, fp_canon(fp_sub_lazy(qq, x3)), acc.y, nppp);
+    acc.x = x3;
 }
 __device__ __forceinline__ XYZZ xyzz_canon(const XYZZ& a) {
     XYZZ r;

@@ -158,6 +158,19 @@ template <int F> __device__ __forceinline__ Fp<F> fp_sqr_lazy(const Fp<F>& a) {
     return r;
 #endif
 }
+// a*b + c*d with one Montgomery reduction: a, c < 2p, b, d CANONICAL (< p) -> result < 2p.  With b or d lazy the sum of
+// the products can exceed p * 2^256 and the result 2p.
+template <int F> __device__ __forceinline__ Fp<F> fp_mul2_lazy(const Fp<F>& a, const Fp<F>& b, const Fp<F>& c, const Fp<F>& d) {
+    Fp<F> r;
+    if (F == FR) fr_mul2_lazy_asm(r.l, a.l, b.l, c.l, d.l); else fq_mul2_lazy_asm(r.l, a.l, b.l, c.l, d.l);
+    return r;
+}
+// p - a for a in [0, p]: a canonical negation whose result is p, not 0, for a == 0
+template <int F> __device__ __forceinline__ Fp<F> fp_neg_lazy(const Fp<F>& a) {
+    Fp<F> r;
+    if (F == FR) fr_neg_lazy_asm(r.l, a.l); else fq_neg_lazy_asm(r.l, a.l);
+    return r;
+}
 template <int F> __device__ __forceinline__ Fp<F> fp_add_lazy(const Fp<F>& a, const Fp<F>& b) {
     Fp<F> r;
     if (F == FR) fr_add_lazy_asm(r.l, a.l, b.l); else fq_add_lazy_asm(r.l, a.l, b.l);
@@ -191,16 +204,20 @@ template <int F> inline void fp_sub_p(uint32_t* t) {
         bw = d >> 32;
     }
 }
-// Montgomery product without the final subtraction: t[0..8] = (ab + Mp) / 2^256
-template <int F> inline void fp_mont_emu(const Fp<F>& a, const Fp<F>& b, uint32_t (&t)[10]) {
+// Montgomery product without the final subtraction: t[0..8] = (ab + Mp) / 2^256 (with c, d: (ab + cd + Mp) / 2^256)
+template <int F> inline void fp_mont_emu(const Fp<F>& a, const Fp<F>& b, uint32_t (&t)[10], const Fp<F>* c2 = nullptr, const Fp<F>* d2 = nullptr) {
     for (int i = 0; i < 8; ++i) {
-        uint64_t c = 0;
-        for (int j = 0; j < 8; ++j) { c += (uint64_t)a.l[j] * b.l[i] + t[j]; t[j] = (uint32_t)c; c >>= 32; }
-        c += t[8]; t[8] = (uint32_t)c; t[9] = (uint32_t)(c >> 32);
+        for (int k = 0; k < (c2 ? 2 : 1); ++k) {
+            const Fp<F>& x = k ? *c2 : a;
+            const uint32_t y = k ? d2->l[i] : b.l[i];
+            uint64_t c = 0;
+            for (int j = 0; j < 8; ++j) { c += (uint64_t)x.l[j] * y + t[j]; t[j] = (uint32_t)c; c >>= 32; }
+            c += t[8]; t[8] = (uint32_t)c; t[9] += (uint32_t)(c >> 32);
+        }
         uint32_t m = t[0] * FpParams<F>::INV;
-        c = (uint64_t)m * FpParams<F>::P(0) + t[0]; c >>= 32;
+        uint64_t c = (uint64_t)m * FpParams<F>::P(0) + t[0]; c >>= 32;
         for (int j = 1; j < 8; ++j) { c += (uint64_t)m * FpParams<F>::P(j) + t[j]; t[j - 1] = (uint32_t)c; c >>= 32; }
-        c += t[8]; t[7] = (uint32_t)c; t[8] = t[9] + (uint32_t)(c >> 32);
+        c += t[8]; t[7] = (uint32_t)c; t[8] = t[9] + (uint32_t)(c >> 32); t[9] = 0;
     }
 }
 template <int F> inline Fp<F> fp_mul(const Fp<F>& a, const Fp<F>& b) {
@@ -241,6 +258,17 @@ template <int F> inline Fp<F> fp_mul_lazy(const Fp<F>& a, const Fp<F>& b) {
     return r;
 }
 template <int F> inline Fp<F> fp_sqr_lazy(const Fp<F>& a) { return fp_mul_lazy(a, a); }
+template <int F> inline Fp<F> fp_mul2_lazy(const Fp<F>& a, const Fp<F>& b, const Fp<F>& c, const Fp<F>& d) {
+    uint32_t t[10] = {0};
+    fp_mont_emu(a, b, t, &c, &d);
+    Fp<F> r; for (int i = 0; i < 8; ++i) r.l[i] = t[i];
+    return r;
+}
+template <int F> inline Fp<F> fp_neg_lazy(const Fp<F>& a) {
+    Fp<F> r; int64_t bw = 0;
+    for (int i = 0; i < 8; ++i) { int64_t d = (int64_t)FpParams<F>::P(i) - a.l[i] + bw; r.l[i] = (uint32_t)d; bw = d >> 32; }
+    return r;
+}
 template <int F> inline Fp<F> fp_add_lazy(const Fp<F>& a, const Fp<F>& b) {
     uint32_t q[8], t[8], s[8]; fp_2p<F>(q);
     uint64_t c = 0; int64_t bw = 0;

@@ -641,7 +641,7 @@ __device__ __forceinline__ uint32_t slice_len(uint32_t total, uint32_t G) {
 }
 
 // ctrl[0] = buckets cut by a slice boundary (split_list), ctrl[1] = those cut into many pieces (heavy_list)
-__global__ void __launch_bounds__(256) msm_accumulate_kernel(MsmPlan pl, const uint4* __restrict__ tables, const uint32_t* __restrict__ offsets,
+__global__ void __launch_bounds__(256, 2) msm_accumulate_kernel(MsmPlan pl, const uint4* __restrict__ tables, const uint32_t* __restrict__ offsets,
                                                            const uint32_t* __restrict__ sorted, uint32_t* __restrict__ ctrl,
                                                            uint32_t* __restrict__ split_list, uint4* __restrict__ bucket_acc,
                                                            uint4* __restrict__ head_partial) {
@@ -662,16 +662,33 @@ __global__ void __launch_bounds__(256) msm_accumulate_kernel(MsmPlan pl, const u
     uint32_t next = offsets[b + 1];
     bool head = offsets[b] < start;      // the bucket began in an earlier slice
 
+    // The next point is gathered into shared memory while this one is added, not into 16 registers held across the
+    // whole addition: with those registers free the addition fits 128 (16 warps per SM) without spilling.  Two slots
+    // per thread, so the copy never overwrites the point being read.
+    __shared__ uint4 pt[2][4][256];
+    const uint32_t tid = threadIdx.x;
     XYZZ acc = xyzz_identity();
     uint32_t e = sorted[start];
-    Affine p = affine_load(tables + 4 * (size_t)(e & ~SIGN_BIT));
+#pragma unroll
+    for (int k = 0; k < 4; ++k) copy16_async(&pt[0][k][tid], tables + 4 * (size_t)(e & ~SIGN_BIT) + k);
+    uint32_t e_next = start + 1 < end ? sorted[start + 1] : 0;
     for (uint32_t j = start; j < end; ++j) {
-        uint32_t e_next = 0;
-        Affine p_next = p;
-        if (j + 1 < end) {      // prefetch the next point while this one is added
-            e_next = sorted[j + 1];
-            p_next = affine_load(tables + 4 * (size_t)(e_next & ~SIGN_BIT));
+        const uint32_t s = (j - start) & 1;
+        copy_async_wait_all();
+        if (j + 1 < end) {
+#pragma unroll
+            for (int k = 0; k < 4; ++k) copy16_async(&pt[s ^ 1][k][tid], tables + 4 * (size_t)(e_next & ~SIGN_BIT) + k);
         }
+        Affine p;
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            const uint4 v = pt[s][k][tid];
+            uint32_t* l = (k < 2 ? p.x.l : p.y.l) + 4 * (k & 1);
+            l[0] = v.x; l[1] = v.y; l[2] = v.z; l[3] = v.w;
+        }
+        const uint32_t e_cur = e;
+        e = e_next;
+        e_next = j + 2 < end ? sorted[j + 2] : 0;
         if (j == next) {        // bucket b is complete: flush, move to the next non-empty bucket
             if (head) xyzz_store(head_partial + 8 * (size_t)t, xyzz_canon(acc));
             else xyzz_store(bucket_acc + 8 * (size_t)b, xyzz_canon(acc));
@@ -679,9 +696,7 @@ __global__ void __launch_bounds__(256) msm_accumulate_kernel(MsmPlan pl, const u
             acc = xyzz_identity();
             do { ++b; next = offsets[b + 1]; } while (next <= j);
         }
-        xyzz_add_affine_lazy(acc, p, (e & SIGN_BIT) != 0);      // acc lazily reduced, canonical when stored
-        e = e_next;
-        p = p_next;
+        xyzz_add_affine_lazy(acc, p, (e_cur & SIGN_BIT) != 0);      // acc lazily reduced, canonical when stored
     }
     if (head) {
         xyzz_store(head_partial + 8 * (size_t)t, xyzz_canon(acc));

@@ -60,22 +60,6 @@ __device__ __forceinline__ void sm_put(uint4* lo, uint4* hi, uint32_t e, const F
     hi[k] = make_uint4(v.l[4], v.l[5], v.l[6], v.l[7]);
 }
 
-// 16-byte global -> shared copy that does not pass through registers (LDGSTS): a thread issues all its copies of a
-// tile back to back and waits once, so the tile load costs one memory latency instead of one per element.
-__device__ __forceinline__ void copy16_async(uint4* smem_dst, const uint4* gmem_src) {
-#ifdef H2B_EMU
-    *smem_dst = *gmem_src;
-#else
-    unsigned sa = (unsigned)__cvta_generic_to_shared(smem_dst);
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(sa), "l"(gmem_src) : "memory");
-#endif
-}
-__device__ __forceinline__ void copy_async_wait_all() {
-#ifndef H2B_EMU
-    asm volatile("cp.async.commit_group;\n\tcp.async.wait_group 0;" ::: "memory");
-#endif
-}
-
 // R consecutive DIF stages (first stage index s) on 2^R elements held in registers: the elements of one work item
 // differ in bits [b-s-R, b-s) of the digit q.  Stage s' multiplies the lower output of each butterfly by
 // Omega^(r * 2^s'), r = position inside the half block (the table index never exceeds N/2).

@@ -110,7 +110,8 @@ int msm_checksum_run(DeviceCtx& ctx, const void* d_scalars, uint64_t seed, uint6
 
 // ---- arithmetic self-tests -------------------------------------------------------------------------------
 // op: 0 add, 1 sub, 2 mul, 3 sqr(a), 4 inv(a), 5 from_mont(a), 6 to_mont(a); lazily reduced (operands < 2p):
-// 7 mul_lazy, 8 sqr_lazy(a), 9 add_lazy, 10 sub_lazy, 11 canon(a), 12 is_zero_lazy(a) (1 or 0 in the low limb)
+// 7 mul_lazy, 8 sqr_lazy(a), 9 add_lazy, 10 sub_lazy, 11 canon(a), 12 is_zero_lazy(a) (1 or 0 in the low limb),
+// 13 mul2_lazy(a, canon(b), b, neg_lazy(canon(a))) = a (b mod p) + b (p - (a mod p)), the form of the mixed addition's Y3
 template <int F>
 __global__ void __launch_bounds__(128) field_selftest_kernel(int op, const uint4* __restrict__ a, const uint4* __restrict__ b, uint32_t n, uint4* __restrict__ out) {
     uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -129,6 +130,7 @@ __global__ void __launch_bounds__(128) field_selftest_kernel(int op, const uint4
         case 9: r = fp_add_lazy(x, y); break;
         case 10: r = fp_sub_lazy(x, y); break;
         case 11: r = fp_canon(x); break;
+        case 13: r = fp_mul2_lazy(x, fp_canon(y), y, fp_neg_lazy(fp_canon(x))); break;
         default: r = fp_zero<F>(); r.l[0] = fp_is_zero_lazy(x) ? 1u : 0u; break;
     }
     fp_store<F>(out + 2 * (size_t)i, r);

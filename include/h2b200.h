@@ -602,7 +602,8 @@ int h2b_gen_scalars_dev(int device, uint64_t seed, size_t n, int kind, void* d_o
 int h2b_msm_checksum_dev(int device, const void* d_scalars /* n x 32 B Montgomery */, uint64_t seed, uint64_t first, size_t n, void* d_out, void* stream);
 /* element-wise field op on host arrays.  field: 0 Fr, 1 Fq.  op: 0 add, 1 sub, 2 mul, 3 sqr(a), 4 inv(a),
  * 5 from_mont(a), 6 to_mont(a); the lazily reduced operations of the MSM and NTT loops (operands in [0, 2p)):
- * 7 mul, 8 sqr(a), 9 add, 10 sub (results in [0, 2p)), 11 canonical form of a, 12 a == 0 mod p (1 or 0 in limb 0) */
+ * 7 mul, 8 sqr(a), 9 add, 10 sub (results in [0, 2p)), 11 canonical form of a, 12 a == 0 mod p (1 or 0 in limb 0),
+ * 13 a (b mod p) + b (p - (a mod p)) with one Montgomery reduction (result in [0, 2p)) */
 int h2b_field_op(int field, int op, const uint64_t* a, const uint64_t* b, size_t n, uint64_t* out);
 /* element-wise group op on host arrays of affine points; op: 0 p+q, 1 p-q, 2 4(p+q) via the general
  * XYZZ adder and doubling, 3 p+q through the Jacobian conversion, 4 p+q by the lazily reduced mixed addition

@@ -147,14 +147,19 @@ class Prog:
 #   T = E + O*2^32 ; E gets the products a_j*b_i with j even, O those with j odd.
 #   After each row the low limb of E is zero, T is divided by 2^32 by *renaming*:
 #   new E = old O (+ old e1 at limb 0), new O = old E >> 64.
+#   pair=True: r = (a*b + c*d) / 2^256 with ONE reduction; row i adds a*b_i and c*d_i before it reduces.  The
+#   running total stays below a + c + p, the pre-division total below 2^288 whenever a, c < 2^255 (both < 2p), so
+#   neither accumulator's top carry is ever lost (chk0).
 # =====================================================================================
-def gen_mont_mul(name, mod, square=False, lazy=False):
+def gen_mont_mul(name, mod, square=False, lazy=False, pair=False):
     p = limbs(mod)
     inv = (-pow(mod, -1, 1 << 32)) & M32
     A = ["a%d" % i for i in range(NL)]
     B = A if square else ["b%d" % i for i in range(NL)]
+    C = ["c%d" % i for i in range(NL)] if pair else []
+    D = ["d%d" % i for i in range(NL)] if pair else []
     R = ["r%d" % i for i in range(NL)]
-    P = Prog(name, A + ([] if square else B), R)
+    P = Prog(name, A + ([] if square else B) + C + D, R)
     ev = [P.tmp("e%d" % i) for i in range(NL)]
     od = [P.tmp("o%d" % i) for i in range(NL)]
     m = P.tmp("m")
@@ -190,11 +195,18 @@ def gen_mont_mul(name, mod, square=False, lazy=False):
                 src_hi = E[2 * j + 3] if 2 * j + 3 < NL else 0
                 P.emit("madc.lo.cc", E[2 * j], a_odd[j], bi, src_lo)
                 P.emit("madc.hi.cc", E[2 * j + 1], a_odd[j], bi, src_hi)
+            P.emit("chk0", None)
             E, O = O, E
             chain_mad(E, a_even, bi)
             P.emit("addc", O[NL - 1], O[NL - 1], 0)
+        if pair:
+            chain_mad(O, [C[1], C[3], C[5], C[7]], D[i])
+            P.emit("chk0", None)
+            chain_mad(E, [C[0], C[2], C[4], C[6]], D[i])
+            P.emit("addc", O[NL - 1], O[NL - 1], 0)
         P.emit("mul.lo", m, E[0], inv)
         chain_mad(O, p_odd, m)
+        P.emit("chk0", None)
         chain_mad(E, p_even, m)
         P.emit("addc", O[NL - 1], O[NL - 1], 0)
     # T = (E >> 32) + O   (E[0] == 0);  T < 2p whenever a*b < p * 2^256
@@ -223,9 +235,8 @@ def gen_mont_mul(name, mod, square=False, lazy=False):
 #   chain inside ONE accumulator, so ptxas keeps it as IMAD.WIDE.U32(.X).  The Montgomery
 #   reduction adds its m_i * p rows into the same accumulators; a carry that leaves a chain goes
 #   into a small per-limb counter C[pos] (or initialises a still untouched limb), never ripples.
-#   Used for the operations whose product phase differs from a plain a*b:
-#     * squaring (28 doubled cross products + 8 squares instead of 64 products),
-#     * a*b + c*d with ONE reduction (the Y3 of the XYZZ mixed addition).
+#   Used for squaring (28 doubled cross products + 8 squares instead of 64 products), whose product phase is not a
+#   sequence of rows a*b_i.
 # =====================================================================================
 class WideAcc:
     def __init__(self, P, nlimbs=16):
@@ -346,13 +357,6 @@ def redc_tail(P, acc, p, inv, R, lazy=False):
         P.emit("selnz", R[i], bw, t[i], s[i])
 
 
-def product_rows(acc, X, Y):
-    """acc += X * Y (8 x 8 limbs), operand scanning, two chains per row."""
-    for i in range(NL):
-        acc.chain(i, [(X[j], Y[i]) for j in (0, 2, 4, 6)])
-        acc.chain(i + 1, [(X[j], Y[i]) for j in (1, 3, 5, 7)])
-
-
 def gen_mont_sqr_sep(name, mod, lazy=False):
     p = limbs(mod)
     inv = (-pow(mod, -1, 1 << 32)) & M32
@@ -371,25 +375,6 @@ def gen_mont_sqr_sep(name, mod, lazy=False):
     acc.chain(0, [(A[i], A[i]) for i in range(NL)])
     redc_tail(P, acc, p, inv, R, lazy)
     return P
-
-
-def gen_mont_mul2_sep(name, mod):
-    """r = (a*b + c*d) / R mod p with a single reduction (a*b + c*d < 2 p^2 < p * 2^256)."""
-    p = limbs(mod)
-    inv = (-pow(mod, -1, 1 << 32)) & M32
-    A = ["a%d" % i for i in range(NL)]
-    B = ["b%d" % i for i in range(NL)]
-    C = ["c%d" % i for i in range(NL)]
-    D = ["d%d" % i for i in range(NL)]
-    R = ["r%d" % i for i in range(NL)]
-    P = Prog(name, A + B + C + D, R)
-    acc = WideAcc(P)
-    product_rows(acc, A, B)
-    product_rows(acc, C, D)
-    redc_tail(P, acc, p, inv, R)
-    return P
-
-
 
 
 def gen_add(name, mod, lazy=False):
@@ -446,6 +431,17 @@ def gen_canon(name, mod):
     return P
 
 
+def gen_neg(name, mod):
+    """[0, p] -> [0, p]: r = p - a (no borrow, no correction)."""
+    p = limbs(mod)
+    A = ["a%d" % i for i in range(NL)]
+    R = ["r%d" % i for i in range(NL)]
+    P = Prog(name, A, R)
+    for i in range(NL):
+        P.emit("sub.cc" if i == 0 else ("subc.cc" if i < NL - 1 else "subc"), R[i], p[i], A[i])
+    return P
+
+
 # =====================================================================================
 # verification
 # =====================================================================================
@@ -497,7 +493,9 @@ def check(prog, mod, kind, trials=3000):
 def check_lazy(prog, mod, kind, trials=3000):
     """Lazily reduced operations: operands in [0, 2p).  Checks the
     congruence, the output bound and, for products, the exact value: (a*b + M*p) / 2^256 with M = -a*b/p mod 2^256
-    is the unique Montgomery value before a final subtraction, so every other implementation must give these bits."""
+    is the unique Montgomery value before a final subtraction, so every other implementation must give these bits.
+    mul2 (a*b + c*d): a, c in [0, 2p), b, d canonical, so a*b + c*d < 4p^2 and the result < p (1 + 4p / 2^256) < 1.76p;
+    with all four operands lazy it could reach 2.51p.  neg: operand in [0, p]."""
     rng = random.Random(0x1A2B + mod % 9973 + len(prog.ins))
     R = 1 << 256
     Rinv = pow(R, -1, mod)
@@ -509,17 +507,27 @@ def check_lazy(prog, mod, kind, trials=3000):
         edge += [((1 << 256) - 1 - ((1 << sh) - 1)) % two_p, ((1 << sh) - 1) % two_p]
     cases = [(x, y) for x in edge for y in edge]
     cases += [(rng.randrange(two_p), rng.randrange(two_p)) for _ in range(trials)]
-    for x, y in cases:
+    for idx, (x, y) in enumerate(cases):
         if kind == "sqr":
             y = x
+        elif kind == "mul2":
+            y %= mod
+            z, w = cases[(idx * 7 + 3) % len(cases)]
+            z, w = (two_p - 1, mod - 1) if idx % 5 == 0 else (z, w % mod)
+        elif kind == "neg":
+            x = x if x <= mod else x - mod
         env = {"z0": 0}
-        for i, l in enumerate(limbs(x)):
-            env["a%d" % i] = l
-        for i, l in enumerate(limbs(y)):
-            env["b%d" % i] = l
+        for reg, v in (("a", x), ("b", y)) + ((("c", z), ("d", w)) if kind == "mul2" else ()):
+            for i, l in enumerate(limbs(v)):
+                env["%s%d" % (reg, i)] = l
         got = sum(v << (32 * i) for i, v in enumerate(prog.run(env)))
         if kind in ("mul", "sqr"):
             ok = got == (x * y + (-x * y * pinv % R) * mod) // R and got < two_p and got % mod == x * y * Rinv % mod
+        elif kind == "mul2":
+            t = x * y + z * w
+            ok = got == (t + (-t * pinv % R) * mod) // R and got < two_p and got % mod == t * Rinv % mod
+        elif kind == "neg":
+            ok = got == mod - x
         elif kind == "add":
             ok = got < two_p and got % mod == (x + y) % mod
         elif kind == "sub":
@@ -540,7 +548,7 @@ def main():
     ]
     total = 0
     for tag, mod in (("fr", FR), ("fq", FQ)):
-        for kind, gen in (("mul", gen_mont_mul), ("sqr", gen_mont_sqr_sep), ("mul2", gen_mont_mul2_sep),
+        for kind, gen in (("mul", gen_mont_mul), ("sqr", gen_mont_sqr_sep), ("mul2", lambda n, m: gen_mont_mul(n, m, pair=True)),
                           ("add", gen_add), ("sub", gen_sub)):
             prog = gen("%s_%s" % (tag, kind), mod)
             total += check(prog, mod, kind)
@@ -556,15 +564,20 @@ def main():
             chunks.append("\n")
     chunks.append("// Lazily reduced operations: operands and results in [0, 2p) (canon: result in [0, p)).\n"
                   "// BN254's p and r are below 2^256 / 5.29, so a Montgomery product of two values < 2p is already < 2p\n"
-                  "// without the final conditional subtraction.\n\n")
+                  "// without the final conditional subtraction.  mul2_lazy (a*b + c*d, one reduction) needs b, d < p for the\n"
+                  "// same bound; neg_lazy maps [0, p] to p - a.\n\n")
     for tag, mod in (("fr", FR), ("fq", FQ)):
         for kind, gen in (("mul", lambda n, m: gen_mont_mul(n, m, lazy=True)), ("sqr", lambda n, m: gen_mont_sqr_sep(n, m, lazy=True)),
+                          ("mul2", lambda n, m: gen_mont_mul(n, m, lazy=True, pair=True)),
                           ("add", lambda n, m: gen_add(n, m, lazy=True)), ("sub", lambda n, m: gen_sub(n, m, lazy=True)),
-                          ("canon", gen_canon)):
+                          ("canon", gen_canon), ("neg", gen_neg)):
             name = "%s_%s" % (tag, kind) if kind == "canon" else "%s_%s_lazy" % (tag, kind)
             prog = gen(name, mod)
             total += check_lazy(prog, mod, kind)
-            if kind in ("sqr", "canon"):
+            if kind == "mul2":
+                sig = ("__device__ __forceinline__ void %s_asm(uint32_t (&r)[8], const uint32_t (&a)[8], const uint32_t (&b)[8], "
+                       "const uint32_t (&c)[8], const uint32_t (&d)[8])" % name)
+            elif kind in ("sqr", "canon", "neg"):
                 sig = "__device__ __forceinline__ void %s_asm(uint32_t (&r)[8], const uint32_t (&a)[8])" % name
             else:
                 sig = "__device__ __forceinline__ void %s_asm(uint32_t (&r)[8], const uint32_t (&a)[8], const uint32_t (&b)[8])" % name
