@@ -89,6 +89,17 @@ __host__ __device__ __forceinline__ uint64_t splitmix64_at(uint64_t seed, uint64
     return z ^ (z >> 31);
 }
 
+// w (4 little-endian words) is below the scalar field modulus r
+inline bool fr_canonical(const uint64_t w[4]) {
+    uint32_t l[8];
+    memcpy(l, w, 32);
+    for (int i = 7; i >= 0; --i) {
+        if (l[i] < FpParams<FR>::P(i)) return true;
+        if (l[i] > FpParams<FR>::P(i)) return false;
+    }
+    return false;
+}
+
 // Optional per-kernel timing with CUDA events on the launching stream (bench.py's roofline numbers).
 enum ProfTag { PROF_BEGIN = 0, PROF_MSM_DECOMPOSE = 1, PROF_MSM_SCAN = 2, PROF_MSM_SCATTER = 3, PROF_MSM_PLAN = 4, PROF_MSM_ACCUMULATE = 5,
                PROF_MSM_COMBINE = 6, PROF_MSM_REDUCE = 7, PROF_MSM_FINAL = 8, PROF_MSM_PRECOMPUTE = 9, PROF_NTT_TWIDDLE = 15, PROF_NTT_PASS0 = 16,
@@ -161,6 +172,12 @@ int host_download_2d(DeviceCtx& ctx, void* h_dst, size_t h_pitch, const void* d_
 void stager_release(DeviceCtx& ctx);
 bool host_is_pageable(const void* p);
 // ---- scan.cu ----
+// polynomial evaluation and division by (X - b) run in levels of POLY_K coefficients; the powers x^(16^l), l < POLY_LEVELS_MAX, of one
+// point take POLY_PTS elements, the last of them the point itself
+static const uint32_t POLY_K = 16;
+static const uint32_t POLY_LEVELS_MAX = 9;                 // 16^8 > 2^31
+static const uint32_t POLY_PTS = POLY_LEVELS_MAX + 1;
+static const uint32_t SCAN_BLOCK = 1024;                   // elements per CTA of u32_exclusive_scan (256 threads x 4)
 int fr_batch_invert_run(DeviceCtx& ctx, void* d_a, size_t n, cudaStream_t stream);
 int fq_batch_invert_run(DeviceCtx& ctx, void* d_a, size_t n, cudaStream_t stream);
 int fr_prefix_product_run(DeviceCtx& ctx, const void* d_in, void* d_out, size_t n, cudaStream_t stream);
@@ -171,6 +188,14 @@ int fr_kate_division_at_run(DeviceCtx& ctx, const void* d_a, size_t n, const voi
 // `count` divisions of length n in one launch sequence: division d divides the n Fr at d_a + d n by (X - d_b[d]) into d_q + d n (n - 1
 // coefficients; d_b: count consecutive Fr on the device, outside ctx.scan_scratch).  count = 1 is fr_kate_division_at_run.
 int fr_kate_division_batch_run(DeviceCtx& ctx, const void* d_a, size_t n, const void* d_b, uint32_t count, void* d_q, cudaStream_t stream);
+// the powers of `count` points (back to back at d_x) into d_pts, point y's at d_pts + y POLY_PTS
+int fr_point_powers_run(const void* d_x, uint32_t count, void* d_pts, cudaStream_t stream);
+// `count` vectors of m values back to back at d_in, vector y at the point whose powers are at d_pts + y POLY_PTS, from `level` on:
+// one launch per level, the partial values of every level in d_buf (count (m / 15 + 1) elements), the count values to d_out
+int fr_horner_levels_run(const void* d_in, size_t m, const void* d_pts, uint32_t level, uint32_t count, void* d_buf, void* d_out, cudaStream_t stream);
+// exclusive scan of `count` 32-bit values: out[i] = in[0] + .. + in[i-1], out[count] = total, out2 (optional) = out[0, count) again;
+// `sums` holds ceil(count / SCAN_BLOCK) + 1 words
+int u32_exclusive_scan(const uint32_t* in, uint32_t count, uint32_t* out, uint32_t* out2, uint32_t* sums, cudaStream_t stream);
 int fr_lincomb_run(DeviceCtx& ctx, const void* const* d_cols, const uint64_t* coeffs, uint32_t m, size_t n, void* d_out, cudaStream_t stream);
 int permutation_product_run(DeviceCtx& ctx, const void* const* d_values, const void* const* d_sigma, uint32_t m, size_t n, const uint64_t* beta,
                             const uint64_t* gamma, const uint64_t* delta, const uint64_t* deltaomega, const uint64_t* omega, const uint64_t* last_z,
@@ -275,7 +300,6 @@ struct ShplonkPlan {
     std::vector<std::vector<uint32_t>> set_slots, set_points;
     uint32_t n_points() const { return (uint32_t)(points.size() / 4); }
 };
-bool fr_canonical(const uint64_t w[4]);
 // need_every_poly: a polynomial that no query names is refused
 int shplonk_plan_build(const char* who, const h2b_opening_query* queries, uint32_t n_queries, uint32_t n_polys, bool need_every_poly, ShplonkPlan* out);
 size_t shplonk_tables_bytes(const ShplonkPlan& p);

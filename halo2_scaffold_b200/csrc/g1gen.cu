@@ -219,12 +219,7 @@ static void fr_mul_host(const uint64_t* a, const uint64_t* b, uint64_t* r) {
 
 int srs_setup_check(uint32_t k, const uint64_t s[4]) {
     if (k > 28) { set_error("h2b_srs_setup: k = %u (at most 28)", k); return H2B_ERR_BAD_ARGUMENT; }
-    uint32_t w[8];
-    memcpy(w, s, 32);
-    for (int i = 7; i >= 0; --i) {
-        if (w[i] < FpParams<FR>::P(i)) break;
-        if (w[i] > FpParams<FR>::P(i) || i == 0) { set_error("h2b_srs_setup: s is not below the scalar field modulus"); return H2B_ERR_BAD_ARGUMENT; }
-    }
+    if (!fr_canonical(s)) { set_error("h2b_srs_setup: s is not below the scalar field modulus"); return H2B_ERR_BAD_ARGUMENT; }
     // s^n == 1 means s = w^j for some j: a denominator s - w^j vanishes (upstream panics in invert().unwrap())
     uint64_t p[4];
     memcpy(p, s, 32);

@@ -1,5 +1,5 @@
-// 256-bit sort keys (canonical Fr values, limb 7 most significant), their sort and the flag scan: shared by the lookup argument's
-// permutation (lookup.cu, which implements both passes) and the MockProver checker (mock.cu).
+// 256-bit sort keys (canonical Fr values, limb 7 most significant) and their sort: shared by the lookup argument's permutation
+// (lookup.cu, which implements the sort) and the MockProver checker (mock.cu).
 #pragma once
 #include "common.h"
 
@@ -32,13 +32,8 @@ __device__ __forceinline__ void key_store(uint4* p, size_t i, const Key& k) {
     p[2 * i + 1] = make_uint4(k.l[4], k.l[5], k.l[6], k.l[7]);
 }
 
-static const uint32_t FLAG_SCAN_BLOCK = 1024;
-
 // ---- lookup.cu ----
 // ascending bitonic sort of `padded` keys (a power of two, at least SORT_TILE)
 int bitonic_sort(uint4* keys, uint32_t padded, cudaStream_t stream);
-// exclusive scan of `count` 32-bit values: out[i] = in[0] + .. + in[i-1], out[count] = total; `sums` holds
-// ceil(count / FLAG_SCAN_BLOCK) + 1 words
-int flag_scan(const uint32_t* in, uint32_t count, uint32_t* out, uint32_t* sums, cudaStream_t stream);
 
 }  // namespace h2b

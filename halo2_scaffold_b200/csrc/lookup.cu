@@ -10,8 +10,8 @@
 //     indistinguishable, so no stability is needed; compare-exchange distances below the tile run in shared memory
 //     (limb-major layout), larger ones as streaming passes, two distances per pass.  Padding up to a power of two is the all-ones key;
 //   * first occurrences, the match of every distinct input value to the first equal table entry (binary search in the
-//     sorted table), the ranks of the repeated rows and of the unmatched table entries (two exclusive scans) and the fill
-//     are elementwise kernels.  The order of the fill is exactly upstream's: the i-th smallest leftover value goes to the
+//     sorted table) and the fill are elementwise kernels; the ranks of the repeated rows and of the unmatched table entries are two
+//     exclusive scans (scan.cu's u32_exclusive_scan).  The order of the fill is exactly upstream's: the i-th smallest leftover value goes to the
 //     i-th repeated row counted from the end.
 // Rows at and beyond usable_rows (the blinding rows) are the caller's.
 #include "keys.cuh"
@@ -144,59 +144,6 @@ int bitonic_sort(uint4* keys, uint32_t padded, cudaStream_t stream) {      // pa
     return H2B_OK;
 }
 
-// ---- exclusive scan of 32-bit flags (out[count] = total) -----------------------------------------------------------------
-__global__ void __launch_bounds__(256) flag_scan_sums_kernel(const uint32_t* __restrict__ in, uint32_t count, uint32_t* __restrict__ sums) {
-    __shared__ uint32_t ws[8];
-    const uint32_t base = blockIdx.x * FLAG_SCAN_BLOCK + threadIdx.x * 4;
-    uint32_t s = 0;
-    for (int q = 0; q < 4; ++q) if (base + q < count) s += in[base + q];
-    for (int o = 16; o > 0; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
-    if ((threadIdx.x & 31) == 0) ws[threadIdx.x >> 5] = s;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        uint32_t t = 0;
-        for (int q = 0; q < 8; ++q) t += ws[q];
-        sums[blockIdx.x] = t;
-    }
-}
-__global__ void flag_scan_top_kernel(uint32_t* sums, uint32_t nblocks) {          // one thread: at most a few thousand sums
-    if (blockIdx.x != 0 || threadIdx.x != 0) return;
-    uint32_t run = 0;
-    for (uint32_t i = 0; i < nblocks; ++i) { const uint32_t v = sums[i]; sums[i] = run; run += v; }
-    sums[nblocks] = run;
-}
-__global__ void __launch_bounds__(256) flag_scan_apply_kernel(const uint32_t* __restrict__ in, uint32_t count, const uint32_t* __restrict__ sums,
-                                                            uint32_t* __restrict__ out) {
-    __shared__ uint32_t ws[8];
-    const uint32_t base = blockIdx.x * FLAG_SCAN_BLOCK + threadIdx.x * 4;
-    uint32_t v[4], s = 0;
-    for (int q = 0; q < 4; ++q) { v[q] = base + q < count ? in[base + q] : 0; s += v[q]; }
-    const uint32_t lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    uint32_t incl = s;
-    for (int o = 1; o < 32; o <<= 1) {
-        const uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= (uint32_t)o) incl += t;
-    }
-    if (lane == 31) ws[wid] = incl;
-    __syncthreads();
-    uint32_t woff = 0;
-    for (uint32_t q = 0; q < wid; ++q) woff += ws[q];
-    uint32_t run = sums[blockIdx.x] + woff + incl - s;
-    for (int q = 0; q < 4; ++q) {
-        if (base + q < count) out[base + q] = run;
-        run += v[q];
-    }
-    if (blockIdx.x == gridDim.x - 1 && threadIdx.x == 255) out[count] = sums[gridDim.x];
-}
-int flag_scan(const uint32_t* in, uint32_t count, uint32_t* out, uint32_t* sums, cudaStream_t stream) {
-    const uint32_t nblocks = (count + FLAG_SCAN_BLOCK - 1) / FLAG_SCAN_BLOCK;
-    H2B_LAUNCH(flag_scan_sums_kernel, nblocks, 256, 0, stream, in, count, sums);
-    H2B_LAUNCH(flag_scan_top_kernel, 1, 32, 0, stream, sums, nblocks);
-    H2B_LAUNCH(flag_scan_apply_kernel, nblocks, 256, 0, stream, in, count, (const uint32_t*)sums, out);
-    H2B_CUDA(cudaGetLastError());
-    return H2B_OK;
-}
-
 // ---- matching the sorted input against the sorted table --------------------------------------------------------------------
 // repeated[r] = 1 when A'[r] == A'[r-1]; a first occurrence claims the first table entry equal to it (used[p] = 1)
 __global__ void __launch_bounds__(256) lookup_match_kernel(const uint4* __restrict__ a, const uint4* __restrict__ t, uint32_t usable,
@@ -257,7 +204,7 @@ int lookup_permute_run(DeviceCtx& ctx, const void* d_input, const void* d_table,
     uint32_t padded = SORT_TILE;
     while (padded < usable_rows) padded <<= 1;
     const size_t key_bytes = (size_t)padded * 32, flag_bytes = ((size_t)usable_rows + 1 + 3) / 4 * 16;
-    const uint32_t nblocks = (usable_rows + FLAG_SCAN_BLOCK - 1) / FLAG_SCAN_BLOCK;
+    const uint32_t nblocks = (usable_rows + SCAN_BLOCK - 1) / SCAN_BLOCK;
     H2B_TRY(ctx.lookup_scratch.reserve(2 * key_bytes + 7 * flag_bytes + ((size_t)nblocks + 2) * 4 + 64));
     char* base = (char*)ctx.lookup_scratch.p;
     uint4* ka = (uint4*)base;
@@ -279,8 +226,8 @@ int lookup_permute_run(DeviceCtx& ctx, const void* d_input, const void* d_table,
     H2B_CUDA(cudaMemsetAsync(missing, 0, 4, stream));
     H2B_LAUNCH(lookup_match_kernel, gu, 256, 0, stream, (const uint4*)ka, (const uint4*)kt, usable_rows, repeated, used, missing);
     H2B_LAUNCH(lookup_invert_flags_kernel, gu, 256, 0, stream, (const uint32_t*)used, usable_rows, unused);
-    H2B_TRY(flag_scan(repeated, usable_rows, rank_r, sums, stream));
-    H2B_TRY(flag_scan(unused, usable_rows, rank_l, sums, stream));
+    H2B_TRY(u32_exclusive_scan(repeated, usable_rows, rank_r, nullptr, sums, stream));
+    H2B_TRY(u32_exclusive_scan(unused, usable_rows, rank_l, nullptr, sums, stream));
     H2B_LAUNCH(lookup_repeated_rows_kernel, gu, 256, 0, stream, (const uint32_t*)repeated, (const uint32_t*)rank_r, usable_rows, rows_of_rank);
     H2B_LAUNCH(lookup_fill_kernel, gu, 256, 0, stream, (const uint4*)ka, (const uint4*)kt, usable_rows, (const uint32_t*)repeated, (const uint32_t*)rank_r,
                (const uint32_t*)unused, (const uint32_t*)rank_l, (const uint32_t*)rows_of_rank, (uint4*)d_permuted_input, (uint4*)d_permuted_table);

@@ -360,7 +360,7 @@ int mock_verify_run(DeviceCtx& ctx, const h2b_mock_circuit* c, h2b_mock_record* 
     }
     group_first.push_back(c->n_roots);
     max_scan = std::max(max_scan, (size_t)n_groups * n);
-    H2B_TRY(mem.get(&sums, max_scan / FLAG_SCAN_BLOCK + 2, "scan sums"));
+    H2B_TRY(mem.get(&sums, max_scan / SCAN_BLOCK + 2, "scan sums"));
     uint8_t* status = nullptr;
     uint32_t *counts = nullptr, *gate_off = nullptr;
     uint32_t totals[3] = {0, 0, 0};
@@ -382,7 +382,7 @@ int mock_verify_run(DeviceCtx& ctx, const h2b_mock_circuit* c, h2b_mock_record* 
         H2B_TRY(mock_launch_graph<0>(ctx, p, cg.n_slots, mr, MockOut{status, counts, nullptr, 0}, st));
         H2B_CUDA(cudaEventRecord(pb->done, st));
         ctx.prof.mark(PROF_MOCK_GATES, st);
-        H2B_TRY(flag_scan(counts, n_groups * n, gate_off, sums, st));
+        H2B_TRY(u32_exclusive_scan(counts, n_groups * n, gate_off, nullptr, sums, st));
         H2B_CUDA(cudaMemcpyAsync(d_totals, gate_off + (size_t)n_groups * n, 4, cudaMemcpyDeviceToDevice, st));
     }
 
@@ -432,7 +432,7 @@ int mock_verify_run(DeviceCtx& ctx, const h2b_mock_circuit* c, h2b_mock_record* 
             H2B_CUDA(cudaGetLastError());
         }
         ctx.prof.mark(PROF_MOCK_LOOKUPS, st);
-        H2B_TRY(flag_scan(lk_flags, c->n_lookups * usable, lk_off, sums, st));
+        H2B_TRY(u32_exclusive_scan(lk_flags, c->n_lookups * usable, lk_off, nullptr, sums, st));
         H2B_CUDA(cudaMemcpyAsync(d_totals + 1, lk_off + (size_t)c->n_lookups * usable, 4, cudaMemcpyDeviceToDevice, st));
     }
 
@@ -465,7 +465,7 @@ int mock_verify_run(DeviceCtx& ctx, const h2b_mock_circuit* c, h2b_mock_record* 
         pc.n_columns = P; pc.n = n; pc.usable = usable;
         H2B_LAUNCH(mock_permutation_kernel, blocks_of((size_t)P * n, 256), 256, 0, st, pc, pm_flags, d_totals + 3);
         ctx.prof.mark(PROF_MOCK_PERMUTATION, st);
-        H2B_TRY(flag_scan(pm_flags, P * n, pm_off, sums, st));
+        H2B_TRY(u32_exclusive_scan(pm_flags, P * n, pm_off, nullptr, sums, st));
         H2B_CUDA(cudaMemcpyAsync(d_totals + 2, pm_off + (size_t)P * n, 4, cudaMemcpyDeviceToDevice, st));
     }
     uint32_t got[4];

@@ -507,75 +507,7 @@ __global__ void __launch_bounds__(256) msm_decompose_kernel(MsmCols cols, MsmPla
     }
 }
 
-// ---- 2. exclusive scan (three small kernels) + scatter -------------------------------------------
-static const uint32_t SCAN_BLOCK = 1024;   // elements per CTA (256 threads x 4)
-
-__global__ void __launch_bounds__(256) scan_block_sums_kernel(const uint32_t* __restrict__ in, uint32_t count, uint32_t* __restrict__ block_sums) {
-    __shared__ uint32_t warp_sums[8];
-    uint32_t base = blockIdx.x * SCAN_BLOCK + threadIdx.x * 4;
-    uint32_t s = 0;
-#pragma unroll
-    for (int k = 0; k < 4; ++k) if (base + k < count) s += in[base + k];
-    for (int o = 16; o > 0; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
-    if ((threadIdx.x & 31) == 0) warp_sums[threadIdx.x >> 5] = s;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        uint32_t t = 0;
-        for (int k = 0; k < 8; ++k) t += warp_sums[k];
-        block_sums[blockIdx.x] = t;
-    }
-}
-// single CTA: exclusive scan of block_sums in place; block_sums[nblocks] = total
-__global__ void __launch_bounds__(1024) scan_top_kernel(uint32_t* block_sums, uint32_t nblocks) {
-    __shared__ uint32_t sh[1024];
-    __shared__ uint32_t carry_sh;
-    if (threadIdx.x == 0) carry_sh = 0;
-    __syncthreads();
-    for (uint32_t start = 0; start < nblocks; start += 1024) {
-        uint32_t idx = start + threadIdx.x;
-        uint32_t v = idx < nblocks ? block_sums[idx] : 0;
-        sh[threadIdx.x] = v;
-        __syncthreads();
-        for (uint32_t o = 1; o < 1024; o <<= 1) {
-            uint32_t add = threadIdx.x >= o ? sh[threadIdx.x - o] : 0;
-            __syncthreads();
-            sh[threadIdx.x] += add;
-            __syncthreads();
-        }
-        uint32_t incl = sh[threadIdx.x], carry = carry_sh;
-        if (idx < nblocks) block_sums[idx] = carry + incl - v;
-        __syncthreads();
-        if (threadIdx.x == 1023) carry_sh = carry + incl;
-        __syncthreads();
-    }
-    if (threadIdx.x == 0) block_sums[nblocks] = carry_sh;
-}
-// per CTA: local exclusive scan + block offset; writes `out` and a second copy `out2` (cursor)
-__global__ void __launch_bounds__(256) scan_apply_kernel(const uint32_t* __restrict__ in, uint32_t count, const uint32_t* __restrict__ block_sums,
-                                                       uint32_t* __restrict__ out, uint32_t* __restrict__ out2) {
-    __shared__ uint32_t warp_sums[8];
-    uint32_t base = blockIdx.x * SCAN_BLOCK + threadIdx.x * 4;
-    uint32_t v[4], s = 0;
-#pragma unroll
-    for (int k = 0; k < 4; ++k) { v[k] = (base + k < count) ? in[base + k] : 0; s += v[k]; }
-    uint32_t lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    uint32_t incl = s;
-    for (int o = 1; o < 32; o <<= 1) {
-        uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
-        if (lane >= (uint32_t)o) incl += t;
-    }
-    if (lane == 31) warp_sums[wid] = incl;
-    __syncthreads();
-    uint32_t woff = 0;
-    for (uint32_t k = 0; k < wid; ++k) woff += warp_sums[k];
-    uint32_t run = block_sums[blockIdx.x] + woff + incl - s;
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        if (base + k < count) { out[base + k] = run; out2[base + k] = run; }
-        run += v[k];
-    }
-    if (blockIdx.x == gridDim.x - 1 && threadIdx.x == 255) out[count] = block_sums[gridDim.x];
-}
+// ---- 2. exclusive scan of the counts (scan.cu's u32_exclusive_scan) + scatter -------------------------
 
 __global__ void __launch_bounds__(256) msm_scatter_kernel(MsmCols cols, MsmPlan pl, const uint32_t* __restrict__ digits, uint32_t* __restrict__ cursor,
                                                         uint32_t* __restrict__ sorted) {
@@ -1072,17 +1004,6 @@ static uint32_t msm_pick_window_tables(size_t n, uint32_t c0) {
     return best;
 }
 
-static int exclusive_scan(MsmScratch& s, const uint32_t* in, uint32_t count, uint32_t* out, uint32_t* out2, cudaStream_t stream) {
-    uint32_t nblocks = (count + SCAN_BLOCK - 1) / SCAN_BLOCK;
-    H2B_TRY(s.block_sums.reserve(((size_t)nblocks + 1) * 4));
-    uint32_t* bs = (uint32_t*)s.block_sums.p;
-    H2B_LAUNCH(scan_block_sums_kernel, nblocks, 256, 0, stream, in, count, bs);
-    H2B_LAUNCH(scan_top_kernel, 1, 1024, 0, stream, bs, nblocks);
-    H2B_LAUNCH(scan_apply_kernel, nblocks, 256, 0, stream, in, count, (const uint32_t*)bs, out, out2);
-    H2B_CUDA(cudaGetLastError());
-    return H2B_OK;
-}
-
 // ---- an MSM = plan + one or more chunks of scalars accumulated into the same buckets + one bucket reduction ----
 static int msm_plan(DeviceCtx& ctx, MsmScratch& s, const MsmBases& bases, size_t n_total, bool chunked, cudaStream_t stream, MsmPlan& pl, uint32_t ncols = 1) {
     (void)ctx;
@@ -1238,7 +1159,8 @@ static int msm_sort_chunk(DeviceCtx& ctx, MsmScratch& s, const MsmPlan& pl, cons
     ctx.prof.mark(PROF_BEGIN, stream);
     H2B_LAUNCH(msm_decompose_kernel, dim3(sort_grid, pl.ncols), 256, 0, stream, cols, pl, (uint32_t*)s.digits.p, counts);
     ctx.prof.mark(PROF_MSM_DECOMPOSE, stream);
-    H2B_TRY(exclusive_scan(s, counts, pl.B, offsets, cursor, stream));
+    H2B_TRY(s.block_sums.reserve((((size_t)pl.B + SCAN_BLOCK - 1) / SCAN_BLOCK + 1) * 4));
+    H2B_TRY(u32_exclusive_scan(counts, pl.B, offsets, cursor, (uint32_t*)s.block_sums.p, stream));
     ctx.prof.mark(PROF_MSM_SCAN, stream);
     H2B_LAUNCH(msm_scatter_kernel, dim3(sort_grid, pl.ncols), 256, 0, stream, cols, pl, (const uint32_t*)s.digits.p, cursor, sorted);
     H2B_CUDA(cudaGetLastError());

@@ -4,9 +4,10 @@
 //
 //   * plan (host, no field arithmetic): construct_intermediate_sets -- polynomials in first-appearance order with their distinct
 //     points, grouped into rotation sets by equal point sets, the super point set T -- packed into one table block on the device;
-//   * query evaluation: one kernel reads a polynomial's 16-coefficient chunk once and runs the chunk Horner of scan.cu for every
-//     point of that polynomial (up to 16, in groups of 4 accumulators); the chunk values of every (polynomial, point) pair then go
-//     down the levels of 16 together, one launch per level for all pairs;
+//   * query evaluation: the table block holds every (polynomial, point) pair's point, and scan.cu's point powers give each pair its
+//     row of powers; one kernel reads a polynomial's 16-coefficient chunk once and runs the chunk Horner for every point of that
+//     polynomial (up to 16, in groups of 4 accumulators); the chunk values of every pair then go down scan.cu's levels of 16 together
+//     (fr_horner_levels_run: its batched chunk kernel, one launch per level for all pairs);
 //   * scalars (one CTA): y^j, v^i and the combined interpolant of every set, R_i = sum_j y^j R_ij = interpolate(S_i, sum_j y^j P_ij(S_i))
 //     (the interpolation is linear, so one interpolation per set replaces one per polynomial); after u: z_i = Z_{T \ S_i}(u), z_0^-1,
 //     every linearisation coefficient v^i z_i y^j / z_0, -Z_T(u) / z_0 and the constant -sum_i v^i z_i R_i(u) / z_0, and a status
@@ -23,23 +24,10 @@
 
 namespace h2b {
 
-static const uint32_t MO_K = 16;                 // coefficients per chunk at every level (scan.cu's POLY_K)
-static const uint32_t MO_LEVELS = 9;             // 16^8 > 2^31
 static const uint32_t MO_GROUP = 4;              // points evaluated together per pass over a chunk
 static const uint32_t MO_SCALAR_THREADS = 128;
 
 // ---- plan -------------------------------------------------------------------------------------------------------------------
-static bool fr_words_canonical(const uint64_t* w) {
-    uint32_t l[8];
-    memcpy(l, w, 32);
-    for (int i = 7; i >= 0; --i) {
-        if (l[i] < FpParams<FR>::P(i)) return true;
-        if (l[i] > FpParams<FR>::P(i)) return false;
-    }
-    return false;
-}
-bool fr_canonical(const uint64_t w[4]) { return fr_words_canonical(w); }
-
 // the refusals every opening makes of its queries, and the distinct points in first-appearance order (compared as words): *points
 // (4 words each), (*query_point)[q] = the point index of query q
 static int opening_points(const char* who, const h2b_opening_query* queries, uint32_t n_queries, uint32_t n_polys, bool need_every_poly,
@@ -50,7 +38,7 @@ static int opening_points(const char* who, const h2b_opening_query* queries, uin
     for (uint32_t q = 0; q < n_queries; ++q) {
         const uint32_t poly = queries[q].poly;
         if (poly >= n_polys) { set_error("%s: query %u names polynomial %u of %u", who, q, poly, n_polys); return H2B_ERR_BAD_ARGUMENT; }
-        if (!fr_words_canonical(queries[q].point)) { set_error("%s: the point of query %u is not below the scalar field modulus", who, q); return H2B_ERR_BAD_ARGUMENT; }
+        if (!fr_canonical(queries[q].point)) { set_error("%s: the point of query %u is not below the scalar field modulus", who, q); return H2B_ERR_BAD_ARGUMENT; }
         const size_t count = points->size() / 4;
         uint32_t t = 0;
         while (t < count && memcmp(&(*points)[4 * (size_t)t], queries[q].point, 32) != 0) ++t;
@@ -115,7 +103,7 @@ int shplonk_plan_build(const char* who, const h2b_opening_query* queries, uint32
 // ---- the plan's tables on the device -----------------------------------------------------------------------------------------
 struct MoSet { uint32_t member0, members, point0, points, pair0, comp0, comps, r0; };
 
-struct MoLayout { size_t ptrs, slot_pairs, pair_pt, query_pair, sets, members, set_pts, pairidx, comp, status, jac, T, end; };
+struct MoLayout { size_t ptrs, slot_pairs, pair_x, query_pair, sets, members, set_pts, pairidx, comp, status, jac, T, end; };
 static size_t up32(size_t b) { return (b + 31) & ~(size_t)31; }
 static MoLayout mo_layout(const ShplonkPlan& p) {
     size_t sum_points = 0, sum_pairs = 0, sum_comp = 0;
@@ -128,7 +116,7 @@ static MoLayout mo_layout(const ShplonkPlan& p) {
     size_t o = 0;
     L.ptrs = o;       o = up32(o + 8 * p.used.size());
     L.slot_pairs = o; o = up32(o + 8 * p.used.size());
-    L.pair_pt = o;    o = up32(o + 4 * p.pair_point.size());
+    L.pair_x = o;     o = up32(o + 32 * p.pair_point.size());
     L.query_pair = o; o = up32(o + 4 * p.query_pair.size());
     L.sets = o;       o = up32(o + sizeof(MoSet) * p.set_slots.size());
     L.members = o;    o = up32(o + 4 * p.used.size());
@@ -159,7 +147,7 @@ int shplonk_tables_upload(const ShplonkPlan& p, const void* const* d_polys_by_sl
         u32s(L.slot_pairs)[2 * s] = p.slot_first[s];
         u32s(L.slot_pairs)[2 * s + 1] = p.slot_count[s];
     }
-    if (!p.pair_point.empty()) memcpy(h.data() + L.pair_pt, p.pair_point.data(), 4 * p.pair_point.size());
+    for (size_t i = 0; i < p.pair_point.size(); ++i) memcpy(h.data() + L.pair_x + 32 * i, &p.points[4 * (size_t)p.pair_point[i]], 32);
     memcpy(h.data() + L.query_pair, p.query_pair.data(), 4 * p.query_pair.size());
     uint32_t member0 = 0, point0 = 0, pair0 = 0, comp0 = 0;
     for (size_t i = 0; i < p.set_slots.size(); ++i) {
@@ -194,34 +182,22 @@ const void* shplonk_tables_status(const ShplonkPlan& p, const void* d_tables) { 
 const void* shplonk_tables_jac(const ShplonkPlan& p, const void* d_tables) { return (const char*)d_tables + mo_layout(p).jac; }
 
 // ---- query evaluation ---------------------------------------------------------------------------------------------------------
-// pow[t * MO_LEVELS + l] = T[t]^(16^l)
-__global__ void __launch_bounds__(128) mo_point_powers_kernel(const uint4* __restrict__ T, uint32_t t_count, uint4* __restrict__ pow) {
-    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= t_count) return;
-    Fr p = fp_load<FR>(T + 2 * (size_t)t);
-    for (uint32_t l = 0; l < MO_LEVELS; ++l) {
-        fp_store<FR>(pow + 2 * ((size_t)t * MO_LEVELS + l), p);
-        for (int k = 0; k < 4; ++k) p = fp_sqr(p);
-    }
-}
-
 // level 0: polynomial blockIdx.y, chunk t: out[pair * chunks + t] = sum_{i < 16} a[16 t + i] * x_pair^i for every pair (point) of the
 // polynomial; the chunk is read from HBM once, the groups of MO_GROUP points after the first re-read it from L1
 __global__ void __launch_bounds__(128) mo_eval_chunk_kernel(const uint64_t* __restrict__ ptrs, const uint32_t* __restrict__ slot_pairs,
-                                                          const uint32_t* __restrict__ pair_pt, const uint4* __restrict__ pow, size_t n, uint32_t chunks,
-                                                          uint4* __restrict__ out) {
+                                                          const uint4* __restrict__ pow, size_t n, uint32_t chunks, uint4* __restrict__ out) {
     const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= chunks) return;
     const uint32_t slot = blockIdx.y, first = slot_pairs[2 * slot], count = slot_pairs[2 * slot + 1];
     const uint4* in = (const uint4*)(uintptr_t)ptrs[slot];
-    const size_t lo = (size_t)t * MO_K, hi = lo + MO_K < n ? lo + MO_K : n;
+    const size_t lo = (size_t)t * POLY_K, hi = lo + POLY_K < n ? lo + POLY_K : n;
     for (uint32_t g0 = 0; g0 < count; g0 += MO_GROUP) {
         const uint32_t gm = count - g0 < MO_GROUP ? count - g0 : MO_GROUP;      // uniform over the block
         Fr x[MO_GROUP], r[MO_GROUP];
         const Fr top = fp_load<FR>(in + 2 * (hi - 1));
 #pragma unroll
         for (uint32_t g = 0; g < MO_GROUP; ++g) {
-            if (g < gm) { x[g] = fp_load<FR>(pow + 2 * (size_t)pair_pt[first + g0 + g] * MO_LEVELS); r[g] = top; }
+            if (g < gm) { x[g] = fp_load<FR>(pow + 2 * (size_t)(first + g0 + g) * POLY_PTS); r[g] = top; }
         }
         for (size_t i = hi - 1; i-- > lo;) {
             const Fr a = fp_load<FR>(in + 2 * i);
@@ -235,21 +211,6 @@ __global__ void __launch_bounds__(128) mo_eval_chunk_kernel(const uint64_t* __re
     }
 }
 
-// level l >= 1, pair blockIdx.y: out[pair * out_stride + t] = sum_{i < 16} in[pair * m + 16 t + i] * (x_pair^(16^l))^i
-__global__ void __launch_bounds__(128) mo_eval_level_kernel(const uint4* __restrict__ in, size_t m, const uint32_t* __restrict__ pair_pt,
-                                                          const uint4* __restrict__ pow, uint32_t level, uint32_t chunks, uint4* __restrict__ out,
-                                                          uint32_t out_stride) {
-    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= chunks) return;
-    const uint32_t pair = blockIdx.y;
-    const uint4* a = in + 2 * (size_t)pair * m;
-    const size_t lo = (size_t)t * MO_K, hi = lo + MO_K < m ? lo + MO_K : m;
-    const Fr x = fp_load<FR>(pow + 2 * ((size_t)pair_pt[pair] * MO_LEVELS + level));
-    Fr r = fp_load<FR>(a + 2 * (hi - 1));
-    for (size_t i = hi - 1; i-- > lo;) r = fp_add(fp_mul(r, x), fp_load<FR>(a + 2 * i));
-    fp_store<FR>(out + 2 * ((size_t)pair * out_stride + t), r);
-}
-
 __global__ void __launch_bounds__(128) mo_gather_kernel(const uint4* __restrict__ evals, const uint32_t* __restrict__ query_pair, uint32_t n_queries,
                                                       uint4* __restrict__ out) {
     const uint32_t q = blockIdx.x * blockDim.x + threadIdx.x;
@@ -261,28 +222,17 @@ __global__ void __launch_bounds__(128) mo_gather_kernel(const uint4* __restrict_
 int shplonk_eval_pairs_run(DeviceCtx& ctx, const ShplonkPlan& p, const void* d_tables, size_t n, void* d_evals, cudaStream_t stream) {
     const MoLayout L = mo_layout(p);
     const char* tb = (const char*)d_tables;
-    const uint32_t pairs = (uint32_t)p.pair_point.size(), slots = (uint32_t)p.used.size(), tc = p.n_points();
-    const uint32_t chunks0 = (uint32_t)((n + MO_K - 1) / MO_K);
+    const uint32_t pairs = (uint32_t)p.pair_point.size(), slots = (uint32_t)p.used.size();
+    const uint32_t chunks0 = (uint32_t)((n + POLY_K - 1) / POLY_K);
     size_t level_elems = 0;
-    for (size_t m = chunks0; m > 1; m = (m + MO_K - 1) / MO_K) level_elems += m;
-    H2B_TRY(ctx.open_scratch.reserve(((size_t)tc * MO_LEVELS + (size_t)pairs * level_elems + 2) * 32));
+    for (size_t m = chunks0; m > 1; m = (m + POLY_K - 1) / POLY_K) level_elems += m;
+    H2B_TRY(ctx.open_scratch.reserve(((size_t)pairs * POLY_PTS + (size_t)pairs * level_elems + 2) * 32));
     uint4* pow = (uint4*)ctx.open_scratch.p;
-    uint4* buf = pow + 2 * (size_t)tc * MO_LEVELS;
-    const uint32_t* pair_pt = (const uint32_t*)(tb + L.pair_pt);
-    H2B_LAUNCH(mo_point_powers_kernel, (tc + 127) / 128, 128, 0, stream, (const uint4*)(tb + L.T), tc, pow);
-    uint4* out0 = chunks0 == 1 ? (uint4*)d_evals : buf;
+    uint4* buf = pow + 2 * (size_t)pairs * POLY_PTS;
+    H2B_TRY(fr_point_powers_run(tb + L.pair_x, pairs, pow, stream));
     H2B_LAUNCH(mo_eval_chunk_kernel, dim3((chunks0 + 127) / 128, slots), 128, 0, stream, (const uint64_t*)(tb + L.ptrs), (const uint32_t*)(tb + L.slot_pairs),
-               pair_pt, (const uint4*)pow, n, chunks0, out0);
-    const uint4* in = buf;
-    size_t m = chunks0;
-    for (uint32_t l = 1; m > 1; ++l) {
-        const uint32_t chunks = (uint32_t)((m + MO_K - 1) / MO_K);
-        uint4* out = chunks == 1 ? (uint4*)d_evals : (uint4*)in + 2 * (size_t)pairs * m;
-        H2B_LAUNCH(mo_eval_level_kernel, dim3((chunks + 127) / 128, pairs), 128, 0, stream, in, m, pair_pt, (const uint4*)pow, l, chunks, out,
-                   chunks == 1 ? 1u : chunks);
-        in = out;
-        m = chunks;
-    }
+               (const uint4*)pow, n, chunks0, chunks0 == 1 ? (uint4*)d_evals : buf);
+    if (chunks0 > 1) H2B_TRY(fr_horner_levels_run(buf, chunks0, pow, 1, pairs, buf + 2 * (size_t)pairs * chunks0, d_evals, stream));
     H2B_CUDA(cudaGetLastError());
     return H2B_OK;
 }

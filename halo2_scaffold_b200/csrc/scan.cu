@@ -6,6 +6,9 @@
 //     inversion per thread), prefix products parked in a scratch column;
 //   * exclusive prefix product: chunk products of 16 consecutive elements, recursive scan of the chunk products (one CTA
 //     Hillis-Steele at the bottom), then every chunk replays its elements from its scanned offset.
+// The file also holds the exclusive scan of u32 values (the MSM's bucket offsets, the lookup argument's ranks, MockProver's record
+// offsets), polynomial evaluation and division by (X - b) in levels of 16 (shared with the SHPLONK query evaluation and the batched
+// divisions of GWC), and the linear combination of columns.
 #include "common.h"
 
 namespace h2b {
@@ -124,6 +127,84 @@ int fr_prefix_product_run(DeviceCtx& ctx, const void* d_in, void* d_out, size_t 
     return prefix_product_rec(ctx, (const uint4*)d_in, (uint4*)d_out, n, (uint4*)ctx.scan_scratch.p, stream);
 }
 
+// ---- exclusive scan of u32 values ----------------------------------------------------------------------------------------
+// block sums of SCAN_BLOCK elements, one CTA scans the block sums, then every block replays its elements from its offset
+__global__ void __launch_bounds__(256) scan_block_sums_kernel(const uint32_t* __restrict__ in, uint32_t count, uint32_t* __restrict__ block_sums) {
+    __shared__ uint32_t warp_sums[8];
+    uint32_t base = blockIdx.x * SCAN_BLOCK + threadIdx.x * 4;
+    uint32_t s = 0;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) if (base + k < count) s += in[base + k];
+    for (int o = 16; o > 0; o >>= 1) s += __shfl_down_sync(0xffffffffu, s, o);
+    if ((threadIdx.x & 31) == 0) warp_sums[threadIdx.x >> 5] = s;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        uint32_t t = 0;
+        for (int k = 0; k < 8; ++k) t += warp_sums[k];
+        block_sums[blockIdx.x] = t;
+    }
+}
+// single CTA: exclusive scan of block_sums in place; block_sums[nblocks] = total
+__global__ void __launch_bounds__(1024) scan_top_kernel(uint32_t* block_sums, uint32_t nblocks) {
+    __shared__ uint32_t sh[1024];
+    __shared__ uint32_t carry_sh;
+    if (threadIdx.x == 0) carry_sh = 0;
+    __syncthreads();
+    for (uint32_t start = 0; start < nblocks; start += 1024) {
+        uint32_t idx = start + threadIdx.x;
+        uint32_t v = idx < nblocks ? block_sums[idx] : 0;
+        sh[threadIdx.x] = v;
+        __syncthreads();
+        for (uint32_t o = 1; o < 1024; o <<= 1) {
+            uint32_t add = threadIdx.x >= o ? sh[threadIdx.x - o] : 0;
+            __syncthreads();
+            sh[threadIdx.x] += add;
+            __syncthreads();
+        }
+        uint32_t incl = sh[threadIdx.x], carry = carry_sh;
+        if (idx < nblocks) block_sums[idx] = carry + incl - v;
+        __syncthreads();
+        if (threadIdx.x == 1023) carry_sh = carry + incl;
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) block_sums[nblocks] = carry_sh;
+}
+// per CTA: local exclusive scan + block offset; writes `out` and, when given, a second copy `out2`
+__global__ void __launch_bounds__(256) scan_apply_kernel(const uint32_t* __restrict__ in, uint32_t count, const uint32_t* __restrict__ block_sums,
+                                                       uint32_t* __restrict__ out, uint32_t* __restrict__ out2) {
+    __shared__ uint32_t warp_sums[8];
+    uint32_t base = blockIdx.x * SCAN_BLOCK + threadIdx.x * 4;
+    uint32_t v[4], s = 0;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) { v[k] = (base + k < count) ? in[base + k] : 0; s += v[k]; }
+    uint32_t lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    uint32_t incl = s;
+    for (int o = 1; o < 32; o <<= 1) {
+        uint32_t t = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= (uint32_t)o) incl += t;
+    }
+    if (lane == 31) warp_sums[wid] = incl;
+    __syncthreads();
+    uint32_t woff = 0;
+    for (uint32_t k = 0; k < wid; ++k) woff += warp_sums[k];
+    uint32_t run = block_sums[blockIdx.x] + woff + incl - s;
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+        if (base + k < count) { out[base + k] = run; if (out2) out2[base + k] = run; }
+        run += v[k];
+    }
+    if (blockIdx.x == gridDim.x - 1 && threadIdx.x == 255) out[count] = block_sums[gridDim.x];
+}
+
+int u32_exclusive_scan(const uint32_t* in, uint32_t count, uint32_t* out, uint32_t* out2, uint32_t* sums, cudaStream_t stream) {
+    const uint32_t nblocks = (count + SCAN_BLOCK - 1) / SCAN_BLOCK;
+    H2B_LAUNCH(scan_block_sums_kernel, nblocks, 256, 0, stream, in, count, sums);
+    H2B_LAUNCH(scan_top_kernel, 1, 1024, 0, stream, sums, nblocks);
+    H2B_LAUNCH(scan_apply_kernel, nblocks, 256, 0, stream, in, count, (const uint32_t*)sums, out, out2);
+    H2B_CUDA(cudaGetLastError());
+    return H2B_OK;
+}
+
 // ---- polynomial evaluation and division by (X - b) ---------------------------------------------------------------------
 // [UP] halo2_proofs::arithmetic::{eval_polynomial, kate_division} (SURVEY.md section 1, layer L0): the prover evaluates
 // every committed polynomial at the challenge points and divides by (X - x) for the multi-open argument.
@@ -131,15 +212,11 @@ int fr_prefix_product_run(DeviceCtx& ctx, const void* d_in, void* d_out, size_t 
 //   eval:  P(x) = sum_t p_t * (x^16)^t with p_t the Horner value of 16 consecutive coefficients -> evaluate {p_t} at x^16;
 //   kate:  q[i-1] = a[i] + b * q[i]  (q = all suffix Horner values): chunk sums with zero carry-in, the same recurrence
 //          on the chunk sums with multiplier b^16 gives every chunk's carry-in, then the chunks replay.
-static const uint32_t POLY_K = 16;
-static const uint32_t POLY_LEVELS_MAX = 9;          // 16^8 > 2^31
-
-// The kernels of the kate levels also run a batch of divisions of one length, division d = blockIdx.y: a level's vectors, quotients,
-// chunk sums and carries lie back to back, each as long as the level's vector (n) or its chunk count, and the point powers of
-// division d at pts + d * POLY_PTS.  The offsets follow from arguments every form already has, and only the BATCH forms compute them,
-// so a single division runs the code it ran before batches existed (with the offsets, SHPLONK's per-point divisions measured 2 %
-// slower on a B200).
-static const uint32_t POLY_PTS = POLY_LEVELS_MAX + 1;      // the powers of one point and the point itself
+// The kernels of the levels also run a batch of vectors of one length, vector d = blockIdx.y (kate divisions, SHPLONK's query
+// evaluation): a level's vectors, quotients, chunk sums and carries lie back to back, each as long as the level's vector (n) or its
+// chunk count, and the point powers of vector d at pts + d * POLY_PTS.  The offsets follow from arguments every form already has, and
+// only the BATCH forms compute them, so a single division or evaluation runs the code it ran before batches existed (with the offsets,
+// SHPLONK's per-point divisions measured 2 % slower on a B200).
 
 // pts[l] = x^(16^l), l < levels (one thread; a handful of squarings)
 template <bool BATCH>
@@ -154,6 +231,12 @@ __global__ void fr_point_powers_kernel(const uint4* __restrict__ x, uint32_t lev
         fp_store<FR>(pts + 2 * l, p);
         for (int k = 0; k < 4; ++k) p = fp_sqr(p);
     }
+}
+
+int fr_point_powers_run(const void* d_x, uint32_t count, void* d_pts, cudaStream_t stream) {
+    H2B_LAUNCH((count > 1 ? fr_point_powers_kernel<true> : fr_point_powers_kernel<false>), dim3(1, count), 32, 0, stream, (const uint4*)d_x, POLY_LEVELS_MAX,
+               (uint4*)d_pts);
+    return H2B_OK;
 }
 
 // out[t] = sum_{i < 16} in[16 t + i] * x^i
@@ -174,29 +257,33 @@ __global__ void __launch_bounds__(128) fr_horner_chunk_kernel(const uint4* __res
     fp_store<FR>(out + 2 * (size_t)t, r);
 }
 
-int fr_eval_polynomial_run(DeviceCtx& ctx, const void* d_coeffs, size_t n, const uint64_t x[4], void* d_out, cudaStream_t stream) {
-    if (!d_out || !x || (n && !d_coeffs)) { set_error("eval_polynomial: null pointer"); return H2B_ERR_BAD_ARGUMENT; }
-    if (n == 0) { H2B_CUDA(cudaMemsetAsync(d_out, 0, 32, stream)); return H2B_OK; }
-    if (n > ((size_t)1 << 31)) { set_error("eval_polynomial: at most 2^31 coefficients"); return H2B_ERR_BAD_ARGUMENT; }
-    // scratch: point powers (POLY_LEVELS_MAX + 1 elements) | the partial values of all levels (< n/15 + slack)
-    H2B_TRY(ctx.scan_scratch.reserve((n / 15 + 64) * 32));
-    uint4* pts = (uint4*)ctx.scan_scratch.p;
-    uint4* buf = pts + 2 * (POLY_LEVELS_MAX + 1);
-    H2B_CUDA(cudaMemcpyAsync(pts + 2 * POLY_LEVELS_MAX, x, 32, cudaMemcpyHostToDevice, stream));
-    H2B_LAUNCH(fr_point_powers_kernel<false>, 1, 32, 0, stream, (const uint4*)(pts + 2 * POLY_LEVELS_MAX), POLY_LEVELS_MAX, pts);
-    const uint4* in = (const uint4*)d_coeffs;
-    size_t m = n;
-    for (uint32_t l = 0;; ++l) {
+int fr_horner_levels_run(const void* d_in, size_t m, const void* d_pts, uint32_t level, uint32_t count, void* d_buf, void* d_out, cudaStream_t stream) {
+    const uint4* in = (const uint4*)d_in;
+    uint4* buf = (uint4*)d_buf;
+    for (;; ++level) {
         const uint32_t chunks = (uint32_t)((m + POLY_K - 1) / POLY_K);
         uint4* out = chunks == 1 ? (uint4*)d_out : buf;
-        H2B_LAUNCH(fr_horner_chunk_kernel<false>, (chunks + 127) / 128, 128, 0, stream, in, m, (const uint4*)(pts + 2 * l), out, chunks);
+        H2B_LAUNCH((count > 1 ? fr_horner_chunk_kernel<true> : fr_horner_chunk_kernel<false>), dim3((chunks + 127) / 128, count), 128, 0, stream, in, m,
+                   (const uint4*)d_pts + 2 * level, out, chunks);
         if (chunks == 1) break;
         in = buf;
-        buf += 2 * (size_t)chunks;
+        buf += 2 * (size_t)chunks * count;
         m = chunks;
     }
     H2B_CUDA(cudaGetLastError());
     return H2B_OK;
+}
+
+int fr_eval_polynomial_run(DeviceCtx& ctx, const void* d_coeffs, size_t n, const uint64_t x[4], void* d_out, cudaStream_t stream) {
+    if (!d_out || !x || (n && !d_coeffs)) { set_error("eval_polynomial: null pointer"); return H2B_ERR_BAD_ARGUMENT; }
+    if (n == 0) { H2B_CUDA(cudaMemsetAsync(d_out, 0, 32, stream)); return H2B_OK; }
+    if (n > ((size_t)1 << 31)) { set_error("eval_polynomial: at most 2^31 coefficients"); return H2B_ERR_BAD_ARGUMENT; }
+    // scratch: point powers (POLY_PTS elements) | the partial values of all levels (< n/15 + slack)
+    H2B_TRY(ctx.scan_scratch.reserve((n / 15 + 64) * 32));
+    uint4* pts = (uint4*)ctx.scan_scratch.p;
+    H2B_CUDA(cudaMemcpyAsync(pts + 2 * POLY_LEVELS_MAX, x, 32, cudaMemcpyHostToDevice, stream));
+    H2B_TRY(fr_point_powers_run(pts + 2 * POLY_LEVELS_MAX, 1, pts, stream));
+    return fr_horner_levels_run(d_coeffs, n, pts, 0, 1, pts + 2 * POLY_PTS, d_out, stream);
 }
 
 // chunk sums with zero carry-in: s[t] = sum_{i < 16} a[16 t + i] * b^i   (the same kernel as the Horner chunks), then
@@ -272,7 +359,7 @@ static int kate_reserve(DeviceCtx& ctx, size_t n, uint32_t count) {
 static int kate_divisions(DeviceCtx& ctx, const void* d_a, size_t n, const uint4* x, uint32_t count, void* d_q, cudaStream_t stream) {
     uint4* pts = (uint4*)ctx.scan_scratch.p;
     uint4* buf = pts + 2 * (size_t)POLY_PTS * count;
-    H2B_LAUNCH((count > 1 ? fr_point_powers_kernel<true> : fr_point_powers_kernel<false>), dim3(1, count), 32, 0, stream, x, POLY_LEVELS_MAX, pts);
+    H2B_TRY(fr_point_powers_run(x, count, pts, stream));
     H2B_TRY(kate_level(ctx, (const uint4*)d_a, n, pts, 0, (uint4*)d_q, buf, count, stream));
     H2B_CUDA(cudaGetLastError());
     return H2B_OK;

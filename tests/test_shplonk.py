@@ -7,7 +7,7 @@ verifier's pairing equation becomes the G1 identity
 checked with the oracle's MSM; P_ij(s) and R_ij(u) come from the inputs on the host.  It fails for a verifier handed another
 polynomial or an evaluation off by one.
 
-CPU: the kernel sources through the emulator at k = 3 .. 7.  GPU: the product library at k = 10, 14, 16 and the lr22-like structure at
+CPU: the kernel sources through the emulator at k = 3 .. 7, and the query evaluation also at k = 13 (three levels of 16).  GPU: the product library at k = 10, 14, 16 and the lr22-like structure at
 k = 20."""
 import ctypes
 import os
@@ -273,7 +273,7 @@ def test_u_at_a_point_of_the_first_set_emu(emu, oc):
 
 def test_eval_queries_emu(emu, oc):
     import oracle_c
-    for k, name in ((3, "duplicates"), (6, "lr22"), (5, "sixteen_points")):
+    for k, name in ((3, "duplicates"), (6, "lr22"), (5, "sixteen_points"), (13, "lr22")):
         case = Case(oracle_c, k, name, 300 + k)
         ptrs = device_polys(emu, case)
         nq = len(case.queries)
